@@ -194,6 +194,42 @@ int sqfa_class_statistics(const float* X, int64_t ldx, const int64_t* labels, in
                           int64_t* counts, int64_t* offsets, int32_t* perm, void* ws, size_t ws_bytes,
                           sqfa_stream_t stream);
 
+/* bfloat16 / float16 points (`elem` = SQFA_ELEM_BF16 or SQFA_ELEM_F16; any other code returns
+ * SQFA_E_INVALID with sqfa_last_error set, and the workspace / signal queries return 0). Same contracts as
+ * the float32 entry points they are named after; only X changes: `const void*` with row stride ldx in
+ * ELEMENTS. Every element is widened to float32 as it is loaded and the kernels then do exactly what they
+ * do for float32 points (same centring, tf32 hi/lo split, MMA order and epilogue): sums, means, counts,
+ * Grams, covariances and Z are float32, and
+ *   - sqfa_class_sums_h, sqfa_class_statistics_h (means, epilogue), and sqfa_class_gram_h wherever the
+ *     float32 Gram runs without a K split, give the SAME BITS as the float32 entry points on a contiguous
+ *     float32 copy of X;
+ *   - elsewhere (K-split Grams, whose parts are summed with red.add in arrival order; transform) the
+ *     results agree with that copy's to float32 rounding.
+ * Rows aligned to 4 elements (8 bytes) are read with one 8-byte load per 4 columns, other rows element by
+ * element. The Gram's K-split rule counts the bytes of a class's rows (2 per element), so the workspace
+ * and completion-signal queries take `elem` too; everything else (label bucketing, sqfa_class_means,
+ * sqfa_stats_epilogue, counts, peer pushes) is dtype-free and shared. */
+#define SQFA_ELEM_BF16 1
+#define SQFA_ELEM_F16 2
+int sqfa_class_sums_h(const void* X, int64_t ldx, int32_t elem, const int32_t* perm, const int64_t* offsets,
+                      const float* shift, int64_t n, int32_t n_dim, int32_t n_classes, float* sums, int accumulate,
+                      void* ws, size_t ws_bytes, sqfa_stream_t stream);
+size_t sqfa_class_gram_workspace_bytes_h(int64_t n, int32_t n_dim, int32_t n_classes, int32_t elem);
+int sqfa_class_gram_h(const void* X, int64_t ldx, int32_t elem, const int32_t* perm, const int64_t* offsets,
+                      const float* shift, int64_t n, int32_t n_dim, int32_t n_classes, float* gram, int accumulate,
+                      int chain_rows, int32_t* done, int32_t n_groups, int32_t first_class, int32_t reserve_sms,
+                      void* ws, size_t ws_bytes, sqfa_stream_t stream);
+int64_t sqfa_class_gram_group_signals_h(int64_t n, int32_t n_dim, int32_t n_classes, int32_t n_groups, int32_t group,
+                                        int32_t elem);
+size_t sqfa_class_statistics_workspace_bytes_h(int64_t n, int32_t n_dim, int32_t n_classes, int32_t elem);
+int sqfa_class_statistics_h(const void* X, int64_t ldx, int32_t elem, const int64_t* labels, int64_t n, int32_t n_dim,
+                            int32_t n_classes, int estimator, int ddof, float* means, float* cov, float* sm,
+                            int64_t* counts, int64_t* offsets, int32_t* perm, void* ws, size_t ws_bytes,
+                            sqfa_stream_t stream);
+/* Z = X F^T with bf16 / fp16 X and float32 F, Z (sqfa_transform; X staged in shared memory as it is) */
+int sqfa_transform_h(const void* X, int64_t ldx, int32_t elem, const float* F, int64_t n, int32_t n_dim,
+                     int32_t n_filters, float* Z, sqfa_stream_t stream);
+
 /* float64 variants (the reference follows the dtype of `points`, statistics.py:28,32-34, and runs its
  * test-suite in float64): same contracts as the float32 entry points above, label bucketing is shared.
  * FP64 pipe (DFMA), 64 x 64 upper tiles, every reduction in a fixed order (bit-reproducible); no

@@ -23,6 +23,9 @@ c_ptr = ctypes.c_void_p
 c_size = ctypes.c_size_t
 c_int = ctypes.c_int
 
+# element codes of the *_h entry points (SQFA_ELEM_* in include/sqfa_b200.h)
+ELEM_CODES = {torch.bfloat16: 1, torch.float16: 2}
+
 # name -> (restype, argtypes); mirrors include/sqfa_b200.h one to one
 SIGNATURES = {
     "sqfa_version": (c_int, []),
@@ -67,6 +70,24 @@ SIGNATURES = {
         [c_ptr, c_i64, c_ptr, c_i64, c_i32, c_i32, c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
          c_size, c_ptr],
     ),
+    "sqfa_class_sums_h": (
+        c_int,
+        [c_ptr, c_i64, c_i32, c_ptr, c_ptr, c_ptr, c_i64, c_i32, c_i32, c_ptr, c_int, c_ptr, c_size, c_ptr],
+    ),
+    "sqfa_class_gram_workspace_bytes_h": (c_size, [c_i64, c_i32, c_i32, c_i32]),
+    "sqfa_class_gram_h": (
+        c_int,
+        [c_ptr, c_i64, c_i32, c_ptr, c_ptr, c_ptr, c_i64, c_i32, c_i32, c_ptr, c_int, c_int, c_ptr, c_i32, c_i32,
+         c_i32, c_ptr, c_size, c_ptr],
+    ),
+    "sqfa_class_gram_group_signals_h": (c_i64, [c_i64, c_i32, c_i32, c_i32, c_i32, c_i32]),
+    "sqfa_class_statistics_workspace_bytes_h": (c_size, [c_i64, c_i32, c_i32, c_i32]),
+    "sqfa_class_statistics_h": (
+        c_int,
+        [c_ptr, c_i64, c_i32, c_ptr, c_i64, c_i32, c_i32, c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
+         c_ptr, c_size, c_ptr],
+    ),
+    "sqfa_transform_h": (c_int, [c_ptr, c_i64, c_i32, c_ptr, c_i64, c_i32, c_i32, c_ptr, c_ptr]),
     "sqfa_class_sums_f64": (c_int, [c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_i64, c_i32, c_i32, c_ptr, c_int, c_ptr]),
     "sqfa_class_means_f64": (c_int, [c_ptr, c_ptr, c_ptr, c_i32, c_i32, c_ptr, c_ptr]),
     "sqfa_class_gram_f64": (c_int, [c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_i64, c_i32, c_i32, c_ptr, c_int, c_ptr]),

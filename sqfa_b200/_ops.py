@@ -75,6 +75,13 @@ def transform_raw(X, F):
     n, D = X.shape
     k = F.shape[0]
     Z = torch.empty(n, k, dtype=torch.float32, device=dev)
+    if X.dtype in _lib.ELEM_CODES:  # bf16 / fp16 points, float32 filters and Z
+        _lib.check(
+            lib.sqfa_transform_h(_lib.ptr(X), X.stride(0), _lib.ELEM_CODES[X.dtype], _lib.ptr(F), n, D, k, _lib.ptr(Z),
+                                 _lib.stream_ptr(dev)),
+            "sqfa_transform_h",
+        )
+        return Z
     _lib.check(
         lib.sqfa_transform(_lib.ptr(X), X.stride(0), _lib.ptr(F), n, D, k, _lib.ptr(Z), _lib.stream_ptr(dev)),
         "sqfa_transform",

@@ -26,11 +26,28 @@ from . import _lib
 
 
 class CudaStatsOps:
-    """Local steps of class_statistics on the current CUDA device (kernels K1, K2a, K2, K3)."""
+    """Local steps of class_statistics on the current CUDA device (kernels K1, K2a, K2, K3).
 
-    def __init__(self):
+    `elem` is the element code of the points: 0 for float32 (the float32 entry points), or
+    `_lib.ELEM_CODES[torch.bfloat16 / torch.float16]` (the `*_h` entry points, which widen every element
+    to float32 as they load it). Sums, means, Grams and statistics are float32 either way."""
+
+    def __init__(self, elem=0):
         self.lib = _lib.load()
+        self.elem = elem
         self.gram_events = None  # set to a list to record (start, end) CUDA events around K2
+
+    def _x_fn(self, name):
+        """Entry point `name` for this element type, and the leading (X, ldx[, elem]) arguments it takes."""
+        if self.elem == 0:
+            return getattr(self.lib, name), lambda X: (_lib.ptr(X), X.stride(0))
+        return getattr(self.lib, name + "_h"), lambda X: (_lib.ptr(X), X.stride(0), self.elem)
+
+    def _query(self, name, *args):
+        """Host-only size query for this element type (the `*_h` queries take the element code last)."""
+        if self.elem == 0:
+            return getattr(self.lib, name)(*args)
+        return getattr(self.lib, name + "_h")(*args, self.elem)
 
     def label_max(self, y):
         mx = torch.empty(1, dtype=torch.int64, device=y.device)
@@ -96,11 +113,10 @@ class CudaStatsOps:
         sums = torch.empty(C, D, dtype=torch.float32, device=dev) if out is None else out
         ws_bytes = lib.sqfa_class_sums_workspace_bytes(n, D, C)
         ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=dev)
+        fn, xa = self._x_fn("sqfa_class_sums")
         _lib.check(
-            lib.sqfa_class_sums(
-                _lib.ptr(X), X.stride(0), _lib.ptr(perm), _lib.ptr(offsets), None, n, D, C, _lib.ptr(sums), 0,
-                _lib.ptr(ws), ws_bytes, _lib.stream_ptr(dev),
-            ),
+            fn(*xa(X), _lib.ptr(perm), _lib.ptr(offsets), None, n, D, C, _lib.ptr(sums), 0, _lib.ptr(ws), ws_bytes,
+               _lib.stream_ptr(dev)),
             "sqfa_class_sums",
         )
         return sums
@@ -112,11 +128,10 @@ class CudaStatsOps:
         sums = torch.empty(C, D, dtype=torch.float32, device=dev)
         ws_bytes = lib.sqfa_class_sums_workspace_bytes(n, D, C)
         ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=dev)
+        fn, xa = self._x_fn("sqfa_class_sums")
         _lib.check(
-            lib.sqfa_class_sums(
-                _lib.ptr(X), X.stride(0), _lib.ptr(perm), _lib.ptr(offsets), _lib.ptr(shift), n, D, C, _lib.ptr(sums),
-                0, _lib.ptr(ws), ws_bytes, _lib.stream_ptr(dev),
-            ),
+            fn(*xa(X), _lib.ptr(perm), _lib.ptr(offsets), _lib.ptr(shift), n, D, C, _lib.ptr(sums), 0, _lib.ptr(ws),
+               ws_bytes, _lib.stream_ptr(dev)),
             "sqfa_class_sums",
         )
         return sums
@@ -162,18 +177,15 @@ class CudaStatsOps:
             gram = torch.empty(lib.sqfa_gram_packed_floats(D, C), dtype=torch.float32, device=dev)
         else:
             gram = torch.empty(C, D, D, dtype=torch.float32, device=dev)
-        ws_bytes = lib.sqfa_class_gram_workspace_bytes(n, D, C)
+        ws_bytes = self._query("sqfa_class_gram_workspace_bytes", n, D, C)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         if self.gram_events is not None:
             ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
             ev[0].record()
+        fn, xa = self._x_fn("sqfa_class_gram")
         _lib.check(
-            lib.sqfa_class_gram(
-                _lib.ptr(X), X.stride(0), _lib.ptr(perm), _lib.ptr(offsets), _lib.ptr(centre), n, D, C,
-                _lib.ptr(gram), 2 if packed else 0, 0, _lib.ptr(done), n_groups, first_class, reserve_sms, _lib.ptr(ws),
-                ws_bytes,
-                _lib.stream_ptr(dev),
-            ),
+            fn(*xa(X), _lib.ptr(perm), _lib.ptr(offsets), _lib.ptr(centre), n, D, C, _lib.ptr(gram), 2 if packed else 0,
+               0, _lib.ptr(done), n_groups, first_class, reserve_sms, _lib.ptr(ws), ws_bytes, _lib.stream_ptr(dev)),
             "sqfa_class_gram",
         )
         if self.gram_events is not None:
@@ -243,7 +255,7 @@ class CudaStatsOps:
             hi = lo
             while hi < C and (hi * G) // C == g:
                 hi += 1
-            expected = lib.sqfa_class_gram_group_signals(n, D, C, G, g)
+            expected = self._query("sqfa_class_gram_group_signals", n, D, C, G, g)
             _lib.check(
                 lib.sqfa_stream_wait_geq(ctypes.c_void_p(side.cuda_stream),
                                          ctypes.c_void_p(done.data_ptr() + 4 * g), int(expected)),
@@ -333,7 +345,7 @@ class CudaStatsOps:
         set_base = k * W * stride
         plan = st.setdefault("plans", {}).get(n)
         if plan is None:  # push order and the counter value that says "group g is final", per row count
-            plan = [(g, lo, hi, int(lib.sqfa_class_gram_group_signals(n, D, C, W, g)))
+            plan = [(g, lo, hi, int(self._query("sqfa_class_gram_group_signals", n, D, C, W, g)))
                     for g, lo, hi in peer_push_schedule(r, W, shares)]
             st["plans"][n] = plan
         for g, lo, hi, expected in plan:
@@ -415,7 +427,7 @@ class CudaStatsOps:
         sm = torch.empty(C, D, D, dtype=torch.float32, device=dev) if want_sm else None
         meta = torch.empty(2 * C + 4, dtype=torch.int64, device=dev)  # counts [C+1] | offsets [C+2]
         perm = torch.empty(n, dtype=torch.int32, device=dev)
-        ws_bytes = lib.sqfa_class_statistics_workspace_bytes(n, D, C)
+        ws_bytes = self._query("sqfa_class_statistics_workspace_bytes", n, D, C)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         return C, want_sm, means, cov, sm, meta, perm, ws, ws_bytes
 
@@ -427,12 +439,10 @@ class CudaStatsOps:
             prepared = self.fused_prepare(X, C, want_sm)
         _, _, means, cov, sm, meta, perm, ws, ws_bytes = prepared
         counts, offsets = meta[: C + 1], meta[C + 1 : 2 * C + 3]
+        fn, xa = self._x_fn("sqfa_class_statistics")
         _lib.check(
-            lib.sqfa_class_statistics(
-                _lib.ptr(X), X.stride(0), _lib.ptr(y), n, D, C, estimator_id, ddof, _lib.ptr(means), _lib.ptr(cov),
-                _lib.ptr(sm), _lib.ptr(counts), _lib.ptr(offsets), _lib.ptr(perm), _lib.ptr(ws), ws_bytes,
-                _lib.stream_ptr(dev),
-            ),
+            fn(*xa(X), _lib.ptr(y), n, D, C, estimator_id, ddof, _lib.ptr(means), _lib.ptr(cov), _lib.ptr(sm),
+               _lib.ptr(counts), _lib.ptr(offsets), _lib.ptr(perm), _lib.ptr(ws), ws_bytes, _lib.stream_ptr(dev)),
             "sqfa_class_statistics",
         )
         return means, cov, sm, (perm, offsets, counts)
@@ -585,18 +595,20 @@ def run_class_statistics(ops, X, y, estimator_id, group=None, n_classes=None, dd
         lease = ops.peer_acquire(D, C, group)  # before the collective below (see peer_acquire)
     if group is not None:
         # ONE small collective: [class sums | counts / 2^20 | counts mod 2^20] in the dtype of the sums
-        small = torch.empty(C * D + 2 * C, dtype=X.dtype, device=X.device)
+        # (float64 for float64 points, float32 otherwise: bf16 / fp16 points have float32 sums)
+        sums_dtype = torch.float64 if X.dtype == torch.float64 else torch.float32
+        small = torch.empty(C * D + 2 * C, dtype=sums_dtype, device=X.device)
         sums = small[: C * D].view(C, D)
         local_sums = ops.class_sums(X, perm, offsets, C, out=sums)
         if local_sums is not sums:  # ops without an `out` argument
             sums.copy_(local_sums)
         local = counts[:C]
-        native_words = X.dtype == torch.float32 and getattr(ops, "counts_pack", None) is not None
+        native_words = small.dtype == torch.float32 and getattr(ops, "counts_pack", None) is not None
         if native_words:  # one launch each way instead of a dozen element-wise torch kernels
             ops.counts_pack(local, small[C * D :])
         else:
-            small[C * D : C * D + C] = torch.div(local, _COUNT_BASE, rounding_mode="floor").to(X.dtype)
-            small[C * D + C :] = torch.remainder(local, _COUNT_BASE).to(X.dtype)
+            small[C * D : C * D + C] = torch.div(local, _COUNT_BASE, rounding_mode="floor").to(sums_dtype)
+            small[C * D + C :] = torch.remainder(local, _COUNT_BASE).to(sums_dtype)
         _all_reduce(small, group)
         if native_words:
             class_counts = ops.counts_unpack(small[C * D :])

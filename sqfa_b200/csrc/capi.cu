@@ -1,4 +1,5 @@
 // extern "C" boundary of libsqfa_b200.so -- see include/sqfa_b200.h for the contract.
+#include <cstdint>
 #include <cstdio>
 #include <cstring>
 #include <cuda_runtime.h>
@@ -34,6 +35,29 @@ int sm_count_cached() {
   }
   return sms[dev];
 }
+
+// element code of the *_h entry points -> sqfa::ElemType; -1 (with sqfa_last_error set) if unknown
+int half_elem(const char* fn, int32_t elem) {
+  if (elem == SQFA_ELEM_BF16) return sqfa::ELEM_BF16;
+  if (elem == SQFA_ELEM_F16) return sqfa::ELEM_F16;
+  snprintf(g_err, sizeof(g_err), "%s: unknown element code %d (SQFA_ELEM_BF16 = 1, SQFA_ELEM_F16 = 2)", fn, (int)elem);
+  return -1;
+}
+
+int class_sums_impl(const char* fn, const void* X, int elem, int64_t ldx, const int32_t* perm,
+                    const int64_t* offsets, const float* shift, int64_t n, int32_t n_dim, int32_t n_classes,
+                    float* sums, int accumulate, void* ws, size_t ws_bytes, sqfa_stream_t stream);
+int class_gram_impl(const char* fn, const void* X, int elem, int64_t ldx, const int32_t* perm,
+                    const int64_t* offsets, const float* shift, int64_t n, int32_t n_dim, int32_t n_classes,
+                    float* gram, int accumulate, int chain_rows, int32_t* done, int32_t n_groups,
+                    int32_t first_class, int32_t reserve_sms, void* ws, size_t ws_bytes, sqfa_stream_t stream);
+size_t class_gram_ws(int64_t n, int32_t n_dim, int32_t n_classes, int elem);
+int64_t class_gram_signals(int64_t n, int32_t n_dim, int32_t n_classes, int32_t n_groups, int32_t group, int elem);
+size_t class_statistics_ws(int64_t n, int32_t n_dim, int32_t n_classes, int elem);
+int class_statistics_impl(const char* fn, const void* X, int elem, int64_t ldx, const int64_t* labels, int64_t n,
+                          int32_t n_dim, int32_t n_classes, int estimator, int ddof, float* means, float* cov,
+                          float* sm, int64_t* counts, int64_t* offsets, int32_t* perm, void* ws, size_t ws_bytes,
+                          sqfa_stream_t stream);
 
 }  // namespace
 
@@ -78,15 +102,17 @@ size_t sqfa_class_sums_workspace_bytes(int64_t n, int32_t n_dim, int32_t n_class
 int sqfa_class_sums(const float* X, int64_t ldx, const int32_t* perm, const int64_t* offsets, const float* shift,
                     int64_t n, int32_t n_dim, int32_t n_classes, float* sums, int accumulate, void* ws,
                     size_t ws_bytes, sqfa_stream_t stream) {
-  if (n < 0 || n_dim <= 0 || n_classes < 0 || offsets == nullptr || sums == nullptr || ws == nullptr ||
-      (n > 0 && (X == nullptr || perm == nullptr)) || ldx < n_dim)
-    return fail_arg(__func__, "bad argument");
-  const int sms = sm_count_cached();
-  const int ns = sqfa::class_sums_splits(n, n_classes, n_dim, sms > 0 ? sms : 148);
-  if (ws_bytes < (size_t)ns * (size_t)n_classes * (size_t)n_dim * sizeof(float))
-    return fail_arg(__func__, "workspace too small", SQFA_E_WORKSPACE);
-  return wrap(__func__, sqfa::launch_class_sums(X, ldx, perm, offsets, shift, n, n_dim, n_classes, sums, accumulate,
-                                                static_cast<float*>(ws), ns, S(stream)));
+  return class_sums_impl(__func__, X, sqfa::ELEM_F32, ldx, perm, offsets, shift, n, n_dim, n_classes, sums,
+                         accumulate, ws, ws_bytes, stream);
+}
+
+int sqfa_class_sums_h(const void* X, int64_t ldx, int32_t elem, const int32_t* perm, const int64_t* offsets,
+                      const float* shift, int64_t n, int32_t n_dim, int32_t n_classes, float* sums, int accumulate,
+                      void* ws, size_t ws_bytes, sqfa_stream_t stream) {
+  const int e = half_elem(__func__, elem);
+  if (e < 0) return SQFA_E_INVALID;
+  return class_sums_impl(__func__, X, e, ldx, perm, offsets, shift, n, n_dim, n_classes, sums, accumulate, ws,
+                         ws_bytes, stream);
 }
 
 int sqfa_class_means(const float* sums, const int64_t* counts, const float* shift, int32_t n_dim,
@@ -97,10 +123,12 @@ int sqfa_class_means(const float* sums, const int64_t* counts, const float* shif
 }
 
 size_t sqfa_class_gram_workspace_bytes(int64_t n, int32_t n_dim, int32_t n_classes) {
-  if (n_classes <= 0 || n_dim <= 0) return 256;
-  const int sms = sm_count_cached();
-  return sqfa::gram_workspace_bytes(n_classes, n_dim,
-                                    sqfa::gram_ksplit(n < 0 ? 0 : n, n_classes, n_dim, sms > 0 ? sms : 148));
+  return class_gram_ws(n, n_dim, n_classes, sqfa::ELEM_F32);
+}
+
+size_t sqfa_class_gram_workspace_bytes_h(int64_t n, int32_t n_dim, int32_t n_classes, int32_t elem) {
+  const int e = half_elem(__func__, elem);
+  return e < 0 ? 0 : class_gram_ws(n, n_dim, n_classes, e);
 }
 
 int64_t sqfa_gram_executed_tile_area(int32_t n_dim) {
@@ -116,31 +144,28 @@ int sqfa_class_gram(const float* X, int64_t ldx, const int32_t* perm, const int6
                     int64_t n, int32_t n_dim, int32_t n_classes, float* gram, int accumulate, int chain_rows,
                     int32_t* done, int32_t n_groups, int32_t first_class, int32_t reserve_sms, void* ws,
                     size_t ws_bytes, sqfa_stream_t stream) {
-  if (n_dim <= 0 || n_classes < 0 || offsets == nullptr || gram == nullptr || ws == nullptr || ldx < n_dim ||
-      X == nullptr || perm == nullptr || (accumulate & ~(SQFA_GRAM_ACCUMULATE | SQFA_GRAM_PACKED)) ||
-      (done != nullptr && (n_groups <= 0 || n_groups > 65536)) || reserve_sms < 0 || first_class < 0 ||
-      (first_class > 0 && (done == nullptr || first_class >= n_classes)))
-    return fail_arg(__func__, "bad argument");
-  if (n < 0) return fail_arg(__func__, "bad argument");
-  if (ws_bytes < sqfa_class_gram_workspace_bytes(n, n_dim, n_classes))
-    return fail_arg(__func__, "workspace too small", SQFA_E_WORKSPACE);
-  if ((int64_t)n_classes * sqfa::gram_tiles_per_class(n_dim, nullptr) > (1ll << 30) / 4096)
-    return fail_arg(__func__, "too many (class, tile) jobs", SQFA_E_UNSUPPORTED);
-  const int sms = sm_count_cached();
-  if (sms <= 0) return fail_arg(__func__, "no CUDA device");
-  return wrap(__func__, sqfa::launch_class_gram(X, ldx, perm, offsets, shift, n, n_dim, n_classes, gram,
-                                                accumulate & SQFA_GRAM_ACCUMULATE, accumulate & SQFA_GRAM_PACKED,
-                                                chain_rows, done, n_groups, first_class, reserve_sms, ws, sms,
-                                                S(stream)));
+  return class_gram_impl(__func__, X, sqfa::ELEM_F32, ldx, perm, offsets, shift, n, n_dim, n_classes, gram, accumulate,
+                         chain_rows, done, n_groups, first_class, reserve_sms, ws, ws_bytes, stream);
+}
+
+int sqfa_class_gram_h(const void* X, int64_t ldx, int32_t elem, const int32_t* perm, const int64_t* offsets,
+                      const float* shift, int64_t n, int32_t n_dim, int32_t n_classes, float* gram, int accumulate,
+                      int chain_rows, int32_t* done, int32_t n_groups, int32_t first_class, int32_t reserve_sms,
+                      void* ws, size_t ws_bytes, sqfa_stream_t stream) {
+  const int e = half_elem(__func__, elem);
+  if (e < 0) return SQFA_E_INVALID;
+  return class_gram_impl(__func__, X, e, ldx, perm, offsets, shift, n, n_dim, n_classes, gram, accumulate, chain_rows,
+                         done, n_groups, first_class, reserve_sms, ws, ws_bytes, stream);
 }
 
 int64_t sqfa_class_gram_group_signals(int64_t n, int32_t n_dim, int32_t n_classes, int32_t n_groups, int32_t group) {
-  if (n_dim <= 0 || n_classes <= 0 || n_groups <= 0 || n_groups > 65536 || group < 0 || group >= n_groups) return 0;
-  const int sms = sm_count_cached();
-  const int64_t ks = sqfa::gram_ksplit(n < 0 ? 0 : n, n_classes, n_dim, sms > 0 ? sms : 148);
-  int64_t classes = 0;  // classes c with c * n_groups / n_classes == group
-  for (int c = 0; c < n_classes; ++c) classes += ((int64_t)c * n_groups) / n_classes == group ? 1 : 0;
-  return classes * sqfa::gram_tiles_per_class(n_dim, nullptr) * ks * 8;  // 2 CTAs x 4 epilogue warps per job
+  return class_gram_signals(n, n_dim, n_classes, n_groups, group, sqfa::ELEM_F32);
+}
+
+int64_t sqfa_class_gram_group_signals_h(int64_t n, int32_t n_dim, int32_t n_classes, int32_t n_groups, int32_t group,
+                                        int32_t elem) {
+  const int e = half_elem(__func__, elem);
+  return e < 0 ? 0 : class_gram_signals(n, n_dim, n_classes, n_groups, group, e);
 }
 
 // cuStreamWaitValue32 through the runtime's driver entry point lookup (no link dependency on libcuda)
@@ -258,7 +283,17 @@ int sqfa_transform(const float* X, int64_t ldx, const float* F, int64_t n, int32
   if (n < 0 || n_dim <= 0 || n_filters <= 0 || F == nullptr || (n > 0 && (X == nullptr || Z == nullptr)) ||
       ldx < n_dim)
     return fail_arg(__func__, "bad argument");
-  return wrap(__func__, sqfa::launch_transform(X, ldx, F, n, n_dim, n_filters, Z, S(stream)));
+  return wrap(__func__, sqfa::launch_transform(X, sqfa::ELEM_F32, ldx, F, n, n_dim, n_filters, Z, S(stream)));
+}
+
+int sqfa_transform_h(const void* X, int64_t ldx, int32_t elem, const float* F, int64_t n, int32_t n_dim,
+                     int32_t n_filters, float* Z, sqfa_stream_t stream) {
+  const int e = half_elem(__func__, elem);
+  if (e < 0) return SQFA_E_INVALID;
+  if (n < 0 || n_dim <= 0 || n_filters <= 0 || F == nullptr || (n > 0 && (X == nullptr || Z == nullptr)) ||
+      ldx < n_dim)
+    return fail_arg(__func__, "bad argument");
+  return wrap(__func__, sqfa::launch_transform(X, e, ldx, F, n, n_dim, n_filters, Z, S(stream)));
 }
 
 static int dist_ok(int32_t dist) {
@@ -414,51 +449,31 @@ int sqfa_closure_eval(const float* S_, const float* M, const float* raw_filters,
 extern "C" {
 
 // ---- the whole of class_statistics for rows resident on one device, in one call ----
-namespace {
-inline size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
-struct StatsWs { size_t bucket, sums_ws, sums, gram, epi, total; };
-inline StatsWs stats_ws(int64_t n, int32_t D, int32_t C) {
-  StatsWs w;
-  w.bucket = align256(sqfa_bucket_workspace_bytes(n, C));
-  w.sums_ws = align256(sqfa_class_sums_workspace_bytes(n, D, C));
-  w.sums = align256((size_t)(C > 0 ? C : 1) * (size_t)(D > 0 ? D : 1) * sizeof(float));
-  w.gram = align256(sqfa_class_gram_workspace_bytes(n, D, C));
-  w.epi = align256(sqfa_stats_epilogue_workspace_bytes(C));
-  w.total = w.bucket + w.sums_ws + w.sums + w.gram + w.epi;
-  return w;
-}
-}  // namespace
-
 size_t sqfa_class_statistics_workspace_bytes(int64_t n, int32_t n_dim, int32_t n_classes) {
-  return stats_ws(n < 0 ? 0 : n, n_dim, n_classes).total;
+  return class_statistics_ws(n, n_dim, n_classes, sqfa::ELEM_F32);
+}
+
+size_t sqfa_class_statistics_workspace_bytes_h(int64_t n, int32_t n_dim, int32_t n_classes, int32_t elem) {
+  const int e = half_elem(__func__, elem);
+  return e < 0 ? 0 : class_statistics_ws(n, n_dim, n_classes, e);
 }
 
 int sqfa_class_statistics(const float* X, int64_t ldx, const int64_t* labels, int64_t n, int32_t n_dim,
                           int32_t n_classes, int estimator, int ddof, float* means, float* cov, float* sm,
                           int64_t* counts, int64_t* offsets, int32_t* perm, void* ws, size_t ws_bytes,
                           sqfa_stream_t stream) {
-  if (X == nullptr || labels == nullptr || means == nullptr || cov == nullptr || counts == nullptr ||
-      offsets == nullptr || perm == nullptr || ws == nullptr || n <= 0 || n_dim <= 0 || n_classes <= 0)
-    return fail_arg(__func__, "bad argument");
-  const StatsWs w = stats_ws(n, n_dim, n_classes);
-  if (ws_bytes < w.total) return fail_arg(__func__, "workspace too small", SQFA_E_WORKSPACE);
-  uint8_t* p = static_cast<uint8_t*>(ws);
-  void* ws_bucket = p;
-  void* ws_sums = p + w.bucket;
-  float* sums = reinterpret_cast<float*>(p + w.bucket + w.sums_ws);
-  void* ws_gram = p + w.bucket + w.sums_ws + w.sums;
-  void* ws_epi = p + w.bucket + w.sums_ws + w.sums + w.gram;
-  int rc = sqfa_bucket_labels(labels, n, n_classes, counts, offsets, perm, ws_bucket, w.bucket, stream);
-  if (rc) return rc;
-  rc = sqfa_class_sums(X, ldx, perm, offsets, nullptr, n, n_dim, n_classes, sums, 0, ws_sums, w.sums_ws, stream);
-  if (rc) return rc;
-  rc = sqfa_class_means(sums, counts, nullptr, n_dim, n_classes, means, stream);
-  if (rc) return rc;
-  rc = sqfa_class_gram(X, ldx, perm, offsets, means, n, n_dim, n_classes, cov, 0, 0, nullptr, 0, 0, 0, ws_gram,
-                       w.gram, stream);
-  if (rc) return rc;
-  return sqfa_stats_epilogue(cov, means, nullptr, counts, n_dim, n_classes, estimator, ddof, cov, sm, ws_epi, w.epi,
-                             stream);
+  return class_statistics_impl(__func__, X, sqfa::ELEM_F32, ldx, labels, n, n_dim, n_classes, estimator, ddof, means,
+                               cov, sm, counts, offsets, perm, ws, ws_bytes, stream);
+}
+
+int sqfa_class_statistics_h(const void* X, int64_t ldx, int32_t elem, const int64_t* labels, int64_t n, int32_t n_dim,
+                            int32_t n_classes, int estimator, int ddof, float* means, float* cov, float* sm,
+                            int64_t* counts, int64_t* offsets, int32_t* perm, void* ws, size_t ws_bytes,
+                            sqfa_stream_t stream) {
+  const int e = half_elem(__func__, elem);
+  if (e < 0) return SQFA_E_INVALID;
+  return class_statistics_impl(__func__, X, e, ldx, labels, n, n_dim, n_classes, estimator, ddof, means, cov, sm,
+                               counts, offsets, perm, ws, ws_bytes, stream);
 }
 
 }  // extern "C"
@@ -553,3 +568,106 @@ int sqfa_gauss_pair_distances(const float* mu_a, const float* sigma_a, const flo
 }
 
 }  // extern "C"
+
+// ------------------------------------------------------ shared bodies of the float32 and *_h entry points
+namespace {
+
+int class_sums_impl(const char* fn, const void* X, int elem, int64_t ldx, const int32_t* perm,
+                    const int64_t* offsets, const float* shift, int64_t n, int32_t n_dim, int32_t n_classes,
+                    float* sums, int accumulate, void* ws, size_t ws_bytes, sqfa_stream_t stream) {
+  if (n < 0 || n_dim <= 0 || n_classes < 0 || offsets == nullptr || sums == nullptr || ws == nullptr ||
+      (n > 0 && (X == nullptr || perm == nullptr)) || ldx < n_dim)
+    return fail_arg(fn, "bad argument");
+  const int sms = sm_count_cached();
+  const int ns = sqfa::class_sums_splits(n, n_classes, n_dim, sms > 0 ? sms : 148);
+  if (ws_bytes < (size_t)ns * (size_t)n_classes * (size_t)n_dim * sizeof(float))
+    return fail_arg(fn, "workspace too small", SQFA_E_WORKSPACE);
+  return wrap(fn, sqfa::launch_class_sums(X, elem, ldx, perm, offsets, shift, n, n_dim, n_classes, sums, accumulate,
+                                          static_cast<float*>(ws), ns, S(stream)));
+}
+
+size_t class_gram_ws(int64_t n, int32_t n_dim, int32_t n_classes, int elem) {
+  if (n_classes <= 0 || n_dim <= 0) return 256;
+  const int sms = sm_count_cached();
+  return sqfa::gram_workspace_bytes(
+      n_classes, n_dim,
+      sqfa::gram_ksplit(n < 0 ? 0 : n, n_classes, n_dim, sms > 0 ? sms : 148, sqfa::elem_bytes(elem)));
+}
+
+int class_gram_impl(const char* fn, const void* X, int elem, int64_t ldx, const int32_t* perm,
+                    const int64_t* offsets, const float* shift, int64_t n, int32_t n_dim, int32_t n_classes,
+                    float* gram, int accumulate, int chain_rows, int32_t* done, int32_t n_groups,
+                    int32_t first_class, int32_t reserve_sms, void* ws, size_t ws_bytes, sqfa_stream_t stream) {
+  if (n_dim <= 0 || n_classes < 0 || offsets == nullptr || gram == nullptr || ws == nullptr || ldx < n_dim ||
+      X == nullptr || perm == nullptr || (accumulate & ~(SQFA_GRAM_ACCUMULATE | SQFA_GRAM_PACKED)) ||
+      (done != nullptr && (n_groups <= 0 || n_groups > 65536)) || reserve_sms < 0 || first_class < 0 ||
+      (first_class > 0 && (done == nullptr || first_class >= n_classes)))
+    return fail_arg(fn, "bad argument");
+  if (n < 0) return fail_arg(fn, "bad argument");
+  if (ws_bytes < class_gram_ws(n, n_dim, n_classes, elem)) return fail_arg(fn, "workspace too small", SQFA_E_WORKSPACE);
+  if ((int64_t)n_classes * sqfa::gram_tiles_per_class(n_dim, nullptr) > (1ll << 30) / 4096)
+    return fail_arg(fn, "too many (class, tile) jobs", SQFA_E_UNSUPPORTED);
+  const int sms = sm_count_cached();
+  if (sms <= 0) return fail_arg(fn, "no CUDA device");
+  return wrap(fn, sqfa::launch_class_gram(X, elem, ldx, perm, offsets, shift, n, n_dim, n_classes, gram,
+                                          accumulate & SQFA_GRAM_ACCUMULATE, accumulate & SQFA_GRAM_PACKED, chain_rows,
+                                          done, n_groups, first_class, reserve_sms, ws, sms, S(stream)));
+}
+
+int64_t class_gram_signals(int64_t n, int32_t n_dim, int32_t n_classes, int32_t n_groups, int32_t group, int elem) {
+  if (n_dim <= 0 || n_classes <= 0 || n_groups <= 0 || n_groups > 65536 || group < 0 || group >= n_groups) return 0;
+  const int sms = sm_count_cached();
+  const int64_t ks = sqfa::gram_ksplit(n < 0 ? 0 : n, n_classes, n_dim, sms > 0 ? sms : 148, sqfa::elem_bytes(elem));
+  int64_t classes = 0;  // classes c with c * n_groups / n_classes == group
+  for (int c = 0; c < n_classes; ++c) classes += ((int64_t)c * n_groups) / n_classes == group ? 1 : 0;
+  return classes * sqfa::gram_tiles_per_class(n_dim, nullptr) * ks * 8;  // 2 CTAs x 4 epilogue warps per job
+}
+
+inline size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
+struct StatsWs { size_t bucket, sums_ws, sums, gram, epi, total; };
+inline StatsWs stats_ws(int64_t n, int32_t D, int32_t C, int elem) {
+  StatsWs w;
+  w.bucket = align256(sqfa_bucket_workspace_bytes(n, C));
+  w.sums_ws = align256(sqfa_class_sums_workspace_bytes(n, D, C));
+  w.sums = align256((size_t)(C > 0 ? C : 1) * (size_t)(D > 0 ? D : 1) * sizeof(float));
+  w.gram = align256(class_gram_ws(n, D, C, elem));
+  w.epi = align256(sqfa_stats_epilogue_workspace_bytes(C));
+  w.total = w.bucket + w.sums_ws + w.sums + w.gram + w.epi;
+  return w;
+}
+
+size_t class_statistics_ws(int64_t n, int32_t n_dim, int32_t n_classes, int elem) {
+  return stats_ws(n < 0 ? 0 : n, n_dim, n_classes, elem).total;
+}
+
+int class_statistics_impl(const char* fn, const void* X, int elem, int64_t ldx, const int64_t* labels, int64_t n,
+                          int32_t n_dim, int32_t n_classes, int estimator, int ddof, float* means, float* cov,
+                          float* sm, int64_t* counts, int64_t* offsets, int32_t* perm, void* ws, size_t ws_bytes,
+                          sqfa_stream_t stream) {
+  if (X == nullptr || labels == nullptr || means == nullptr || cov == nullptr || counts == nullptr ||
+      offsets == nullptr || perm == nullptr || ws == nullptr || n <= 0 || n_dim <= 0 || n_classes <= 0)
+    return fail_arg(fn, "bad argument");
+  const StatsWs w = stats_ws(n, n_dim, n_classes, elem);
+  if (ws_bytes < w.total) return fail_arg(fn, "workspace too small", SQFA_E_WORKSPACE);
+  uint8_t* p = static_cast<uint8_t*>(ws);
+  void* ws_bucket = p;
+  void* ws_sums = p + w.bucket;
+  float* sums = reinterpret_cast<float*>(p + w.bucket + w.sums_ws);
+  void* ws_gram = p + w.bucket + w.sums_ws + w.sums;
+  void* ws_epi = p + w.bucket + w.sums_ws + w.sums + w.gram;
+  int rc = sqfa_bucket_labels(labels, n, n_classes, counts, offsets, perm, ws_bucket, w.bucket, stream);
+  if (rc) return rc;
+  const bool f32 = elem == sqfa::ELEM_F32;  // failures name the step, as the step's own entry point would
+  rc = class_sums_impl(f32 ? "sqfa_class_sums" : "sqfa_class_sums_h", X, elem, ldx, perm, offsets, nullptr, n, n_dim, n_classes, sums, 0, ws_sums, w.sums_ws,
+                       stream);
+  if (rc) return rc;
+  rc = sqfa_class_means(sums, counts, nullptr, n_dim, n_classes, means, stream);
+  if (rc) return rc;
+  rc = class_gram_impl(f32 ? "sqfa_class_gram" : "sqfa_class_gram_h", X, elem, ldx, perm, offsets, means, n, n_dim, n_classes, cov, 0, 0, nullptr, 0, 0, 0,
+                       ws_gram, w.gram, stream);
+  if (rc) return rc;
+  return sqfa_stats_epilogue(cov, means, nullptr, counts, n_dim, n_classes, estimator, ddof, cov, sm, ws_epi, w.epi,
+                             stream);
+}
+
+}  // namespace

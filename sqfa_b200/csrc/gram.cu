@@ -41,6 +41,7 @@
 #include <cuda_runtime.h>
 #include <type_traits>
 
+#include "elem.cuh"
 #include "ptx.cuh"
 #include "sqfa_internal.h"
 
@@ -74,7 +75,7 @@ constexpr uint32_t TMEM_COLS2 = 512, TMEM_SMALL2 = 256;
 __device__ __align__(16) float g_zero[4] = {0.f, 0.f, 0.f, 0.f};  // read with 16-byte loads
 
 struct GramParams {
-  const float* X;
+  const void* X;     // float, __nv_bfloat16 or __half (the kernel's template argument)
   int64_t ldx;
   int64_t n;         // rows of X (= entries of perm)
   const int32_t* perm;
@@ -93,10 +94,59 @@ struct GramParams {
   int packed;        // gram = packed list of upper tiles [class][tile][256][256] instead of (C, D, D)
   int T, TT;         // tiles per class, tiles per side
   int vec_ok;
-  int vecx;          // rows of X are 16-byte aligned: LDG.128
+  int vecx;          // rows of X are aligned to 4 elements: LDG.128 (float32) / LDG.64 (bf16, fp16)
   int flags;         // tuning switches (env SQFA_GRAM_FLAGS): 1 = no A-as-B reuse on diagonal tiles,
                      // 2 = A / B producer warps share the A operand of diagonal tiles, 4 = scalar loads,
                      // 8 = no early cross-term MMAs during a chain drain
+};
+
+__device__ __forceinline__ uint32_t ldg_nc_u16(const void* p) {  // zero-extended
+  uint32_t v;
+  asm volatile("ld.global.nc.u16 %0, [%1];" : "=r"(v) : "l"(p));
+  return v;
+}
+
+// How a producer thread's 4 adjacent columns of one sample arrive in registers: ONE aligned unit per
+// sample (16 bytes of float32 or 8 bytes of bf16 / fp16), or element loads where the rows are not
+// aligned to 4 elements or the last column tile ends inside the four. The element type changes nothing
+// else: widen() gives the float32 values the float32 path would have loaded.
+template <typename T>
+struct GramLoad {  // bf16 / fp16
+  using raw = uint64_t;
+  static __device__ __forceinline__ raw vec(const T* p) {
+    uint64_t v;
+    asm volatile("ld.global.nc.b64 %0, [%1];" : "=l"(v) : "l"(p));
+    return v;
+  }
+  static __device__ __forceinline__ raw scalar(const T* p, int ncol) {
+    uint32_t e0 = 0u, e1 = 0u, e2 = 0u, e3 = 0u;  // past D: zero bits, which widen to 0.f like the float32 zeros
+    if (ncol > 0) e0 = ldg_nc_u16(p);
+    if (ncol > 1) e1 = ldg_nc_u16(p + 1);
+    if (ncol > 2) e2 = ldg_nc_u16(p + 2);
+    if (ncol > 3) e3 = ldg_nc_u16(p + 3);
+    uint64_t v;
+    asm("mov.b64 %0, {%1, %2};" : "=l"(v) : "r"(e0 | (e1 << 16)), "r"(e2 | (e3 << 16)));
+    return v;
+  }
+  static __device__ __forceinline__ float4 widen(raw q) {
+    uint2 w;  // volatile like unpack_b128: the split stays where it is written, after the batch's wait
+    asm volatile("mov.b64 {%0, %1}, %2;" : "=r"(w.x), "=r"(w.y) : "l"(q));
+    return widen4<T>(w);
+  }
+};
+template <>
+struct GramLoad<float> {
+  using raw = b128_t;
+  static __device__ __forceinline__ raw vec(const float* p) { return ldg_nc_b128(p); }
+  static __device__ __forceinline__ raw scalar(const float* p, int ncol) {
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (ncol > 0) v.x = ldg_nc_f32(p);
+    if (ncol > 1) v.y = ldg_nc_f32(p + 1);
+    if (ncol > 2) v.z = ldg_nc_f32(p + 2);
+    if (ncol > 3) v.w = ldg_nc_f32(p + 3);
+    return pack_b128(v);
+  }
+  static __device__ __forceinline__ float4 widen(raw q) { return unpack_b128(q); }
 };
 
 // Job list: classes in descending size; within a class the K parts, and within a K part its tiles:
@@ -159,8 +209,10 @@ __device__ __forceinline__ JobGeom decode_job(const GramParams& P, int j) {
 //               n_dim <= 128, where a class has a single (diagonal) tile and a 256 x 256 tile would execute
 //               (256 / D)^2 times the useful MMA work. A launch without cluster dimensions is a cluster of
 //               one CTA, so the cluster-window barrier addressing below is valid in both variants.
-template <bool PAIR, int TN>
+template <typename T, bool PAIR, int TN>
 __device__ __forceinline__ void gram_body(const GramParams& P) {
+  using Load = GramLoad<T>;
+  using raw_t = typename Load::raw;
   constexpr int TM = PAIR ? 256 : 128;
   constexpr int NCTA = PAIR ? 2 : 1;
   extern __shared__ uint8_t smem_raw[];
@@ -248,9 +300,9 @@ __device__ __forceinline__ void gram_body(const GramParams& P) {
         if (ncol > 3) sh.w = __ldg(sp + 3);
       }
       // a thread without columns (past D) reads a fixed zero vector with row stride 0
-      const float* const xcol = ncol > 0 ? P.X + col : g_zero;
-      const uint32_t stride = ncol > 0 ? (uint32_t)P.ldx * 4u : 0u;
-      // warp-uniform choice of the load path: LDG.128 when rows are 16-byte aligned and every
+      const T* const xcol = ncol > 0 ? static_cast<const T*>(P.X) + col : reinterpret_cast<const T*>(g_zero);
+      const uint32_t stride = ncol > 0 ? (uint32_t)P.ldx * (uint32_t)sizeof(T) : 0u;
+      // warp-uniform choice of the load path: one vector load when rows are 4-element aligned and every
       // thread of the warp owns all four of its columns or none (straight-line code, no
       // per-load branches); scalar loads only in the last column tile of a D not divisible by 4
       const bool fastw = __all_sync(0xffffffffu, vecx && (ncol == 4 || ncol == 0));
@@ -267,7 +319,7 @@ __device__ __forceinline__ void gram_body(const GramParams& P) {
         // j + 1 are issued right after the single wait of batch j and have the whole time batch j
         // is being written to shared memory (GB stage periods) to land. All loads are volatile
         // asm so they stay where they are written relative to the barrier waits and stores.
-        b128_t bufA[GB][4], bufB[GB][4];
+        raw_t bufA[GB][4], bufB[GB][4];
         // lane r < 4 holds the row id of sample (4 quad + r) of a stage; refilled one batch ahead,
         // unconditional and clamped (a predicated load needs a select that waits on it)
         auto load_row = [&](int kb) -> uint32_t {
@@ -284,24 +336,19 @@ __device__ __forceinline__ void gram_body(const GramParams& P) {
           if (++stage == STAGES2) { stage = 0; phase ^= 1; }
           ++ring_kb;
         };
-        auto issue = [&](int kb, b128_t(&b)[GB][4]) {  // loads of stages kb, kb + S, .. kb + (GB - 1) S
+        auto issue = [&](int kb, raw_t(&b)[GB][4]) {  // loads of stages kb, kb + S, .. kb + (GB - 1) S
 #pragma unroll
           for (int u = 0; u < GB; ++u) {
 #pragma unroll
             for (int r = 0; r < 4; ++r) {
               const uint32_t row = __shfl_sync(0xffffffffu, rowreg[u], r);
-              uint64_t addr;  // xcol + row * ldx floats
+              uint64_t addr;  // xcol + row * ldx elements
               asm("mad.wide.u32 %0, %1, %2, %3;" : "=l"(addr) : "r"(row), "r"(stride), "l"(xcol));
-              const float* ptr = reinterpret_cast<const float*>(addr);
+              const T* ptr = reinterpret_cast<const T*>(addr);
               if constexpr (FAST) {
-                b[u][r] = ldg_nc_b128(ptr);
+                b[u][r] = Load::vec(ptr);
               } else {
-                float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (ncol > 0) v.x = ldg_nc_f32(ptr);
-                if (ncol > 1) v.y = ldg_nc_f32(ptr + 1);
-                if (ncol > 2) v.z = ldg_nc_f32(ptr + 2);
-                if (ncol > 3) v.w = ldg_nc_f32(ptr + 3);
-                b[u][r] = pack_b128(v);
+                b[u][r] = Load::scalar(ptr, ncol);
               }
             }
           }
@@ -317,7 +364,7 @@ __device__ __forceinline__ void gram_body(const GramParams& P) {
           st_shared_v4(hp, h);
           st_shared_v4(lp, l);
         };
-        auto consume = [&](int kb, const b128_t(&bq)[4]) {
+        auto consume = [&](int kb, const raw_t(&bq)[4]) {
           if constexpr (SHARE) {
             while (ring_kb < kb) skip_stage();
             ++ring_kb;
@@ -325,7 +372,7 @@ __device__ __forceinline__ void gram_body(const GramParams& P) {
           mbar_wait(&empty_bar[stage], phase ^ 1);
           float4 b[4];
 #pragma unroll
-          for (int r = 0; r < 4; ++r) b[r] = unpack_b128(bq[r]);
+          for (int r = 0; r < 4; ++r) b[r] = Load::widen(bq[r]);
           const int64_t nv = n_c - (int64_t)kb * BK - 4 * quad;  // valid samples among this thread's four
           if (nv < 4) {  // ragged last stage of the class: padded samples must be exact zeros
             const float4 z = make_float4(sh.x, sh.y, sh.z, sh.w);
@@ -347,7 +394,7 @@ __device__ __forceinline__ void gram_body(const GramParams& P) {
         };
         // one batch: the first stage's write (which contains the one wait for the batch's loads),
         // then the loads of the next batch into the other register set, then the remaining stages
-        auto batch = [&](int kb, b128_t(&cur)[GB][4], b128_t(&nxt)[GB][4]) {
+        auto batch = [&](int kb, raw_t(&cur)[GB][4], raw_t(&nxt)[GB][4]) {
           if (kb < kb1) consume(kb, cur[0]);
           issue(kb + S * GB, nxt);  // unconditional: stages past the end re-read valid rows, never consumed
 #pragma unroll
@@ -619,13 +666,15 @@ __device__ __forceinline__ void gram_body(const GramParams& P) {
   }
 }
 
+template <typename T>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GRAM2_THREADS, 1)
-gram_tf32x3_kernel(const GramParams P) { gram_body<true, TN2>(P); }
+gram_tf32x3_kernel(const GramParams P) { gram_body<T, true, TN2>(P); }
 
 constexpr int TN1 = 128;  // tile edge of the single-CTA variant
 constexpr int GRAM1_SMEM = STAGES2 * STAGE2_BYTES + 128 * TN1 * 4 + 1024;
+template <typename T>
 __global__ void __launch_bounds__(GRAM2_THREADS, 1)
-gram_tf32x3_small_kernel(const GramParams P) { gram_body<false, TN1>(P); }
+gram_tf32x3_small_kernel(const GramParams P) { gram_body<T, false, TN1>(P); }
 
 }  // namespace
 
@@ -662,8 +711,9 @@ int gram_ksplit_small(int64_t n, int C, int num_sms) {
   return (int)(ks < 1 ? 1 : ks);
 }
 
-// K parts per tile so that small problems still fill the CTA pairs
-int gram_ksplit(int64_t n, int C, int D, int num_sms) {
+// K parts per tile so that small problems still fill the CTA pairs. elem_size: bytes per element of X
+// (the L2-residency rule below counts the bytes of a class's rows, so bf16 / fp16 rows split half as often)
+int gram_ksplit(int64_t n, int C, int D, int num_sms, int elem_size) {
   const int T = gram_tiles_per_class(D, nullptr);
   const int64_t tiles = (int64_t)C * T;
   const int pairs = num_sms / 2 > 0 ? num_sms / 2 : 1;
@@ -677,7 +727,7 @@ int gram_ksplit(int64_t n, int C, int D, int num_sms) {
     const int64_t avg = C > 0 ? n / C : n;
     const double groups_in_flight = (double)pairs / T > 1.0 ? (double)pairs / T : 1.0;
     const double part_bytes = 96e6 / groups_in_flight;
-    const double class_bytes = (double)avg * D * 4.0;
+    const double class_bytes = (double)avg * D * (double)elem_size;
     if (class_bytes <= part_bytes) return 1;
     int64_t ks = (int64_t)(class_bytes / part_bytes + 0.999);
     const int64_t cap = avg / 2048 > 1 ? avg / 2048 : 1;  // keep >= 2048 samples per part (epilogue amortised)
@@ -700,40 +750,41 @@ size_t gram_workspace_bytes(int C, int D, int ksplit_max) {
   return (pair > small ? pair : small) * sizeof(int4) + 256;
 }
 
-cudaError_t launch_class_gram(const float* X, int64_t ldx, const int32_t* perm, const int64_t* offsets,
-                               const float* shift, int64_t n, int D, int C, float* gram, int accumulate, int packed,
-                               int chain_rows, int32_t* done, int n_groups, int first_class, int reserve_sms, void* ws,
-                               int num_sms, cudaStream_t stream) {
+template <typename T>
+static cudaError_t launch_class_gram_t(const T* X, int64_t ldx, const int32_t* perm, const int64_t* offsets,
+                                       const float* shift, int64_t n, int D, int C, float* gram, int accumulate,
+                                       int packed, int chain_rows, int32_t* done, int n_groups, int first_class,
+                                       int reserve_sms, void* ws, int num_sms, cudaStream_t stream) {
   const bool small = gram_use_small(D, packed);
-  static int smem_set[kMaxDevices] = {0}, smem_set1[kMaxDevices] = {0};
+  static int smem_set[kMaxDevices] = {0}, smem_set1[kMaxDevices] = {0};  // per element type
   {
-    cudaError_t e = small ? ensure_dynamic_smem(gram_tf32x3_small_kernel, GRAM1_SMEM, smem_set1)
-                          : ensure_dynamic_smem(gram_tf32x3_kernel, GRAM2_SMEM, smem_set);
+    cudaError_t e = small ? ensure_dynamic_smem(gram_tf32x3_small_kernel<T>, GRAM1_SMEM, smem_set1)
+                          : ensure_dynamic_smem(gram_tf32x3_kernel<T>, GRAM2_SMEM, smem_set);
     if (e != cudaSuccess) return e;
   }
   if (C <= 0) return cudaSuccess;
   GramParams P;
   int TT = 0;
-  int T = gram_tiles_per_class(D, &TT);
-  if (small) { TT = 1; T = 1; }
+  int T_ = gram_tiles_per_class(D, &TT);
+  if (small) { TT = 1; T_ = 1; }
   P.X = X; P.ldx = ldx; P.n = n; P.perm = perm; P.offsets = offsets; P.shift = shift; P.gram = gram;
   P.done = done; P.n_groups = n_groups > 0 ? n_groups : 1; P.class_order = done != nullptr ? 1 : 0;
   P.first_class = (P.class_order && first_class > 0 && first_class < C) ? first_class : 0;
   P.jobs = reinterpret_cast<const int4*>(ws);
   P.D = D; P.C = C;
-  P.KS = small ? gram_ksplit_small(n, C, num_sms) : gram_ksplit(n, C, D, num_sms);
-  P.njobs = C * T * P.KS;
+  P.KS = small ? gram_ksplit_small(n, C, num_sms) : gram_ksplit(n, C, D, num_sms, (int)sizeof(T));
+  P.njobs = C * T_ * P.KS;
   const int cr = chain_rows > 0 ? chain_rows : 512;
   P.chain_kb = (cr + BK - 1) / BK;
   P.atomic_out = (accumulate || P.KS > 1) ? 1 : 0;
-  P.packed = packed ? 1 : 0; P.T = T; P.TT = TT;
+  P.packed = packed ? 1 : 0; P.T = T_; P.TT = TT;
   P.vec_ok = (D % 4 == 0) && ((reinterpret_cast<uintptr_t>(gram) & 15) == 0);
   static const int env_flags = [] { const char* e = getenv("SQFA_GRAM_FLAGS"); return e ? atoi(e) : 0; }();
   P.flags = env_flags;
-  P.vecx = ((ldx % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0) && !(env_flags & 4)) ? 1 : 0;
-  if ((uint64_t)ldx * 4ull >= (1ull << 32)) return cudaErrorInvalidValue;
+  P.vecx = ((ldx % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & (4 * sizeof(T) - 1)) == 0) && !(env_flags & 4)) ? 1 : 0;
+  if ((uint64_t)ldx * sizeof(T) >= (1ull << 32)) return cudaErrorInvalidValue;
   if (P.atomic_out && !accumulate) {  // K parts are summed with red.add -> start from zero
-    const size_t floats = packed ? (size_t)C * T * TM2 * TN2 : (size_t)C * D * D;
+    const size_t floats = packed ? (size_t)C * T_ * TM2 * TN2 : (size_t)C * D * D;
     cudaError_t e = cudaMemsetAsync(gram, 0, floats * sizeof(float), stream);
     if (e != cudaSuccess) return e;
   }
@@ -744,13 +795,28 @@ cudaError_t launch_class_gram(const float* X, int64_t ldx, const int32_t* perm, 
   if (small) {
     int grid = usable > 1 ? usable : 1;
     if (grid > P.njobs) grid = P.njobs;
-    gram_tf32x3_small_kernel<<<grid, GRAM2_THREADS, GRAM1_SMEM, stream>>>(P);
+    gram_tf32x3_small_kernel<T><<<grid, GRAM2_THREADS, GRAM1_SMEM, stream>>>(P);
     return cudaGetLastError();
   }
   int grid = ((usable > 2 ? usable : 2) / 2) * 2;
   if (grid > 2 * P.njobs) grid = 2 * P.njobs;
-  gram_tf32x3_kernel<<<grid, GRAM2_THREADS, GRAM2_SMEM, stream>>>(P);
+  gram_tf32x3_kernel<T><<<grid, GRAM2_THREADS, GRAM2_SMEM, stream>>>(P);
   return cudaGetLastError();
+}
+
+cudaError_t launch_class_gram(const void* X, int elem, int64_t ldx, const int32_t* perm, const int64_t* offsets,
+                              const float* shift, int64_t n, int D, int C, float* gram, int accumulate, int packed,
+                              int chain_rows, int32_t* done, int n_groups, int first_class, int reserve_sms, void* ws,
+                              int num_sms, cudaStream_t stream) {
+  if (elem == ELEM_BF16)
+    return launch_class_gram_t(static_cast<const __nv_bfloat16*>(X), ldx, perm, offsets, shift, n, D, C, gram,
+                               accumulate, packed, chain_rows, done, n_groups, first_class, reserve_sms, ws, num_sms,
+                               stream);
+  if (elem == ELEM_F16)
+    return launch_class_gram_t(static_cast<const __half*>(X), ldx, perm, offsets, shift, n, D, C, gram, accumulate,
+                               packed, chain_rows, done, n_groups, first_class, reserve_sms, ws, num_sms, stream);
+  return launch_class_gram_t(static_cast<const float*>(X), ldx, perm, offsets, shift, n, D, C, gram, accumulate,
+                             packed, chain_rows, done, n_groups, first_class, reserve_sms, ws, num_sms, stream);
 }
 
 }  // namespace sqfa

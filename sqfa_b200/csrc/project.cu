@@ -14,6 +14,7 @@
 #include <cuda_runtime.h>
 
 #include "../../include/sqfa_b200.h"
+#include "elem.cuh"
 #include "sqfa_internal.h"
 
 namespace sqfa {
@@ -356,10 +357,11 @@ __global__ void project_bwd_finalize_kernel(const float* __restrict__ partial, i
   dF[idx] = a;
 }
 
-// Z[n][f] = sum_j X[n][j] F[f][j]; one warp per row, F chunk in shared memory.
-template <int KT>
+// Z[n][f] = sum_j X[n][j] F[f][j]; one warp per row, F chunk in shared memory. T = float, __nv_bfloat16
+// or __half (widened as it is loaded).
+template <int KT, typename T>
 __global__ void __launch_bounds__(256)
-transform_kernel(const float* __restrict__ X, int64_t ldx, const float* __restrict__ F, int64_t n, int D, int k,
+transform_kernel(const T* __restrict__ X, int64_t ldx, const float* __restrict__ F, int64_t n, int D, int k,
                  int f0, float* __restrict__ Z) {
   extern __shared__ float Fs[];  // [KT][512]
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -381,9 +383,9 @@ transform_kernel(const float* __restrict__ X, int64_t ldx, const float* __restri
     for (int r = 0; r < 8; ++r) {
       const int64_t row = r0 + warp * 8 + r;
       if (row >= n) break;
-      const float* xr = X + row * ldx + j0;
+      const T* xr = X + row * ldx + j0;
       for (int jj = lane; jj < 512 && j0 + jj < D; jj += 32) {
-        const float x = __ldg(xr + jj);
+        const float x = ldg_widen(xr + jj);
 #pragma unroll
         for (int f = 0; f < KT; ++f) acc[r][f] += x * Fs[f * 512 + jj];
       }
@@ -409,7 +411,15 @@ transform_kernel(const float* __restrict__ X, int64_t ldx, const float* __restri
 // filters of TWO rows (every F value loaded from shared memory feeds two FMAs), accumulated as
 // packed pairs: one fma.rn.f32x2 per two filters, row and column.
 // HBM-bound for k <= 16 (one read of X), about FMA-bound at k = 32.
+// bf16 / fp16 X is staged in shared memory as it is (16-byte cp.async of 8 elements, rows padded to 72
+// elements: LDS.128 of 8 elements, conflict-free per quarter warp) and widened after the LDS: half the
+// HBM and half the shared-memory bytes of a float32 row; the columns are multiplied in the same order.
 constexpr int TT_ROWS = 128, TT_COLS = 64, TT_LDX = TT_COLS + 4, TT_THREADS = 256;
+constexpr int TT_LDX_H = TT_COLS + 8;  // row pitch (elements) of a bf16 / fp16 X tile
+template <typename T>
+constexpr int tt_x_bytes() {  // both X buffers
+  return sizeof(T) == 4 ? 2 * TT_ROWS * TT_LDX * 4 : 2 * TT_ROWS * TT_LDX_H * 2;
+}
 
 __device__ __forceinline__ void cp_async_16(uint32_t dst, const void* src, int src_bytes) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");
@@ -423,14 +433,17 @@ __device__ __forceinline__ void cp_async_wait() {
   asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
 }
 
-template <int KF>
+template <int KF, typename T>
 __global__ void __launch_bounds__(TT_THREADS)
-transform_tile_kernel(const float* __restrict__ X, int64_t ldx, const float* __restrict__ F, int64_t n, int D, int k,
+transform_tile_kernel(const T* __restrict__ X, int64_t ldx, const float* __restrict__ F, int64_t n, int D, int k,
                       float* __restrict__ Z) {
   constexpr int KT = 4 * KF;
+  constexpr bool F32 = sizeof(T) == 4;
+  constexpr int LDX = F32 ? TT_LDX : TT_LDX_H;  // row pitch of the X tile (elements)
+  constexpr int XV = 16 / sizeof(T);            // elements per 16-byte cp.async
   extern __shared__ __align__(16) float tsm[];
-  float* Xs = tsm;                              // [2][TT_ROWS][TT_LDX]
-  float* Fs = tsm + 2 * TT_ROWS * TT_LDX;       // [2][TT_COLS][KT]
+  T* Xs = reinterpret_cast<T*>(tsm);                                    // [2][TT_ROWS][LDX]
+  float* Fs = tsm + tt_x_bytes<T>() / 4;                                // [2][TT_COLS][KT]
   const int tid = threadIdx.x;
   const int rp = tid & 63, fg = tid >> 6;  // rows rp and rp + 64; a warp: 32 consecutive rows, one filter group
   const int nchunks = (D + TT_COLS - 1) / TT_COLS;
@@ -438,14 +451,17 @@ transform_tile_kernel(const float* __restrict__ X, int64_t ldx, const float* __r
   const uint32_t xs_u = (uint32_t)__cvta_generic_to_shared(Xs), fs_u = (uint32_t)__cvta_generic_to_shared(Fs);
 
   auto load_chunk = [&](int64_t r0, int c0, int buf) {
-    // X tile: 128 rows x 16 float4; rows past n and columns past D are zero-filled (src_bytes = 0)
-    for (int idx = tid; idx < TT_ROWS * (TT_COLS / 4); idx += TT_THREADS) {
-      const int r = idx >> 4, c4 = idx & 15;
+    // X tile: 128 rows x 16-byte pieces; rows past n and columns past D are zero-filled (src_bytes = 0).
+    // D % 4 == 0 on this path: a piece is inside, outside, or (bf16 / fp16, 8 elements) half inside.
+    constexpr int PIECES = TT_COLS / XV;
+    for (int idx = tid; idx < TT_ROWS * PIECES; idx += TT_THREADS) {
+      const int r = idx / PIECES, cv = idx % PIECES;
       const int64_t gr = r0 + r;
-      const int gc = c0 + 4 * c4;
-      const bool ok = gr < n && gc < D;  // D % 4 == 0 on this path: a float4 is all inside or all outside
-      const float* src = ok ? X + gr * ldx + gc : X;
-      cp_async_16(xs_u + (uint32_t)(((buf * TT_ROWS + r) * TT_LDX + 4 * c4) * 4), src, ok ? 16 : 0);
+      const int gc = c0 + XV * cv;
+      const bool ok = gr < n && gc < D;
+      const int bytes = !ok ? 0 : (D - gc >= XV ? 16 : (D - gc) * (int)sizeof(T));
+      const T* src = ok ? X + gr * ldx + gc : X;
+      cp_async_16(xs_u + (uint32_t)(((buf * TT_ROWS + r) * LDX + XV * cv) * (int)sizeof(T)), src, bytes);
     }
     // F^T tile: Fs[c][f] = F[f][c0 + c]
     for (int idx = tid; idx < TT_COLS * KT; idx += TT_THREADS) {
@@ -472,18 +488,30 @@ transform_tile_kernel(const float* __restrict__ X, int64_t ldx, const float* __r
         cp_async_wait<0>();
       }
       __syncthreads();
-      const float* xr0 = Xs + (buf * TT_ROWS + rp) * TT_LDX;
-      const float* xr1 = xr0 + 64 * TT_LDX;
+      const T* xr0 = Xs + (buf * TT_ROWS + rp) * LDX;
+      const T* xr1 = xr0 + 64 * LDX;
       const float* fb = Fs + buf * TT_COLS * KT + fg * KF;
-#pragma unroll 4
-      for (int c4 = 0; c4 < TT_COLS / 4; ++c4) {
-        const float4 xa = *reinterpret_cast<const float4*>(xr0 + 4 * c4);
-        const float4 xb = *reinterpret_cast<const float4*>(xr1 + 4 * c4);
-        const float va[4] = {xa.x, xa.y, xa.z, xa.w}, vb[4] = {xb.x, xb.y, xb.z, xb.w};
+      // one LDS.128 per row and step: 4 float32 or 8 bf16 / fp16 columns, multiplied in column order
+#pragma unroll(F32 ? 4 : 2)
+      for (int cv = 0; cv < TT_COLS / XV; ++cv) {
+        float va[XV], vb[XV];
+        if constexpr (F32) {
+          const float4 xa = *reinterpret_cast<const float4*>(xr0 + 4 * cv);
+          const float4 xb = *reinterpret_cast<const float4*>(xr1 + 4 * cv);
+          va[0] = xa.x; va[1] = xa.y; va[2] = xa.z; va[3] = xa.w;
+          vb[0] = xb.x; vb[1] = xb.y; vb[2] = xb.z; vb[3] = xb.w;
+        } else {
+          const uint4 xa = *reinterpret_cast<const uint4*>(xr0 + 8 * cv);
+          const uint4 xb = *reinterpret_cast<const uint4*>(xr1 + 8 * cv);
+          const float4 a0 = widen4<T>(make_uint2(xa.x, xa.y)), a1 = widen4<T>(make_uint2(xa.z, xa.w));
+          const float4 b0 = widen4<T>(make_uint2(xb.x, xb.y)), b1 = widen4<T>(make_uint2(xb.z, xb.w));
+          va[0] = a0.x; va[1] = a0.y; va[2] = a0.z; va[3] = a0.w; va[4] = a1.x; va[5] = a1.y; va[6] = a1.z; va[7] = a1.w;
+          vb[0] = b0.x; vb[1] = b0.y; vb[2] = b0.z; vb[3] = b0.w; vb[4] = b1.x; vb[5] = b1.y; vb[6] = b1.z; vb[7] = b1.w;
+        }
 #pragma unroll
-        for (int u = 0; u < 4; ++u) {
+        for (int u = 0; u < XV; ++u) {
           const float2 a2 = make_float2(va[u], va[u]), b2 = make_float2(vb[u], vb[u]);
-          const float* fr = fb + (4 * c4 + u) * KT;
+          const float* fr = fb + (XV * cv + u) * KT;
           if constexpr (KF >= 4) {
 #pragma unroll
             for (int g = 0; g < KF / 4; ++g) {
@@ -566,18 +594,18 @@ cudaError_t run_project_stream(const float* S, const float* F, int C, int D, int
   return cudaGetLastError();
 }
 
-template <int KT>
-cudaError_t run_transform(const float* X, int64_t ldx, const float* F, int64_t n, int D, int k, float* Z,
+template <int KT, typename T>
+cudaError_t run_transform(const T* X, int64_t ldx, const float* F, int64_t n, int D, int k, float* Z,
                           cudaStream_t st) {
   const int smem = KT * 512 * (int)sizeof(float);
   static int smem_set[kMaxDevices] = {0};
   {
-    cudaError_t e = ensure_dynamic_smem(transform_kernel<KT>, smem, smem_set);
+    cudaError_t e = ensure_dynamic_smem(transform_kernel<KT, T>, smem, smem_set);
     if (e != cudaSuccess) return e;
   }
   const int64_t blocks = (n + 63) / 64;
   for (int f0 = 0; f0 < k; f0 += KT)
-    transform_kernel<KT><<<(unsigned)blocks, 256, smem, st>>>(X, ldx, F, n, D, k, f0, Z);
+    transform_kernel<KT, T><<<(unsigned)blocks, 256, smem, st>>>(X, ldx, F, n, D, k, f0, Z);
   return cudaGetLastError();
 }
 
@@ -741,27 +769,30 @@ cudaError_t launch_constraint_fwd(const float* Wraw, int D, int k, float* F, flo
   return cudaGetLastError();
 }
 
-template <int KF>
-static cudaError_t run_transform_tile(const float* X, int64_t ldx, const float* F, int64_t n, int D, int k, float* Z,
+template <int KF, typename T>
+static cudaError_t run_transform_tile(const T* X, int64_t ldx, const float* F, int64_t n, int D, int k, float* Z,
                                       cudaStream_t st) {
-  const int smem = (2 * TT_ROWS * TT_LDX + 2 * TT_COLS * 4 * KF) * (int)sizeof(float);
+  const int smem = tt_x_bytes<T>() + 2 * TT_COLS * 4 * KF * (int)sizeof(float);
   static int smem_set[kMaxDevices] = {0};
   {
-    cudaError_t e = ensure_dynamic_smem(transform_tile_kernel<KF>, smem, smem_set);
+    cudaError_t e = ensure_dynamic_smem(transform_tile_kernel<KF, T>, smem, smem_set);
     if (e != cudaSuccess) return e;
   }
   int dev = 0, sms = 148;
   if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const int64_t ntiles = (n + TT_ROWS - 1) / TT_ROWS;
   const int64_t grid = ntiles < 2 * (int64_t)sms ? ntiles : 2 * (int64_t)sms;
-  transform_tile_kernel<KF><<<(unsigned)grid, TT_THREADS, smem, st>>>(X, ldx, F, n, D, k, Z);
+  transform_tile_kernel<KF, T><<<(unsigned)grid, TT_THREADS, smem, st>>>(X, ldx, F, n, D, k, Z);
   return cudaGetLastError();
 }
 
-cudaError_t launch_transform(const float* X, int64_t ldx, const float* F, int64_t n, int D, int k, float* Z,
-                             cudaStream_t st) {
+template <typename T>
+static cudaError_t launch_transform_t(const T* X, int64_t ldx, const float* F, int64_t n, int D, int k, float* Z,
+                                      cudaStream_t st) {
   if (n <= 0) return cudaSuccess;
-  if (D % 4 == 0 && ldx % 4 == 0 && (reinterpret_cast<uintptr_t>(X) & 15) == 0 && k <= 32) {
+  // the tile kernel's 16-byte cp.async: every row starts 16-byte aligned (4 float32 / 8 bf16 / fp16 elements)
+  constexpr int64_t XV = 16 / sizeof(T);
+  if (D % 4 == 0 && ldx % XV == 0 && (reinterpret_cast<uintptr_t>(X) & 15) == 0 && k <= 32) {
     if (k <= 8) return run_transform_tile<2>(X, ldx, F, n, D, k, Z, st);
     if (k <= 16) return run_transform_tile<4>(X, ldx, F, n, D, k, Z, st);
     return run_transform_tile<8>(X, ldx, F, n, D, k, Z, st);
@@ -769,6 +800,13 @@ cudaError_t launch_transform(const float* X, int64_t ldx, const float* F, int64_
   if (k <= 4) return run_transform<4>(X, ldx, F, n, D, k, Z, st);
   if (k <= 8) return run_transform<8>(X, ldx, F, n, D, k, Z, st);
   return run_transform<16>(X, ldx, F, n, D, k, Z, st);
+}
+
+cudaError_t launch_transform(const void* X, int elem, int64_t ldx, const float* F, int64_t n, int D, int k, float* Z,
+                             cudaStream_t st) {
+  if (elem == ELEM_BF16) return launch_transform_t(static_cast<const __nv_bfloat16*>(X), ldx, F, n, D, k, Z, st);
+  if (elem == ELEM_F16) return launch_transform_t(static_cast<const __half*>(X), ldx, F, n, D, k, Z, st);
+  return launch_transform_t(static_cast<const float*>(X), ldx, F, n, D, k, Z, st);
 }
 
 cudaError_t launch_embed_fwd(const float* Psi, const float* Mu, float noise, int C, int k, int fr, float* E,

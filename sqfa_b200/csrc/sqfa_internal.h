@@ -21,6 +21,10 @@ inline cudaError_t ensure_dynamic_smem(Kernel kernel, int bytes, int (&set_bytes
   return e;
 }
 
+// Element type of the data points X (same values as SQFA_ELEM_* of the C ABI); see elem.cuh.
+enum ElemType { ELEM_F32 = 0, ELEM_BF16 = 1, ELEM_F16 = 2 };
+inline int elem_bytes(int elem) { return elem == ELEM_F32 ? 4 : 2; }
+
 // ---- bucket.cu (K1) ----
 cudaError_t launch_label_max(const int64_t* labels, int64_t n, int64_t* out_max, cudaStream_t stream);
 size_t bucket_workspace_bytes(int64_t n, int32_t C);
@@ -29,7 +33,7 @@ cudaError_t launch_bucket_labels(const int64_t* labels, int64_t n, int32_t C, in
 
 // ---- stats.cu (K2a, K3) ----
 int class_sums_splits(int64_t n, int C, int D, int num_sms);
-cudaError_t launch_class_sums(const float* X, int64_t ldx, const int32_t* perm, const int64_t* offsets,
+cudaError_t launch_class_sums(const void* X, int elem, int64_t ldx, const int32_t* perm, const int64_t* offsets,
                               const float* shift, int64_t n, int D, int C, float* sums, int accumulate,
                               float* partial_ws, int nsplit, cudaStream_t stream);
 cudaError_t launch_class_means(const float* sums, const int64_t* counts, const float* shift, int D, int C,
@@ -52,9 +56,9 @@ cudaError_t launch_stats_epilogue(const float* gram, int packed, const float* me
 // ---- gram.cu (K2: tcgen05 cta_group::2 Gram on CTA pairs) ----
 int gram_tiles_per_class(int D, int* TT_out);
 int64_t gram_executed_tile_area(int D);
-int gram_ksplit(int64_t n, int C, int D, int num_sms);
+int gram_ksplit(int64_t n, int C, int D, int num_sms, int elem_size);
 size_t gram_workspace_bytes(int C, int D, int ksplit_max);
-cudaError_t launch_class_gram(const float* X, int64_t ldx, const int32_t* perm, const int64_t* offsets,
+cudaError_t launch_class_gram(const void* X, int elem, int64_t ldx, const int32_t* perm, const int64_t* offsets,
                               const float* shift, int64_t n, int D, int C, float* gram, int accumulate, int packed,
                               int chain_rows, int32_t* done, int n_groups, int first_class, int reserve_sms, void* ws,
                               int num_sms, cudaStream_t stream);
@@ -82,7 +86,7 @@ cudaError_t launch_project_bwd_constrained(const float* gPsi, const float* gMu, 
                                            int n_fixed, float* grad, float* out, float* out_host,
                                            unsigned int* ticket, float* ws, cudaStream_t st);
 cudaError_t launch_constraint_fwd(const float* Wraw, int D, int k, float* F, float* inv_norm, cudaStream_t st);
-cudaError_t launch_transform(const float* X, int64_t ldx, const float* F, int64_t n, int D, int k, float* Z,
+cudaError_t launch_transform(const void* X, int elem, int64_t ldx, const float* F, int64_t n, int D, int k, float* Z,
                              cudaStream_t st);
 cudaError_t launch_embed_fwd(const float* Psi, const float* Mu, float noise, int C, int k, int fr, float* E,
                              cudaStream_t st);

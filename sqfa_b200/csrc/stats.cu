@@ -11,6 +11,7 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
+#include "elem.cuh"
 #include "sqfa_internal.h"
 
 namespace sqfa {
@@ -34,10 +35,15 @@ __host__ __device__ inline int sums_threads_per_row(int D) {
 }
 
 // partial[c][split][D] = sum over the split's rows of (x - shift_c)
+// T = float, __nv_bfloat16 or __half: elements are widened to float32 as they are loaded. `blk_ok` selects
+// the summation order (rows in groups of four into four accumulators), `vec_ok` the 4-element vector loads;
+// for float32 they are the same flag. A bf16 / fp16 X keeps the order of a float32 copy of it (contiguous,
+// so blocked whenever D % 4 == 0) even where its rows only allow element loads: the sums are bit-identical.
+template <typename T>
 __global__ void __launch_bounds__(SUM_THREADS)
-class_sums_kernel(const float* __restrict__ X, int64_t ldx, const int32_t* __restrict__ perm,
+class_sums_kernel(const T* __restrict__ X, int64_t ldx, const int32_t* __restrict__ perm,
                   const int64_t* __restrict__ offsets, const float* __restrict__ shift, int D, int nsplit,
-                  float* __restrict__ partial, int vec_ok) {
+                  float* __restrict__ partial, int vec_ok, int blk_ok) {
   __shared__ float4 red[SUM_THREADS];
   const int tpr = sums_threads_per_row(D), nlanes = SUM_THREADS / tpr;
   const int rlane = threadIdx.x / tpr, tcol = threadIdx.x % tpr;
@@ -51,7 +57,8 @@ class_sums_kernel(const float* __restrict__ X, int64_t ldx, const int32_t* __res
   const int col = (blockIdx.x * tpr + tcol) * 4;
   const bool live = col < D;
   float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
-  const bool full = vec_ok && (col + 4 <= D);
+  const bool full = blk_ok && (col + 4 <= D);
+  const bool vec = vec_ok != 0;
   if (shift != nullptr && live) {
     const float* sh = shift + (int64_t)c * D + col;
     s.x = sh[0];
@@ -66,14 +73,19 @@ class_sums_kernel(const float* __restrict__ X, int64_t ldx, const int32_t* __res
     int64_t k = kb;
     if (full) {
       for (; k + 4 <= ke; k += 4) {  // 4 independent 16-byte loads in flight per thread
-        const float* r0 = X + (int64_t)perm[begin + k + 0] * ldx + col;
-        const float* r1 = X + (int64_t)perm[begin + k + 1] * ldx + col;
-        const float* r2 = X + (int64_t)perm[begin + k + 2] * ldx + col;
-        const float* r3 = X + (int64_t)perm[begin + k + 3] * ldx + col;
-        const float4 v0 = __ldg(reinterpret_cast<const float4*>(r0));
-        const float4 v1 = __ldg(reinterpret_cast<const float4*>(r1));
-        const float4 v2 = __ldg(reinterpret_cast<const float4*>(r2));
-        const float4 v3 = __ldg(reinterpret_cast<const float4*>(r3));
+        const T* r0 = X + (int64_t)perm[begin + k + 0] * ldx + col;
+        const T* r1 = X + (int64_t)perm[begin + k + 1] * ldx + col;
+        const T* r2 = X + (int64_t)perm[begin + k + 2] * ldx + col;
+        const T* r3 = X + (int64_t)perm[begin + k + 3] * ldx + col;
+        float4 v0, v1, v2, v3;
+        if (sizeof(T) == 4 || vec) {  // float32: vec_ok == blk_ok
+          v0 = ldg_widen4(r0); v1 = ldg_widen4(r1); v2 = ldg_widen4(r2); v3 = ldg_widen4(r3);
+        } else {
+          v0 = make_float4(ldg_widen(r0), ldg_widen(r0 + 1), ldg_widen(r0 + 2), ldg_widen(r0 + 3));
+          v1 = make_float4(ldg_widen(r1), ldg_widen(r1 + 1), ldg_widen(r1 + 2), ldg_widen(r1 + 3));
+          v2 = make_float4(ldg_widen(r2), ldg_widen(r2 + 1), ldg_widen(r2 + 2), ldg_widen(r2 + 3));
+          v3 = make_float4(ldg_widen(r3), ldg_widen(r3 + 1), ldg_widen(r3 + 2), ldg_widen(r3 + 3));
+        }
         a0 = f4add(a0, make_float4(v0.x - s.x, v0.y - s.y, v0.z - s.z, v0.w - s.w));
         a1 = f4add(a1, make_float4(v1.x - s.x, v1.y - s.y, v1.z - s.z, v1.w - s.w));
         a2 = f4add(a2, make_float4(v2.x - s.x, v2.y - s.y, v2.z - s.z, v2.w - s.w));
@@ -81,12 +93,12 @@ class_sums_kernel(const float* __restrict__ X, int64_t ldx, const int32_t* __res
       }
     }
     for (; k < ke; ++k) {
-      const float* r = X + (int64_t)perm[begin + k] * ldx + col;
+      const T* r = X + (int64_t)perm[begin + k] * ldx + col;
       float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-      v.x = __ldg(r) - s.x;
-      if (col + 1 < D) v.y = __ldg(r + 1) - s.y;
-      if (col + 2 < D) v.z = __ldg(r + 2) - s.z;
-      if (col + 3 < D) v.w = __ldg(r + 3) - s.w;
+      v.x = ldg_widen(r) - s.x;
+      if (col + 1 < D) v.y = ldg_widen(r + 1) - s.y;
+      if (col + 2 < D) v.z = ldg_widen(r + 2) - s.z;
+      if (col + 3 < D) v.w = ldg_widen(r + 3) - s.w;
       a0 = f4add(a0, v);
     }
     outer = f4add(outer, f4add(f4add(a0, a1), f4add(a2, a3)));
@@ -422,15 +434,26 @@ int class_sums_splits(int64_t n, int C, int D, int num_sms) {
   return (int)want;
 }
 
-cudaError_t launch_class_sums(const float* X, int64_t ldx, const int32_t* perm, const int64_t* offsets,
+cudaError_t launch_class_sums(const void* X, int elem, int64_t ldx, const int32_t* perm, const int64_t* offsets,
                               const float* shift, int64_t n, int D, int C, float* sums, int accumulate,
                               float* partial_ws, int nsplit, cudaStream_t stream) {
   (void)n;
   if (C <= 0 || D <= 0) return cudaSuccess;
-  const int vec_ok = (D % 4 == 0) && (ldx % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0);
+  // 4-element loads: rows aligned to 4 elements (16 bytes for float32, 8 for bf16 / fp16)
+  const uintptr_t al = 4u * (uintptr_t)elem_bytes(elem) - 1u;
+  const int vec_ok = (D % 4 == 0) && (ldx % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & al) == 0);
+  const int blk_ok = elem == ELEM_F32 ? vec_ok : (D % 4 == 0);
   const int tpr = sums_threads_per_row(D);
   dim3 grid((D + tpr * 4 - 1) / (tpr * 4), nsplit, C);
-  class_sums_kernel<<<grid, SUM_THREADS, 0, stream>>>(X, ldx, perm, offsets, shift, D, nsplit, partial_ws, vec_ok);
+  if (elem == ELEM_BF16)
+    class_sums_kernel<<<grid, SUM_THREADS, 0, stream>>>(static_cast<const __nv_bfloat16*>(X), ldx, perm, offsets,
+                                                        shift, D, nsplit, partial_ws, vec_ok, blk_ok);
+  else if (elem == ELEM_F16)
+    class_sums_kernel<<<grid, SUM_THREADS, 0, stream>>>(static_cast<const __half*>(X), ldx, perm, offsets, shift, D,
+                                                        nsplit, partial_ws, vec_ok, blk_ok);
+  else
+    class_sums_kernel<<<grid, SUM_THREADS, 0, stream>>>(static_cast<const float*>(X), ldx, perm, offsets, shift, D,
+                                                        nsplit, partial_ws, vec_ok, blk_ok);
   const int64_t total = (int64_t)C * D;
   class_sums_finalize_kernel<<<(int)((total + 255) / 256), 256, 0, stream>>>(partial_ws, nsplit, D, C, sums,
                                                                                accumulate);

@@ -128,8 +128,8 @@ class _Transform(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gZ):
         Fc, X = ctx.saved_tensors
-        dF = gZ.t() @ X if ctx.needs_input_grad[0] else None
-        dX = gZ @ Fc if ctx.needs_input_grad[1] else None
+        dF = gZ.t() @ X.float() if ctx.needs_input_grad[0] else None  # bf16 / fp16 X: float32 like Z
+        dX = (gZ @ Fc).to(X.dtype) if ctx.needs_input_grad[1] else None
         return dF, dX
 
 
@@ -230,7 +230,8 @@ class SecondMomentsSQFA(nn.Module):
         """Project data points (n_samples, n_dim) to feature space (n_samples, n_filters)
         (reference model.py:222-237)."""
         dev = _lib.compute_device(data_points, self.filters)
-        if data_points.dim() != 2 or data_points.dtype != torch.float32:
+        # float32, bf16 and fp16 points run the native kernel (Z is float32); float64 stays with torch
+        if data_points.dim() != 2 or data_points.dtype not in (torch.float32, torch.bfloat16, torch.float16):
             return torch.einsum("ij,nj->ni", self.filters.to(dev), data_points.to(dev)).to(data_points.device)
         with torch.cuda.device(dev):
             X = data_points.to(dev)

@@ -15,17 +15,24 @@ from ._stats_driver import CudaStatsOps, CudaStatsOps64, run_class_statistics
 __all__ = ["class_statistics", "oas_covariance", "pca", "pca_from_scatter"]  # the reference's; extensions below
 
 _ESTIMATORS = {"empirical": 0, "oas": 1}
+_POINT_DTYPES = (torch.float32, torch.float64, torch.bfloat16, torch.float16)
 _ops_singleton = None
 _ops64_singleton = None
+_ops_half = {}
 
 
 def _cuda_ops(dtype=torch.float32):
-    """The local kernels for the dtype of the points: float32 (tcgen05 3xTF32) or float64 (DFMA)."""
+    """The local kernels for the dtype of the points: float32 (tcgen05 3xTF32), float64 (DFMA), or
+    bfloat16 / float16 (the float32 kernels, every element widened to float32 as it is loaded)."""
     global _ops_singleton, _ops64_singleton
     if dtype == torch.float64:
         if _ops64_singleton is None:
             _ops64_singleton = CudaStatsOps64()
         return _ops64_singleton
+    if dtype in _lib.ELEM_CODES:
+        if dtype not in _ops_half:
+            _ops_half[dtype] = CudaStatsOps(_lib.ELEM_CODES[dtype])
+        return _ops_half[dtype]
     if _ops_singleton is None:
         _ops_singleton = CudaStatsOps()
     return _ops_singleton
@@ -36,8 +43,9 @@ def _as_device_points(points, dev):
         raise TypeError("points must be a torch.Tensor")
     if points.dim() != 2:
         raise ValueError("points must have shape (n_points, n_dim)")
-    if points.dtype not in (torch.float32, torch.float64):
-        raise TypeError(f"points must be float32 or float64 (the output follows their dtype); got {points.dtype}")
+    if points.dtype not in _POINT_DTYPES:
+        raise TypeError("points must be float32, float64, bfloat16 or float16 (the output follows their dtype; "
+                        f"float32 for bfloat16 / float16); got {points.dtype}")
     X = points.detach().to(dev, non_blocking=True)
     if X.stride(1) != 1 or X.stride(0) < X.shape[1]:
         X = X.contiguous()
@@ -85,6 +93,12 @@ def class_statistics(points, labels, estimator="empirical", keep_on_device=False
     points : torch.Tensor
         Data points with shape (n_points, n_dim), float32 or float64 (the statistics have the dtype of
         the points, like the reference's), on the CPU or a CUDA device.
+        (extension) bfloat16 and float16 points are accepted too, and their statistics are FLOAT32: the
+        reference would accumulate them in bf16, whose 8-bit mantissa loses the small eigenvalues the
+        affine-invariant distance depends on, and the fitting closure takes float32 or float64 only.
+        Every element is widened to float32 as the kernels load it, so the result is what
+        `class_statistics(points.float(), labels)` returns -- bit for bit where that path is
+        deterministic -- while half the bytes are read and no float32 copy of the points is made.
     labels : torch.Tensor
         Class labels of each point with shape (n_points).
     estimator:
@@ -169,9 +183,12 @@ class StreamingClassStatistics:
         self._rows_at_shift = 0
 
     def _first_shift(self, X, perm, offsets, counts):
-        ops = _cuda_ops()
+        ops = _cuda_ops(X.dtype)
         m = ops.class_means(ops.class_sums(X, perm, offsets, self.C), counts[: self.C].clone())
-        fallback = X.mean(dim=0, keepdim=True).expand_as(m)  # classes absent from the first chunk
+        # classes absent from the first chunk. Computed on the chunk's float32 values (a copy of the first
+        # chunk only, for bf16 / fp16) with the same reduction a float32 stream runs, so that a bf16 / fp16
+        # stream and a float32 stream of the same values hold identical state
+        fallback = X.float().mean(dim=0, keepdim=True).expand_as(m)
         shift = torch.where(torch.isfinite(m), m, fallback).contiguous()
         if self.group is not None:
             import torch.distributed as dist
@@ -180,20 +197,22 @@ class StreamingClassStatistics:
         return shift
 
     def update(self, points, labels):
-        """Fold a chunk of rows (n, n_dim) float32 with labels (n,) into the state. Rows whose label is
-        outside [0, n_classes) are ignored, like rows no `labels == i` selects in the reference."""
-        lib, dev, C, D = self.lib, self.dev, self.C, self.D
+        """Fold a chunk of rows (n, n_dim) float32 (or bfloat16 / float16, widened to float32 as they are
+        loaded: the same state as the chunk's float32 copy would give) with labels (n,) into the state.
+        Rows whose label is outside [0, n_classes) are ignored, like rows no `labels == i` selects in
+        the reference."""
+        dev, C, D = self.dev, self.C, self.D
         X = _as_device_points(points, dev)
         y = _as_device_labels(labels, dev)
-        if X.dtype != torch.float32:
-            raise TypeError("StreamingClassStatistics accumulates float32 chunks")
+        if X.dtype == torch.float64:
+            raise TypeError("StreamingClassStatistics accumulates float32, bfloat16 or float16 chunks")
         if X.shape[1] != D or y.numel() != X.shape[0]:
             raise ValueError("chunk must have shape (n, n_dim) and one label per row")
         n = X.shape[0]
         if n == 0:
             return self
         with torch.cuda.device(dev):
-            ops = _cuda_ops()
+            ops = _cuda_ops(X.dtype)
             perm, offsets, counts = ops.bucket(y, C)
             if self.shift is None:
                 self.shift = self._first_shift(X, perm, offsets, counts)
@@ -201,18 +220,20 @@ class StreamingClassStatistics:
             elif self._auto_shift and self.n_rows + n >= 4 * self._rows_at_shift:
                 self._recentre(X, perm, offsets, counts)
             st = _lib.stream_ptr(dev)
-            nb = lib.sqfa_class_sums_workspace_bytes(n, D, C)
+            nb = self.lib.sqfa_class_sums_workspace_bytes(n, D, C)
             ws = torch.empty(max(nb, 1), dtype=torch.uint8, device=dev)
+            fn, xa = ops._x_fn("sqfa_class_sums")
             _lib.check(
-                lib.sqfa_class_sums(_lib.ptr(X), X.stride(0), _lib.ptr(perm), _lib.ptr(offsets), _lib.ptr(self.shift),
-                                    n, D, C, _lib.ptr(self.sums), 1, _lib.ptr(ws), nb, st),
+                fn(*xa(X), _lib.ptr(perm), _lib.ptr(offsets), _lib.ptr(self.shift), n, D, C, _lib.ptr(self.sums), 1,
+                   _lib.ptr(ws), nb, st),
                 "sqfa_class_sums",
             )
-            nb = lib.sqfa_class_gram_workspace_bytes(n, D, C)
+            nb = ops._query("sqfa_class_gram_workspace_bytes", n, D, C)
             ws = torch.empty(nb, dtype=torch.uint8, device=dev)
+            fn, xa = ops._x_fn("sqfa_class_gram")
             _lib.check(
-                lib.sqfa_class_gram(_lib.ptr(X), X.stride(0), _lib.ptr(perm), _lib.ptr(offsets), _lib.ptr(self.shift),
-                                    n, D, C, _lib.ptr(self.gram), 1, 0, None, 0, 0, 0, _lib.ptr(ws), nb, st),
+                fn(*xa(X), _lib.ptr(perm), _lib.ptr(offsets), _lib.ptr(self.shift), n, D, C, _lib.ptr(self.gram), 1, 0,
+                   None, 0, 0, 0, _lib.ptr(ws), nb, st),
                 "sqfa_class_gram",
             )
             self.counts += counts[:C]
@@ -225,7 +246,7 @@ class StreamingClassStatistics:
         u - n m. Done every time the number of rows grows 4x, so the shift stays within a few
         standard errors of the means whatever the first chunk looked like -- a shift far from the
         mean inflates the accumulated Gram by n d d^T and with it the fp32 rounding error."""
-        ops = _cuda_ops()
+        ops = _cuda_ops(X.dtype)
         u_c = ops.class_sums_shifted(X, perm, offsets, self.shift, self.C)
         n_old = self.counts.to(torch.float32)[:, None]
         n_all = n_old + counts[: self.C].to(torch.float32)[:, None]
@@ -277,7 +298,9 @@ def _single_class(points, estimator_id, assume_centered):
     n, D = X.shape
     with torch.cuda.device(dev):
         y = torch.zeros(n, dtype=torch.int64, device=dev)
-        centre = torch.zeros(1, D, dtype=X.dtype, device=dev) if assume_centered else None
+        # the centring vector has the dtype of the statistics: float32 for bf16 / fp16 points
+        centre = torch.zeros(1, D, dtype=torch.float64 if X.dtype == torch.float64 else torch.float32,
+                             device=dev) if assume_centered else None
         _, cov, _, _ = run_class_statistics(
             _cuda_ops(X.dtype), X, y, estimator_id, n_classes=1, ddof=0 if assume_centered else 1, centre=centre,
             want_sm=False,
