@@ -52,6 +52,14 @@ typedef void* sqfa_stream_t; /* cudaStream_t */
 #define SQFA_DIST_AFFINE_INVARIANT 0 /* distances.py:70-89  sqrt(sum log^2 lambda + 1e-6)      */
 #define SQFA_DIST_FISHER_RAO_LB 1    /* distances.py:210-237 sqrt(AI^2(E_i,E_j)/2 + 1e-6)       */
 #define SQFA_DIST_LOG_EUCLIDEAN 2    /* distances.py:119-138 sqrt(|logA - logB|_F^2 + 1e-6)     */
+/* Bures-Wasserstein between SPD matrices (an extension, not reference API):
+ *   d^2 = tr A + tr B - 2 tr((B^1/2 A B^1/2)^1/2), clamped at 0; sqrt(d^2 + 1e-6). m <= 34, else SQFA_E_UNSUPPORTED;
+ *   no eig_out. */
+#define SQFA_DIST_BURES_WASSERSTEIN 3
+/* 2-Wasserstein between Gaussians: |mu_A - mu_B|^2 + Bures-Wasserstein^2 of the covariances. Closures only
+ * (sqfa_fused_loss, sqfa_fused_loss_sharded, sqfa_closure_eval; M required, m = n_filters): sqfa_class_factor
+ * and sqfa_pair_distances take no means and reject it. */
+#define SQFA_DIST_WASSERSTEIN_GAUSSIAN 4
 /* add SQFA_DIST_SQUARED to get the squared variants (no sqrt, no epsilon) */
 #define SQFA_DIST_SQUARED 16
 

@@ -14,8 +14,11 @@ from . import _lib
 DIST_AI = 0  # SQFA_DIST_AFFINE_INVARIANT
 DIST_FR = 1  # SQFA_DIST_FISHER_RAO_LB
 DIST_LE = 2  # SQFA_DIST_LOG_EUCLIDEAN
+DIST_BW = 3  # SQFA_DIST_BURES_WASSERSTEIN
+DIST_W2 = 4  # SQFA_DIST_WASSERSTEIN_GAUSSIAN
 SQUARED = 16  # SQFA_DIST_SQUARED
 MAX_M = 64
+MAX_M_BW = 34  # Bures-Wasserstein: column-pair kernel only
 MAX_FILTERS = 32
 
 

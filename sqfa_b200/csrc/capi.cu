@@ -299,7 +299,26 @@ int sqfa_transform_h(const void* X, int64_t ldx, int32_t elem, const float* F, i
 static int dist_ok(int32_t dist) {
   const int b = dist & 15;
   return (dist & ~(15 | SQFA_DIST_SQUARED)) == 0 &&
-         (b == SQFA_DIST_AFFINE_INVARIANT || b == SQFA_DIST_FISHER_RAO_LB || b == SQFA_DIST_LOG_EUCLIDEAN);
+         (b == SQFA_DIST_AFFINE_INVARIANT || b == SQFA_DIST_FISHER_RAO_LB || b == SQFA_DIST_LOG_EUCLIDEAN ||
+          b == SQFA_DIST_BURES_WASSERSTEIN || b == SQFA_DIST_WASSERSTEIN_GAUSSIAN);
+}
+
+// distances whose closure reads the class means
+static int dist_uses_means(int32_t dist) {
+  const int b = dist & 15;
+  return b == SQFA_DIST_FISHER_RAO_LB || b == SQFA_DIST_WASSERSTEIN_GAUSSIAN;
+}
+
+// Bures-Wasserstein runs in the column-pair kernel only (m <= 34); the Gaussian form needs means, which the
+// per-matrix entry points do not take. Returns 0 or the fail_arg code.
+static int check_bw_matrices(const char* fn, int32_t dist, int32_t m) {
+  const int b = dist & 15;
+  if (b == SQFA_DIST_WASSERSTEIN_GAUSSIAN)
+    return fail_arg(fn, "SQFA_DIST_WASSERSTEIN_GAUSSIAN needs class means: use SQFA_DIST_BURES_WASSERSTEIN on the "
+                        "covariances and add |mu_A - mu_B|^2");
+  if (b == SQFA_DIST_BURES_WASSERSTEIN && m > 34)
+    return fail_arg(fn, "Bures-Wasserstein supports m <= 34", SQFA_E_UNSUPPORTED);
+  return 0;
 }
 
 int sqfa_embed_fwd(const float* Psi, const float* Mu, float noise, int32_t n_classes, int32_t n_filters,
@@ -326,6 +345,7 @@ int sqfa_class_factor(const float* E, int32_t n_classes, int32_t m, int32_t dist
   if (!dist_ok(dist) || E == nullptr || W == nullptr || flag == nullptr || n_classes < 0 || m <= 0)
     return fail_arg(__func__, "bad argument");
   if (m > SQFA_MAX_M) return fail_arg(__func__, "m exceeds SQFA_MAX_M", SQFA_E_UNSUPPORTED);
+  if (const int rc = check_bw_matrices(__func__, dist, m)) return rc;
   return wrap(__func__, sqfa::launch_class_factor(E, n_classes, m, dist, W, flag, S(stream)));
 }
 
@@ -344,6 +364,9 @@ int sqfa_pair_distances(const float* Wa, const float* Wb, int32_t n_a, int32_t n
       (triangular && (n_a != n_b || Wa != Wb)) || ((gEa == nullptr) != (gEb == nullptr)) ||
       (eig_out != nullptr && (triangular || (dist & 15) == SQFA_DIST_LOG_EUCLIDEAN)))
     return fail_arg(__func__, "bad argument");
+  if (const int rc = check_bw_matrices(__func__, dist, m)) return rc;
+  if (eig_out != nullptr && (dist & 15) == SQFA_DIST_BURES_WASSERSTEIN)
+    return fail_arg(__func__, "eig_out is not defined for Bures-Wasserstein");
   const int64_t P = triangular ? (int64_t)n_a * (n_a - 1) / 2 : (int64_t)n_a * n_b;
   if (pair_begin < 0 || pair_end > P || pair_begin > pair_end) return fail_arg(__func__, "bad pair range");
   if (m > SQFA_MAX_M) return fail_arg(__func__, "m exceeds SQFA_MAX_M", SQFA_E_UNSUPPORTED);
@@ -380,7 +403,7 @@ static int closure_common(const char* fn, const float* S_, const float* M, const
                           size_t ws_bytes, sqfa_stream_t stream) {
   const int base = dist & 15;
   if (!dist_ok(dist) || S_ == nullptr || filters == nullptr || out == nullptr || grad == nullptr || ws == nullptr ||
-      n_classes <= 0 || n_dim <= 0 || n_filters <= 0 || (base == SQFA_DIST_FISHER_RAO_LB && M == nullptr) ||
+      n_classes <= 0 || n_dim <= 0 || n_filters <= 0 || (dist_uses_means(dist) && M == nullptr) ||
       n_fixed < 0 || n_fixed > n_filters || (reinterpret_cast<uintptr_t>(ws) & 15) != 0)
     return fail_arg(fn, "bad argument");
   const int m = base == SQFA_DIST_FISHER_RAO_LB ? n_filters + 1 : n_filters;
@@ -417,7 +440,7 @@ int sqfa_fused_loss_sharded(int32_t phase, const float* S_, const float* M, cons
                             size_t ws_bytes, sqfa_stream_t stream) {
   const int base = dist & 15;
   if (!dist_ok(dist) || S_ == nullptr || F == nullptr || ws == nullptr || n_classes <= 0 || n_dim <= 0 ||
-      n_filters <= 0 || (base == SQFA_DIST_FISHER_RAO_LB && M == nullptr) || phase < 0 || phase > 2 ||
+      n_filters <= 0 || (dist_uses_means(dist) && M == nullptr) || phase < 0 || phase > 2 ||
       (phase == 2 && dF == nullptr) || class_begin < 0 || class_end > n_classes || class_begin > class_end ||
       (reinterpret_cast<uintptr_t>(ws) & 15) != 0)
     return fail_arg(__func__, "bad argument");

@@ -13,7 +13,8 @@
 //   pair_reduce             dLoss/dE_c in fixed order -> embedding adjoint (gPsi, gMu); loss
 //   project_bwd             class-split partials of dLoss/dF
 //   closure_finish          dLoss/dF, constraint adjoint -> grad, max |grad|
-// Log-Euclidean adds le_grad + le_factor_bwd + embed_bwd between the pair kernel and project_bwd.
+// Log-Euclidean adds le_grad + le_factor_bwd + embed_bwd between the pair kernel and project_bwd; the
+// Gaussian Wasserstein distance projects the means too (no embedding) and adds le_grad for their gradient.
 #include <cstdint>
 #include <cuda_runtime.h>
 
@@ -71,6 +72,7 @@ cudaError_t launch_fused_loss(const float* S, const float* M, const float* filte
   const int base = dist & 15;
   const bool fr = base == SQFA_DIST_FISHER_RAO_LB;
   const bool le = base == SQFA_DIST_LOG_EUCLIDEAN;
+  const bool means = fr || base == SQFA_DIST_WASSERSTEIN_GAUSSIAN;  // this distance uses the class means
   const int m = fr ? k + 1 : k;
   const ClosureLayout L = closure_layout(C, D, k, dist, pair_begin, pair_end);
   float* Fbuf = ws + L.F;
@@ -88,7 +90,7 @@ cudaError_t launch_fused_loss(const float* S, const float* M, const float* filte
   float* PsiPart = ws + L.psipart;
   float* MuPart = ws + L.mupart;
   float* pairws = ws + L.pair;
-  const float* Mfr = fr ? M : nullptr;
+  const float* Mfr = means ? M : nullptr;
   const int64_t P = (int64_t)C * (C - 1) / 2;
   const float weight = -1.0f / (float)(P > 0 ? P : 1);
   const int sphere = constraint == 1 ? 1 : 0;
@@ -99,9 +101,9 @@ cudaError_t launch_fused_loss(const float* S, const float* M, const float* filte
     if ((e = launch_constraint_fwd(filters, D, k, Fbuf, inv_norm, st)) != cudaSuccess) return e;
     F = Fbuf;
   }
-  if ((e = launch_project_partials(S, Mfr, F, C, D, k, T, proj, PsiPart, fr ? MuPart : nullptr, st)) != cudaSuccess)
+  if ((e = launch_project_partials(S, Mfr, F, C, D, k, T, proj, PsiPart, means ? MuPart : nullptr, st)) != cudaSuccess)
     return e;
-  if ((e = launch_class_prepare(PsiPart, fr ? MuPart : nullptr, project_nchunk(D), noise, C, k, dist, Mu, E, W, flag,
+  if ((e = launch_class_prepare(PsiPart, means ? MuPart : nullptr, project_nchunk(D), noise, C, k, dist, Mu, E, W, flag,
                                 st)) != cudaSuccess)
     return e;
   if ((e = launch_pair_closure(W, C, m, dist, pair_begin, pair_end, weight, Mu, k, out, gPsi, gMu, gLog, pairws, st)) !=
@@ -112,7 +114,7 @@ cudaError_t launch_fused_loss(const float* S, const float* M, const float* filte
     if ((e = launch_class_factor_bwd(W, gLog, C, m, dist, gE, st)) != cudaSuccess) return e;
     if ((e = launch_embed_bwd(gE, Mu, C, k, 0, gPsi, gMu, st)) != cudaSuccess) return e;
   }
-  return launch_project_bwd_constrained(gPsi, fr ? gMu : nullptr, T, Mfr, C, D, k, F, inv_norm, sphere, n_fixed, grad,
+  return launch_project_bwd_constrained(gPsi, means ? gMu : nullptr, T, Mfr, C, D, k, F, inv_norm, sphere, n_fixed, grad,
                                         out, out_host, reinterpret_cast<unsigned int*>(flag + 1), proj, st);
 }
 
@@ -144,6 +146,7 @@ cudaError_t launch_fused_loss_sharded(int phase, const float* S, const float* M,
                                       float* dF, float* ws, cudaStream_t st) {
   const int base = dist & 15;
   const bool fr = base == SQFA_DIST_FISHER_RAO_LB;
+  const bool means = fr || base == SQFA_DIST_WASSERSTEIN_GAUSSIAN;
   if (base == SQFA_DIST_LOG_EUCLIDEAN) return cudaErrorNotSupported;
   const int m = fr ? k + 1 : k;
   const ClosureLayout L = closure_layout(C, D, k, dist, pair_begin, pair_end);
@@ -154,28 +157,28 @@ cudaError_t launch_fused_loss_sharded(int phase, const float* S, const float* M,
   float* PsiPart = ws + L.psipart;
   float* MuPart = ws + L.mupart;
   float* proj = ws + L.proj;
-  const float* Mfr = fr ? M : nullptr;
+  const float* Mfr = means ? M : nullptr;
   const int nchunk = project_nchunk(D);
   const int n_own = c1 > c0 ? c1 - c0 : 0;
   cudaError_t e;
   if (phase == 0) {
     if ((e = cudaMemsetAsync(PsiPart, 0, (L.pair - L.psipart) * sizeof(float), st)) != cudaSuccess) return e;
     if (n_own == 0) return cudaSuccess;
-    return launch_project_partials(S + (size_t)c0 * D * D, fr ? M + (size_t)c0 * D : nullptr, F, n_own, D, k,
+    return launch_project_partials(S + (size_t)c0 * D * D, means ? M + (size_t)c0 * D : nullptr, F, n_own, D, k,
                                    T + (size_t)c0 * k * D, proj, PsiPart + (size_t)c0 * nchunk * k * k,
-                                   fr ? MuPart + (size_t)c0 * nchunk * k : nullptr, st);
+                                   means ? MuPart + (size_t)c0 * nchunk * k : nullptr, st);
   }
   if (phase == 1) {
     const int64_t P = (int64_t)C * (C - 1) / 2;
     const float weight = -1.0f / (float)(P > 0 ? P : 1);
-    if ((e = launch_class_prepare(PsiPart, fr ? MuPart : nullptr, nchunk, noise, C, k, dist, Mu, ws + L.E, ws + L.W,
+    if ((e = launch_class_prepare(PsiPart, means ? MuPart : nullptr, nchunk, noise, C, k, dist, Mu, ws + L.E, ws + L.W,
                                   reinterpret_cast<int32_t*>(ws + L.flag), st)) != cudaSuccess)
       return e;
     return launch_pair_closure(ws + L.W, C, m, dist, pair_begin, pair_end, weight, Mu, k, ws + L.red_out, gPsi, gMu,
                                nullptr, ws + L.pair, st);
   }
   // phase 2: (gPsi, gMu) are now the sums over all pairs
-  return launch_project_bwd(gPsi + (size_t)c0 * k * k, fr ? gMu + (size_t)c0 * k : nullptr, T + (size_t)c0 * k * D,
+  return launch_project_bwd(gPsi + (size_t)c0 * k * k, means ? gMu + (size_t)c0 * k : nullptr, T + (size_t)c0 * k * D,
                             Mfr != nullptr ? Mfr + (size_t)c0 * D : nullptr, n_own, D, k, dF, proj, st);
 }
 

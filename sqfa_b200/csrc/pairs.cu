@@ -18,6 +18,13 @@
 // -- no 1/(lambda_a - lambda_b) terms (the eigh backward of the reference has them and NaNs on
 // repeated eigenvalues). Only the strict lower triangle (i > j) is evaluated: the reference
 // computes all C*C pairs and then reads the lower triangle (_optim.py:94).
+//
+// Bures-Wasserstein (m <= 34, column-pair kernel): the same Jacobi on A = L_i^T L_j instead. Its singular
+// values sigma_q = |a_q| sum to the fidelity tr((E_j^1/2 E_i E_j^1/2)^1/2), so
+//   d^2 = |L_i|_F^2 + |L_j|_F^2 - 2 sum_q sigma_q                         (clamped at 0)
+//   d(d^2)/dE_i = I - sum_q sigma_q^-1 y_q y_q^T,   y_q = L_i^-T a_q
+//   d(d^2)/dE_j = I - sum_q sigma_q^-3 z_q z_q^T,   z_q = L_i a_q
+// -- again no 1/(sigma_a - sigma_b) terms. The Gaussian form adds |mu_i - mu_j|^2 (closure only).
 #include <cmath>
 #include <cstdint>
 #include <cstdlib>
@@ -299,6 +306,7 @@ class_factor_kernel(const float* __restrict__ E, int C, int m, int dist, float* 
 //   E_c = Psi_c + noise I (+ Calvo-Oller embedding with mu'_c for Fisher-Rao)
 //         (reference model.py:216-217 / 537-538, distances.py:162-174),
 //   W_c = factorisation of E_c (above).  E is also written out (m x m per class).
+// mu'_c is formed whenever MuPart is given (Fisher-Rao, Gaussian Wasserstein); only Fisher-Rao embeds it.
 __global__ void __launch_bounds__(PAIR_WARPS * 32)
 class_prepare_kernel(const float* __restrict__ PsiPart, const float* __restrict__ MuPart, int nchunk, float noise,
                      int C, int k, int dist, float* __restrict__ Mu, float* __restrict__ E, float* __restrict__ W,
@@ -313,7 +321,7 @@ class_prepare_kernel(const float* __restrict__ PsiPart, const float* __restrict_
   float* scratch = smem + (size_t)warp * per_warp;
   float* Es = scratch + factor_scratch_floats(m);
   float* mus = Es + m * m;
-  if (fr) {
+  if (MuPart != nullptr) {
     for (int r = lane; r < k; r += 32) {
       float a = 0.f;
       const float* mp_ = MuPart + (int64_t)c * nchunk * k + r;
@@ -647,7 +655,8 @@ __device__ __forceinline__ void cp_rotation(float alpha, float beta, float ab, b
   }
 }
 
-template <int MJ>
+// BW = true: Bures-Wasserstein (A = L_i^T L_j; L_j^T is staged where Linv_j is) -- see the file header.
+template <int MJ, bool BW>
 __global__ void __launch_bounds__(PAIR_WARPS * 32, (MJ <= 12 ? 6 : (MJ <= 20 ? 5 : 3)))
 pair_cp_kernel(const PairArgs A) {
   using G = CpGeom<MJ>;
@@ -686,6 +695,10 @@ pair_cp_kernel(const PairArgs A) {
         float* rp = A.rowpart + ((int64_t)t * R + ii) * m2;
         for (int idx = lane; idx < m2; idx += 32) rp[idx] = 0.f;
       }
+      if constexpr (BW) {
+        if (A.pwpart != nullptr)
+          for (int idx = lane; idx < R; idx += 32) A.pwpart[((int64_t)t * R + ii) * R + idx] = 0.f;
+      }
       continue;
     }
     const float* Wi = A.Wa + (int64_t)i * 2 * m2;
@@ -695,14 +708,23 @@ pair_cp_kernel(const PairArgs A) {
       sLi[idx] = c < m ? Wi[r * m + c] : 0.f;
     }
     if (active) {  // Linv_j of this problem's column class (row MJ - 1 of sJ stays zero: Y never reaches it)
-      const float* Wj = A.Wb + (int64_t)j * 2 * m2 + m2;
-      for (int idx = lg; idx < m2; idx += LP) {
-        const int q = div_m(idx);
-        sJ[q * LDJ + (idx - q * m)] = Wj[idx];
+      if constexpr (BW) {  // L_j^T: sJ[q][r] = L_j[r][q]
+        const float* Wj = A.Wb + (int64_t)j * 2 * m2;
+        for (int idx = lg; idx < m2; idx += LP) {
+          const int r = div_m(idx);
+          sJ[(idx - r * m) * LDJ + r] = Wj[idx];
+        }
+      } else {
+        const float* Wj = A.Wb + (int64_t)j * 2 * m2 + m2;
+        for (int idx = lg; idx < m2; idx += LP) {
+          const int q = div_m(idx);
+          sJ[q * LDJ + (idx - q * m)] = Wj[idx];
+        }
       }
     }
     __syncwarp();
-    // ---- columns 2 lg and 2 lg + 1 of A: a[s] = sum_r Linv_j[q][r] L_i[r][s]  (row MJ - 1 of sJ is zero for odd m)
+    // ---- columns 2 lg and 2 lg + 1 of A: a[s] = sum_r Linv_j[q][r] L_i[r][s]  (row MJ - 1 of sJ is zero for odd m;
+    // BW: L_j^T[q][r] in place of Linv_j[q][r])
     float2 a[MH], b[MH];
 #pragma unroll
     for (int s = 0; s < MH; ++s) { a[s] = make_float2(0.f, 0.f); b[s] = make_float2(0.f, 0.f); }
@@ -829,15 +851,48 @@ pair_cp_kernel(const PairArgs A) {
     const bool pad_first = m_odd && (sweeps & 1);
     const bool real_a = active && !(pad_first && lg == 0);
     const bool real_b = active && !(m_odd && !pad_first && lg == LP - 1);
-    const float lla = real_a ? logf(n2a) : 0.f, llb = real_b ? logf(n2b) : 0.f;
+    // AI: log lambda; BW: sigma
+    const float lla = BW ? (real_a ? sqrtf(n2a) : 0.f) : (real_a ? logf(n2a) : 0.f);
+    const float llb = BW ? (real_b ? sqrtf(n2b) : 0.f) : (real_b ? logf(n2b) : 0.f);
     const int g0 = (g * LP) & 31;
     float d2 = 0.f;
-    {
+    bool bw_live = true;  // BW: d^2 of the matrices was not clamped (its gradient is live)
+    if constexpr (BW) {
+      // |L_i|_F^2 + |L_j|_F^2 - 2 (sigma_a + sigma_b) over this lane's rows 2 lg, 2 lg + 1 of L_i and L_j^T;
+      // Gaussian form: the lane's share of |mu_i - mu_j|^2 (components lg, lg + LP, ...)
+      float part = -2.f * (lla + llb), pmu = 0.f;
+      if (active) {
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          const int row = 2 * lg + h;
+          if (row < m) {
+            for (int c = 0; c <= row; ++c) part = fmaf(sLi[row * MP4 + c], sLi[row * MP4 + c], part);
+            for (int c = row; c < m; ++c) part = fmaf(sJ[row * LDJ + c], sJ[row * LDJ + c], part);
+          }
+        }
+        if (A.Mu != nullptr) {
+          const float* mui = A.Mu + (int64_t)i * A.k;
+          const float* muj = A.Mu + (int64_t)j * A.k;
+          for (int e = lg; e < A.k; e += LP) {
+            const float df = mui[e] - muj[e];
+            pmu = fmaf(df, df, pmu);
+          }
+        }
+      }
+      float dmu = 0.f;
+#pragma unroll
+      for (int u = 0; u < LP; ++u) {  // fixed order, same in every lane
+        d2 += __shfl_sync(FULL, part, (g0 + u) & 31);
+        dmu += __shfl_sync(FULL, pmu, (g0 + u) & 31);
+      }
+      bw_live = d2 > 0.f;
+      d2 = (d2 < 0.f ? 0.f : d2) + dmu;  // not fmaxf: a NaN (failed Cholesky) must reach the non-finite count
+    } else {
       const float part = lla * lla + llb * llb;
 #pragma unroll
       for (int u = 0; u < LP; ++u) d2 += __shfl_sync(FULL, part, (g0 + u) & 31);  // fixed order, same in every lane
     }
-    if (A.eig_out != nullptr) {  // descending order (linalg.py:69-70); the padding column has norm 0 and ranks last
+    if (!BW && A.eig_out != nullptr) {  // descending order (linalg.py:69-70); the padding column has norm 0 and ranks last
       int ra = 0, rb = 0;
 #pragma unroll
       for (int u = 0; u < LP; ++u) {
@@ -867,6 +922,127 @@ pair_cp_kernel(const PairArgs A) {
         w = A.weight * dd_dd2;
         if (A.gD != nullptr)
           w *= tri ? (A.gD[(int64_t)i * nB + j] + A.gD[(int64_t)j * nB + i]) : A.gD[(int64_t)i * nB + j];
+      }
+      if constexpr (BW) {
+        if (A.pwpart != nullptr && alive && lg == 0 && g < R) A.pwpart[((int64_t)t * R + ii) * R + g] = 2.f * w;
+        if (!bw_live) w = 0.f;
+        // G of the positions' vectors V (rows of sY = component, columns = position) with one coefficient per
+        // position (sCo), plus w I: a lane owns the rows s0 = lg and s1 = lg + LP, packed in the two halves.
+        // toRow: G_i, summed over the problems of the row in a fixed order and stored by the first one;
+        // else G_j, added to the problem's column accumulator.
+        float* rp = A.rowpart + ((int64_t)t * R + ii) * m2;
+        auto gram_pass = [&](bool toRow) {
+          const int s0 = lg, s1 = lg + LP;
+          const bool mine0 = alive && s0 < m, mine1 = alive && s1 < m;
+          float2 cij[MP4];
+          {
+            const float* v0 = sY + (mine0 ? s0 : 0) * MP4;
+            const float* v1 = sY + (mine1 ? s1 : 0) * MP4;
+#pragma unroll
+            for (int q4 = 0; q4 < MP4 / 4; ++q4) {
+              const float4 y0 = *reinterpret_cast<const float4*>(v0 + 4 * q4);
+              const float4 y1 = *reinterpret_cast<const float4*>(v1 + 4 * q4);
+              const float4 c = *reinterpret_cast<const float4*>(sCo + 4 * q4);
+              cij[4 * q4] = make_float2(y0.x * c.x, y1.x * c.x);
+              cij[4 * q4 + 1] = make_float2(y0.y * c.y, y1.y * c.y);
+              cij[4 * q4 + 2] = make_float2(y0.z * c.z, y1.z * c.z);
+              cij[4 * q4 + 3] = make_float2(y0.w * c.w, y1.w * c.w);
+            }
+          }
+#pragma unroll 1
+          for (int r = 0; r < m; ++r) {
+            float2 gab = make_float2(r == s0 ? w : 0.f, r == s1 ? w : 0.f);
+#pragma unroll
+            for (int q4 = 0; q4 < MP4 / 4; ++q4) {
+              const float4 yr = *reinterpret_cast<const float4*>(sY + r * MP4 + 4 * q4);
+              gab = __ffma2_rn(make_float2(yr.x, yr.x), cij[4 * q4], gab);
+              gab = __ffma2_rn(make_float2(yr.y, yr.y), cij[4 * q4 + 1], gab);
+              gab = __ffma2_rn(make_float2(yr.z, yr.z), cij[4 * q4 + 2], gab);
+              gab = __ffma2_rn(make_float2(yr.w, yr.w), cij[4 * q4 + 3], gab);
+            }
+            if (toRow) {
+              const float g0v = (active && mine0) ? gab.x : 0.f, g1v = (active && mine1) ? gab.y : 0.f;
+              float t0 = 0.f, t1 = 0.f;
+#pragma unroll
+              for (int gg = 0; gg < NP; ++gg) {
+                t0 += __shfl_sync(FULL, g0v, (gg * LP + lg) & 31);
+                t1 += __shfl_sync(FULL, g1v, (gg * LP + lg) & 31);
+              }
+              if (g == 0 && mine0) rp[r * m + s0] = t0;
+              if (g == 0 && mine1) rp[r * m + s1] = t1;
+            } else if (active) {
+              if (mine0) sC[r * m + s0] += gab.x;
+              if (mine1) sC[r * m + s1] += gab.y;
+            }
+          }
+        };
+        // ---- pass 1: Z = L_i A_f (sLi still holds L_i; L_j^T in sJ is dead) -> G_j with -w sigma^-3
+        __syncwarp();
+        if constexpr (MP4 > MJ) {  // the two padding columns of sY lie on what was L_j^T: zero them
+          for (int idx = lg; idx < 2 * m; idx += LP) sY[(idx >> 1) * MP4 + MJ + (idx & 1)] = 0.f;
+        }
+        if (alive) {
+#pragma unroll
+          for (int r = 0; r < MJ; ++r) {
+            if (r < m) {
+              float2 za = make_float2(0.f, 0.f), zb = za;
+#pragma unroll
+              for (int s4 = 0; s4 <= r / 4; ++s4) {  // L_i is lower triangular: row r ends at column r
+                const float4 wv = *reinterpret_cast<const float4*>(sLi + r * MP4 + 4 * s4);
+                const float2 w0 = make_float2(wv.x, wv.y), w1 = make_float2(wv.z, wv.w);
+                za = __ffma2_rn(w0, a[2 * s4], za);
+                za = __ffma2_rn(w1, a[2 * s4 + 1], za);
+                zb = __ffma2_rn(w0, b[2 * s4], zb);
+                zb = __ffma2_rn(w1, b[2 * s4 + 1], zb);
+              }
+              *reinterpret_cast<float2*>(sY + r * MP4 + 2 * lg) = make_float2(za.x + za.y, zb.x + zb.y);
+            }
+          }
+          *reinterpret_cast<float2*>(sCo + 2 * lg) =
+              make_float2(real_a ? -w / (lla * n2a) : 0.f, real_b ? -w / (llb * n2b) : 0.f);
+        }
+        __syncwarp();
+        gram_pass(false);
+        // ---- pass 2: Y = L_i^-T A_f -> G_i with -w sigma^-1
+        __syncwarp();
+        for (int idx = lane; idx < m * MP4; idx += 32) {
+          const int r = idx / MP4, c = idx - r * MP4;
+          sLi[idx] = c < m ? Wi[m2 + r * m + c] : 0.f;
+        }
+        __syncwarp();
+        float2 ya[MH], yb[MH];
+#pragma unroll
+        for (int s = 0; s < MH; ++s) { ya[s] = make_float2(0.f, 0.f); yb[s] = make_float2(0.f, 0.f); }
+#pragma unroll
+        for (int s = 0; s < MJ; ++s) {
+          if (s < m) {
+            const float as = (s & 1) ? a[s / 2].y : a[s / 2].x, bs = (s & 1) ? b[s / 2].y : b[s / 2].x;
+            const float2 as2 = make_float2(as, as), bs2 = make_float2(bs, bs);
+#pragma unroll
+            for (int r4 = 0; r4 <= s / 4; ++r4) {  // Linv_i is lower triangular
+              const float4 wv = *reinterpret_cast<const float4*>(sLi + s * MP4 + 4 * r4);
+              const float2 w0 = make_float2(wv.x, wv.y), w1 = make_float2(wv.z, wv.w);
+              ya[2 * r4] = __ffma2_rn(as2, w0, ya[2 * r4]);
+              ya[2 * r4 + 1] = __ffma2_rn(as2, w1, ya[2 * r4 + 1]);
+              yb[2 * r4] = __ffma2_rn(bs2, w0, yb[2 * r4]);
+              yb[2 * r4 + 1] = __ffma2_rn(bs2, w1, yb[2 * r4 + 1]);
+            }
+          }
+        }
+        __syncwarp();  // every lane has read Z
+        if (alive) {
+#pragma unroll
+          for (int r = 0; r < MJ; ++r) {
+            if (r < m) {
+              const float y0 = (r & 1) ? ya[r / 2].y : ya[r / 2].x, y1 = (r & 1) ? yb[r / 2].y : yb[r / 2].x;
+              *reinterpret_cast<float2*>(sY + r * MP4 + 2 * lg) = make_float2(y0, y1);
+            }
+          }
+          *reinterpret_cast<float2*>(sCo + 2 * lg) = make_float2(real_a ? -w / lla : 0.f, real_b ? -w / llb : 0.f);
+        }
+        __syncwarp();
+        gram_pass(true);
+        continue;
       }
       // ---- Y = L_i^-T A_f for this lane's two columns: y[r] = sum_s Linv_i[s][r] a[s]
       __syncwarp();
@@ -976,17 +1152,26 @@ pair_cp_kernel(const PairArgs A) {
   }
 }
 
-template <int MJ>
-static cudaError_t launch_pair_cp(const PairArgs& A, cudaStream_t st) {
+template <int MJ, bool BW>
+static cudaError_t launch_pair_cp_t(const PairArgs& A, cudaStream_t st) {
   const int smem = PAIR_WARPS * cp_warp_floats(MJ, A.m) * (int)sizeof(float);
   static int smem_set[kMaxDevices] = {0};
   {
-    cudaError_t e = ensure_dynamic_smem(pair_cp_kernel<MJ>, smem, smem_set);
+    cudaError_t e = ensure_dynamic_smem(pair_cp_kernel<MJ, BW>, smem, smem_set);
     if (e != cudaSuccess) return e;
   }
   const unsigned blocks = (unsigned)((A.T.ntiles + PAIR_WARPS - 1) / PAIR_WARPS);
-  pair_cp_kernel<MJ><<<blocks, PAIR_WARPS * 32, smem, st>>>(A);
+  pair_cp_kernel<MJ, BW><<<blocks, PAIR_WARPS * 32, smem, st>>>(A);
   return cudaGetLastError();
+}
+
+__host__ __device__ inline bool is_bw_family(int dist) {
+  return (dist & 15) == SQFA_DIST_BURES_WASSERSTEIN || (dist & 15) == SQFA_DIST_WASSERSTEIN_GAUSSIAN;
+}
+
+template <int MJ>
+static cudaError_t launch_pair_cp(const PairArgs& A, cudaStream_t st) {
+  return is_bw_family(A.dist) ? launch_pair_cp_t<MJ, true>(A, st) : launch_pair_cp_t<MJ, false>(A, st);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1033,35 +1218,39 @@ pair_le_kernel(const PairArgs A) {
   }
 }
 
-// gLa[c] += sum_b pw(c, b) (logA_c - logB_b)   and   gLb[c] -= sum_a pw(a, c) (logA_a - logB_c),
-// pairs in launch order; block = class, thread = matrix element. Self distances (tri): one sum over
-// all other classes.
+// gLa[c] += sum_b pw(c, b) (xA_c - xB_b)   and   gLb[c] -= sum_a pw(a, c) (xA_a - xB_c),
+// pairs in launch order; block = class, thread = element. x = the ne floats at Wa / Wb + class * stride + off
+// (log-Euclidean: the matrix logs; Gaussian Wasserstein: the means), pw = one factor per pair in the R x R
+// tiles of T. Self distances (tri): one sum over all other classes.
 __global__ void __launch_bounds__(256)
-le_grad_kernel(const PairTiles T, const float* __restrict__ Wa, const float* __restrict__ Wb, int nA, int nB, int m,
-               const float* __restrict__ pw, float* gLa, float* gLb) {
+le_grad_kernel(const PairTiles T, const float* __restrict__ Wa, const float* __restrict__ Wb, int nA, int nB, int ne,
+               int stride, int off, const float* __restrict__ pw, float* gLa, float* gLb) {
   const int c = blockIdx.x;
-  const int m2 = m * m, stride = 2 * m2 + 2 * m, off = m2 + 2 * m;
-  for (int e = threadIdx.x; e < m2; e += blockDim.x) {
+  const int R = T.R, R2 = R * R;
+  // factor of pair (i, j): tile (i / R, j / R), slot (i % R, j % R)
+  auto pw_at = [&](int i, int j) {
+    const int64_t bi = i / R;
+    const int64_t tt = (T.tri ? bi * (bi + 1) / 2 : bi * T.nbj) + j / R - T.tile0;
+    return pw[tt * R2 + (i % R) * R + j % R];
+  };
+  for (int e = threadIdx.x; e < ne; e += blockDim.x) {
     float ga = 0.f, gb = 0.f;
-    if (c < nA && c >= T.bi0 && c <= T.bi1) {  // row side: pairs (c, j)
+    if (c < nA && c / R >= T.bi0 && c / R <= T.bi1) {  // row side: pairs (c, j)
       const float lc = Wa[(int64_t)c * stride + off + e];
-      const int nj = T.tri ? c : nB;  // (c, c) itself holds pw = 0
-      const int64_t base = (T.tri ? (int64_t)c * (c + 1) / 2 : (int64_t)c * T.nbj) - T.tile0;
-      for (int j = 0; j < nj; ++j) ga += pw[base + j] * (lc - Wb[(int64_t)j * stride + off + e]);
+      const int nj = T.tri ? c : nB;
+      for (int j = 0; j < nj; ++j) ga += pw_at(c, j) * (lc - Wb[(int64_t)j * stride + off + e]);
     }
     if (c < nB) {  // column side: pairs (i, c)
       const float lc = Wb[(int64_t)c * stride + off + e];
-      const int i0 = T.tri ? max(T.bi0, c + 1) : T.bi0;
-      for (int i = i0; i <= T.bi1; ++i) {
-        const int64_t tt = (T.tri ? (int64_t)i * (i + 1) / 2 : (int64_t)i * T.nbj) + c - T.tile0;
-        gb -= pw[tt] * (Wa[(int64_t)i * stride + off + e] - lc);
-      }
+      const int i0 = T.tri ? max(T.bi0 * R, c + 1) : T.bi0 * R;
+      const int i1 = min((T.bi1 + 1) * R, nA);
+      for (int i = i0; i < i1; ++i) gb -= pw_at(i, c) * (Wa[(int64_t)i * stride + off + e] - lc);
     }
     if (gLa == gLb) {
-      if (c < nA) gLa[(int64_t)c * m2 + e] += ga + gb;
+      if (c < nA) gLa[(int64_t)c * ne + e] += ga + gb;
     } else {
-      if (c < nA) gLa[(int64_t)c * m2 + e] += ga;
-      if (c < nB) gLb[(int64_t)c * m2 + e] += gb;
+      if (c < nA) gLa[(int64_t)c * ne + e] += ga;
+      if (c < nB) gLb[(int64_t)c * ne + e] += gb;
     }
   }
 }
@@ -1326,12 +1515,14 @@ PairWorkspace pair_workspace(int nA, int nB, int m, int dist, int tri, int64_t p
   const int64_t npairs = pair_end > pair_begin ? pair_end - pair_begin : 0;
   w.T = make_pair_tiles(nA, nB, tri, pair_begin, pair_end, pair_tile_edge(m, dist, npairs));
   const bool le = (dist & 15) == SQFA_DIST_LOG_EUCLIDEAN;
+  const bool w2 = (dist & 15) == SQFA_DIST_WASSERSTEIN_GAUSSIAN;
   const size_t part = le ? (size_t)w.T.ntiles : (size_t)w.T.ntiles * w.T.R * m * m;
   auto al = [](size_t n) { return (n + 63) & ~size_t(63); };
   w.rowpart = 0;
   w.colpart = al(part);
   w.losspart = w.colpart + (le ? 0 : al(part));
-  w.total_floats = w.losspart + al((size_t)2 * w.T.ntiles) + 64;
+  w.pwpart = w.losspart + al((size_t)2 * w.T.ntiles);
+  w.total_floats = w.pwpart + (w2 ? al((size_t)w.T.ntiles * w.T.R * w.T.R) : 0) + 64;
   return w;
 }
 
@@ -1343,6 +1534,7 @@ static cudaError_t launch_pair_kernel(const PairArgs& A, cudaStream_t st) {
     pair_le_kernel<<<blocks, PAIR_WARPS * 32, 0, st>>>(A);
     return cudaGetLastError();
   }
+  if (is_bw_family(A.dist) && m > 34) return cudaErrorNotSupported;
   if (pair_use_cp(m, A.dist)) {  // two columns per lane, several problems per warp
     switch ((m + 1) / 2) {
       case 1: return launch_pair_cp<2>(A, st);
@@ -1391,6 +1583,9 @@ static PairArgs make_pair_args(const float* Wa, const float* Wb, int nA, int nB,
   A.rowpart = want_grad ? ws + L.rowpart : nullptr;
   A.colpart = want_grad ? ws + L.colpart : nullptr;
   A.losspart = want_loss ? ws + L.losspart : nullptr;
+  A.Mu = nullptr;
+  A.k = 0;
+  A.pwpart = nullptr;
   A.T = L.T;
   return A;
 }
@@ -1413,7 +1608,8 @@ cudaError_t launch_pair_distances(const float* Wa, const float* Wb, int nA, int 
   if (!want_grad && !want_loss) return cudaSuccess;
   const int nC = nA > nB ? nA : nB;
   const bool le = (dist & 15) == SQFA_DIST_LOG_EUCLIDEAN;
-  if (le && want_grad) le_grad_kernel<<<nC, 256, 0, st>>>(L.T, Wa, Wb, nA, nB, m, A.rowpart, gEa, gEb);
+  if (le && want_grad)
+    le_grad_kernel<<<nC, 256, 0, st>>>(L.T, Wa, Wb, nA, nB, m * m, 2 * m * m + 2 * m, m * m + 2 * m, A.rowpart, gEa, gEb);
   pair_reduce_kernel<false><<<nC + 1, pair_reduce_threads(m), 0, st>>>(L.T, nA, nB, m, le ? nullptr : A.rowpart, A.colpart, A.losspart,
                                                     gEa, gEb, loss, 1.f, nullptr, 0, 0, nullptr, nullptr);
   return cudaGetLastError();
@@ -1428,14 +1624,26 @@ cudaError_t launch_pair_closure(const float* W, int C, int m, int dist, int64_t 
                                 float* ws, cudaStream_t st) {
   const bool le = (dist & 15) == SQFA_DIST_LOG_EUCLIDEAN;
   const bool fr = (dist & 15) == SQFA_DIST_FISHER_RAO_LB;
+  const bool w2 = (dist & 15) == SQFA_DIST_WASSERSTEIN_GAUSSIAN;
   const PairWorkspace L = pair_workspace(C, C, m, dist, 1, pair_begin, pair_end);
-  const PairArgs A = make_pair_args(W, W, C, C, m, dist, 1, pair_begin, pair_end, weight, nullptr, nullptr, nullptr,
-                                    true, true, ws, L);
+  PairArgs A = make_pair_args(W, W, C, C, m, dist, 1, pair_begin, pair_end, weight, nullptr, nullptr, nullptr,
+                              true, true, ws, L);
+  if (w2) {  // |mu'_i - mu'_j|^2 joins d^2; the pair factors give gMu below
+    A.Mu = Mu;
+    A.k = k;
+    A.pwpart = ws + L.pwpart;
+  }
   cudaError_t e = launch_pair_kernel(A, st);
   if (e != cudaSuccess) return e;
+  if (w2) {  // gMu[c] = sum_o pw(c, o) (mu'_c - mu'_o), fixed order
+    if ((e = cudaMemsetAsync(gMu, 0, (size_t)C * k * sizeof(float), st)) != cudaSuccess) return e;
+    if (L.T.ntiles > 0) le_grad_kernel<<<C, 256, 0, st>>>(L.T, Mu, Mu, C, C, k, k, 0, A.pwpart, gMu, gMu);
+  }
   if (le) {
     if ((e = cudaMemsetAsync(gLog, 0, (size_t)C * m * m * sizeof(float), st)) != cudaSuccess) return e;
-    if (L.T.ntiles > 0) le_grad_kernel<<<C, 256, 0, st>>>(L.T, W, W, C, C, m, A.rowpart, gLog, gLog);
+    if (L.T.ntiles > 0)
+      le_grad_kernel<<<C, 256, 0, st>>>(L.T, W, W, C, C, m * m, 2 * m * m + 2 * m, m * m + 2 * m, A.rowpart, gLog,
+                                        gLog);
     pair_reduce_kernel<true><<<C + 1, pair_reduce_threads(m), 0, st>>>(L.T, C, C, m, nullptr, nullptr, A.losspart, nullptr, nullptr, out,
                                                     weight, nullptr, k, 0, nullptr, nullptr);
     return cudaGetLastError();

@@ -112,10 +112,13 @@ struct PairArgs {
   float* rowpart;   // [ntiles][R][m*m] per-tile partial gradients of the row classes (LE: one factor per pair)
   float* colpart;   // [ntiles][R][m*m] ... of the column classes
   float* losspart;  // [ntiles][2] {sum of distances, non-finite count}
+  const float* Mu;  // Gaussian Wasserstein: class means [nA][k] (rows and columns are the same classes)
+  int k;
+  float* pwpart;    // Gaussian Wasserstein: [ntiles][R][R] per-pair factor of the means gradient
   PairTiles T;
 };
 struct PairWorkspace {
-  size_t rowpart, colpart, losspart, total_floats;  // offsets in floats
+  size_t rowpart, colpart, losspart, pwpart, total_floats;  // offsets in floats
   PairTiles T;
 };
 PairTiles make_pair_tiles(int nA, int nB, int tri, int64_t pair_begin, int64_t pair_end, int R);

@@ -8,6 +8,10 @@ distances of the reference (Bhattacharyya, Mahalanobis, Hellinger, Fisher-Rao wi
 covariance; alternative `distance_fun` plug-ins, SURVEY.md section 8(f) row 4) run in a warp-per-pair
 Cholesky kernel with an analytic backward. float64 inputs and matrices above 64 x 64 take the
 reference's own composition with device-side library calls, in the dtype of the inputs.
+
+Extension (not reference API): the Bures-Wasserstein distance between SPD matrices and the
+2-Wasserstein distance between Gaussians run in the same Jacobi pair kernel (up to 34 x 34) and
+can be used as `distance_fun` of the models' native fitting closure.
 """
 
 import torch
@@ -26,6 +30,10 @@ __all__ = [
     "mahalanobis",
     "hellinger",
     "fisher_rao_same_cov",
+    "bures_wasserstein_sq",
+    "bures_wasserstein",
+    "wasserstein_sq",
+    "wasserstein",
 ]
 
 
@@ -52,6 +60,12 @@ def _pairwise_composed(a3, b3, dist):
     if (dist & 15) == _ops.DIST_LE:
         diff = linalg.spd_log(a3)[:, None] - linalg.spd_log(b3)[None]
         d2 = (diff * diff).sum(dim=(-2, -1))
+    elif (dist & 15) == _ops.DIST_BW:
+        R = linalg.spd_sqrt(b3)
+        inner = torch.linalg.eigvalsh(R[None] @ a3[:, None] @ R[None]).clamp_min(0)
+        tr_a = torch.diagonal(a3, dim1=-2, dim2=-1).sum(-1)
+        tr_b = torch.diagonal(b3, dim1=-2, dim2=-1).sum(-1)
+        d2 = (tr_a[:, None] + tr_b[None] - 2 * torch.sqrt(inner).sum(dim=-1)).clamp_min(0)
     else:
         W = linalg.spd_inv_sqrt(b3)
         conj = W[None] @ a3[:, None] @ W.transpose(-2, -1)[None]
@@ -69,7 +83,8 @@ def _pairwise(A, B, dist):
         raise ValueError("expected SPD matrices of equal size, shapes (n, m, m)")
     dev = _lib.compute_device(A, B)
     with torch.cuda.device(dev):
-        if a3.dtype == torch.float32 and b3.dtype == torch.float32 and a3.shape[-1] <= _ops.MAX_M:
+        max_m = _ops.MAX_M_BW if (dist & 15) == _ops.DIST_BW else _ops.MAX_M
+        if a3.dtype == torch.float32 and b3.dtype == torch.float32 and a3.shape[-1] <= max_m:
             D = _ops.PairDistance.apply(a3.to(dev), None if same else b3.to(dev), dist, same)
         else:
             D = _pairwise_composed(a3.to(dev), b3.to(dev), dist)
@@ -95,6 +110,44 @@ def log_euclidean_sq(A, B):
 def log_euclidean(A, B):
     """Log-Euclidean distance, sqrt(d^2 + 1e-6) (reference distances.py:119-138)."""
     return _pairwise(A, B, _ops.DIST_LE)
+
+
+def bures_wasserstein_sq(A, B):
+    """Squared Bures-Wasserstein distance between SPD matrices, shape (n_batch_A, n_batch_B), squeezed
+    like `affine_invariant_sq`: tr A + tr B - 2 tr((B^1/2 A B^1/2)^1/2), clamped at 0.
+
+    Extension, not reference API (the reference's tutorial writes it as a custom `distance_fun`).
+    float32 matrices up to 34 x 34 run in the native pair kernel with an analytic backward; float64
+    and larger matrices take a composition of device-side library calls in the input dtype."""
+    return _pairwise(A, B, _ops.DIST_BW | _ops.SQUARED)
+
+
+def bures_wasserstein(A, B):
+    """Bures-Wasserstein distance, sqrt(d^2 + 1e-6) (extension, not reference API; see
+    `bures_wasserstein_sq`)."""
+    return _pairwise(A, B, _ops.DIST_BW)
+
+
+def _wasserstein_sq(statistics_A, statistics_B):
+    mu_a, mu_b = _unsq_mean(statistics_A["means"]), _unsq_mean(statistics_B["means"])
+    cov_a = statistics_A["covariances"]
+    cov_b = cov_a if statistics_B is statistics_A else statistics_B["covariances"]
+    bw = bures_wasserstein_sq(cov_a, cov_b)
+    diff = mu_a[:, None] - mu_b.to(mu_a.device)[None]
+    return torch.squeeze((diff * diff).sum(dim=-1)).to(bw.device) + bw
+
+
+def wasserstein_sq(statistics_A, statistics_B):
+    """Squared 2-Wasserstein distance between Gaussians given as dicts with "means" (n, k) and
+    "covariances" (n, k, k): |mu_A - mu_B|^2 + `bures_wasserstein_sq` of the covariances, shape
+    (n_A, n_B), squeezed. Extension, not reference API."""
+    return _wasserstein_sq(statistics_A, statistics_B)
+
+
+def wasserstein(statistics_A, statistics_B):
+    """2-Wasserstein distance between Gaussians, sqrt(max(d^2, 0) + 1e-6) (extension, not reference
+    API; see `wasserstein_sq`)."""
+    return torch.sqrt(_wasserstein_sq(statistics_A, statistics_B).clamp_min(0) + EPSILON)
 
 
 def _embed_gaussian(statistics):

@@ -37,11 +37,15 @@ _TENSOR_DISTANCES = {
     distances.affine_invariant_sq: _ops.DIST_AI | _ops.SQUARED,
     distances.log_euclidean: _ops.DIST_LE,
     distances.log_euclidean_sq: _ops.DIST_LE | _ops.SQUARED,
+    distances.bures_wasserstein: _ops.DIST_BW,
+    distances.bures_wasserstein_sq: _ops.DIST_BW | _ops.SQUARED,
 }
 # full models: dicts {"means", "covariances"} in
 _DICT_DISTANCES = {
     distances.fisher_rao_lower_bound: _ops.DIST_FR,
     distances.fisher_rao_lower_bound_sq: _ops.DIST_FR | _ops.SQUARED,
+    distances.wasserstein: _ops.DIST_W2,
+    distances.wasserstein_sq: _ops.DIST_W2 | _ops.SQUARED,
 }
 
 
