@@ -60,6 +60,17 @@ typedef void* sqfa_stream_t; /* cudaStream_t */
  * (sqfa_fused_loss, sqfa_fused_loss_sharded, sqfa_closure_eval; M required, m = n_filters): sqfa_class_factor
  * and sqfa_pair_distances take no means and reject it. */
 #define SQFA_DIST_WASSERSTEIN_GAUSSIAN 4
+/* Distances between Gaussians under the mean covariance M = (Sigma_i + Sigma_j) / 2 of the pair, d = mu_i - mu_j,
+ * x = d^T M^-1 d (distances.py:240-393). Closures only (sqfa_fused_loss, sqfa_fused_loss_sharded,
+ * sqfa_closure_eval; M required, n_filters <= 32); the per-matrix entry points reject them, and
+ * sqfa_gauss_pair_distances evaluates these distances pair by pair.
+ *   SQFA_DIST_MAHALANOBIS    sqrt(x + 1e-6), or x with SQFA_DIST_SQUARED
+ *   SQFA_DIST_BHATTACHARYYA  B = x / 8 + (logdet M - (logdet Sigma_i + logdet Sigma_j) / 2) / 2
+ *   SQFA_DIST_HELLINGER      sqrt(1 - exp(-B) + 1e-6), no clamp
+ * SQFA_DIST_SQUARED with Bhattacharyya or Hellinger is rejected. */
+#define SQFA_DIST_MAHALANOBIS 5
+#define SQFA_DIST_BHATTACHARYYA 6
+#define SQFA_DIST_HELLINGER 7
 /* add SQFA_DIST_SQUARED to get the squared variants (no sqrt, no epsilon) */
 #define SQFA_DIST_SQUARED 16
 

@@ -16,6 +16,9 @@ DIST_FR = 1  # SQFA_DIST_FISHER_RAO_LB
 DIST_LE = 2  # SQFA_DIST_LOG_EUCLIDEAN
 DIST_BW = 3  # SQFA_DIST_BURES_WASSERSTEIN
 DIST_W2 = 4  # SQFA_DIST_WASSERSTEIN_GAUSSIAN
+DIST_MAHA = 5  # SQFA_DIST_MAHALANOBIS (closures only)
+DIST_BHATT = 6  # SQFA_DIST_BHATTACHARYYA (closures only)
+DIST_HELL = 7  # SQFA_DIST_HELLINGER (closures only)
 SQUARED = 16  # SQFA_DIST_SQUARED
 MAX_M = 64
 MAX_M_BW = 34  # Bures-Wasserstein: column-pair kernel only

@@ -298,15 +298,26 @@ int sqfa_transform_h(const void* X, int64_t ldx, int32_t elem, const float* F, i
 
 static int dist_ok(int32_t dist) {
   const int b = dist & 15;
+  if ((dist & SQFA_DIST_SQUARED) && (b == SQFA_DIST_BHATTACHARYYA || b == SQFA_DIST_HELLINGER))
+    return 0;  // the reference has no squared form of these
   return (dist & ~(15 | SQFA_DIST_SQUARED)) == 0 &&
          (b == SQFA_DIST_AFFINE_INVARIANT || b == SQFA_DIST_FISHER_RAO_LB || b == SQFA_DIST_LOG_EUCLIDEAN ||
-          b == SQFA_DIST_BURES_WASSERSTEIN || b == SQFA_DIST_WASSERSTEIN_GAUSSIAN);
+          b == SQFA_DIST_BURES_WASSERSTEIN || b == SQFA_DIST_WASSERSTEIN_GAUSSIAN || sqfa::is_gauss_closure(dist));
 }
 
 // distances whose closure reads the class means
 static int dist_uses_means(int32_t dist) {
   const int b = dist & 15;
-  return b == SQFA_DIST_FISHER_RAO_LB || b == SQFA_DIST_WASSERSTEIN_GAUSSIAN;
+  return b == SQFA_DIST_FISHER_RAO_LB || b == SQFA_DIST_WASSERSTEIN_GAUSSIAN || sqfa::is_gauss_closure(dist);
+}
+
+// The mean-covariance codes exist for closures only: the per-matrix entry points have no means and no
+// pair-mean covariance. Returns 0 or the fail_arg code.
+static int check_not_gauss_closure(const char* fn, int32_t dist) {
+  if (sqfa::is_gauss_closure(dist))
+    return fail_arg(fn, "SQFA_DIST_MAHALANOBIS / BHATTACHARYYA / HELLINGER are closure codes: evaluate these "
+                        "distances with sqfa_gauss_pair_distances");
+  return 0;
 }
 
 // Bures-Wasserstein runs in the column-pair kernel only (m <= 34); the Gaussian form needs means, which the
@@ -326,6 +337,7 @@ int sqfa_embed_fwd(const float* Psi, const float* Mu, float noise, int32_t n_cla
   const int fr = (dist & 15) == SQFA_DIST_FISHER_RAO_LB;
   if (!dist_ok(dist) || Psi == nullptr || E == nullptr || n_classes < 0 || n_filters <= 0 || (fr && Mu == nullptr))
     return fail_arg(__func__, "bad argument");
+  if (const int rc = check_not_gauss_closure(__func__, dist)) return rc;
   return wrap(__func__, sqfa::launch_embed_fwd(Psi, Mu, noise, n_classes, n_filters, fr, E, S(stream)));
 }
 
@@ -335,6 +347,7 @@ int sqfa_embed_bwd(const float* gE, const float* Mu, int32_t n_classes, int32_t 
   if (!dist_ok(dist) || gE == nullptr || gPsi == nullptr || n_classes < 0 || n_filters <= 0 ||
       (fr && (Mu == nullptr || gMu == nullptr)))
     return fail_arg(__func__, "bad argument");
+  if (const int rc = check_not_gauss_closure(__func__, dist)) return rc;
   return wrap(__func__, sqfa::launch_embed_bwd(gE, Mu, n_classes, n_filters, fr, gPsi, gMu, S(stream)));
 }
 
@@ -344,6 +357,7 @@ int sqfa_class_factor(const float* E, int32_t n_classes, int32_t m, int32_t dist
                       sqfa_stream_t stream) {
   if (!dist_ok(dist) || E == nullptr || W == nullptr || flag == nullptr || n_classes < 0 || m <= 0)
     return fail_arg(__func__, "bad argument");
+  if (const int rc = check_not_gauss_closure(__func__, dist)) return rc;
   if (m > SQFA_MAX_M) return fail_arg(__func__, "m exceeds SQFA_MAX_M", SQFA_E_UNSUPPORTED);
   if (const int rc = check_bw_matrices(__func__, dist, m)) return rc;
   return wrap(__func__, sqfa::launch_class_factor(E, n_classes, m, dist, W, flag, S(stream)));
@@ -351,7 +365,7 @@ int sqfa_class_factor(const float* E, int32_t n_classes, int32_t m, int32_t dist
 
 size_t sqfa_pair_distances_workspace_bytes(int32_t n_a, int32_t n_b, int32_t m, int32_t dist, int32_t triangular,
                                            int64_t pair_begin, int64_t pair_end) {
-  if (n_a <= 0 || n_b <= 0 || m <= 0 || !dist_ok(dist)) return 256;
+  if (n_a <= 0 || n_b <= 0 || m <= 0 || !dist_ok(dist) || sqfa::is_gauss_closure(dist)) return 256;
   return sqfa::pair_workspace(n_a, n_b, m, dist, triangular ? 1 : 0, pair_begin, pair_end).total_floats *
              sizeof(float) + 256;
 }
@@ -364,6 +378,7 @@ int sqfa_pair_distances(const float* Wa, const float* Wb, int32_t n_a, int32_t n
       (triangular && (n_a != n_b || Wa != Wb)) || ((gEa == nullptr) != (gEb == nullptr)) ||
       (eig_out != nullptr && (triangular || (dist & 15) == SQFA_DIST_LOG_EUCLIDEAN)))
     return fail_arg(__func__, "bad argument");
+  if (const int rc = check_not_gauss_closure(__func__, dist)) return rc;
   if (const int rc = check_bw_matrices(__func__, dist, m)) return rc;
   if (eig_out != nullptr && (dist & 15) == SQFA_DIST_BURES_WASSERSTEIN)
     return fail_arg(__func__, "eig_out is not defined for Bures-Wasserstein");
@@ -383,6 +398,7 @@ int sqfa_class_factor_bwd(const float* W, const float* gLog, int32_t n_classes, 
                           float* gE, sqfa_stream_t stream) {
   if (!dist_ok(dist) || W == nullptr || gLog == nullptr || gE == nullptr || n_classes < 0 || m <= 0)
     return fail_arg(__func__, "bad argument");
+  if (const int rc = check_not_gauss_closure(__func__, dist)) return rc;
   if (m > SQFA_MAX_M) return fail_arg(__func__, "m exceeds SQFA_MAX_M", SQFA_E_UNSUPPORTED);
   return wrap(__func__, sqfa::launch_class_factor_bwd(W, gLog, n_classes, m, dist, gE, S(stream)));
 }

@@ -15,6 +15,8 @@
 //   closure_finish          dLoss/dF, constraint adjoint -> grad, max |grad|
 // Log-Euclidean adds le_grad + le_factor_bwd + embed_bwd between the pair kernel and project_bwd; the
 // Gaussian Wasserstein distance projects the means too (no embedding) and adds le_grad for their gradient.
+// The mean-covariance distances (Mahalanobis, Bhattacharyya, Hellinger) project the means and replace
+// class_prepare / pair kernel / pair_reduce with the class, pair and reduce stages of gauss.cu.
 #include <cstdint>
 #include <cuda_runtime.h>
 
@@ -28,13 +30,16 @@ namespace {
 inline size_t al(size_t n) { return (n + 63) & ~size_t(63); }  // floats, 256-byte granules
 
 struct ClosureLayout {
-  size_t F, inv_norm, T, Mu, E, W, gE, gLog, gPsi, gMu, red_out, flag, proj, psipart, mupart, pair, total;
+  size_t F, inv_norm, T, Mu, E, W, logdet, sinv, gE, gLog, gPsi, gMu, red_out, flag, proj, psipart, mupart, pair,
+      total;
 };
 
 ClosureLayout closure_layout(int C, int D, int k, int dist, int64_t pair_begin, int64_t pair_end) {
   const int base = dist & 15;
   const int m = (base == SQFA_DIST_FISHER_RAO_LB) ? k + 1 : k;
   const bool le = base == SQFA_DIST_LOG_EUCLIDEAN;
+  const bool gauss = is_gauss_closure(dist);  // E holds Psi_c; no factorisation W
+  const bool ld = gauss_closure_needs_logdet(dist);
   ClosureLayout L;
   size_t o = 0;
   L.F = o;        o += al((size_t)k * D);
@@ -42,7 +47,9 @@ ClosureLayout closure_layout(int C, int D, int k, int dist, int64_t pair_begin, 
   L.T = o;        o += al((size_t)C * k * D);
   L.Mu = o;       o += al((size_t)C * k);
   L.E = o;        o += al((size_t)C * m * m);
-  L.W = o;        o += al((size_t)C * class_factor_floats(m, dist));
+  L.W = o;        o += gauss ? 0 : al((size_t)C * class_factor_floats(m, dist));
+  L.logdet = o;   o += ld ? al(C) : 0;
+  L.sinv = o;     o += ld ? al((size_t)C * k * k) : 0;
   L.gE = o;       o += le ? al((size_t)C * m * m) : 0;
   L.gLog = o;     o += le ? al((size_t)C * m * m) : 0;
   L.gPsi = o;     o += al((size_t)C * k * k);
@@ -52,7 +59,8 @@ ClosureLayout closure_layout(int C, int D, int k, int dist, int64_t pair_begin, 
   L.proj = o;     o += al(project_workspace_bytes(C, D, k) / sizeof(float) + 1);
   L.psipart = o;  o += project_psipart_floats(C, D, k);
   L.mupart = o;   o += project_mupart_floats(C, D, k);
-  L.pair = o;     o += al(pair_workspace(C, C, m, dist, 1, pair_begin, pair_end).total_floats);
+  L.pair = o;     o += al(gauss ? gauss_closure_workspace_floats(C, k, pair_begin, pair_end)
+                            : pair_workspace(C, C, m, dist, 1, pair_begin, pair_end).total_floats);
   L.total = o;
   return L;
 }
@@ -72,7 +80,8 @@ cudaError_t launch_fused_loss(const float* S, const float* M, const float* filte
   const int base = dist & 15;
   const bool fr = base == SQFA_DIST_FISHER_RAO_LB;
   const bool le = base == SQFA_DIST_LOG_EUCLIDEAN;
-  const bool means = fr || base == SQFA_DIST_WASSERSTEIN_GAUSSIAN;  // this distance uses the class means
+  const bool gauss = is_gauss_closure(dist);
+  const bool means = fr || base == SQFA_DIST_WASSERSTEIN_GAUSSIAN || gauss;  // this distance uses the class means
   const int m = fr ? k + 1 : k;
   const ClosureLayout L = closure_layout(C, D, k, dist, pair_begin, pair_end);
   float* Fbuf = ws + L.F;
@@ -103,12 +112,21 @@ cudaError_t launch_fused_loss(const float* S, const float* M, const float* filte
   }
   if ((e = launch_project_partials(S, Mfr, F, C, D, k, T, proj, PsiPart, means ? MuPart : nullptr, st)) != cudaSuccess)
     return e;
-  if ((e = launch_class_prepare(PsiPart, means ? MuPart : nullptr, project_nchunk(D), noise, C, k, dist, Mu, E, W, flag,
-                                st)) != cudaSuccess)
-    return e;
-  if ((e = launch_pair_closure(W, C, m, dist, pair_begin, pair_end, weight, Mu, k, out, gPsi, gMu, gLog, pairws, st)) !=
-      cudaSuccess)
-    return e;
+  if (gauss) {
+    if ((e = launch_gauss_closure_class(PsiPart, MuPart, project_nchunk(D), noise, C, k, dist, E, Mu, ws + L.logdet,
+                                        ws + L.sinv, flag, st)) != cudaSuccess)
+      return e;
+    if ((e = launch_gauss_closure_pairs(E, Mu, ws + L.logdet, ws + L.sinv, C, k, dist, pair_begin, pair_end, weight, out,
+                                        gPsi, gMu, pairws, st)) != cudaSuccess)
+      return e;
+  } else {
+    if ((e = launch_class_prepare(PsiPart, means ? MuPart : nullptr, project_nchunk(D), noise, C, k, dist, Mu, E, W,
+                                  flag, st)) != cudaSuccess)
+      return e;
+    if ((e = launch_pair_closure(W, C, m, dist, pair_begin, pair_end, weight, Mu, k, out, gPsi, gMu, gLog, pairws,
+                                 st)) != cudaSuccess)
+      return e;
+  }
   if (le) {
     if ((e = cudaMemsetAsync(gE, 0, (size_t)C * m * m * sizeof(float), st)) != cudaSuccess) return e;
     if ((e = launch_class_factor_bwd(W, gLog, C, m, dist, gE, st)) != cudaSuccess) return e;
@@ -146,7 +164,8 @@ cudaError_t launch_fused_loss_sharded(int phase, const float* S, const float* M,
                                       float* dF, float* ws, cudaStream_t st) {
   const int base = dist & 15;
   const bool fr = base == SQFA_DIST_FISHER_RAO_LB;
-  const bool means = fr || base == SQFA_DIST_WASSERSTEIN_GAUSSIAN;
+  const bool gauss = is_gauss_closure(dist);
+  const bool means = fr || base == SQFA_DIST_WASSERSTEIN_GAUSSIAN || gauss;
   if (base == SQFA_DIST_LOG_EUCLIDEAN) return cudaErrorNotSupported;
   const int m = fr ? k + 1 : k;
   const ClosureLayout L = closure_layout(C, D, k, dist, pair_begin, pair_end);
@@ -171,6 +190,13 @@ cudaError_t launch_fused_loss_sharded(int phase, const float* S, const float* M,
   if (phase == 1) {
     const int64_t P = (int64_t)C * (C - 1) / 2;
     const float weight = -1.0f / (float)(P > 0 ? P : 1);
+    if (gauss) {
+      if ((e = launch_gauss_closure_class(PsiPart, MuPart, nchunk, noise, C, k, dist, ws + L.E, Mu, ws + L.logdet,
+                                          ws + L.sinv, reinterpret_cast<int32_t*>(ws + L.flag), st)) != cudaSuccess)
+        return e;
+      return launch_gauss_closure_pairs(ws + L.E, Mu, ws + L.logdet, ws + L.sinv, C, k, dist, pair_begin, pair_end,
+                                        weight, ws + L.red_out, gPsi, gMu, ws + L.pair, st);
+    }
     if ((e = launch_class_prepare(PsiPart, means ? MuPart : nullptr, nchunk, noise, C, k, dist, Mu, ws + L.E, ws + L.W,
                                   reinterpret_cast<int32_t*>(ws + L.flag), st)) != cudaSuccess)
       return e;

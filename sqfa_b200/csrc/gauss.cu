@@ -9,11 +9,14 @@
 //   d maha / d mu_a = 2 u,  d maha / d mu_b = -2 u,  d maha / d Sigma_a = d maha / d Sigma_b = -u u^T / 2
 //   d logdet M / d Sigma_a = M^-1 / 2,               d logdet Sigma_a / d Sigma_a = Sigma_a^-1
 // Per-pair gradient partials are stored and summed per class in a fixed order (no float atomics).
+// The second half of this file is the fitting closure of these distances (SQFA_DIST_MAHALANOBIS / BHATTACHARYYA /
+// HELLINGER): strict lower triangle only, the scalar map inside, tile partials instead of per-pair ones.
 #include <cstdint>
 #include <cuda_runtime.h>
 
 #include "../../include/sqfa_b200.h"
 #include "sqfa_internal.h"
+#include "pair_tiles.cuh"
 
 namespace sqfa {
 
@@ -59,6 +62,25 @@ __device__ void gp_tri_inverse(const float* L, float* Li, int k, int ld, int lan
   __syncwarp();
 }
 
+// logdet of the k x k SPD matrix staged in L (row stride ld) and, if Sinv_c != NULL, its inverse L^-T L^-1;
+// one warp, Li is scratch. A failed Cholesky sets *flag and leaves a NaN or -inf logdet.
+__device__ __forceinline__ void gp_logdet_inverse(float* L, float* Li, int k, int ld, int lane, float* logdet_c,
+                                                  float* Sinv_c, int32_t* flag) {
+  bool ok = true;
+  const float ldv = gp_cholesky(L, k, ld, lane, ok);
+  if (!ok && lane == 0) atomicOr(flag, 1);
+  if (lane == 0) *logdet_c = ldv;
+  if (Sinv_c != nullptr) {
+    gp_tri_inverse(L, Li, k, ld, lane);
+    for (int idx = lane; idx < k * k; idx += 32) {  // Sigma^-1 = L^-T L^-1
+      const int r = idx / k, s = idx % k;
+      float a = 0.f;
+      for (int q = (r > s ? r : s); q < k; ++q) a += Li[q * ld + r] * Li[q * ld + s];
+      Sinv_c[idx] = a;
+    }
+  }
+}
+
 // per class: logdet Sigma_c and (optionally) Sigma_c^-1; one warp per class
 __global__ void __launch_bounds__(GP_WARPS * 32)
 gauss_class_kernel(const float* __restrict__ Sigma, int C, int k, float* __restrict__ logdet,
@@ -72,19 +94,7 @@ gauss_class_kernel(const float* __restrict__ Sigma, int C, int k, float* __restr
   float* Li = L + k * ld;
   for (int idx = lane; idx < k * k; idx += 32) L[(idx / k) * ld + idx % k] = Sigma[(int64_t)c * k * k + idx];
   __syncwarp();
-  bool ok = true;
-  const float ldv = gp_cholesky(L, k, ld, lane, ok);
-  if (!ok && lane == 0) atomicOr(flag, 1);
-  if (lane == 0) logdet[c] = ldv;
-  if (Sinv != nullptr) {
-    gp_tri_inverse(L, Li, k, ld, lane);
-    for (int idx = lane; idx < k * k; idx += 32) {  // Sigma^-1 = L^-T L^-1
-      const int r = idx / k, s = idx % k;
-      float a = 0.f;
-      for (int q = (r > s ? r : s); q < k; ++q) a += Li[q * ld + r] * Li[q * ld + s];
-      Sinv[(int64_t)c * k * k + idx] = a;
-    }
-  }
+  gp_logdet_inverse(L, Li, k, ld, lane, logdet + c, Sinv != nullptr ? Sinv + (int64_t)c * k * k : nullptr, flag);
 }
 
 // One warp per pair (a, b), a in [a0, a1), b in [0, nB). mode 0: mahalanobis_sq, 1: bhattacharyya.
@@ -196,6 +206,244 @@ gauss_reduce_kernel(const float* __restrict__ rowpart, const float* __restrict__
   }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Fitting closure of the mean-covariance distances (SQFA_DIST_MAHALANOBIS / BHATTACHARYYA / HELLINGER):
+//   class stage   one warp per class: Psi_c = sum of the projection's chunk partials + noise I, mu'_c;
+//                 Bhattacharyya / Hellinger also logdet Psi_c and Psi_c^-1 (gp_cholesky, gp_tri_inverse)
+//   pair stage    a warp owns an R x R tile of the strict lower triangle; a group of G lanes (G = k rounded
+//                 up to a power of two, the matrix padded with the identity) owns one pair, so 32 / G pairs
+//                 run side by side. Lane r holds row r of M = (Psi_i + Psi_j) / 2 in registers; an in-place
+//                 Gauss-Jordan sweep with the pivot rows broadcast by shuffles leaves row r of M^-1. Its
+//                 pivots are the squared Cholesky pivots: their logs sum to logdet M, and a pivot that is not
+//                 positive and finite makes the distance NaN (as a failed Cholesky does). u = M^-1 d and
+//                 x = d^T u follow with G more shuffles.
+//   reduce        per class, the tile partials of its block row and block column in a fixed order
+// Per pair, with g = weight * d'(x or B) and (c_m, c_l) = (1, 0) for Mahalanobis, (1/8, 1/2) otherwise:
+//   dL/dPsi_i = dL/dPsi_j = g (-c_m / 2 u u^T + c_l / 2 M^-1),   dL/dmu'_i = -dL/dmu'_j = 2 c_m g u,
+// and the class term -1/4 Psi_c^-1 sum_o g(c, o) of the logdet Psi_c in B is added once per class.
+// ------------------------------------------------------------------------------------------------
+constexpr int GC_WARPS = 4;
+constexpr float GC_EPS = 1e-6f;  // distances.py:29 EPSILON
+
+// floats of one class slot of a tile partial: [dL/dPsi (k*k) | dL/dmu' (k) | sum of g]
+__host__ __device__ inline int gc_slot_floats(int k) { return k * k + k + 1; }
+
+struct GaussClosureArgs {
+  const float* Psi;     // [C][k][k]
+  const float* Mu;      // [C][k]
+  const float* logdet;  // [C] (Bhattacharyya / Hellinger)
+  int C, k, dist, Q;    // a tile row is processed as Q batches of 32 / G pairs
+  int64_t pair_begin, pair_end;
+  float weight;
+  PairTiles T;
+  float* rowpart;   // [ntiles][R][slot]
+  float* colpart;   // [ntiles][R][slot]
+  float* losspart;  // [ntiles][2] {sum of distances, non-finite count}
+};
+
+template <int G>
+__device__ __forceinline__ float gc_group_sum(float v) {
+#pragma unroll
+  for (int o = G / 2; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  return v;
+}
+
+__global__ void __launch_bounds__(GP_WARPS * 32)
+gauss_closure_class_kernel(const float* __restrict__ PsiPart, const float* __restrict__ MuPart, int nchunk, float noise,
+                           int C, int k, int want_logdet, float* __restrict__ Psi, float* __restrict__ Mu,
+                           float* __restrict__ logdet, float* __restrict__ Sinv, int32_t* __restrict__ flag) {
+  extern __shared__ float sm[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int c = blockIdx.x * GP_WARPS + warp;
+  if (c >= C) return;
+  const int ld = k + 1;
+  float* L = sm + (size_t)warp * 2 * k * ld;
+  float* Li = L + k * ld;
+  for (int r = lane; r < k; r += 32) {  // chunks added in order, as class_prepare does
+    float a = 0.f;
+    for (int ch = 0; ch < nchunk; ++ch) a += MuPart[((int64_t)c * nchunk + ch) * k + r];
+    Mu[(int64_t)c * k + r] = a;
+  }
+  for (int idx = lane; idx < k * k; idx += 32) {
+    float v = 0.f;
+    for (int ch = 0; ch < nchunk; ++ch) v += PsiPart[((int64_t)c * nchunk + ch) * k * k + idx];
+    if (idx / k == idx % k) v += noise;
+    Psi[(int64_t)c * k * k + idx] = v;
+    L[(idx / k) * ld + idx % k] = v;
+  }
+  if (!want_logdet) return;
+  __syncwarp();
+  gp_logdet_inverse(L, Li, k, ld, lane, logdet + c, Sinv + (int64_t)c * k * k, flag);
+}
+
+template <int G>
+__global__ void __launch_bounds__(GC_WARPS * 32)
+gauss_closure_pair_kernel(const GaussClosureArgs A) {
+  constexpr int NP = 32 / G;  // pairs side by side in a warp
+  extern __shared__ float gc_smem[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int64_t t = (int64_t)blockIdx.x * GC_WARPS + warp;
+  if (t >= A.T.ntiles) return;
+  const int grp = lane / G, r = lane % G;
+  const int k = A.k, Q = A.Q, R = A.T.R, base = A.dist & 15;
+  const int per = gc_slot_floats(k);
+  const bool bhat = base != SQFA_DIST_MAHALANOBIS;
+  const float cm = bhat ? 0.125f : 1.f, cl = bhat ? 0.5f : 0.f;
+  // column-slot accumulators [Q][G + 2][32]: every lane owns its own column, so no synchronisation
+  float* colacc = gc_smem + (size_t)warp * Q * (G + 2) * 32;
+  for (int e = 0; e < Q * (G + 2); ++e) colacc[e * 32 + lane] = 0.f;
+  int bi, bj;
+  decode_tile(A.T, t, bi, bj);
+  float dsum = 0.f, nbad = 0.f;
+  for (int ii = 0; ii < R; ++ii) {
+    const int i = bi * R + ii;
+    float racc[G + 2];
+#pragma unroll
+    for (int e = 0; e < G + 2; ++e) racc[e] = 0.f;
+    for (int q = 0; q < Q; ++q) {
+      const int j = bj * R + q * NP + grp;
+      const bool valid = pair_in_launch(i, j, A.C, A.C, 1, A.pair_begin, A.pair_end);
+      const bool live = valid && r < k;
+      float Mr[G];
+      const float* pi = A.Psi + ((int64_t)i * k + r) * k;
+      const float* pj = A.Psi + ((int64_t)j * k + r) * k;
+#pragma unroll
+      for (int l = 0; l < G; ++l) Mr[l] = (live && l < k) ? 0.5f * (pi[l] + pj[l]) : (l == r ? 1.f : 0.f);
+      const float dv = live ? A.Mu[(int64_t)i * k + r] - A.Mu[(int64_t)j * k + r] : 0.f;
+      // Gauss-Jordan: after step p the rows hold [M^-1 of the leading p x p block | eliminated rest]
+      float mypiv = 1.f;
+#pragma unroll
+      for (int p = 0; p < G; ++p) {
+        const float piv = __shfl_sync(0xffffffffu, Mr[p], p, G);
+        const float pinv = 1.f / piv;
+        const float f = Mr[p];
+        const bool prow = r == p;
+        if (prow) mypiv = piv;
+#pragma unroll
+        for (int l = 0; l < G; ++l) {
+          const float pl = __shfl_sync(0xffffffffu, Mr[l], p, G) * pinv;
+          if (l == p) Mr[l] = prow ? pinv : -f * pinv;
+          else Mr[l] = prow ? pl : fmaf(-f, pl, Mr[l]);
+        }
+      }
+      float u = 0.f;  // u_r = (M^-1 d)_r
+#pragma unroll
+      for (int l = 0; l < G; ++l) u = fmaf(Mr[l], __shfl_sync(0xffffffffu, dv, l, G), u);
+      const float x = gc_group_sum<G>(dv * u);
+      const bool pos = mypiv > 0.f && mypiv <= 3.402823466e38f;
+      const bool ok = gc_group_sum<G>(pos ? 0.f : 1.f) == 0.f;
+      float pre = x;
+      if (bhat) {
+        const float ldM = gc_group_sum<G>(logf(mypiv));  // padded rows: log 1 = 0
+        pre = valid ? 0.125f * x + 0.5f * (ldM - 0.5f * (A.logdet[i] + A.logdet[j])) : 0.f;
+      }
+      if (!ok) pre = __int_as_float(0x7fffffff);
+      float dval, dmap;  // distance and its derivative w.r.t. x (Mahalanobis) or B
+      if (base == SQFA_DIST_HELLINGER) {
+        const float e = expf(-pre);
+        dval = sqrtf(1.f - e + GC_EPS);
+        dmap = 0.5f * e / dval;
+      } else if (base == SQFA_DIST_MAHALANOBIS && !(A.dist & SQFA_DIST_SQUARED)) {
+        dval = sqrtf(pre + GC_EPS);
+        dmap = 0.5f / dval;
+      } else {
+        dval = pre;
+        dmap = 1.f;
+      }
+      const float g = valid ? A.weight * dmap : 0.f;
+      if (valid && r == 0) {
+        dsum += dval;
+        if (!isfinite(dval)) nbad += 1.f;
+      }
+      const float gu = g * u;
+      float* ca = colacc + q * (G + 2) * 32 + lane;
+#pragma unroll
+      for (int l = 0; l < G; ++l) {
+        const float ul = __shfl_sync(0xffffffffu, u, l, G);
+        const float v = fmaf(0.5f * cl * g, Mr[l], -0.5f * cm * gu * ul);
+        racc[l] += v;
+        ca[l * 32] += v;
+      }
+      racc[G] += 2.f * cm * gu;
+      ca[G * 32] -= 2.f * cm * gu;
+      racc[G + 1] += g;
+      ca[(G + 1) * 32] += g;
+    }
+    // row slot ii: sum over the NP pairs side by side (butterfly: every group ends with the same bits)
+#pragma unroll
+    for (int e = 0; e < G + 2; ++e)
+#pragma unroll
+      for (int o = G; o < 32; o <<= 1) racc[e] += __shfl_xor_sync(0xffffffffu, racc[e], o);
+    if (grp == 0 && r < k) {
+      float* rp = A.rowpart + (t * R + ii) * per;
+#pragma unroll
+      for (int l = 0; l < G; ++l)
+        if (l < k) rp[r * k + l] = racc[l];
+      rp[k * k + r] = racc[G];
+      if (r == 0) rp[k * k + k] = racc[G + 1];
+    }
+  }
+  if (r < k) {
+    for (int q = 0; q < Q; ++q) {
+      float* cp = A.colpart + (t * R + q * NP + grp) * per;
+      const float* ca = colacc + q * (G + 2) * 32 + lane;
+      for (int l = 0; l < k; ++l) cp[r * k + l] = ca[l * 32];
+      cp[k * k + r] = ca[G * 32];
+      if (r == 0) cp[k * k + k] = ca[(G + 1) * 32];
+    }
+  }
+  dsum = gp_warp_sum(dsum);
+  nbad = gp_warp_sum(nbad);
+  if (lane == 0) {
+    A.losspart[2 * t] = dsum;
+    A.losspart[2 * t + 1] = nbad;
+  }
+}
+
+// Per class c (blocks 0 .. C - 1): the slot partials of the tiles of its block row (ascending block column)
+// and block column (ascending block row) -> gPsi[c] (+ the logdet class term), gMu[c]. Block C: out =
+// {weight * sum d, #non-finite, 0} from the loss partials. Fixed order throughout.
+__global__ void __launch_bounds__(1024)
+gauss_closure_reduce_kernel(const PairTiles T, int C, int k, int dist, const float* __restrict__ rowpart,
+                            const float* __restrict__ colpart, const float* __restrict__ losspart,
+                            const float* __restrict__ Sinv, float weight, float* __restrict__ out,
+                            float* __restrict__ gPsi, float* __restrict__ gMu) {
+  extern __shared__ float sg[];  // the reduced slot of this class
+  const int c = blockIdx.x;
+  if (c == C) {
+    float sum, bad;
+    reduce_loss_partials(losspart, T.ntiles, sum, bad);
+    if (threadIdx.x == 0) {
+      out[0] = weight * sum;
+      out[1] = bad;
+      out[2] = 0.f;  // max |grad|, filled by closure_finish_kernel
+    }
+    return;
+  }
+  const int per = gc_slot_floats(k), R = T.R, slot = c % R, bc = c / R;
+  const int64_t pstride = (int64_t)R * per;
+  for (int e = threadIdx.x; e < per; e += blockDim.x) {
+    float a = 0.f, b = 0.f;
+    if (bc >= T.bi0 && bc <= T.bi1) {  // row side: tiles (bc, 0 .. bc)
+      const float* p = rowpart + ((int64_t)bc * (bc + 1) / 2 - T.tile0) * pstride + (int64_t)slot * per + e;
+#pragma unroll 4
+      for (int bj = 0; bj <= bc; ++bj) a += p[bj * pstride];
+    }
+    const int i0 = max(T.bi0, bc);  // column side: tiles (i0 .. bi1, bc)
+#pragma unroll 4
+    for (int bi = i0; bi <= T.bi1; ++bi)
+      b += colpart[((int64_t)bi * (bi + 1) / 2 + bc - T.tile0) * pstride + (int64_t)slot * per + e];
+    sg[e] = a + b;
+  }
+  __syncthreads();
+  const bool bhat = gauss_closure_needs_logdet(dist);
+  const float gsum = sg[k * k + k];
+  for (int e = threadIdx.x; e < k * k + k; e += blockDim.x) {
+    if (e < k * k) gPsi[(int64_t)c * k * k + e] = bhat ? sg[e] - 0.25f * gsum * Sinv[(int64_t)c * k * k + e] : sg[e];
+    else gMu[(int64_t)c * k + e - k * k] = sg[e];
+  }
+}
+
 }  // namespace
 
 size_t gauss_workspace_floats(int nA, int nB, int k, int want_grad) {
@@ -265,6 +513,99 @@ cudaError_t launch_gauss_pairs(const float* muA, const float* SigA, const float*
   if (flag_out != nullptr) {
     if ((e = cudaMemcpyAsync(flag_out, flag, sizeof(int32_t), cudaMemcpyDeviceToDevice, st)) != cudaSuccess) return e;
   }
+  return cudaGetLastError();
+}
+
+// ---- fitting closure of the mean-covariance distances ----
+// group width G and tile edge R = (32 / G) Q: Q grows with the pair count while tiles stay plentiful, up to
+// R = 16 / 8 / 4 at G <= 8 / 16 / 32, so that the partials (2 R (k^2 + k + 1) floats per tile of R^2 pairs) stay
+// below the affine-invariant closure's
+static int gc_group(int k) {
+  int G = 2;
+  while (G < k) G *= 2;
+  return G;
+}
+
+static int gc_batches(int G, int64_t npairs) {
+  const int np = 32 / G, qmax = G <= 2 ? 1 : (G == 4 ? 2 : 4);
+  int Q = 1;
+  while (Q < qmax && npairs / ((int64_t)(2 * Q * np) * (2 * Q * np)) >= 4096) Q *= 2;
+  return Q;
+}
+
+struct GcWorkspace {
+  size_t rowpart, colpart, losspart, total_floats;
+  PairTiles T;
+  int Q;
+};
+
+static GcWorkspace gc_workspace(int C, int k, int64_t pair_begin, int64_t pair_end) {
+  GcWorkspace w;
+  const int64_t npairs = pair_end > pair_begin ? pair_end - pair_begin : 0;
+  const int G = gc_group(k);
+  w.Q = gc_batches(G, npairs);
+  w.T = make_pair_tiles(C, C, 1, pair_begin, pair_end, (32 / G) * w.Q);
+  auto al = [](size_t n) { return (n + 63) & ~size_t(63); };
+  const size_t part = (size_t)w.T.ntiles * w.T.R * gc_slot_floats(k);
+  w.rowpart = 0;
+  w.colpart = al(part);
+  w.losspart = w.colpart + al(part);
+  w.total_floats = w.losspart + al((size_t)2 * w.T.ntiles) + 64;
+  return w;
+}
+
+size_t gauss_closure_workspace_floats(int C, int k, int64_t pair_begin, int64_t pair_end) {
+  return gc_workspace(C, k, pair_begin, pair_end).total_floats;
+}
+
+cudaError_t launch_gauss_closure_class(const float* PsiPart, const float* MuPart, int nchunk, float noise, int C, int k,
+                                       int dist, float* Psi, float* Mu, float* logdet, float* Sinv, int32_t* flag,
+                                       cudaStream_t st) {
+  cudaError_t e = cudaMemsetAsync(flag, 0, 2 * sizeof(int32_t), st);  // flag[1]: closure_finish's arrival ticket
+  if (e != cudaSuccess || C <= 0) return e;
+  const int smem = GP_WARPS * 2 * k * (k + 1) * (int)sizeof(float);
+  gauss_closure_class_kernel<<<(C + GP_WARPS - 1) / GP_WARPS, GP_WARPS * 32, smem, st>>>(
+      PsiPart, MuPart, nchunk, noise, C, k, gauss_closure_needs_logdet(dist) ? 1 : 0, Psi, Mu, logdet, Sinv, flag);
+  return cudaGetLastError();
+}
+
+template <int G>
+static cudaError_t launch_gc_pair(const GaussClosureArgs& A, cudaStream_t st) {
+  const int smem = GC_WARPS * A.Q * (G + 2) * 32 * (int)sizeof(float);
+  static int smem_set[kMaxDevices] = {0};
+  cudaError_t e = ensure_dynamic_smem(gauss_closure_pair_kernel<G>, smem, smem_set);
+  if (e != cudaSuccess) return e;
+  const unsigned blocks = (unsigned)((A.T.ntiles + GC_WARPS - 1) / GC_WARPS);
+  gauss_closure_pair_kernel<G><<<blocks, GC_WARPS * 32, smem, st>>>(A);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_gauss_closure_pairs(const float* Psi, const float* Mu, const float* logdet, const float* Sinv, int C,
+                                       int k, int dist, int64_t pair_begin, int64_t pair_end, float weight, float* out,
+                                       float* gPsi, float* gMu, float* ws, cudaStream_t st) {
+  const GcWorkspace W = gc_workspace(C, k, pair_begin, pair_end);
+  GaussClosureArgs A;
+  A.Psi = Psi; A.Mu = Mu; A.logdet = logdet;
+  A.C = C; A.k = k; A.dist = dist; A.Q = W.Q;
+  A.pair_begin = pair_begin; A.pair_end = pair_end; A.weight = weight; A.T = W.T;
+  A.rowpart = ws + W.rowpart; A.colpart = ws + W.colpart; A.losspart = ws + W.losspart;
+  cudaError_t e = cudaSuccess;
+  if (W.T.ntiles > 0) {
+    switch (gc_group(k)) {
+      case 2: e = launch_gc_pair<2>(A, st); break;
+      case 4: e = launch_gc_pair<4>(A, st); break;
+      case 8: e = launch_gc_pair<8>(A, st); break;
+      case 16: e = launch_gc_pair<16>(A, st); break;
+      case 32: e = launch_gc_pair<32>(A, st); break;
+      default: return cudaErrorNotSupported;
+    }
+    if (e != cudaSuccess) return e;
+  }
+  const int per = gc_slot_floats(k), passes = (per + 1023) / 1024;
+  int nt = (((per + passes - 1) / passes) + 31) & ~31;
+  if (nt < 128) nt = 128;
+  gauss_closure_reduce_kernel<<<C + 1, nt, per * sizeof(float), st>>>(W.T, C, k, dist, A.rowpart, A.colpart,
+                                                                     A.losspart, Sinv, weight, out, gPsi, gMu);
   return cudaGetLastError();
 }
 

@@ -32,6 +32,7 @@
 
 #include "../../include/sqfa_b200.h"
 #include "sqfa_internal.h"
+#include "pair_tiles.cuh"
 
 namespace sqfa {
 
@@ -186,29 +187,6 @@ __device__ float* warp_jacobi(float* cur, float* nxt, int m, int mp, int ld, int
     if (!__any_sync(0xffffffffu, rotated)) break;
   }
   return cur;
-}
-
-// local tile t of the launch -> block row / block column
-__device__ __forceinline__ void decode_tile(const PairTiles& T, int64_t t, int& bi, int& bj) {
-  const int64_t gt = T.tile0 + t;
-  if (T.tri) {
-    long long b = (long long)((sqrt(8.0 * (double)gt + 1.0) - 1.0) * 0.5);
-    while (b * (b + 1) / 2 > gt) --b;
-    while ((b + 1) * (b + 2) / 2 <= gt) ++b;
-    bi = (int)b;
-    bj = (int)(gt - b * (b + 1) / 2);
-  } else {
-    bi = (int)(gt / T.nbj);
-    bj = (int)(gt % T.nbj);
-  }
-}
-
-// pair (i, j) of a tile: is it part of this launch, and which linear pair index does it have
-__device__ __forceinline__ bool pair_in_launch(int i, int j, int nA, int nB, int tri, int64_t pair_begin,
-                                               int64_t pair_end) {
-  if (i >= nA || j >= nB || (tri && j >= i)) return false;
-  const int64_t p = tri ? (int64_t)i * (i - 1) / 2 + j : (int64_t)i * nB + j;
-  return p >= pair_begin && p < pair_end;
 }
 
 __device__ __forceinline__ float finish_distance(float d2, int dist, float* dd_dd2) {
@@ -1253,30 +1231,6 @@ le_grad_kernel(const PairTiles T, const float* __restrict__ Wa, const float* __r
       if (c < nB) gLb[(int64_t)c * ne + e] += gb;
     }
   }
-}
-
-// fixed-order sum of the per-tile {sum of distances, non-finite count}: every thread sums a strided
-// subset in ascending tile order, then a fixed tree over the block (any block size up to 1024)
-__device__ void reduce_loss_partials(const float* __restrict__ losspart, int64_t ntiles, float& sum, float& bad) {
-  __shared__ float red[2][1024];
-  const int nt = blockDim.x;
-  float a = 0.f, b = 0.f;
-  for (int64_t t = threadIdx.x; t < ntiles; t += nt) {
-    a += losspart[2 * t];
-    b += losspart[2 * t + 1];
-  }
-  red[0][threadIdx.x] = a;
-  red[1][threadIdx.x] = b;
-  __syncthreads();
-  for (int o = 512; o > 0; o >>= 1) {
-    if ((int)threadIdx.x < o && (int)threadIdx.x + o < nt) {
-      red[0][threadIdx.x] += red[0][threadIdx.x + o];
-      red[1][threadIdx.x] += red[1][threadIdx.x + o];
-    }
-    __syncthreads();
-  }
-  sum = red[0][0];
-  bad = red[1][0];
 }
 
 // dLoss/dE of class c = its row partials (tiles of block row c / R, ascending block column) + its

@@ -180,4 +180,14 @@ size_t gauss_workspace_floats(int nA, int nB, int k, int want_grad);
 cudaError_t launch_gauss_pairs(const float* muA, const float* SigA, const float* muB, const float* SigB, int nA,
                                int nB, int k, int mode, const float* gD, float* dist_out, float* gSigA, float* gMuA,
                                float* gSigB, float* gMuB, float* ws, int32_t* flag_out, cudaStream_t st);
+// closure codes SQFA_DIST_MAHALANOBIS / BHATTACHARYYA / HELLINGER
+__host__ __device__ inline bool is_gauss_closure(int dist) { return (dist & 15) >= 5 && (dist & 15) <= 7; }
+__host__ __device__ inline bool gauss_closure_needs_logdet(int dist) { return (dist & 15) == 6 || (dist & 15) == 7; }
+size_t gauss_closure_workspace_floats(int C, int k, int64_t pair_begin, int64_t pair_end);
+cudaError_t launch_gauss_closure_class(const float* PsiPart, const float* MuPart, int nchunk, float noise, int C, int k,
+                                       int dist, float* Psi, float* Mu, float* logdet, float* Sinv, int32_t* flag,
+                                       cudaStream_t st);
+cudaError_t launch_gauss_closure_pairs(const float* Psi, const float* Mu, const float* logdet, const float* Sinv, int C,
+                                       int k, int dist, int64_t pair_begin, int64_t pair_end, float weight, float* out,
+                                       float* gPsi, float* gMu, float* ws, cudaStream_t st);
 }  // namespace sqfa

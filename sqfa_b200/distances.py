@@ -7,7 +7,9 @@ warp-per-pair Jacobi kernels and are differentiable through analytic backward pa
 distances of the reference (Bhattacharyya, Mahalanobis, Hellinger, Fisher-Rao with shared
 covariance; alternative `distance_fun` plug-ins, SURVEY.md section 8(f) row 4) run in a warp-per-pair
 Cholesky kernel with an analytic backward. float64 inputs and matrices above 64 x 64 take the
-reference's own composition with device-side library calls, in the dtype of the inputs.
+reference's own composition with device-side library calls, in the dtype of the inputs. As `distance_fun`
+of `SQFA`, `mahalanobis`, `mahalanobis_sq`, `bhattacharyya` and `hellinger` also fit through the models'
+single-call native closure (up to 32 filters); `fisher_rao_same_cov` keeps the generic path.
 
 Extension (not reference API): the Bures-Wasserstein distance between SPD matrices and the
 2-Wasserstein distance between Gaussians run in the same Jacobi pair kernel (up to 34 x 34) and
@@ -207,6 +209,8 @@ def fisher_rao_lower_bound(statistics_A, statistics_B):
 # The reference's other distance_fun plug-ins (distances.py:240-432): distances between Gaussians under
 # the MEAN covariance of the pair. Native: one warp per pair (Cholesky of the mean covariance), analytic
 # backward; mahalanobis, hellinger and fisher_rao_same_cov are scalar maps of the two kernels' outputs.
+# In a fit, all but fisher_rao_same_cov run the closure of gauss.cu instead (strict lower triangle only, the
+# scalar map and its derivative inside the pair stage; DESIGN.md section 17).
 # ------------------------------------------------------------------------------------------------
 def _gauss_pairs(statistics_A, statistics_B, mode):
     """(n_a, n_b) matrix of mahalanobis_sq / bhattacharyya values (not squeezed)."""

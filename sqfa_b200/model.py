@@ -46,7 +46,14 @@ _DICT_DISTANCES = {
     distances.fisher_rao_lower_bound_sq: _ops.DIST_FR | _ops.SQUARED,
     distances.wasserstein: _ops.DIST_W2,
     distances.wasserstein_sq: _ops.DIST_W2 | _ops.SQUARED,
+    distances.mahalanobis: _ops.DIST_MAHA,
+    distances.mahalanobis_sq: _ops.DIST_MAHA | _ops.SQUARED,
+    distances.bhattacharyya: _ops.DIST_BHATT,
+    distances.hellinger: _ops.DIST_HELL,
 }
+# fisher_rao_same_cov stays on the generic path on purpose: with the reference's closure its gradient is NaN
+# (acosh' is infinite at the diagonal's x = 0, and 0 * inf = NaN), so those fits fail. A native closure
+# that only touches the pairs i > j would turn such a fit into a working one.
 
 
 _GRAPH_CLOSURE = os.environ.get("SQFA_GRAPH_CLOSURE", "1") != "0"
