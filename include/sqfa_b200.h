@@ -389,6 +389,20 @@ int sqfa_closure_eval(const float* S, const float* M, const float* raw_filters, 
                       int64_t pair_begin, int64_t pair_end, float* out, float* out_host, float* grad, void* ws,
                       size_t ws_bytes, sqfa_stream_t stream);
 
+/* sqfa_closure_eval in float64: S, M, raw_filters, out, out_host and grad are double. For
+ * SQFA_DIST_AFFINE_INVARIANT and SQFA_DIST_FISHER_RAO_LB (each optionally + SQFA_DIST_SQUARED) and
+ * n_filters <= 32; other codes and n_filters > 32 return SQFA_E_UNSUPPORTED (M is required for Fisher-Rao).
+ * `noise` points to ONE double in device memory (read by the kernels, so a captured graph picks up a new
+ * value). As in float32, out[0] over a sub-range [pair_begin, pair_end) is scaled by 1/P of ALL pairs, so
+ * the losses and gradients of disjoint ranges add up. Deterministic: no floating-point atomics. The
+ * workspace query returns 0 for arguments the evaluation rejects. */
+size_t sqfa_fused_loss_workspace_bytes_f64(int32_t n_classes, int32_t n_dim, int32_t n_filters, int32_t dist,
+                                           int64_t pair_begin, int64_t pair_end);
+int sqfa_closure_eval_f64(const double* S, const double* M, const double* raw_filters, int32_t n_classes,
+                          int32_t n_dim, int32_t n_filters, const double* noise, int32_t dist, int32_t constraint,
+                          int32_t n_fixed, int64_t pair_begin, int64_t pair_end, double* out, double* out_host,
+                          double* grad, void* ws, size_t ws_bytes, sqfa_stream_t stream);
+
 /* Plug-in distances between Gaussians that use the mean covariance of the pair (distances.py:240-432),
  * one warp per pair (Cholesky of (Sigma_a + Sigma_b) / 2 in shared memory), all n_a * n_b pairs:
  *   SQFA_GAUSS_MAHALANOBIS_SQ  d^T M^-1 d                                             (:283-330)

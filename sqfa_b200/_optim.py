@@ -115,6 +115,9 @@ def fitting_loop(
             if bad != 0 or loss_value != loss_value:
                 raise ValueError(_NAN_MSG if loss_value != loss_value else _INF_MSG)
             optimizer._last_grad_absmax = grad_absmax
+            if getattr(direct, "dtype", None) == torch.float64:
+                # a float64 fit keeps its loss in float64, as on the composed path
+                return torch.tensor(loss_value, dtype=torch.float64)
             return torch.tensor(loss_value)
         optimizer.zero_grad()
         if fused is not None:

@@ -1,6 +1,6 @@
 // Device helpers of the R x R pair tiles (PairTiles, sqfa_internal.h) shared by the pair kernels of
-// pairs.cu and the mean-covariance closure of gauss.cu: tile decoding, the pair mask of a launch and the
-// fixed-order reduction of the per-tile loss partials.
+// pairs.cu, the mean-covariance closure of gauss.cu and the float64 closure of closure64.cu: tile
+// decoding, the pair mask of a launch and the fixed-order reduction of the per-tile loss partials.
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
@@ -35,10 +35,11 @@ __device__ __forceinline__ bool pair_in_launch(int i, int j, int nA, int nB, int
 
 // fixed-order sum of the per-tile {sum of distances, non-finite count}: every thread sums a strided
 // subset in ascending tile order, then a fixed tree over the block (any block size up to 1024)
-__device__ void reduce_loss_partials(const float* __restrict__ losspart, int64_t ntiles, float& sum, float& bad) {
-  __shared__ float red[2][1024];
+template <typename T>
+__device__ void reduce_loss_partials(const T* __restrict__ losspart, int64_t ntiles, T& sum, T& bad) {
+  __shared__ T red[2][1024];
   const int nt = blockDim.x;
-  float a = 0.f, b = 0.f;
+  T a = T(0), b = T(0);
   for (int64_t t = threadIdx.x; t < ntiles; t += nt) {
     a += losspart[2 * t];
     b += losspart[2 * t + 1];

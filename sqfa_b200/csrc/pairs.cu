@@ -33,6 +33,7 @@
 #include "../../include/sqfa_b200.h"
 #include "sqfa_internal.h"
 #include "pair_tiles.cuh"
+#include "spd_factor.cuh"
 
 namespace sqfa {
 
@@ -109,42 +110,6 @@ __device__ __forceinline__ int rr_partner(int p, int r, int mp) {
   if (q < 0) q += n1;
   else if (q >= n1) q -= n1;
   return q == p ? n1 : q;
-}
-
-// Cholesky E = L L^T and L^-1 of an m x m SPD matrix, one warp. La / Li: shared, row stride ld.
-// Returns false (all lanes) if a pivot is not positive / finite.
-__device__ bool warp_cholesky_inverse(const float* __restrict__ E, float* La, float* Li, int m, int ld, int lane) {
-  for (int idx = lane; idx < m * m; idx += 32) {
-    const int r = idx / m, c = idx % m;
-    La[r * ld + c] = E[idx];
-    Li[r * ld + c] = 0.f;
-  }
-  __syncwarp();
-  bool ok = true;
-  for (int j = 0; j < m; ++j) {
-    float d = La[j * ld + j];
-    for (int k = 0; k < j; ++k) d -= La[j * ld + k] * La[j * ld + k];
-    if (!(d > 0.f) || !isfinite(d)) ok = false;
-    const float ljj = sqrtf(d);
-    __syncwarp();
-    for (int i = j + 1 + lane; i < m; i += 32) {
-      float v = La[i * ld + j];
-      for (int k = 0; k < j; ++k) v -= La[i * ld + k] * La[j * ld + k];
-      La[i * ld + j] = v / ljj;
-    }
-    if (lane == 0) La[j * ld + j] = ljj;
-    __syncwarp();
-  }
-  // inverse by forward substitution, one column per lane
-  for (int c = lane; c < m; c += 32) {
-    for (int i = 0; i < m; ++i) {
-      float s = (i == c) ? 1.f : 0.f;
-      for (int k = 0; k < i; ++k) s -= La[i * ld + k] * Li[k * ld + c];
-      Li[i * ld + c] = (i < c) ? 0.f : s / La[i * ld + i];
-    }
-  }
-  __syncwarp();
-  return ok;
 }
 
 // One-sided Jacobi on the columns of the m x mp matrix in `cur` (row stride ld, column q of slot

@@ -149,6 +149,12 @@ cudaError_t launch_fused_loss_sharded(int phase, const float* S, const float* M,
 cudaError_t launch_fused_loss(const float* S, const float* M, const float* filters, int C, int D, int k, float noise,
                               int dist, int constraint, int n_fixed, int64_t pair_begin, int64_t pair_end, float* out,
                               float* out_host, float* grad, float* ws, cudaStream_t st);
+// ---- closure64.cu (float64 closure: affine-invariant / Fisher-Rao lower bound, k <= 32) ----
+size_t fused_loss_workspace_bytes_f64(int C, int D, int k, int dist, int64_t pair_begin, int64_t pair_end);
+cudaError_t launch_closure_f64(const double* S, const double* M, const double* raw_filters, int C, int D, int k,
+                               const double* noise, int dist, int constraint, int n_fixed, int64_t pair_begin,
+                               int64_t pair_end, double* out, double* out_host, double* grad, double* ws,
+                               cudaStream_t st);
 }  // namespace sqfa
 
 

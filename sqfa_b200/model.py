@@ -116,8 +116,8 @@ def _check_statistics(data_statistics, needs_dict=False):
 def _statistics_to(data_statistics, dev, dtype=torch.float32):
     """The statistics on the compute device in the model's dtype (no copy if already so). float32 models
     run the native closure; a model converted with `.double()` -- the reference's remedy for NaN / inf
-    distances, _optim.py:28-30 -- keeps float64 statistics and evaluates the closure with float64
-    device-side library calls (SURVEY.md 8(f) row 3)."""
+    distances, _optim.py:28-30 -- keeps float64 statistics; its affine-invariant / Fisher-Rao closure is native
+    (closure64.cu), every other float64 closure uses float64 device-side library calls (SURVEY.md 8(f) row 3)."""
 
     def put(t):
         return t.detach().to(device=dev, dtype=dtype).contiguous()
@@ -309,21 +309,27 @@ class SecondMomentsSQFA(nn.Module):
         vector [loss, #non-finite distances, max|grad|]. Available when every constraint on the
         filters has a closed-form adjoint (Sphere: (I - f f^T)/|w| per row; Identity; FixedFilters:
         zero rows) -- torch's `orthogonal` keeps the autograd path. Saves the ~15 micro-kernels and
-        the autograd engine round trip per evaluation that dominate small-C fits."""
+        the autograd engine round trip per evaluation that dominate small-C fits. A float64 parameter with
+        float64 statistics takes the float64 closure for the affine-invariant / Fisher-Rao distances on one
+        device, and None otherwise."""
         if not parametrize_is_parametrized(self, "filters"):
             return None
         chain = list(self.parametrizations.filters)
         if any(type(m) not in (Sphere, Identity, FixedFilters) for m in chain):
             return None
         p = self.parametrizations.filters.original
-        if not (p.is_cuda and p.dtype == torch.float32) or p.shape[0] > _ops.MAX_FILTERS:
+        if not (p.is_cuda and p.dtype in (torch.float32, torch.float64)) or p.shape[0] > _ops.MAX_FILTERS:
             return None
         plan = self._fused_inputs(data_statistics)
         noise = self._noise_scalar()
         if plan is None or noise is None:
             return None
         S, M, dist = plan
-        if S.dtype != torch.float32 or (M is not None and M.dtype != torch.float32):
+        if S.dtype != p.dtype or (M is not None and M.dtype != p.dtype):
+            return None
+        f64 = p.dtype == torch.float64
+        # float64 (a `.double()` model): the native closure covers affine-invariant / Fisher-Rao on one device
+        if f64 and ((dist & 15) not in (_ops.DIST_AI, _ops.DIST_FR) or self._process_group is not None):
             return None
         group = self._process_group
         k, D = p.shape
@@ -368,15 +374,21 @@ class SecondMomentsSQFA(nn.Module):
         # single device: ONE native call per evaluation (constraint and its adjoint included), all
         # buffers static, captured in a CUDA graph after the first evaluations
         P = C * (C - 1) // 2
-        ws = torch.empty(max(int(lib.sqfa_fused_loss_workspace_bytes(C, D, k, dist, 0, P)), 1), dtype=torch.uint8,
-                         device=S.device)
-        out = torch.zeros(_ops.N_OUT, dtype=torch.float32, device=S.device)
-        out_host = torch.zeros(_ops.N_OUT, dtype=torch.float32).pin_memory()  # mirror, filled by every evaluation
-        grad = torch.zeros(k, D, dtype=torch.float32, device=S.device)
+        ws_bytes = (lib.sqfa_fused_loss_workspace_bytes_f64 if f64 else lib.sqfa_fused_loss_workspace_bytes)(
+            C, D, k, dist, 0, P)
+        ws = torch.empty(max(int(ws_bytes), 1), dtype=torch.uint8, device=S.device)
+        out = torch.zeros(_ops.N_OUT, dtype=p.dtype, device=S.device)
+        out_host = torch.zeros(_ops.N_OUT, dtype=p.dtype).pin_memory()  # mirror, filled by every evaluation
+        grad = torch.zeros(k, D, dtype=p.dtype, device=S.device)
         state = {"calls": 0, "graph": None, "param_ptr": None}
+        if f64:
+            noise_dev = torch.full((1,), noise, dtype=torch.float64, device=S.device)
 
-        def launch():
-            _ops.closure_eval_raw(p.detach(), S, M, noise, dist, sphere, n_fixed, out, grad, ws, out_host)
+            def launch():
+                _ops.closure_eval_f64_raw(p.detach(), S, M, noise_dev, dist, sphere, n_fixed, out, grad, ws, out_host)
+        else:
+            def launch():
+                _ops.closure_eval_raw(p.detach(), S, M, noise, dist, sphere, n_fixed, out, grad, ws, out_host)
 
         @torch.no_grad()
         def enqueue():
@@ -397,7 +409,7 @@ class SecondMomentsSQFA(nn.Module):
             enqueue()
             return out
 
-        run.enqueue, run.host_out = enqueue, out_host
+        run.enqueue, run.host_out, run.dtype = enqueue, out_host, p.dtype
         return run
 
     # ------------------------------------------------------------------ training
