@@ -27,8 +27,6 @@ namespace sqfa {
 
 namespace {
 
-inline size_t al(size_t n) { return (n + 63) & ~size_t(63); }  // floats, 256-byte granules
-
 struct ClosureLayout {
   size_t F, inv_norm, T, Mu, E, W, logdet, sinv, gE, gLog, gPsi, gMu, red_out, flag, proj, psipart, mupart, pair,
       total;
@@ -42,24 +40,24 @@ ClosureLayout closure_layout(int C, int D, int k, int dist, int64_t pair_begin, 
   const bool ld = gauss_closure_needs_logdet(dist);
   ClosureLayout L;
   size_t o = 0;
-  L.F = o;        o += al((size_t)k * D);
-  L.inv_norm = o; o += al(k);
-  L.T = o;        o += al((size_t)C * k * D);
-  L.Mu = o;       o += al((size_t)C * k);
-  L.E = o;        o += al((size_t)C * m * m);
-  L.W = o;        o += gauss ? 0 : al((size_t)C * class_factor_floats(m, dist));
-  L.logdet = o;   o += ld ? al(C) : 0;
-  L.sinv = o;     o += ld ? al((size_t)C * k * k) : 0;
-  L.gE = o;       o += le ? al((size_t)C * m * m) : 0;
-  L.gLog = o;     o += le ? al((size_t)C * m * m) : 0;
-  L.gPsi = o;     o += al((size_t)C * k * k);
-  L.gMu = o;      o += al((size_t)C * k);
-  L.red_out = o;  o += al(16);  // {loss, #non-finite, -} of a rank's pairs: [gPsi | gMu | red_out] is one exchange span
-  L.flag = o;     o += al(16);
-  L.proj = o;     o += al(project_workspace_bytes(C, D, k) / sizeof(float) + 1);
+  L.F = o;        o += al<float>((size_t)k * D);
+  L.inv_norm = o; o += al<float>(k);
+  L.T = o;        o += al<float>((size_t)C * k * D);
+  L.Mu = o;       o += al<float>((size_t)C * k);
+  L.E = o;        o += al<float>((size_t)C * m * m);
+  L.W = o;        o += gauss ? 0 : al<float>((size_t)C * class_factor_floats(m, dist));
+  L.logdet = o;   o += ld ? al<float>(C) : 0;
+  L.sinv = o;     o += ld ? al<float>((size_t)C * k * k) : 0;
+  L.gE = o;       o += le ? al<float>((size_t)C * m * m) : 0;
+  L.gLog = o;     o += le ? al<float>((size_t)C * m * m) : 0;
+  L.gPsi = o;     o += al<float>((size_t)C * k * k);
+  L.gMu = o;      o += al<float>((size_t)C * k);
+  L.red_out = o;  o += al<float>(16);  // {loss, #non-finite, -} of a rank's pairs: [gPsi | gMu | red_out] is one exchange span
+  L.flag = o;     o += al<float>(16);
+  L.proj = o;     o += al<float>(project_workspace_bytes(C, D, k) / sizeof(float) + 1);
   L.psipart = o;  o += project_psipart_floats(C, D, k);
   L.mupart = o;   o += project_mupart_floats(C, D, k);
-  L.pair = o;     o += al(gauss ? gauss_closure_workspace_floats(C, k, pair_begin, pair_end)
+  L.pair = o;     o += al<float>(gauss ? gauss_closure_workspace_floats(C, k, pair_begin, pair_end)
                             : pair_workspace(C, C, m, dist, 1, pair_begin, pair_end).total_floats);
   L.total = o;
   return L;

@@ -3,15 +3,16 @@
 // filters frozen. It is what a model converted with `.double()` evaluates: the reference's remedy for NaN / inf
 // distances (_optim.py:28-30). Same formulation as the float32 closure (pairs.cu header), every operation in
 // double, with exact division, square root and logarithm. Eight launches and one 4-byte memset, no
-// floating-point atomics (loss and gradient are bit-reproducible):
-//   constraint64_fwd_kernel   F = W / |W| row-wise                              (sphere only)
+// floating-point atomics (loss and gradient are bit-reproducible). The kernels marked * are the float32
+// closure's, instantiated for double (project.cu, pairs.cu); this file holds what differs in float64:
+//   constraint_fwd_kernel*    F = W / |W| row-wise                              (sphere only)
 //   project64_stream_kernel   row-split partials of T_c = F S_c                 (the one pass over C D^2 doubles)
 //   project64_finish_kernel   T_c; per-chunk partials of Psi_c = T_c F^T and mu'_c = F m_c
-//   class64_kernel            E_c = Psi_c + noise I (Calvo-Oller embedding for FR), L_c and L_c^-1 (one warp)
+//   class64_kernel            E_c (assemble_class_matrix*, spd_factor.cuh), L_c and L_c^-1 (one warp per class)
 //   pair64_kernel             one-sided Jacobi per pair, distances, per-tile partial dLoss/dE (one warp per tile)
-//   reduce64_kernel           dLoss/dE_c in a fixed order -> embedding adjoint (gPsi, gMu); loss, #non-finite
-//   project64_bwd_kernel      class-split partials of dLoss/dF
-//   closure64_finish_kernel   dLoss/dF, constraint adjoint -> grad, max |grad|; the last block publishes out
+//   pair_reduce_kernel*       dLoss/dE_c in a fixed order -> embedding adjoint (gPsi, gMu); loss, #non-finite
+//   project_bwd_kernel*       class-split partials of dLoss/dF
+//   closure_finish_kernel*    dLoss/dF, constraint adjoint -> grad, max |grad|; the last block publishes out
 //
 // Pair stage. A = (L_j^-1 L_i)^T; the one-sided Jacobi orthogonalises its columns, A_f = A V, and
 // lambda_q = |a_q|^2 are the generalized eigenvalues of (E_i, E_j). d^2 = sum_q log^2 lambda_q (FR: / 2).
@@ -41,36 +42,10 @@ constexpr int W64 = 4;               // warps per block of the per-class and pai
 constexpr int PS64_THREADS = 128;    // projection stream: threads per block
 constexpr int PS64_FROWS = 64;       // rows of F^T staged in shared memory at a time
 constexpr int PF64_COLS = 64;        // columns per chunk of the Psi / mu' partials
-constexpr int PB64_MAX_CSPLIT = 128;
-constexpr int CF64_THREADS = 512;
-
-__device__ __forceinline__ double warp_sum64(double v) {
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
 
 // ---------------------------------------------------------------------------------------------------------------
-// constraint and projection
+// projection
 // ---------------------------------------------------------------------------------------------------------------
-// F[f] = W[f] / |W[f]|, inv_norm[f] = 1 / |W[f]| (reference constraints.py:37). One block per filter, fixed tree.
-__global__ void __launch_bounds__(256)
-constraint64_fwd_kernel(const double* __restrict__ Wraw, int D, double* __restrict__ F, double* __restrict__ inv_norm) {
-  __shared__ double red[256];
-  const int f = blockIdx.x;
-  const double* w = Wraw + (int64_t)f * D;
-  double a = 0.0;
-  for (int j = threadIdx.x; j < D; j += 256) a = fma(w[j], w[j], a);
-  red[threadIdx.x] = a;
-  __syncthreads();
-  for (int o = 128; o > 0; o >>= 1) {
-    if ((int)threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
-    __syncthreads();
-  }
-  const double nrm = sqrt(red[0]);
-  for (int j = threadIdx.x; j < D; j += 256) F[(int64_t)f * D + j] = w[j] / nrm;
-  if (threadIdx.x == 0) inv_norm[f] = 1.0 / nrm;
-}
-
 // part[split][c][f][j] = sum_{i in the rows of split} F[f][i] S[c][i][j]. A thread owns VEC adjacent columns
 // (VEC = 2: one 16-byte load per row) and all KT filters; F^T arrives in shared memory PS64_FROWS rows at a
 // time and is read as double2 broadcasts (two filters per load, four DFMAs per load when VEC = 2).
@@ -195,32 +170,7 @@ class64_kernel(const double* __restrict__ PsiPart, const double* __restrict__ Mu
   double* Li = La + m * ld;
   double* Es = Li + m * ld;
   double* mus = Es + m * m;
-  const double noise = *noise_p;
-  if (fr) {
-    for (int r = lane; r < k; r += 32) {
-      double a = 0.0;
-      for (int ch = 0; ch < nchunk; ++ch) a += MuPart[((int64_t)c * nchunk + ch) * k + r];
-      mus[r] = a;
-      Mu[(int64_t)c * k + r] = a;
-    }
-    __syncwarp();
-  }
-  for (int idx = lane; idx < m * m; idx += 32) {
-    const int r = idx / m, s = idx % m;
-    double v;
-    if (r < k && s < k) {
-      v = 0.0;
-      const double* pp = PsiPart + (int64_t)c * nchunk * k * k + r * k + s;
-      for (int ch = 0; ch < nchunk; ++ch) v += pp[(int64_t)ch * k * k];
-      if (r == s) v += noise;
-      if (fr) v = fma(mus[r], mus[s], v);
-    } else if (r == k && s == k) {
-      v = 1.0;
-    } else {
-      v = mus[r < k ? r : s];
-    }
-    Es[idx] = v;
-  }
+  assemble_class_matrix(PsiPart, fr ? MuPart : nullptr, nchunk, *noise_p, c, k, fr != 0, Mu, mus, Es, nullptr, lane);
   __syncwarp();
   const bool ok = warp_cholesky_inverse<double>(Es, La, Li, m, ld, lane);
   double* Wc = W + (int64_t)c * 2 * m * m;
@@ -385,7 +335,7 @@ pair64_kernel(const Pair64Args A) {
           cj[q] = -2.0 * ll;
         }
       }
-      d2 = warp_sum64(d2);
+      d2 = warp_sum(d2);
       double dd_dd2;
       const double dval = finish_distance64(d2, A.dist, &dd_dd2);
       dsum += dval;
@@ -426,167 +376,9 @@ pair64_kernel(const Pair64Args A) {
   }
 }
 
-// dLoss/dE_c = its row partials (tiles of block row c / R, ascending block column) + its column partials
-// (tiles of block column c / R, ascending block row), then the adjoint of the embedding:
-//   gPsi_c = G[:k, :k];  gMu_c[r] = sum_s (G[r][s] + G[s][r]) mu_s + G[r][k] + G[k][r]   (Fisher-Rao).
-// Block C reduces the loss partials: out = {weight * sum d, #non-finite}.
-__global__ void __launch_bounds__(1024)
-reduce64_kernel(const PairTiles T, int C, int m, int k, int fr, const double* __restrict__ rowpart,
-                const double* __restrict__ colpart, const double* __restrict__ losspart, double weight,
-                const double* __restrict__ Mu, double* __restrict__ gPsi, double* __restrict__ gMu,
-                double* __restrict__ out) {
-  extern __shared__ double sg64[];
-  const int c = blockIdx.x;
-  if (c == C) {
-    double sum = 0.0, bad = 0.0;
-    if (T.ntiles > 0) reduce_loss_partials<double>(losspart, T.ntiles, sum, bad);
-    if (threadIdx.x == 0) {
-      out[0] = weight * sum;
-      out[1] = bad;
-    }
-    return;
-  }
-  const int R = T.R, m2 = m * m;
-  const int slot = c % R, bc = c / R;
-  const int64_t pstride = (int64_t)R * m2;
-  for (int e = threadIdx.x; e < m2; e += blockDim.x) {
-    double a = 0.0, b = 0.0;
-    if (bc >= T.bi0 && bc <= T.bi1) {
-      const double* p = rowpart + ((int64_t)bc * (bc + 1) / 2 - T.tile0) * pstride + (int64_t)slot * m2 + e;
-      for (int bj = 0; bj <= bc; ++bj, p += pstride) a += *p;
-    }
-    for (int bi = max(T.bi0, bc); bi <= T.bi1; ++bi)
-      b += colpart[((int64_t)bi * (bi + 1) / 2 + bc - T.tile0) * pstride + (int64_t)slot * m2 + e];
-    sg64[e] = a + b;
-  }
-  __syncthreads();
-  for (int idx = threadIdx.x; idx < k * (k + 1); idx += blockDim.x) {
-    const int r = idx / (k + 1), s = idx % (k + 1);
-    if (s < k) {
-      gPsi[(int64_t)c * k * k + r * k + s] = sg64[r * m + s];
-    } else if (fr) {
-      double v = sg64[r * m + k] + sg64[k * m + r];
-      for (int u = 0; u < k; ++u) v = fma(sg64[r * m + u] + sg64[u * m + r], Mu[(int64_t)c * k + u], v);
-      gMu[(int64_t)c * k + r] = v;
-    }
-  }
-}
-
-// partial[split][f][j] = sum_{c in split} ( sum_g (gPsi[c][f][g] + gPsi[c][g][f]) T[c][g][j] + gMu[c][f] M[c][j] )
-__global__ void __launch_bounds__(128)
-project64_bwd_kernel(const double* __restrict__ gPsi, const double* __restrict__ gMu, const double* __restrict__ T,
-                     const double* __restrict__ M, int C, int D, int k, int csplit, double* __restrict__ partial) {
-  __shared__ double Gs[32 * 32];
-  __shared__ double gm[32];
-  const int j = blockIdx.x * 128 + threadIdx.x;
-  const int c0 = (int)(((int64_t)C * blockIdx.y) / csplit), c1 = (int)(((int64_t)C * (blockIdx.y + 1)) / csplit);
-  double acc[32];
-#pragma unroll
-  for (int f = 0; f < 32; ++f) acc[f] = 0.0;
-  for (int c = c0; c < c1; ++c) {
-    __syncthreads();
-    for (int idx = threadIdx.x; idx < k * k; idx += 128) {
-      const int f = idx / k, g = idx % k;
-      Gs[idx] = gPsi[(int64_t)c * k * k + f * k + g] + gPsi[(int64_t)c * k * k + g * k + f];
-    }
-    if (gMu != nullptr)
-      for (int f = threadIdx.x; f < k; f += 128) gm[f] = gMu[(int64_t)c * k + f];
-    __syncthreads();
-    if (j < D) {
-      for (int g = 0; g < k; ++g) {
-        const double tv = T[((int64_t)c * k + g) * D + j];
-#pragma unroll
-        for (int f = 0; f < 32; ++f)
-          if (f < k) acc[f] = fma(Gs[f * k + g], tv, acc[f]);
-      }
-      if (gMu != nullptr) {
-        const double mj = M[(int64_t)c * D + j];
-#pragma unroll
-        for (int f = 0; f < 32; ++f)
-          if (f < k) acc[f] = fma(gm[f], mj, acc[f]);
-      }
-    }
-  }
-  if (j < D) {
-#pragma unroll
-    for (int f = 0; f < 32; ++f)
-      if (f < k) partial[((int64_t)blockIdx.y * k + f) * D + j] = acc[f];
-  }
-}
-
-__device__ double block_reduce64(double v, double* red, bool take_max) {
-  red[threadIdx.x] = v;
-  __syncthreads();
-  for (int o = CF64_THREADS / 2; o > 0; o >>= 1) {
-    if ((int)threadIdx.x < o)
-      red[threadIdx.x] = take_max ? fmax(red[threadIdx.x], red[threadIdx.x + o]) : red[threadIdx.x] + red[threadIdx.x + o];
-    __syncthreads();
-  }
-  const double r = red[0];
-  __syncthreads();
-  return r;
-}
-
-// One block per filter f: dF[f] = the class-split partials summed in split order; the constraint's adjoint
-// (sphere: grad[f] = (dF[f] - (dF[f] . F[f]) F[f]) / |W[f]|, none: grad[f] = dF[f]); zero rows for f < n_fixed.
-// Every block stores max |grad[f]|; the last block to arrive (integer ticket) takes the maximum over the filters
-// and writes out[2], then copies out[0..2] to the mapped host buffer.
-__global__ void __launch_bounds__(CF64_THREADS)
-closure64_finish_kernel(const double* __restrict__ partial, int D, int k, int csplit, const double* __restrict__ F,
-                        const double* __restrict__ inv_norm, int sphere, int n_fixed, double* __restrict__ grad,
-                        double* fmax_f, double* out, double* out_host, unsigned int* ticket) {
-  __shared__ double red[CF64_THREADS];
-  __shared__ bool last;
-  const int f = blockIdx.x;
-  double* g = grad + (int64_t)f * D;
-  const int64_t sstride = (int64_t)k * D;
-  double dot = 0.0;
-  for (int j = threadIdx.x; j < D; j += CF64_THREADS) {
-    const double* p = partial + (int64_t)f * D + j;
-    double a = 0.0;
-    for (int s = 0; s < csplit; ++s) a += p[(int64_t)s * sstride];
-    g[j] = a;  // re-read below by the same thread
-    if (sphere) dot = fma(a, F[(int64_t)f * D + j], dot);
-  }
-  if (sphere) dot = block_reduce64(dot, red, false);
-  const double inv = sphere ? inv_norm[f] : 1.0;
-  double amax = 0.0;
-  for (int j = threadIdx.x; j < D; j += CF64_THREADS) {
-    double v = g[j];
-    if (f < n_fixed) v = 0.0;
-    else if (sphere) v = (v - dot * F[(int64_t)f * D + j]) * inv;
-    g[j] = v;
-    amax = fmax(amax, fabs(v));
-  }
-  amax = block_reduce64(amax, red, true);  // NaN gradients: fmax drops NaN, the loss carries that information
-  if (threadIdx.x == 0) {
-    fmax_f[f] = amax;
-    __threadfence();
-    last = atomicAdd(ticket, 1u) == gridDim.x - 1;
-  }
-  __syncthreads();
-  if (last && threadIdx.x == 0) {
-    __threadfence();
-    volatile double* fm = fmax_f;
-    double mx = 0.0;
-    for (int u = 0; u < k; ++u) mx = fmax(mx, fm[u]);
-    out[2] = mx;
-    if (out_host != nullptr) {
-      volatile double* o = out;
-      volatile double* h = out_host;
-      h[0] = o[0];
-      h[1] = o[1];
-      h[2] = mx;
-      __threadfence_system();
-    }
-  }
-}
-
 // ---------------------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------------------
-inline size_t al(size_t n) { return (n + 31) & ~size_t(31); }  // doubles, 256-byte granules
-
 // row splits of the streaming pass: enough (column block, split, class) blocks for about eight per SM, at least
 // 64 rows per split
 int p64_nsplit(int C, int D) {
@@ -598,14 +390,6 @@ int p64_nsplit(int C, int D) {
   return n < 1 ? 1 : n;
 }
 
-int p64_csplit(int C, int D) {
-  const int colblocks = (D + 127) / 128;
-  int csplit = (8 * 148 + colblocks - 1) / colblocks;
-  if (csplit > PB64_MAX_CSPLIT) csplit = PB64_MAX_CSPLIT;
-  if (csplit > C) csplit = C > 0 ? C : 1;
-  return csplit < 1 ? 1 : csplit;
-}
-
 // Tile edge: single pairs for short pair lists (every pair its own warp), up to 4 x 4 once there are enough tiles
 // to fill the GPU several times over (the per-tile partials shrink with R: 2 R m^2 doubles per R^2 pairs).
 int p64_tile_edge(int64_t npairs) {
@@ -615,7 +399,7 @@ int p64_tile_edge(int64_t npairs) {
 }
 
 struct Closure64Layout {
-  size_t F, inv_norm, fmax, T, Mu, W, gPsi, gMu, ticket, proj, psipart, mupart, rowpart, colpart, losspart, total;
+  size_t F, inv_norm, T, Mu, W, gPsi, gMu, ticket, proj, psipart, mupart, rowpart, colpart, losspart, total;
   int rows, nsplit, nchunk, csplit;
   PairTiles tiles;
 };
@@ -628,27 +412,26 @@ Closure64Layout closure64_layout(int C, int D, int k, int dist, int64_t pair_beg
   L.rows = (D + L.nsplit - 1) / L.nsplit;
   L.nsplit = (D + L.rows - 1) / L.rows;
   L.nchunk = (D + PF64_COLS - 1) / PF64_COLS;
-  L.csplit = p64_csplit(C, D);
+  L.csplit = project_bwd_csplit<double>(C, D);
   const int64_t npairs = pair_end > pair_begin ? pair_end - pair_begin : 0;
   L.tiles = make_pair_tiles(C, C, 1, pair_begin, pair_end, p64_tile_edge(npairs));
   const size_t part = (size_t)L.tiles.ntiles * L.tiles.R * m * m;
   const size_t fwd = (size_t)L.nsplit * C * k * D, bwd = (size_t)L.csplit * k * D;
   size_t o = 0;
-  L.F = o;        o += al((size_t)k * D);
-  L.inv_norm = o; o += al(k);
-  L.fmax = o;     o += al(k);
-  L.T = o;        o += al((size_t)C * k * D);
-  L.Mu = o;       o += al((size_t)C * k);
-  L.W = o;        o += al((size_t)C * 2 * m * m);
-  L.gPsi = o;     o += al((size_t)C * k * k);
-  L.gMu = o;      o += al((size_t)C * k);
-  L.ticket = o;   o += al(1);  // uint32 arrival ticket of the finish kernel
-  L.proj = o;     o += al(fwd > bwd ? fwd : bwd);  // row-split partials of T, later the class-split partials of dF
-  L.psipart = o;  o += al((size_t)C * L.nchunk * k * k);
-  L.mupart = o;   o += al((size_t)C * L.nchunk * k);
-  L.rowpart = o;  o += al(part);
-  L.colpart = o;  o += al(part);
-  L.losspart = o; o += al((size_t)2 * L.tiles.ntiles);
+  L.F = o;        o += al<double>((size_t)k * D);
+  L.inv_norm = o; o += al<double>(k);
+  L.T = o;        o += al<double>((size_t)C * k * D);
+  L.Mu = o;       o += al<double>((size_t)C * k);
+  L.W = o;        o += al<double>((size_t)C * 2 * m * m);
+  L.gPsi = o;     o += al<double>((size_t)C * k * k);
+  L.gMu = o;      o += al<double>((size_t)C * k);
+  L.ticket = o;   o += al<double>(1);  // uint32 arrival ticket of closure_finish_kernel
+  L.proj = o;     o += al<double>(fwd > bwd ? fwd : bwd);  // row-split partials of T, later the class-split partials of dF
+  L.psipart = o;  o += al<double>((size_t)C * L.nchunk * k * k);
+  L.mupart = o;   o += al<double>((size_t)C * L.nchunk * k);
+  L.rowpart = o;  o += al<double>(part);
+  L.colpart = o;  o += al<double>(part);
+  L.losspart = o; o += al<double>((size_t)2 * L.tiles.ntiles);
   L.total = o;
   return L;
 }
@@ -668,11 +451,6 @@ cudaError_t run_project64_k(const double* S, const double* F, int C, int D, int 
   if (k <= 8) return run_project64<8, VEC>(S, F, C, D, k, L, part, st);
   if (k <= 16) return run_project64<16, VEC>(S, F, C, D, k, L, part, st);
   return run_project64<32, VEC>(S, F, C, D, k, L, part, st);
-}
-
-int warps_for64(int per_warp_bytes) {
-  int nw = (200 * 1024) / (per_warp_bytes > 0 ? per_warp_bytes : 1);
-  return nw > W64 ? W64 : (nw < 1 ? 1 : nw);
 }
 
 }  // namespace
@@ -696,8 +474,7 @@ cudaError_t launch_closure_f64(const double* S, const double* M, const double* r
   cudaError_t e;
   const double* F = raw_filters;
   if (sphere) {
-    constraint64_fwd_kernel<<<k, 256, 0, st>>>(raw_filters, D, ws + L.F, ws + L.inv_norm);
-    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    if ((e = launch_constraint_fwd(raw_filters, D, k, ws + L.F, ws + L.inv_norm, st)) != cudaSuccess) return e;
     F = ws + L.F;
   }
   if ((e = cudaMemsetAsync(ticket, 0, sizeof(unsigned int), st)) != cudaSuccess) return e;
@@ -710,7 +487,7 @@ cudaError_t launch_closure_f64(const double* S, const double* M, const double* r
   if ((e = cudaGetLastError()) != cudaSuccess) return e;
   {
     const int per_warp = class64_smem_doubles(m, k) * (int)sizeof(double);
-    const int nw = warps_for64(per_warp);
+    const int nw = warps_for(per_warp, W64);
     static int smem_set[kMaxDevices] = {0};
     if ((e = ensure_dynamic_smem(class64_kernel, nw * per_warp, smem_set)) != cudaSuccess) return e;
     class64_kernel<<<(C + nw - 1) / nw, nw * 32, nw * per_warp, st>>>(ws + L.psipart, ws + L.mupart, L.nchunk, noise,
@@ -728,28 +505,18 @@ cudaError_t launch_closure_f64(const double* S, const double* M, const double* r
     A.losspart = ws + L.losspart;
     A.T = L.tiles;
     const int per_warp = p64_smem_doubles(m) * (int)sizeof(double);
-    const int nw = warps_for64(per_warp);
+    const int nw = warps_for(per_warp, W64);
     static int smem_set[kMaxDevices] = {0};
     if ((e = ensure_dynamic_smem(pair64_kernel, nw * per_warp, smem_set)) != cudaSuccess) return e;
     pair64_kernel<<<(unsigned)((L.tiles.ntiles + nw - 1) / nw), nw * 32, nw * per_warp, st>>>(A);
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
   }
-  {
-    const int m2 = m * m;
-    int nt = ((m2 < 1024 ? m2 : 1024) + 31) & ~31;
-    if (nt < 128) nt = 128;
-    reduce64_kernel<<<C + 1, nt, m2 * sizeof(double), st>>>(L.tiles, C, m, k, fr, ws + L.rowpart, ws + L.colpart,
-                                                            ws + L.losspart, weight, ws + L.Mu, ws + L.gPsi,
-                                                            fr ? ws + L.gMu : nullptr, out);
-    if ((e = cudaGetLastError()) != cudaSuccess) return e;
-  }
-  project64_bwd_kernel<<<dim3((D + 127) / 128, L.csplit), 128, 0, st>>>(ws + L.gPsi, fr ? ws + L.gMu : nullptr, ws + L.T,
-                                                                        Mfr, C, D, k, L.csplit, ws + L.proj);
-  if ((e = cudaGetLastError()) != cudaSuccess) return e;
-  closure64_finish_kernel<<<k, CF64_THREADS, 0, st>>>(ws + L.proj, D, k, L.csplit, F, ws + L.inv_norm, sphere, n_fixed,
-                                                      grad, ws + L.fmax, out, out_host,
-                                                      ticket);
-  return cudaGetLastError();
+  double* gMu = fr ? ws + L.gMu : nullptr;
+  if ((e = launch_pair_reduce_closure(L.tiles, C, m, k, fr, ws + L.rowpart, ws + L.colpart, ws + L.losspart, weight,
+                                      ws + L.Mu, out, ws + L.gPsi, gMu, st)) != cudaSuccess)
+    return e;
+  return launch_project_bwd_constrained(ws + L.gPsi, gMu, ws + L.T, Mfr, C, D, k, F, ws + L.inv_norm, sphere, n_fixed,
+                                        grad, out, out_host, ticket, ws + L.proj, st);
 }
 
 }  // namespace sqfa

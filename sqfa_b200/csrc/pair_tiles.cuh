@@ -10,6 +10,12 @@
 namespace sqfa {
 namespace {
 
+template <typename T>
+__device__ __forceinline__ T warp_sum(T v) {
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  return v;
+}
+
 // local tile t of the launch -> block row / block column
 __device__ __forceinline__ void decode_tile(const PairTiles& T, int64_t t, int& bi, int& bj) {
   const int64_t gt = T.tile0 + t;

@@ -84,11 +84,6 @@ constexpr int JACOBI_MAX_SWEEPS = 24;
 constexpr float JACOBI_LAST = 3e-4f;  // a sweep of rotations all below this is the last (they leave ~1e-7)
 constexpr float DIST_EPS = 1e-6f;    // distances.py:29 EPSILON
 
-__device__ __forceinline__ float warp_sum(float v) {
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-
 __device__ __forceinline__ float rcp_approx(float x) {
   float r;
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
@@ -245,9 +240,7 @@ class_factor_kernel(const float* __restrict__ E, int C, int m, int dist, float* 
 }
 
 // Closure: everything between the projection and the pair kernel for one class, one warp:
-//   Psi_c = sum over column chunks of the partial T_c F^T (fixed order), mu'_c likewise,
-//   E_c = Psi_c + noise I (+ Calvo-Oller embedding with mu'_c for Fisher-Rao)
-//         (reference model.py:216-217 / 537-538, distances.py:162-174),
+//   E_c from the chunk partials of Psi_c and mu'_c (assemble_class_matrix, spd_factor.cuh),
 //   W_c = factorisation of E_c (above).  E is also written out (m x m per class).
 // mu'_c is formed whenever MuPart is given (Fisher-Rao, Gaussian Wasserstein); only Fisher-Rao embeds it.
 __global__ void __launch_bounds__(PAIR_WARPS * 32)
@@ -264,50 +257,7 @@ class_prepare_kernel(const float* __restrict__ PsiPart, const float* __restrict_
   float* scratch = smem + (size_t)warp * per_warp;
   float* Es = scratch + factor_scratch_floats(m);
   float* mus = Es + m * m;
-  if (MuPart != nullptr) {
-    for (int r = lane; r < k; r += 32) {
-      float a = 0.f;
-      const float* mp_ = MuPart + (int64_t)c * nchunk * k + r;
-      int ch = 0;
-      for (; ch + 8 <= nchunk; ch += 8) {
-        float u[8];
-#pragma unroll
-        for (int q = 0; q < 8; ++q) u[q] = mp_[(int64_t)(ch + q) * k];
-#pragma unroll
-        for (int q = 0; q < 8; ++q) a += u[q];
-      }
-      for (; ch < nchunk; ++ch) a += mp_[(int64_t)ch * k];
-      mus[r] = a;
-      Mu[(int64_t)c * k + r] = a;
-    }
-    __syncwarp();
-  }
-  for (int idx = lane; idx < m * m; idx += 32) {
-    const int r = idx / m, s = idx % m;
-    float v;
-    if (r < k && s < k) {
-      v = 0.f;
-      const float* pp = PsiPart + (int64_t)c * nchunk * k * k + r * k + s;
-      const int kk = k * k;
-      int ch = 0;
-      for (; ch + 8 <= nchunk; ch += 8) {  // eight loads in flight, added in chunk order
-        float u[8];
-#pragma unroll
-        for (int q = 0; q < 8; ++q) u[q] = pp[(int64_t)(ch + q) * kk];
-#pragma unroll
-        for (int q = 0; q < 8; ++q) v += u[q];
-      }
-      for (; ch < nchunk; ++ch) v += pp[(int64_t)ch * kk];
-      if (r == s) v += noise;
-      if (fr) v += mus[r] * mus[s];
-    } else if (r == k && s == k) {
-      v = 1.f;
-    } else {
-      v = mus[r < k ? r : s];
-    }
-    Es[idx] = v;
-    E[(int64_t)c * m * m + idx] = v;
-  }
+  assemble_class_matrix(PsiPart, MuPart, nchunk, noise, c, k, fr, Mu, mus, Es, E, lane);
   __syncwarp();
   const int64_t wfl = ((dist & 15) == SQFA_DIST_LOG_EUCLIDEAN) ? 2 * m * m + 2 * m : 2 * m * m;
   warp_factor_class(Es, m, dist, W + c * wfl, flag, scratch, lane);
@@ -1206,24 +1156,25 @@ le_grad_kernel(const PairTiles T, const float* __restrict__ Wa, const float* __r
 //   CLOSURE = true : the closure's tail fused in: (gPsi, gMu) = adjoint of the embedding applied to the
 //                    reduced dLoss/dE (reference model.py:216-217 / 537-538, distances.py:162-174) and
 //                    loss = {weight * sum d, #bad, 0}
-template <bool CLOSURE>
+template <typename Real, bool CLOSURE>
 __global__ void __launch_bounds__(1024)
-pair_reduce_kernel(const PairTiles T, int nA, int nB, int m, const float* __restrict__ rowpart,
-                   const float* __restrict__ colpart, const float* __restrict__ losspart, float* gEa, float* gEb,
-                   float* loss, float weight, const float* __restrict__ Mu, int k, int fr, float* __restrict__ gPsi,
-                   float* __restrict__ gMu) {
-  extern __shared__ float sg[];  // CLOSURE: the reduced m x m gradient of this class
+pair_reduce_kernel(const PairTiles T, int nA, int nB, int m, const Real* __restrict__ rowpart,
+                   const Real* __restrict__ colpart, const Real* __restrict__ losspart, Real* gEa, Real* gEb, Real* loss,
+                   Real weight, const Real* __restrict__ Mu, int k, int fr, Real* __restrict__ gPsi,
+                   Real* __restrict__ gMu) {
+  extern __shared__ __align__(16) unsigned char pr_smem[];
+  Real* sg = reinterpret_cast<Real*>(pr_smem);  // CLOSURE: the reduced m x m gradient of this class
   const int nC = max(nA, nB);
   const int c = blockIdx.x;
   if (c == nC) {
     if (loss == nullptr || losspart == nullptr) return;
-    float sum, bad;
+    Real sum, bad;
     reduce_loss_partials(losspart, T.ntiles, sum, bad);
     if (threadIdx.x == 0) {
       if (CLOSURE) {
         loss[0] = weight * sum;
         loss[1] = bad;
-        loss[2] = 0.f;  // max |grad|, filled by closure_finish_kernel with atomicMax on the float bits
+        loss[2] = Real(0);  // max |grad|, filled by closure_finish_kernel with atomicMax on the bits
       } else {
         loss[0] += sum;
         loss[1] += bad;
@@ -1236,14 +1187,14 @@ pair_reduce_kernel(const PairTiles T, int nA, int nB, int m, const float* __rest
   const int slot = c % R, bc = c / R;
   const int64_t pstride = (int64_t)R * m2;
   for (int e = threadIdx.x; e < m2; e += blockDim.x) {
-    float a = 0.f, b = 0.f;
+    Real a = Real(0), b = Real(0);
     if (c < nA && bc >= T.bi0 && bc <= T.bi1) {
       const int nb = T.tri ? bc + 1 : T.nbj;
-      const float* p = rowpart + ((T.tri ? (int64_t)bc * (bc + 1) / 2 : (int64_t)bc * T.nbj) - T.tile0) * pstride +
+      const Real* p = rowpart + ((T.tri ? (int64_t)bc * (bc + 1) / 2 : (int64_t)bc * T.nbj) - T.tile0) * pstride +
                        (int64_t)slot * m2 + e;
       int bj = 0;
       for (; bj + 8 <= nb; bj += 8) {  // eight loads in flight, added in order
-        float v[8];
+        Real v[8];
 #pragma unroll
         for (int u = 0; u < 8; ++u) v[u] = p[u * pstride];
 #pragma unroll
@@ -1260,7 +1211,7 @@ pair_reduce_kernel(const PairTiles T, int nA, int nB, int m, const float* __rest
         return colpart[tt * pstride + (int64_t)slot * m2 + e];
       };
       for (; bi + 8 <= T.bi1 + 1; bi += 8) {
-        float v[8];
+        Real v[8];
 #pragma unroll
         for (int u = 0; u < 8; ++u) v[u] = cp(bi + u);
 #pragma unroll
@@ -1285,8 +1236,8 @@ pair_reduce_kernel(const PairTiles T, int nA, int nB, int m, const float* __rest
       if (s < k) {
         gPsi[(int64_t)c * k * k + r * k + s] = sg[r * m + s];
       } else if (fr) {
-        float v = sg[r * m + k] + sg[k * m + r];
-        for (int u = 0; u < k; ++u) v += (sg[r * m + u] + sg[u * m + r]) * Mu[(int64_t)c * k + u];
+        Real v = sg[r * m + k] + sg[k * m + r];
+        for (int u = 0; u < k; ++u) v = fma(sg[r * m + u] + sg[u * m + r], Mu[(int64_t)c * k + u], v);
         gMu[(int64_t)c * k + r] = v;
       }
     }
@@ -1359,12 +1310,6 @@ __global__ void fill_diagonal_kernel(float* dist_out, int C, float v) {
 
 }  // namespace
 
-// warps per block so that the per-warp shared-memory scratch fits (large m -> fewer warps)
-static int warps_for(int per_warp_bytes) {
-  int nw = (200 * 1024) / (per_warp_bytes > 0 ? per_warp_bytes : 1);
-  return nw > PAIR_WARPS ? PAIR_WARPS : (nw < 1 ? 1 : nw);
-}
-
 size_t class_factor_floats(int m, int dist) {
   return ((dist & 15) == SQFA_DIST_LOG_EUCLIDEAN) ? (size_t)(2 * m * m + 2 * m) : (size_t)(2 * m * m);
 }
@@ -1372,7 +1317,7 @@ size_t class_factor_floats(int m, int dist) {
 cudaError_t launch_class_factor(const float* E, int C, int m, int dist, float* W, int32_t* flag, cudaStream_t st) {
   if (C <= 0) return cudaSuccess;
   const int per_warp = factor_scratch_floats(m) * (int)sizeof(float);
-  const int nw = warps_for(per_warp);
+  const int nw = warps_for(per_warp, PAIR_WARPS);
   const int smem = nw * per_warp;
   static int smem_set[kMaxDevices] = {0};
   {
@@ -1390,7 +1335,7 @@ cudaError_t launch_class_prepare(const float* PsiPart, const float* MuPart, int 
   if (C <= 0) return cudaSuccess;
   const int m = ((dist & 15) == SQFA_DIST_FISHER_RAO_LB) ? k + 1 : k;
   const int per_warp = (factor_scratch_floats(m) + m * m + k) * (int)sizeof(float);
-  const int nw = warps_for(per_warp);
+  const int nw = warps_for(per_warp, PAIR_WARPS);
   const int smem = nw * per_warp;
   static int smem_set[kMaxDevices] = {0};
   {
@@ -1436,12 +1381,11 @@ PairWorkspace pair_workspace(int nA, int nB, int m, int dist, int tri, int64_t p
   const bool le = (dist & 15) == SQFA_DIST_LOG_EUCLIDEAN;
   const bool w2 = (dist & 15) == SQFA_DIST_WASSERSTEIN_GAUSSIAN;
   const size_t part = le ? (size_t)w.T.ntiles : (size_t)w.T.ntiles * w.T.R * m * m;
-  auto al = [](size_t n) { return (n + 63) & ~size_t(63); };
   w.rowpart = 0;
-  w.colpart = al(part);
-  w.losspart = w.colpart + (le ? 0 : al(part));
-  w.pwpart = w.losspart + al((size_t)2 * w.T.ntiles);
-  w.total_floats = w.pwpart + (w2 ? al((size_t)w.T.ntiles * w.T.R * w.T.R) : 0) + 64;
+  w.colpart = al<float>(part);
+  w.losspart = w.colpart + (le ? 0 : al<float>(part));
+  w.pwpart = w.losspart + al<float>((size_t)2 * w.T.ntiles);
+  w.total_floats = w.pwpart + (w2 ? al<float>((size_t)w.T.ntiles * w.T.R * w.T.R) : 0) + 64;
   return w;
 }
 
@@ -1476,7 +1420,7 @@ static cudaError_t launch_pair_kernel(const PairArgs& A, cudaStream_t st) {
     }
   }
   const int per_warp = pair_smem_floats(m) * (int)sizeof(float);
-  const int nw = warps_for(per_warp);
+  const int nw = warps_for(per_warp, PAIR_WARPS);
   const int smem = nw * per_warp;
   const unsigned blocks = (unsigned)((A.T.ntiles + nw - 1) / nw);
   static int smem_set12[kMaxDevices] = {0}, smem_set17[kMaxDevices] = {0};
@@ -1529,7 +1473,7 @@ cudaError_t launch_pair_distances(const float* Wa, const float* Wb, int nA, int 
   const bool le = (dist & 15) == SQFA_DIST_LOG_EUCLIDEAN;
   if (le && want_grad)
     le_grad_kernel<<<nC, 256, 0, st>>>(L.T, Wa, Wb, nA, nB, m * m, 2 * m * m + 2 * m, m * m + 2 * m, A.rowpart, gEa, gEb);
-  pair_reduce_kernel<false><<<nC + 1, pair_reduce_threads(m), 0, st>>>(L.T, nA, nB, m, le ? nullptr : A.rowpart, A.colpart, A.losspart,
+  pair_reduce_kernel<float, false><<<nC + 1, pair_reduce_threads(m), 0, st>>>(L.T, nA, nB, m, le ? nullptr : A.rowpart, A.colpart, A.losspart,
                                                     gEa, gEb, loss, 1.f, nullptr, 0, 0, nullptr, nullptr);
   return cudaGetLastError();
 }
@@ -1563,21 +1507,34 @@ cudaError_t launch_pair_closure(const float* W, int C, int m, int dist, int64_t 
     if (L.T.ntiles > 0)
       le_grad_kernel<<<C, 256, 0, st>>>(L.T, W, W, C, C, m * m, 2 * m * m + 2 * m, m * m + 2 * m, A.rowpart, gLog,
                                         gLog);
-    pair_reduce_kernel<true><<<C + 1, pair_reduce_threads(m), 0, st>>>(L.T, C, C, m, nullptr, nullptr, A.losspart, nullptr, nullptr, out,
+    pair_reduce_kernel<float, true><<<C + 1, pair_reduce_threads(m), 0, st>>>(L.T, C, C, m, nullptr, nullptr, A.losspart, nullptr, nullptr, out,
                                                     weight, nullptr, k, 0, nullptr, nullptr);
     return cudaGetLastError();
   }
-  pair_reduce_kernel<true><<<C + 1, pair_reduce_threads(m), m * m * sizeof(float), st>>>(L.T, C, C, m, A.rowpart, A.colpart, A.losspart,
-                                                                     nullptr, nullptr, out, weight, Mu, k, fr ? 1 : 0,
-                                                                     gPsi, gMu);
+  return launch_pair_reduce_closure(L.T, C, m, k, fr ? 1 : 0, A.rowpart, A.colpart, A.losspart, weight, Mu, out, gPsi,
+                                    gMu, st);
+}
+
+template <typename T>
+cudaError_t launch_pair_reduce_closure(const PairTiles& tiles, int C, int m, int k, int fr, const T* rowpart,
+                                       const T* colpart, const T* losspart, T weight, const T* Mu, T* out, T* gPsi,
+                                       T* gMu, cudaStream_t st) {
+  pair_reduce_kernel<T, true><<<C + 1, pair_reduce_threads(m), m * m * sizeof(T), st>>>(
+      tiles, C, C, m, rowpart, colpart, losspart, nullptr, nullptr, out, weight, Mu, k, fr, gPsi, gMu);
   return cudaGetLastError();
 }
+template cudaError_t launch_pair_reduce_closure<float>(const PairTiles&, int, int, int, int, const float*, const float*,
+                                                       const float*, float, const float*, float*, float*, float*,
+                                                       cudaStream_t);
+template cudaError_t launch_pair_reduce_closure<double>(const PairTiles&, int, int, int, int, const double*,
+                                                        const double*, const double*, double, const double*, double*,
+                                                        double*, double*, cudaStream_t);
 
 cudaError_t launch_class_factor_bwd(const float* W, const float* gLog, int C, int m, int dist, float* gE,
                                     cudaStream_t st) {
   if ((dist & 15) != SQFA_DIST_LOG_EUCLIDEAN || C <= 0) return cudaSuccess;
   const int per_warp = 3 * m * m * (int)sizeof(float);
-  const int nw = warps_for(per_warp);
+  const int nw = warps_for(per_warp, PAIR_WARPS);
   const int smem = nw * per_warp;
   static int smem_set[kMaxDevices] = {0};
   {

@@ -209,23 +209,24 @@ __global__ void psi_reduce_kernel(const float* __restrict__ PsiPart, const float
 }
 
 // Sphere constraint (reference constraints.py:37): F[f] = W[f] / |W[f]|, inv_norm[f] = 1 / |W[f]|.
-// One block per filter, fixed reduction tree.
+// One block per filter, fixed reduction tree. T = float or double (the float64 closure).
+template <typename T>
 __global__ void __launch_bounds__(256)
-constraint_fwd_kernel(const float* __restrict__ Wraw, int D, float* __restrict__ F, float* __restrict__ inv_norm) {
-  __shared__ float red[256];
+constraint_fwd_kernel(const T* __restrict__ Wraw, int D, T* __restrict__ F, T* __restrict__ inv_norm) {
+  __shared__ T red[256];
   const int f = blockIdx.x;
-  const float* w = Wraw + (int64_t)f * D;
-  float a = 0.f;
-  for (int j = threadIdx.x; j < D; j += 256) a += w[j] * w[j];
+  const T* w = Wraw + (int64_t)f * D;
+  T a = T(0);
+  for (int j = threadIdx.x; j < D; j += 256) a = fma(w[j], w[j], a);
   red[threadIdx.x] = a;
   __syncthreads();
   for (int o = 128; o > 0; o >>= 1) {
     if ((int)threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
     __syncthreads();
   }
-  const float nrm = sqrtf(red[0]);
+  const T nrm = sqrt(red[0]);
   for (int j = threadIdx.x; j < D; j += 256) F[(int64_t)f * D + j] = w[j] / nrm;
-  if (threadIdx.x == 0) inv_norm[f] = 1.f / nrm;
+  if (threadIdx.x == 0) inv_norm[f] = T(1) / nrm;
 }
 
 // Last kernel of a closure evaluation, one block per filter f:
@@ -233,37 +234,47 @@ constraint_fwd_kernel(const float* __restrict__ Wraw, int D, float* __restrict__
 //   the constraint's adjoint: sphere  grad[f] = (dF[f] - (dF[f] . F[f]) F[f]) / |W[f]|
 //                             (autograd through constraints.py:37), none: grad[f] = dF[f];
 //   rows f < n_fixed get a zero gradient (FixedFilters detaches them, constraints.py:95-141),
-//   out[2] = max |grad| over all filters (atomicMax on the float bits; order-independent).
+//   out[2] = max |grad| over all filters (atomicMax on the bits of the non-negative value: non-negative
+//   IEEE numbers order like their bit patterns, so the result does not depend on the order of the blocks).
 constexpr int CF_THREADS = 1024;
 
-__device__ __forceinline__ float block_reduce_1024(float v, float* red, bool take_max) {
+template <typename T>
+__device__ __forceinline__ T block_reduce_1024(T v, T* red, bool take_max) {
   red[threadIdx.x] = v;
   __syncthreads();
   for (int o = CF_THREADS / 2; o > 0; o >>= 1) {
     if ((int)threadIdx.x < o)
-      red[threadIdx.x] = take_max ? fmaxf(red[threadIdx.x], red[threadIdx.x + o]) : red[threadIdx.x] + red[threadIdx.x + o];
+      red[threadIdx.x] = take_max ? fmax(red[threadIdx.x], red[threadIdx.x + o]) : red[threadIdx.x] + red[threadIdx.x + o];
     __syncthreads();
   }
-  const float r = red[0];
+  const T r = red[0];
   __syncthreads();
   return r;
 }
 
+__device__ __forceinline__ void atomic_max_nonneg(float* p, float v) {
+  atomicMax(reinterpret_cast<unsigned int*>(p), __float_as_uint(v));
+}
+__device__ __forceinline__ void atomic_max_nonneg(double* p, double v) {
+  atomicMax(reinterpret_cast<unsigned long long*>(p), (unsigned long long)__double_as_longlong(v));
+}
+
+template <typename T>
 __global__ void __launch_bounds__(CF_THREADS)
-closure_finish_kernel(const float* __restrict__ partial, int D, int k, int csplit, const float* __restrict__ F,
-                      const float* __restrict__ inv_norm, int sphere, int n_fixed, float* __restrict__ grad,
-                      float* out, float* out_host, unsigned int* ticket) {
-  __shared__ float red[CF_THREADS];
+closure_finish_kernel(const T* __restrict__ partial, int D, int k, int csplit, const T* __restrict__ F,
+                      const T* __restrict__ inv_norm, int sphere, int n_fixed, T* __restrict__ grad,
+                      T* out, T* out_host, unsigned int* ticket) {
+  __shared__ T red[CF_THREADS];
   const int f = blockIdx.x;
-  float* g = grad + (int64_t)f * D;
+  T* g = grad + (int64_t)f * D;
   const int64_t sstride = (int64_t)k * D;
-  float dot = 0.f;
+  T dot = T(0);
   for (int j = threadIdx.x; j < D; j += CF_THREADS) {
-    const float* p = partial + (int64_t)f * D + j;
-    float a = 0.f;
+    const T* p = partial + (int64_t)f * D + j;
+    T a = T(0);
     int s = 0;
     for (; s + 8 <= csplit; s += 8) {  // eight loads in flight, added in split order
-      float u[8];
+      T u[8];
 #pragma unroll
       for (int q = 0; q < 8; ++q) u[q] = p[(int64_t)(s + q) * sstride];
 #pragma unroll
@@ -271,30 +282,30 @@ closure_finish_kernel(const float* __restrict__ partial, int D, int k, int cspli
     }
     for (; s < csplit; ++s) a += p[(int64_t)s * sstride];
     g[j] = a;  // re-read below by the same thread
-    if (sphere) dot += a * F[(int64_t)f * D + j];
+    if (sphere) dot = fma(a, F[(int64_t)f * D + j], dot);
   }
   if (sphere) dot = block_reduce_1024(dot, red, false);
-  const float inv = sphere ? inv_norm[f] : 1.f;
-  float amax = 0.f;
+  const T inv = sphere ? inv_norm[f] : T(1);
+  T amax = T(0);
   for (int j = threadIdx.x; j < D; j += CF_THREADS) {
-    float v = g[j];
-    if (f < n_fixed) v = 0.f;
+    T v = g[j];
+    if (f < n_fixed) v = T(0);
     else if (sphere) v = (v - dot * F[(int64_t)f * D + j]) * inv;
     g[j] = v;
-    amax = fmaxf(amax, fabsf(v));
+    amax = fmax(amax, fabs(v));
   }
   amax = block_reduce_1024(amax, red, true);
-  // NaN gradients: fmaxf drops NaN, the loss / non-finite counter carry that information
+  // NaN gradients: fmax drops NaN, the loss / non-finite counter carry that information
   if (threadIdx.x == 0 && out != nullptr) {
-    atomicMax(reinterpret_cast<unsigned int*>(out + 2), __float_as_uint(amax));
+    atomic_max_nonneg(out + 2, amax);
     if (out_host != nullptr) {
       // the last block to arrive publishes {loss, #non-finite, max |grad|} in the caller's mapped host
-      // memory: the host then needs an event wait and no copy (`ticket` is zeroed by class_prepare's memset)
+      // memory: the host then needs an event wait and no copy (`ticket` is zeroed by the closure's memset)
       __threadfence();
       if (atomicAdd(ticket, 1u) == gridDim.x - 1) {
         __threadfence();
-        volatile float* o = out;
-        volatile float* h = out_host;
+        volatile T* o = out;
+        volatile T* h = out_host;
         h[0] = o[0];
         h[1] = o[1];
         h[2] = o[2];
@@ -305,18 +316,20 @@ closure_finish_kernel(const float* __restrict__ partial, int D, int k, int cspli
 }
 
 // dF[f][j] = sum_c ( sum_g (gPsi[c][f][g] + gPsi[c][g][f]) T[c][g][j] + gMu[c][f] M[c][j] )
-// grid: (ceil(D/128), class splits); partial results reduced by project_bwd_finalize_kernel.
+// grid: (ceil(D/128), class splits); partial results reduced by project_bwd_finalize_kernel or
+// closure_finish_kernel. k <= 32.
+template <typename Real>
 __global__ void __launch_bounds__(128)
-project_bwd_kernel(const float* __restrict__ gPsi, const float* __restrict__ gMu, const float* __restrict__ T,
-                   const float* __restrict__ M, int C, int D, int k, int csplit, float* __restrict__ partial) {
-  extern __shared__ float sm[];  // Gs[k][k] symmetrised, gm[k]
-  float* Gs = sm;
-  float* gm = sm + k * k;
+project_bwd_kernel(const Real* __restrict__ gPsi, const Real* __restrict__ gMu, const Real* __restrict__ T,
+                   const Real* __restrict__ M, int C, int D, int k, int csplit, Real* __restrict__ partial) {
+  extern __shared__ __align__(16) unsigned char pb_smem[];
+  Real* Gs = reinterpret_cast<Real*>(pb_smem);  // Gs[k][k] symmetrised, gm[k]
+  Real* gm = Gs + k * k;
   const int j = blockIdx.x * 128 + threadIdx.x;
   const int c0 = (int)(((int64_t)C * blockIdx.y) / csplit), c1 = (int)(((int64_t)C * (blockIdx.y + 1)) / csplit);
-  float acc[32];
+  Real acc[32];
 #pragma unroll
-  for (int f = 0; f < 32; ++f) acc[f] = 0.f;
+  for (int f = 0; f < 32; ++f) acc[f] = Real(0);
   for (int c = c0; c < c1; ++c) {
     __syncthreads();
     for (int idx = threadIdx.x; idx < k * k; idx += 128) {
@@ -327,17 +340,17 @@ project_bwd_kernel(const float* __restrict__ gPsi, const float* __restrict__ gMu
       for (int f = threadIdx.x; f < k; f += 128) gm[f] = gMu[(int64_t)c * k + f];
     __syncthreads();
     if (j < D) {
-      const float mj = (gMu != nullptr) ? M[(int64_t)c * D + j] : 0.f;
+      const Real mj = (gMu != nullptr) ? M[(int64_t)c * D + j] : Real(0);
       for (int g = 0; g < k; ++g) {
-        const float t = T[((int64_t)c * k + g) * D + j];
+        const Real t = T[((int64_t)c * k + g) * D + j];
 #pragma unroll
         for (int f = 0; f < 32; ++f)
-          if (f < k) acc[f] += Gs[f * k + g] * t;
+          if (f < k) acc[f] = fma(Gs[f * k + g], t, acc[f]);
       }
       if (gMu != nullptr) {
 #pragma unroll
         for (int f = 0; f < 32; ++f)
-          if (f < k) acc[f] += gm[f] * mj;
+          if (f < k) acc[f] = fma(gm[f], mj, acc[f]);
       }
     }
   }
@@ -674,26 +687,30 @@ static size_t project_partial_floats(int C, int D, int k) {
 }
 
 int project_nchunk(int D) { return (D + PF_COLS - 1) / PF_COLS; }
-static size_t al64(size_t n) { return (n + 63) & ~size_t(63); }
-size_t project_psipart_floats(int C, int D, int k) { return al64((size_t)C * project_nchunk(D) * k * k); }
-size_t project_mupart_floats(int C, int D, int k) { return al64((size_t)C * project_nchunk(D) * k); }
-constexpr int PB_MAX_CSPLIT = 256;
+size_t project_psipart_floats(int C, int D, int k) { return al<float>((size_t)C * project_nchunk(D) * k * k); }
+size_t project_mupart_floats(int C, int D, int k) { return al<float>((size_t)C * project_nchunk(D) * k); }
+// most class splits of the projection adjoint (the float64 closure's workspace is sized for 128)
+template <typename T> constexpr int PB_MAX_CSPLIT = 256;
+template <> constexpr int PB_MAX_CSPLIT<double> = 128;
+template <typename T>
 int project_bwd_csplit(int C, int D) {
   // enough (column block, class split) blocks to fill the GPU about 8 times over: every block walks its
   // classes serially (one dependent round of loads per class), so short class lists hide latency
   const int colblocks = (D + 127) / 128;
   int csplit = (8 * 148 + colblocks - 1) / colblocks;
-  if (csplit > PB_MAX_CSPLIT) csplit = PB_MAX_CSPLIT;
+  if (csplit > PB_MAX_CSPLIT<T>) csplit = PB_MAX_CSPLIT<T>;
   if (csplit > C) csplit = C > 0 ? C : 1;
   return csplit < 1 ? 1 : csplit;
 }
+template int project_bwd_csplit<float>(int, int);
+template int project_bwd_csplit<double>(int, int);
 
 // workspace (floats): [ row-split partials | PsiPart | MuPart ] for the forward, [ class-split partials ] for
 // the adjoint (they alias: the two are never live together)
 size_t project_workspace_bytes(int C, int D, int k) {
-  const size_t fwd = al64(project_partial_floats(C, D, k)) + project_psipart_floats(C, D, k) +
+  const size_t fwd = al<float>(project_partial_floats(C, D, k)) + project_psipart_floats(C, D, k) +
                      project_mupart_floats(C, D, k);
-  const size_t bwd = (size_t)PB_MAX_CSPLIT * k * D;
+  const size_t bwd = (size_t)PB_MAX_CSPLIT<float> * k * D;
   return (fwd > bwd ? fwd : bwd) * sizeof(float);
 }
 
@@ -723,7 +740,7 @@ cudaError_t launch_project_partials(const float* S, const float* M, const float*
 cudaError_t launch_project_fwd(const float* S, const float* M, const float* F, int C, int D, int k, float* T,
                                float* Psi, float* Mu, float* ws, cudaStream_t st) {
   if (C <= 0) return cudaSuccess;
-  float* PsiPart = ws + al64(project_partial_floats(C, D, k));
+  float* PsiPart = ws + al<float>(project_partial_floats(C, D, k));
   float* MuPart = PsiPart + project_psipart_floats(C, D, k);
   cudaError_t e = launch_project_partials(S, M, F, C, D, k, T, ws, PsiPart, M != nullptr ? MuPart : nullptr, st);
   if (e != cudaSuccess) return e;
@@ -733,17 +750,18 @@ cudaError_t launch_project_fwd(const float* S, const float* M, const float* F, i
   return cudaGetLastError();
 }
 
-static cudaError_t launch_project_bwd_partials(const float* gPsi, const float* gMu, const float* T, const float* M,
-                                               int C, int D, int k, float* ws, int csplit, cudaStream_t st) {
+template <typename Real>
+static cudaError_t launch_project_bwd_partials(const Real* gPsi, const Real* gMu, const Real* T, const Real* M, int C,
+                                               int D, int k, Real* ws, int csplit, cudaStream_t st) {
   const int colblocks = (D + 127) / 128;
-  const int smem = (k * k + k) * (int)sizeof(float);
-  project_bwd_kernel<<<dim3(colblocks, csplit), 128, smem, st>>>(gPsi, gMu, T, M, C, D, k, csplit, ws);
+  const int smem = (k * k + k) * (int)sizeof(Real);
+  project_bwd_kernel<Real><<<dim3(colblocks, csplit), 128, smem, st>>>(gPsi, gMu, T, M, C, D, k, csplit, ws);
   return cudaGetLastError();
 }
 
 cudaError_t launch_project_bwd(const float* gPsi, const float* gMu, const float* T, const float* M, int C, int D,
                                int k, float* dF, float* ws, cudaStream_t st) {
-  const int csplit = project_bwd_csplit(C, D);
+  const int csplit = project_bwd_csplit<float>(C, D);
   cudaError_t e = launch_project_bwd_partials(gPsi, gMu, T, M, C, D, k, ws, csplit, st);
   if (e != cudaSuccess) return e;
   const int64_t total = (int64_t)k * D;
@@ -752,22 +770,33 @@ cudaError_t launch_project_bwd(const float* gPsi, const float* gMu, const float*
 }
 
 // adjoint of the projection followed by the adjoint of the filter constraint (closure tail)
-cudaError_t launch_project_bwd_constrained(const float* gPsi, const float* gMu, const float* T, const float* M, int C,
-                                           int D, int k, const float* F, const float* inv_norm, int sphere,
-                                           int n_fixed, float* grad, float* out, float* out_host,
-                                           unsigned int* ticket, float* ws, cudaStream_t st) {
-  const int csplit = project_bwd_csplit(C, D);
+template <typename Real>
+cudaError_t launch_project_bwd_constrained(const Real* gPsi, const Real* gMu, const Real* T, const Real* M, int C,
+                                           int D, int k, const Real* F, const Real* inv_norm, int sphere, int n_fixed,
+                                           Real* grad, Real* out, Real* out_host, unsigned int* ticket, Real* ws,
+                                           cudaStream_t st) {
+  const int csplit = project_bwd_csplit<Real>(C, D);
   cudaError_t e = launch_project_bwd_partials(gPsi, gMu, T, M, C, D, k, ws, csplit, st);
   if (e != cudaSuccess) return e;
-  closure_finish_kernel<<<k, CF_THREADS, 0, st>>>(ws, D, k, csplit, F, inv_norm, sphere, n_fixed, grad, out, out_host,
-                                                  ticket);
+  closure_finish_kernel<Real><<<k, CF_THREADS, 0, st>>>(ws, D, k, csplit, F, inv_norm, sphere, n_fixed, grad, out,
+                                                     out_host, ticket);
   return cudaGetLastError();
 }
+template cudaError_t launch_project_bwd_constrained<float>(const float*, const float*, const float*, const float*, int,
+                                                           int, int, const float*, const float*, int, int, float*,
+                                                           float*, float*, unsigned int*, float*, cudaStream_t);
+template cudaError_t launch_project_bwd_constrained<double>(const double*, const double*, const double*,
+                                                            const double*, int, int, int, const double*,
+                                                            const double*, int, int, double*, double*, double*,
+                                                            unsigned int*, double*, cudaStream_t);
 
-cudaError_t launch_constraint_fwd(const float* Wraw, int D, int k, float* F, float* inv_norm, cudaStream_t st) {
-  constraint_fwd_kernel<<<k, 256, 0, st>>>(Wraw, D, F, inv_norm);
+template <typename T>
+cudaError_t launch_constraint_fwd(const T* Wraw, int D, int k, T* F, T* inv_norm, cudaStream_t st) {
+  constraint_fwd_kernel<T><<<k, 256, 0, st>>>(Wraw, D, F, inv_norm);
   return cudaGetLastError();
 }
+template cudaError_t launch_constraint_fwd<float>(const float*, int, int, float*, float*, cudaStream_t);
+template cudaError_t launch_constraint_fwd<double>(const double*, int, int, double*, double*, cudaStream_t);
 
 template <int KF, typename T>
 static cudaError_t run_transform_tile(const T* X, int64_t ldx, const float* F, int64_t n, int D, int k, float* Z,

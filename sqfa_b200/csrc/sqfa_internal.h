@@ -21,6 +21,20 @@ inline cudaError_t ensure_dynamic_smem(Kernel kernel, int bytes, int (&set_bytes
   return e;
 }
 
+// warps per block of a one-warp-per-problem kernel: at most max_warps, fewer when the per-warp shared-memory
+// scratch would not fit in 200 KB (large m)
+inline int warps_for(int per_warp_bytes, int max_warps) {
+  const int nw = (200 * 1024) / (per_warp_bytes > 0 ? per_warp_bytes : 1);
+  return nw > max_warps ? max_warps : (nw < 1 ? 1 : nw);
+}
+
+// n elements of T rounded up to whole 256-byte granules (workspace offsets)
+template <typename T>
+inline size_t al(size_t n) {
+  constexpr size_t g = 256 / sizeof(T);
+  return (n + g - 1) & ~(g - 1);
+}
+
 // Element type of the data points X (same values as SQFA_ELEM_* of the C ABI); see elem.cuh.
 enum ElemType { ELEM_F32 = 0, ELEM_BF16 = 1, ELEM_F16 = 2 };
 inline int elem_bytes(int elem) { return elem == ELEM_F32 ? 4 : 2; }
@@ -81,11 +95,18 @@ cudaError_t launch_project_fwd(const float* S, const float* M, const float* F, i
                                float* Psi, float* Mu, float* ws, cudaStream_t st);
 cudaError_t launch_project_bwd(const float* gPsi, const float* gMu, const float* T, const float* M, int C, int D,
                                int k, float* dF, float* ws, cudaStream_t st);
-cudaError_t launch_project_bwd_constrained(const float* gPsi, const float* gMu, const float* T, const float* M, int C,
-                                           int D, int k, const float* F, const float* inv_norm, int sphere,
-                                           int n_fixed, float* grad, float* out, float* out_host,
-                                           unsigned int* ticket, float* ws, cudaStream_t st);
-cudaError_t launch_constraint_fwd(const float* Wraw, int D, int k, float* F, float* inv_norm, cudaStream_t st);
+// The closure's tail, shared by the float32 and float64 closures (T = float, double): class-split partials of the
+// projection adjoint, then one block per filter sums them, applies the constraint's adjoint, zeroes the frozen rows
+// and publishes max |grad| into out[2] (which the pair stage's reduce kernel zeroes) and out_host.
+template <typename T>
+int project_bwd_csplit(int C, int D);
+template <typename Real>
+cudaError_t launch_project_bwd_constrained(const Real* gPsi, const Real* gMu, const Real* T, const Real* M, int C,
+                                           int D, int k, const Real* F, const Real* inv_norm, int sphere, int n_fixed,
+                                           Real* grad, Real* out, Real* out_host, unsigned int* ticket, Real* ws,
+                                           cudaStream_t st);
+template <typename T>
+cudaError_t launch_constraint_fwd(const T* Wraw, int D, int k, T* F, T* inv_norm, cudaStream_t st);
 cudaError_t launch_transform(const void* X, int elem, int64_t ldx, const float* F, int64_t n, int D, int k, float* Z,
                              cudaStream_t st);
 cudaError_t launch_embed_fwd(const float* Psi, const float* Mu, float noise, int C, int k, int fr, float* E,
@@ -134,6 +155,12 @@ cudaError_t launch_pair_distances(const float* Wa, const float* Wb, int nA, int 
 cudaError_t launch_pair_closure(const float* W, int C, int m, int dist, int64_t pair_begin, int64_t pair_end,
                                 float weight, const float* Mu, int k, float* out, float* gPsi, float* gMu, float* gLog,
                                 float* ws, cudaStream_t st);
+// Per class c < C: dLoss/dE_c summed from the per-tile row / column partials in a fixed order, then the adjoint
+// of the embedding -> (gPsi, gMu); out = {weight * sum d, #non-finite, 0}. T = float, double.
+template <typename T>
+cudaError_t launch_pair_reduce_closure(const PairTiles& tiles, int C, int m, int k, int fr, const T* rowpart,
+                                       const T* colpart, const T* losspart, T weight, const T* Mu, T* out, T* gPsi,
+                                       T* gMu, cudaStream_t st);
 cudaError_t launch_class_factor_bwd(const float* W, const float* gLog, int C, int m, int dist, float* gE,
                                     cudaStream_t st);
 }  // namespace sqfa
