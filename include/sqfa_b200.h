@@ -391,7 +391,8 @@ int sqfa_closure_eval(const float* S, const float* M, const float* raw_filters, 
 
 /* sqfa_closure_eval in float64: S, M, raw_filters, out, out_host and grad are double. For
  * SQFA_DIST_AFFINE_INVARIANT and SQFA_DIST_FISHER_RAO_LB (each optionally + SQFA_DIST_SQUARED) and
- * n_filters <= 32; other codes and n_filters > 32 return SQFA_E_UNSUPPORTED (M is required for Fisher-Rao).
+ * n_filters <= 32; other codes and n_filters > 32 return SQFA_E_UNSUPPORTED (M is required for Fisher-Rao; the
+ * mean-covariance distances have their own entry point, sqfa_gauss_closure_eval_f64).
  * `noise` points to ONE double in device memory (read by the kernels, so a captured graph picks up a new
  * value). As in float32, out[0] over a sub-range [pair_begin, pair_end) is scaled by 1/P of ALL pairs, so
  * the losses and gradients of disjoint ranges add up. Deterministic: no floating-point atomics. The
@@ -402,6 +403,19 @@ int sqfa_closure_eval_f64(const double* S, const double* M, const double* raw_fi
                           int32_t n_dim, int32_t n_filters, const double* noise, int32_t dist, int32_t constraint,
                           int32_t n_fixed, int64_t pair_begin, int64_t pair_end, double* out, double* out_host,
                           double* grad, void* ws, size_t ws_bytes, sqfa_stream_t stream);
+
+/* The float64 closure of the mean-covariance distances: the same 18 parameters and contracts as
+ * sqfa_closure_eval_f64, for SQFA_DIST_MAHALANOBIS (optionally + SQFA_DIST_SQUARED), SQFA_DIST_BHATTACHARYYA
+ * and SQFA_DIST_HELLINGER. M is required, n_filters <= 32, constraint NONE or SPHERE. Every other code,
+ * SQFA_DIST_SQUARED with Bhattacharyya or Hellinger and n_filters > 32 return SQFA_E_UNSUPPORTED (the codes of
+ * sqfa_closure_eval_f64 with a message naming it); the workspace query returns 0 for them. */
+size_t sqfa_gauss_closure_workspace_bytes_f64(int32_t n_classes, int32_t n_dim, int32_t n_filters, int32_t dist,
+                                              int64_t pair_begin, int64_t pair_end);
+int sqfa_gauss_closure_eval_f64(const double* S, const double* M, const double* raw_filters, int32_t n_classes,
+                                int32_t n_dim, int32_t n_filters, const double* noise, int32_t dist,
+                                int32_t constraint, int32_t n_fixed, int64_t pair_begin, int64_t pair_end,
+                                double* out, double* out_host, double* grad, void* ws, size_t ws_bytes,
+                                sqfa_stream_t stream);
 
 /* Plug-in distances between Gaussians that use the mean covariance of the pair (distances.py:240-432),
  * one warp per pair (Cholesky of (Sigma_a + Sigma_b) / 2 in shared memory), all n_a * n_b pairs:

@@ -443,20 +443,30 @@ def closure_eval_raw(W, S, M, noise, dist, sphere, n_fixed, out, grad, ws, out_h
     )
 
 
-def closure_eval_f64_raw(W, S, M, noise, dist, sphere, n_fixed, out, grad, ws, out_host=None):
-    """`closure_eval_raw` in float64 (affine-invariant / Fisher-Rao lower bound): every tensor is float64 and
-    `noise` is a one-element float64 device tensor, read by the kernels."""
+def _closure_eval_f64(fn, W, S, M, noise, dist, sphere, n_fixed, out, grad, ws, out_host):
     lib = _lib.load()
     C, D, _ = S.shape
     k = W.shape[0]
     P = C * (C - 1) // 2
     _lib.check(
-        lib.sqfa_closure_eval_f64(
+        getattr(lib, fn)(
             _lib.ptr(S), _lib.ptr(M), _lib.ptr(W), C, D, k, _lib.ptr(noise), dist, 1 if sphere else 0, int(n_fixed), 0,
             P, _lib.ptr(out), _lib.ptr(out_host), _lib.ptr(grad), _lib.ptr(ws), ws.numel(), _lib.stream_ptr(S.device),
         ),
-        "sqfa_closure_eval_f64",
+        fn,
     )
+
+
+def closure_eval_f64_raw(W, S, M, noise, dist, sphere, n_fixed, out, grad, ws, out_host=None):
+    """`closure_eval_raw` in float64 (affine-invariant / Fisher-Rao lower bound): every tensor is float64 and
+    `noise` is a one-element float64 device tensor, read by the kernels."""
+    _closure_eval_f64("sqfa_closure_eval_f64", W, S, M, noise, dist, sphere, n_fixed, out, grad, ws, out_host)
+
+
+def gauss_closure_eval_f64_raw(W, S, M, noise, dist, sphere, n_fixed, out, grad, ws, out_host=None):
+    """`closure_eval_f64_raw` for the mean-covariance distances (Mahalanobis, Bhattacharyya, Hellinger); M, the
+    class means, is required."""
+    _closure_eval_f64("sqfa_gauss_closure_eval_f64", W, S, M, noise, dist, sphere, n_fixed, out, grad, ws, out_host)
 
 
 class FusedLoss(torch.autograd.Function):

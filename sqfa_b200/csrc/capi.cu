@@ -503,8 +503,13 @@ int sqfa_closure_eval_f64(const double* S_, const double* M, const double* raw_f
                           int32_t n_fixed, int64_t pair_begin, int64_t pair_end, double* out, double* out_host,
                           double* grad, void* ws, size_t ws_bytes, sqfa_stream_t stream) {
   if (!f64_dist_ok(dist))
-    return fail_arg(__func__, "the float64 closure supports SQFA_DIST_AFFINE_INVARIANT and SQFA_DIST_FISHER_RAO_LB "
-                              "(optionally + SQFA_DIST_SQUARED)", SQFA_E_UNSUPPORTED);
+    return fail_arg(__func__, sqfa::is_gauss_closure(dist)
+                                  ? "the float64 closure supports SQFA_DIST_AFFINE_INVARIANT and SQFA_DIST_FISHER_RAO_LB "
+                                    "(optionally + SQFA_DIST_SQUARED); the mean-covariance distances take "
+                                    "sqfa_gauss_closure_eval_f64"
+                                  : "the float64 closure supports SQFA_DIST_AFFINE_INVARIANT and SQFA_DIST_FISHER_RAO_LB "
+                                    "(optionally + SQFA_DIST_SQUARED)",
+                    SQFA_E_UNSUPPORTED);
   if (constraint != SQFA_CONSTRAINT_NONE && constraint != SQFA_CONSTRAINT_SPHERE)
     return fail_arg(__func__, "constraint must be SQFA_CONSTRAINT_NONE or SQFA_CONSTRAINT_SPHERE");
   if (S_ == nullptr || raw_filters == nullptr || noise == nullptr || out == nullptr || grad == nullptr ||
@@ -519,6 +524,50 @@ int sqfa_closure_eval_f64(const double* S_, const double* M, const double* raw_f
   return wrap(__func__, sqfa::launch_closure_f64(S_, M, raw_filters, n_classes, n_dim, n_filters, noise, dist,
                                                  constraint, n_fixed, pair_begin, pair_end, out, out_host, grad,
                                                  static_cast<double*>(ws), S(stream)));
+}
+
+// float64 closure of the mean-covariance distances: Mahalanobis (plain or squared), Bhattacharyya, Hellinger
+static int gauss_f64_dist_ok(int32_t dist) {
+  const int b = dist & 15;
+  return (dist & ~(15 | SQFA_DIST_SQUARED)) == 0 && sqfa::is_gauss_closure(dist) &&
+         (b == SQFA_DIST_MAHALANOBIS || (dist & SQFA_DIST_SQUARED) == 0);
+}
+
+size_t sqfa_gauss_closure_workspace_bytes_f64(int32_t n_classes, int32_t n_dim, int32_t n_filters, int32_t dist,
+                                              int64_t pair_begin, int64_t pair_end) {
+  const int64_t P = (int64_t)n_classes * (n_classes - 1) / 2;
+  if (n_classes <= 0 || n_dim <= 0 || n_filters <= 0 || n_filters > 32 || !gauss_f64_dist_ok(dist) ||
+      pair_begin < 0 || pair_end > P || pair_begin > pair_end)
+    return 0;
+  return sqfa::fused_loss_workspace_bytes_f64(n_classes, n_dim, n_filters, dist, pair_begin, pair_end);
+}
+
+int sqfa_gauss_closure_eval_f64(const double* S_, const double* M, const double* raw_filters, int32_t n_classes,
+                                int32_t n_dim, int32_t n_filters, const double* noise, int32_t dist,
+                                int32_t constraint, int32_t n_fixed, int64_t pair_begin, int64_t pair_end,
+                                double* out, double* out_host, double* grad, void* ws, size_t ws_bytes,
+                                sqfa_stream_t stream) {
+  if (f64_dist_ok(dist))
+    return fail_arg(__func__, "SQFA_DIST_AFFINE_INVARIANT and SQFA_DIST_FISHER_RAO_LB take sqfa_closure_eval_f64",
+                    SQFA_E_UNSUPPORTED);
+  if (!gauss_f64_dist_ok(dist))
+    return fail_arg(__func__, "the float64 mean-covariance closure supports SQFA_DIST_MAHALANOBIS (optionally + "
+                              "SQFA_DIST_SQUARED), SQFA_DIST_BHATTACHARYYA and SQFA_DIST_HELLINGER",
+                    SQFA_E_UNSUPPORTED);
+  if (constraint != SQFA_CONSTRAINT_NONE && constraint != SQFA_CONSTRAINT_SPHERE)
+    return fail_arg(__func__, "constraint must be SQFA_CONSTRAINT_NONE or SQFA_CONSTRAINT_SPHERE");
+  if (S_ == nullptr || M == nullptr || raw_filters == nullptr || noise == nullptr || out == nullptr ||
+      grad == nullptr || ws == nullptr || n_classes <= 0 || n_dim <= 0 || n_filters <= 0 || n_fixed < 0 ||
+      n_fixed > n_filters || (reinterpret_cast<uintptr_t>(ws) & 15) != 0)
+    return fail_arg(__func__, "bad argument");
+  if (n_filters > 32) return fail_arg(__func__, "n_filters must be <= 32", SQFA_E_UNSUPPORTED);
+  const int64_t P = (int64_t)n_classes * (n_classes - 1) / 2;
+  if (pair_begin < 0 || pair_end > P || pair_begin > pair_end) return fail_arg(__func__, "bad pair range");
+  if (ws_bytes < sqfa_gauss_closure_workspace_bytes_f64(n_classes, n_dim, n_filters, dist, pair_begin, pair_end))
+    return fail_arg(__func__, "workspace too small", SQFA_E_WORKSPACE);
+  return wrap(__func__, sqfa::launch_gauss_closure_f64(S_, M, raw_filters, n_classes, n_dim, n_filters, noise, dist,
+                                                       constraint, n_fixed, pair_begin, pair_end, out, out_host, grad,
+                                                       static_cast<double*>(ws), S(stream)));
 }
 
 }  // extern "C"

@@ -57,7 +57,7 @@ ClosureLayout closure_layout(int C, int D, int k, int dist, int64_t pair_begin, 
   L.proj = o;     o += al<float>(project_workspace_bytes(C, D, k) / sizeof(float) + 1);
   L.psipart = o;  o += project_psipart_floats(C, D, k);
   L.mupart = o;   o += project_mupart_floats(C, D, k);
-  L.pair = o;     o += al<float>(gauss ? gauss_closure_workspace_floats(C, k, pair_begin, pair_end)
+  L.pair = o;     o += al<float>(gauss ? gauss_closure_workspace_elems(C, k, pair_begin, pair_end)
                             : pair_workspace(C, C, m, dist, 1, pair_begin, pair_end).total_floats);
   L.total = o;
   return L;

@@ -13,6 +13,9 @@
 //   pair_reduce_kernel*       dLoss/dE_c in a fixed order -> embedding adjoint (gPsi, gMu); loss, #non-finite
 //   project_bwd_kernel*       class-split partials of dLoss/dF
 //   closure_finish_kernel*    dLoss/dF, constraint adjoint -> grad, max |grad|; the last block publishes out
+// The mean-covariance distances (Mahalanobis, Bhattacharyya, Hellinger; launch_gauss_closure_f64) share the
+// constraint, the projection and its adjoint, and replace class64 / pair64 / pair_reduce with the class, pair and
+// reduce stages of gauss.cu instantiated for double (DESIGN.md section 19).
 //
 // Pair stage. A = (L_j^-1 L_i)^T; the one-sided Jacobi orthogonalises its columns, A_f = A V, and
 // lambda_q = |a_q|^2 are the generalized eigenvalues of (E_i, E_j). d^2 = sum_q log^2 lambda_q (FR: / 2).
@@ -399,13 +402,19 @@ int p64_tile_edge(int64_t npairs) {
 }
 
 struct Closure64Layout {
-  size_t F, inv_norm, T, Mu, W, gPsi, gMu, ticket, proj, psipart, mupart, rowpart, colpart, losspart, total;
+  size_t F, inv_norm, T, Mu, W, logdet, sinv, gPsi, gMu, ticket, proj, psipart, mupart, rowpart, colpart, losspart, pair,
+      total;
   int rows, nsplit, nchunk, csplit;
   PairTiles tiles;
 };
 
+// One layout for both float64 closures. The mean-covariance distances (gauss) keep Psi_c in W, logdet Psi_c and
+// Psi_c^-1 for Bhattacharyya / Hellinger, and the pair stage's workspace of gauss.cu in `pair`; the
+// affine-invariant / Fisher-Rao closure keeps [L_c | L_c^-1] in W and its tile partials.
 Closure64Layout closure64_layout(int C, int D, int k, int dist, int64_t pair_begin, int64_t pair_end) {
   const bool fr = (dist & 15) == SQFA_DIST_FISHER_RAO_LB;
+  const bool gauss = is_gauss_closure(dist);
+  const bool ld = gauss_closure_needs_logdet(dist);
   const int m = fr ? k + 1 : k;
   Closure64Layout L;
   L.nsplit = p64_nsplit(C, D);
@@ -414,24 +423,27 @@ Closure64Layout closure64_layout(int C, int D, int k, int dist, int64_t pair_beg
   L.nchunk = (D + PF64_COLS - 1) / PF64_COLS;
   L.csplit = project_bwd_csplit<double>(C, D);
   const int64_t npairs = pair_end > pair_begin ? pair_end - pair_begin : 0;
-  L.tiles = make_pair_tiles(C, C, 1, pair_begin, pair_end, p64_tile_edge(npairs));
-  const size_t part = (size_t)L.tiles.ntiles * L.tiles.R * m * m;
+  L.tiles = make_pair_tiles(C, C, 1, pair_begin, pair_end, gauss ? 1 : p64_tile_edge(npairs));
+  const size_t part = gauss ? 0 : (size_t)L.tiles.ntiles * L.tiles.R * m * m;
   const size_t fwd = (size_t)L.nsplit * C * k * D, bwd = (size_t)L.csplit * k * D;
   size_t o = 0;
   L.F = o;        o += al<double>((size_t)k * D);
   L.inv_norm = o; o += al<double>(k);
   L.T = o;        o += al<double>((size_t)C * k * D);
   L.Mu = o;       o += al<double>((size_t)C * k);
-  L.W = o;        o += al<double>((size_t)C * 2 * m * m);
+  L.W = o;        o += al<double>(gauss ? (size_t)C * k * k : (size_t)C * 2 * m * m);
+  L.logdet = o;   o += ld ? al<double>(C) : 0;
+  L.sinv = o;     o += ld ? al<double>((size_t)C * k * k) : 0;
   L.gPsi = o;     o += al<double>((size_t)C * k * k);
   L.gMu = o;      o += al<double>((size_t)C * k);
-  L.ticket = o;   o += al<double>(1);  // uint32 arrival ticket of closure_finish_kernel
+  L.ticket = o;   o += al<double>(1);  // uint32 arrival ticket of closure_finish_kernel; int32 [2, 4): gauss class flag
   L.proj = o;     o += al<double>(fwd > bwd ? fwd : bwd);  // row-split partials of T, later the class-split partials of dF
   L.psipart = o;  o += al<double>((size_t)C * L.nchunk * k * k);
   L.mupart = o;   o += al<double>((size_t)C * L.nchunk * k);
   L.rowpart = o;  o += al<double>(part);
   L.colpart = o;  o += al<double>(part);
-  L.losspart = o; o += al<double>((size_t)2 * L.tiles.ntiles);
+  L.losspart = o; o += gauss ? 0 : al<double>((size_t)2 * L.tiles.ntiles);
+  L.pair = o;     o += gauss ? al<double>(gauss_closure_workspace_elems(C, k, pair_begin, pair_end)) : 0;
   L.total = o;
   return L;
 }
@@ -453,6 +465,38 @@ cudaError_t run_project64_k(const double* S, const double* F, int C, int D, int 
   return run_project64<32, VEC>(S, F, C, D, k, L, part, st);
 }
 
+// The front of both float64 closures: the sphere constraint (F = W / |W| into the workspace; *F_out is the
+// filters the rest reads), the ticket memset, the streaming pass over S and the per-chunk partials of Psi_c and,
+// with M, mu'_c.
+cudaError_t closure64_front(const double* S, const double* M, const double* raw_filters, int C, int D, int k,
+                            int sphere, const Closure64Layout& L, double* ws, const double** F_out, cudaStream_t st) {
+  cudaError_t e;
+  const double* F = raw_filters;
+  if (sphere) {
+    if ((e = launch_constraint_fwd(raw_filters, D, k, ws + L.F, ws + L.inv_norm, st)) != cudaSuccess) return e;
+    F = ws + L.F;
+  }
+  *F_out = F;
+  if ((e = cudaMemsetAsync(ws + L.ticket, 0, sizeof(unsigned int), st)) != cudaSuccess) return e;
+  // 16-byte loads of S when every row starts 16-byte aligned
+  const bool vec2 = (D % 2 == 0) && (reinterpret_cast<uintptr_t>(S) & 15) == 0;
+  e = vec2 ? run_project64_k<2>(S, F, C, D, k, L, ws + L.proj, st) : run_project64_k<1>(S, F, C, D, k, L, ws + L.proj, st);
+  if (e != cudaSuccess) return e;
+  project64_finish_kernel<<<dim3(L.nchunk, C), PF64_COLS, 0, st>>>(ws + L.proj, F, M, C, D, k, L.nsplit, ws + L.T,
+                                                                   ws + L.psipart, ws + L.mupart);
+  return cudaGetLastError();
+}
+
+// The back of both float64 closures: the projection adjoint with gMu when M is given, the constraint's adjoint,
+// the frozen rows, max |grad| and the published out.
+cudaError_t closure64_back(const double* M, int C, int D, int k, const double* F, int sphere, int n_fixed,
+                           const Closure64Layout& L, double* out, double* out_host, double* grad, double* ws,
+                           cudaStream_t st) {
+  return launch_project_bwd_constrained(ws + L.gPsi, M != nullptr ? ws + L.gMu : nullptr, ws + L.T, M, C, D, k, F,
+                                        ws + L.inv_norm, sphere, n_fixed, grad, out, out_host,
+                                        reinterpret_cast<unsigned int*>(ws + L.ticket), ws + L.proj, st);
+}
+
 }  // namespace
 
 size_t fused_loss_workspace_bytes_f64(int C, int D, int k, int dist, int64_t pair_begin, int64_t pair_end) {
@@ -468,23 +512,11 @@ cudaError_t launch_closure_f64(const double* S, const double* M, const double* r
   const Closure64Layout L = closure64_layout(C, D, k, dist, pair_begin, pair_end);
   const int sphere = constraint == 1 ? 1 : 0;
   const double* Mfr = fr ? M : nullptr;
-  unsigned int* ticket = reinterpret_cast<unsigned int*>(ws + L.ticket);
   const int64_t P = (int64_t)C * (C - 1) / 2;
   const double weight = -1.0 / (double)(P > 0 ? P : 1);
+  const double* F;
   cudaError_t e;
-  const double* F = raw_filters;
-  if (sphere) {
-    if ((e = launch_constraint_fwd(raw_filters, D, k, ws + L.F, ws + L.inv_norm, st)) != cudaSuccess) return e;
-    F = ws + L.F;
-  }
-  if ((e = cudaMemsetAsync(ticket, 0, sizeof(unsigned int), st)) != cudaSuccess) return e;
-  // 16-byte loads of S when every row starts 16-byte aligned
-  const bool vec2 = (D % 2 == 0) && (reinterpret_cast<uintptr_t>(S) & 15) == 0;
-  e = vec2 ? run_project64_k<2>(S, F, C, D, k, L, ws + L.proj, st) : run_project64_k<1>(S, F, C, D, k, L, ws + L.proj, st);
-  if (e != cudaSuccess) return e;
-  project64_finish_kernel<<<dim3(L.nchunk, C), PF64_COLS, 0, st>>>(ws + L.proj, F, Mfr, C, D, k, L.nsplit, ws + L.T,
-                                                                   ws + L.psipart, ws + L.mupart);
-  if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  if ((e = closure64_front(S, Mfr, raw_filters, C, D, k, sphere, L, ws, &F, st)) != cudaSuccess) return e;
   {
     const int per_warp = class64_smem_doubles(m, k) * (int)sizeof(double);
     const int nw = warps_for(per_warp, W64);
@@ -515,8 +547,30 @@ cudaError_t launch_closure_f64(const double* S, const double* M, const double* r
   if ((e = launch_pair_reduce_closure(L.tiles, C, m, k, fr, ws + L.rowpart, ws + L.colpart, ws + L.losspart, weight,
                                       ws + L.Mu, out, ws + L.gPsi, gMu, st)) != cudaSuccess)
     return e;
-  return launch_project_bwd_constrained(ws + L.gPsi, gMu, ws + L.T, Mfr, C, D, k, F, ws + L.inv_norm, sphere, n_fixed,
-                                        grad, out, out_host, ticket, ws + L.proj, st);
+  return closure64_back(Mfr, C, D, k, F, sphere, n_fixed, L, out, out_host, grad, ws, st);
+}
+
+// The mean-covariance distances (Mahalanobis, Bhattacharyya, Hellinger) in float64: the front above, the class,
+// pair and reduce stages of gauss.cu instantiated for double, and the back with gMu.
+cudaError_t launch_gauss_closure_f64(const double* S, const double* M, const double* raw_filters, int C, int D, int k,
+                                     const double* noise, int dist, int constraint, int n_fixed, int64_t pair_begin,
+                                     int64_t pair_end, double* out, double* out_host, double* grad, double* ws,
+                                     cudaStream_t st) {
+  const Closure64Layout L = closure64_layout(C, D, k, dist, pair_begin, pair_end);
+  const int sphere = constraint == 1 ? 1 : 0;
+  const int64_t P = (int64_t)C * (C - 1) / 2;
+  const double weight = -1.0 / (double)(P > 0 ? P : 1);
+  const double* F;
+  cudaError_t e;
+  if ((e = closure64_front(S, M, raw_filters, C, D, k, sphere, L, ws, &F, st)) != cudaSuccess) return e;
+  int32_t* flag = reinterpret_cast<int32_t*>(ws + L.ticket) + 2;
+  if ((e = launch_gauss_closure_class(ws + L.psipart, ws + L.mupart, L.nchunk, noise, C, k, dist, ws + L.W, ws + L.Mu,
+                                      ws + L.logdet, ws + L.sinv, flag, st)) != cudaSuccess)
+    return e;
+  if ((e = launch_gauss_closure_pairs(ws + L.W, ws + L.Mu, ws + L.logdet, ws + L.sinv, C, k, dist, pair_begin,
+                                      pair_end, weight, out, ws + L.gPsi, ws + L.gMu, ws + L.pair, st)) != cudaSuccess)
+    return e;
+  return closure64_back(M, C, D, k, F, sphere, n_fixed, L, out, out_host, grad, ws, st);
 }
 
 }  // namespace sqfa

@@ -11,6 +11,7 @@
 // Per-pair gradient partials are stored and summed per class in a fixed order (no float atomics).
 // The second half of this file is the fitting closure of these distances (SQFA_DIST_MAHALANOBIS / BHATTACHARYYA /
 // HELLINGER): strict lower triangle only, the scalar map inside, tile partials instead of per-pair ones.
+#include <cfloat>
 #include <cstdint>
 #include <cuda_runtime.h>
 
@@ -29,18 +30,19 @@ __device__ __forceinline__ float gp_warp_sum(float v) {
   return v;
 }
 
-// in-place lower Cholesky of the k x k matrix M (row stride ld), one warp; returns logdet, sets ok
-__device__ float gp_cholesky(float* M, int k, int ld, int lane, bool& ok) {
-  float logdet = 0.f;
+// in-place lower Cholesky of the k x k matrix M (row stride ld), one warp; returns logdet, sets ok. T = float, double.
+template <typename T>
+__device__ T gp_cholesky(T* M, int k, int ld, int lane, bool& ok) {
+  T logdet = T(0);
   for (int j = 0; j < k; ++j) {
-    float d = M[j * ld + j];
+    T d = M[j * ld + j];
     for (int q = 0; q < j; ++q) d -= M[j * ld + q] * M[j * ld + q];
-    if (!(d > 0.f) || !isfinite(d)) ok = false;
-    const float ljj = sqrtf(d);
-    logdet += 2.f * logf(ljj);
+    if (!(d > T(0)) || !isfinite(d)) ok = false;
+    const T ljj = sqrt(d);
+    logdet += T(2) * log(ljj);
     __syncwarp();
     for (int i = j + 1 + lane; i < k; i += 32) {
-      float v = M[i * ld + j];
+      T v = M[i * ld + j];
       for (int q = 0; q < j; ++q) v -= M[i * ld + q] * M[j * ld + q];
       M[i * ld + j] = v / ljj;
     }
@@ -51,30 +53,33 @@ __device__ float gp_cholesky(float* M, int k, int ld, int lane, bool& ok) {
 }
 
 // Linv (row stride ld) = L^-1 for lower triangular L, one column per lane
-__device__ void gp_tri_inverse(const float* L, float* Li, int k, int ld, int lane) {
+template <typename T>
+__device__ void gp_tri_inverse(const T* L, T* Li, int k, int ld, int lane) {
   for (int c = lane; c < k; c += 32) {
     for (int i = 0; i < k; ++i) {
-      float s = (i == c) ? 1.f : 0.f;
+      T s = (i == c) ? T(1) : T(0);
       for (int q = c; q < i; ++q) s -= L[i * ld + q] * Li[q * ld + c];
-      Li[i * ld + c] = (i < c) ? 0.f : s / L[i * ld + i];
+      Li[i * ld + c] = (i < c) ? T(0) : s / L[i * ld + i];
     }
   }
   __syncwarp();
 }
 
 // logdet of the k x k SPD matrix staged in L (row stride ld) and, if Sinv_c != NULL, its inverse L^-T L^-1;
-// one warp, Li is scratch. A failed Cholesky sets *flag and leaves a NaN or -inf logdet.
-__device__ __forceinline__ void gp_logdet_inverse(float* L, float* Li, int k, int ld, int lane, float* logdet_c,
-                                                  float* Sinv_c, int32_t* flag) {
+// one warp, Li is scratch. A failed Cholesky sets *flag. In float32 the logdet is left as the factorisation made
+// it (NaN, or +-inf for a zero or infinite pivot); in float64 it is NaN, so every distance of the class is NaN.
+template <typename T>
+__device__ __forceinline__ void gp_logdet_inverse(T* L, T* Li, int k, int ld, int lane, T* logdet_c, T* Sinv_c,
+                                                  int32_t* flag) {
   bool ok = true;
-  const float ldv = gp_cholesky(L, k, ld, lane, ok);
+  const T ldv = gp_cholesky(L, k, ld, lane, ok);
   if (!ok && lane == 0) atomicOr(flag, 1);
-  if (lane == 0) *logdet_c = ldv;
+  if (lane == 0) *logdet_c = (ok || sizeof(T) == sizeof(float)) ? ldv : T(NAN);
   if (Sinv_c != nullptr) {
     gp_tri_inverse(L, Li, k, ld, lane);
     for (int idx = lane; idx < k * k; idx += 32) {  // Sigma^-1 = L^-T L^-1
       const int r = idx / k, s = idx % k;
-      float a = 0.f;
+      T a = T(0);
       for (int q = (r > s ? r : s); q < k; ++q) a += Li[q * ld + r] * Li[q * ld + s];
       Sinv_c[idx] = a;
     }
@@ -221,51 +226,65 @@ gauss_reduce_kernel(const float* __restrict__ rowpart, const float* __restrict__
 // Per pair, with g = weight * d'(x or B) and (c_m, c_l) = (1, 0) for Mahalanobis, (1/8, 1/2) otherwise:
 //   dL/dPsi_i = dL/dPsi_j = g (-c_m / 2 u u^T + c_l / 2 M^-1),   dL/dmu'_i = -dL/dmu'_j = 2 c_m g u,
 // and the class term -1/4 Psi_c^-1 sum_o g(c, o) of the logdet Psi_c in B is added once per class.
+// The three kernels are templates on the scalar type: float for the float32 closure (closure.cu), double for
+// the float64 one (closure64.cu, launch_gauss_closure_f64; DESIGN.md section 19).
 // ------------------------------------------------------------------------------------------------
 constexpr int GC_WARPS = 4;
-constexpr float GC_EPS = 1e-6f;  // distances.py:29 EPSILON
+constexpr double GC_EPS = 1e-6;  // distances.py:29 EPSILON
 
-// floats of one class slot of a tile partial: [dL/dPsi (k*k) | dL/dmu' (k) | sum of g]
+// elements of one class slot of a tile partial: [dL/dPsi (k*k) | dL/dmu' (k) | sum of g]
 __host__ __device__ inline int gc_slot_floats(int k) { return k * k + k + 1; }
 
+// The closure's kernels are templates on the scalar type T = float, double. The float64 closure reads the noise
+// from one device double (a captured graph picks up a new value), the float32 closure takes it by value.
+__device__ __forceinline__ float gc_noise(float noise) { return noise; }
+__device__ __forceinline__ double gc_noise(const double* noise) { return *noise; }
+__device__ __forceinline__ float gc_nan(float) { return __int_as_float(0x7fffffff); }
+__device__ __forceinline__ double gc_nan(double) { return __longlong_as_double(0x7fffffffffffffffll); }
+__device__ __forceinline__ float gc_max(float) { return FLT_MAX; }
+__device__ __forceinline__ double gc_max(double) { return DBL_MAX; }
+
+template <typename Real>
 struct GaussClosureArgs {
-  const float* Psi;     // [C][k][k]
-  const float* Mu;      // [C][k]
-  const float* logdet;  // [C] (Bhattacharyya / Hellinger)
+  const Real* Psi;     // [C][k][k]
+  const Real* Mu;      // [C][k]
+  const Real* logdet;  // [C] (Bhattacharyya / Hellinger)
   int C, k, dist, Q;    // a tile row is processed as Q batches of 32 / G pairs
   int64_t pair_begin, pair_end;
-  float weight;
+  Real weight;
   PairTiles T;
-  float* rowpart;   // [ntiles][R][slot]
-  float* colpart;   // [ntiles][R][slot]
-  float* losspart;  // [ntiles][2] {sum of distances, non-finite count}
+  Real* rowpart;   // [ntiles][R][slot]
+  Real* colpart;   // [ntiles][R][slot]
+  Real* losspart;  // [ntiles][2] {sum of distances, non-finite count}
 };
 
-template <int G>
-__device__ __forceinline__ float gc_group_sum(float v) {
+template <int G, typename T>
+__device__ __forceinline__ T gc_group_sum(T v) {
 #pragma unroll
   for (int o = G / 2; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
 }
 
+template <typename T, typename Noise>
 __global__ void __launch_bounds__(GP_WARPS * 32)
-gauss_closure_class_kernel(const float* __restrict__ PsiPart, const float* __restrict__ MuPart, int nchunk, float noise,
-                           int C, int k, int want_logdet, float* __restrict__ Psi, float* __restrict__ Mu,
-                           float* __restrict__ logdet, float* __restrict__ Sinv, int32_t* __restrict__ flag) {
-  extern __shared__ float sm[];
+gauss_closure_class_kernel(const T* __restrict__ PsiPart, const T* __restrict__ MuPart, int nchunk, Noise noise_arg,
+                           int C, int k, int want_logdet, T* __restrict__ Psi, T* __restrict__ Mu,
+                           T* __restrict__ logdet, T* __restrict__ Sinv, int32_t* __restrict__ flag) {
+  extern __shared__ __align__(16) unsigned char gc_class_smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int c = blockIdx.x * GP_WARPS + warp;
   if (c >= C) return;
+  const T noise = gc_noise(noise_arg);
   const int ld = k + 1;
-  float* L = sm + (size_t)warp * 2 * k * ld;
-  float* Li = L + k * ld;
+  T* L = reinterpret_cast<T*>(gc_class_smem) + (size_t)warp * 2 * k * ld;
+  T* Li = L + k * ld;
   for (int r = lane; r < k; r += 32) {  // chunks added in order, as class_prepare does
-    float a = 0.f;
+    T a = T(0);
     for (int ch = 0; ch < nchunk; ++ch) a += MuPart[((int64_t)c * nchunk + ch) * k + r];
     Mu[(int64_t)c * k + r] = a;
   }
   for (int idx = lane; idx < k * k; idx += 32) {
-    float v = 0.f;
+    T v = T(0);
     for (int ch = 0; ch < nchunk; ++ch) v += PsiPart[((int64_t)c * nchunk + ch) * k * k + idx];
     if (idx / k == idx % k) v += noise;
     Psi[(int64_t)c * k * k + idx] = v;
@@ -276,11 +295,39 @@ gauss_closure_class_kernel(const float* __restrict__ PsiPart, const float* __res
   gp_logdet_inverse(L, Li, k, ld, lane, logdet + c, Sinv + (int64_t)c * k * k, flag);
 }
 
-template <int G>
+// Where a lane keeps its row-slot accumulator racc[G + 2]: registers, or for double at G = 32 (where M's row
+// alone takes 64 registers) a [G + 2][32] block of shared memory after the warp's column accumulators, one
+// column per lane like colacc.
+template <typename T, int G>
+struct GcRowAcc {
+  static constexpr bool in_smem = sizeof(T) == 8 && G == 32;
+};
+
+template <typename T, int G>
+__host__ __device__ inline int gc_pair_smem_elems(int Q) {
+  return (Q + (GcRowAcc<T, G>::in_smem ? 1 : 0)) * (G + 2) * 32;
+}
+
+template <typename T, int G, bool SMEM>
+struct GcRowSlot;
+template <typename T, int G>
+struct GcRowSlot<T, G, false> {
+  T v[G + 2];
+  __device__ __forceinline__ GcRowSlot(T*, int, int) {}
+  __device__ __forceinline__ T& operator[](int e) { return v[e]; }
+};
+template <typename T, int G>
+struct GcRowSlot<T, G, true> {
+  T* p;
+  __device__ __forceinline__ GcRowSlot(T* colacc, int Q, int lane) : p(colacc + Q * (G + 2) * 32 + lane) {}
+  __device__ __forceinline__ T& operator[](int e) { return p[e * 32]; }
+};
+
+template <typename T, int G>
 __global__ void __launch_bounds__(GC_WARPS * 32)
-gauss_closure_pair_kernel(const GaussClosureArgs A) {
+gauss_closure_pair_kernel(const GaussClosureArgs<T> A) {
   constexpr int NP = 32 / G;  // pairs side by side in a warp
-  extern __shared__ float gc_smem[];
+  extern __shared__ __align__(16) unsigned char gc_pair_smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t t = (int64_t)blockIdx.x * GC_WARPS + warp;
   if (t >= A.T.ntiles) return;
@@ -288,84 +335,85 @@ gauss_closure_pair_kernel(const GaussClosureArgs A) {
   const int k = A.k, Q = A.Q, R = A.T.R, base = A.dist & 15;
   const int per = gc_slot_floats(k);
   const bool bhat = base != SQFA_DIST_MAHALANOBIS;
-  const float cm = bhat ? 0.125f : 1.f, cl = bhat ? 0.5f : 0.f;
+  const T cm = bhat ? T(0.125) : T(1), cl = bhat ? T(0.5) : T(0);
   // column-slot accumulators [Q][G + 2][32]: every lane owns its own column, so no synchronisation
-  float* colacc = gc_smem + (size_t)warp * Q * (G + 2) * 32;
-  for (int e = 0; e < Q * (G + 2); ++e) colacc[e * 32 + lane] = 0.f;
+  constexpr int QR = GcRowAcc<T, G>::in_smem ? 1 : 0;  // batches of column slots that hold the row slot
+  T* colacc = reinterpret_cast<T*>(gc_pair_smem) + (size_t)warp * (Q + QR) * (G + 2) * 32;
+  for (int e = 0; e < Q * (G + 2); ++e) colacc[e * 32 + lane] = T(0);
   int bi, bj;
   decode_tile(A.T, t, bi, bj);
-  float dsum = 0.f, nbad = 0.f;
+  T dsum = T(0), nbad = T(0);
   for (int ii = 0; ii < R; ++ii) {
     const int i = bi * R + ii;
-    float racc[G + 2];
+    GcRowSlot<T, G, GcRowAcc<T, G>::in_smem> racc(colacc, Q, lane);
 #pragma unroll
-    for (int e = 0; e < G + 2; ++e) racc[e] = 0.f;
+    for (int e = 0; e < G + 2; ++e) racc[e] = T(0);
     for (int q = 0; q < Q; ++q) {
       const int j = bj * R + q * NP + grp;
       const bool valid = pair_in_launch(i, j, A.C, A.C, 1, A.pair_begin, A.pair_end);
       const bool live = valid && r < k;
-      float Mr[G];
-      const float* pi = A.Psi + ((int64_t)i * k + r) * k;
-      const float* pj = A.Psi + ((int64_t)j * k + r) * k;
+      T Mr[G];
+      const T* pi = A.Psi + ((int64_t)i * k + r) * k;
+      const T* pj = A.Psi + ((int64_t)j * k + r) * k;
 #pragma unroll
-      for (int l = 0; l < G; ++l) Mr[l] = (live && l < k) ? 0.5f * (pi[l] + pj[l]) : (l == r ? 1.f : 0.f);
-      const float dv = live ? A.Mu[(int64_t)i * k + r] - A.Mu[(int64_t)j * k + r] : 0.f;
+      for (int l = 0; l < G; ++l) Mr[l] = (live && l < k) ? T(0.5) * (pi[l] + pj[l]) : (l == r ? T(1) : T(0));
+      const T dv = live ? A.Mu[(int64_t)i * k + r] - A.Mu[(int64_t)j * k + r] : T(0);
       // Gauss-Jordan: after step p the rows hold [M^-1 of the leading p x p block | eliminated rest]
-      float mypiv = 1.f;
+      T mypiv = T(1);
 #pragma unroll
       for (int p = 0; p < G; ++p) {
-        const float piv = __shfl_sync(0xffffffffu, Mr[p], p, G);
-        const float pinv = 1.f / piv;
-        const float f = Mr[p];
+        const T piv = __shfl_sync(0xffffffffu, Mr[p], p, G);
+        const T pinv = T(1) / piv;
+        const T f = Mr[p];
         const bool prow = r == p;
         if (prow) mypiv = piv;
 #pragma unroll
         for (int l = 0; l < G; ++l) {
-          const float pl = __shfl_sync(0xffffffffu, Mr[l], p, G) * pinv;
+          const T pl = __shfl_sync(0xffffffffu, Mr[l], p, G) * pinv;
           if (l == p) Mr[l] = prow ? pinv : -f * pinv;
-          else Mr[l] = prow ? pl : fmaf(-f, pl, Mr[l]);
+          else Mr[l] = prow ? pl : fma(-f, pl, Mr[l]);
         }
       }
-      float u = 0.f;  // u_r = (M^-1 d)_r
+      T u = T(0);  // u_r = (M^-1 d)_r
 #pragma unroll
-      for (int l = 0; l < G; ++l) u = fmaf(Mr[l], __shfl_sync(0xffffffffu, dv, l, G), u);
-      const float x = gc_group_sum<G>(dv * u);
-      const bool pos = mypiv > 0.f && mypiv <= 3.402823466e38f;
-      const bool ok = gc_group_sum<G>(pos ? 0.f : 1.f) == 0.f;
-      float pre = x;
+      for (int l = 0; l < G; ++l) u = fma(Mr[l], __shfl_sync(0xffffffffu, dv, l, G), u);
+      const T x = gc_group_sum<G>(dv * u);
+      const bool pos = mypiv > T(0) && mypiv <= gc_max(T(0));
+      const bool ok = gc_group_sum<G>(pos ? T(0) : T(1)) == T(0);
+      T pre = x;
       if (bhat) {
-        const float ldM = gc_group_sum<G>(logf(mypiv));  // padded rows: log 1 = 0
-        pre = valid ? 0.125f * x + 0.5f * (ldM - 0.5f * (A.logdet[i] + A.logdet[j])) : 0.f;
+        const T ldM = gc_group_sum<G>(log(mypiv));  // padded rows: log 1 = 0
+        pre = valid ? T(0.125) * x + T(0.5) * (ldM - T(0.5) * (A.logdet[i] + A.logdet[j])) : T(0);
       }
-      if (!ok) pre = __int_as_float(0x7fffffff);
-      float dval, dmap;  // distance and its derivative w.r.t. x (Mahalanobis) or B
+      if (!ok) pre = gc_nan(T(0));
+      T dval, dmap;  // distance and its derivative w.r.t. x (Mahalanobis) or B
       if (base == SQFA_DIST_HELLINGER) {
-        const float e = expf(-pre);
-        dval = sqrtf(1.f - e + GC_EPS);
-        dmap = 0.5f * e / dval;
+        const T e = exp(-pre);
+        dval = sqrt(T(1) - e + T(GC_EPS));
+        dmap = T(0.5) * e / dval;
       } else if (base == SQFA_DIST_MAHALANOBIS && !(A.dist & SQFA_DIST_SQUARED)) {
-        dval = sqrtf(pre + GC_EPS);
-        dmap = 0.5f / dval;
+        dval = sqrt(pre + T(GC_EPS));
+        dmap = T(0.5) / dval;
       } else {
         dval = pre;
-        dmap = 1.f;
+        dmap = T(1);
       }
-      const float g = valid ? A.weight * dmap : 0.f;
+      const T g = valid ? A.weight * dmap : T(0);
       if (valid && r == 0) {
         dsum += dval;
-        if (!isfinite(dval)) nbad += 1.f;
+        if (!isfinite(dval)) nbad += T(1);
       }
-      const float gu = g * u;
-      float* ca = colacc + q * (G + 2) * 32 + lane;
+      const T gu = g * u;
+      T* ca = colacc + q * (G + 2) * 32 + lane;
 #pragma unroll
       for (int l = 0; l < G; ++l) {
-        const float ul = __shfl_sync(0xffffffffu, u, l, G);
-        const float v = fmaf(0.5f * cl * g, Mr[l], -0.5f * cm * gu * ul);
+        const T ul = __shfl_sync(0xffffffffu, u, l, G);
+        const T v = fma(T(0.5) * cl * g, Mr[l], T(-0.5) * cm * gu * ul);
         racc[l] += v;
         ca[l * 32] += v;
       }
-      racc[G] += 2.f * cm * gu;
-      ca[G * 32] -= 2.f * cm * gu;
+      racc[G] += T(2) * cm * gu;
+      ca[G * 32] -= T(2) * cm * gu;
       racc[G + 1] += g;
       ca[(G + 1) * 32] += g;
     }
@@ -375,7 +423,7 @@ gauss_closure_pair_kernel(const GaussClosureArgs A) {
 #pragma unroll
       for (int o = G; o < 32; o <<= 1) racc[e] += __shfl_xor_sync(0xffffffffu, racc[e], o);
     if (grp == 0 && r < k) {
-      float* rp = A.rowpart + (t * R + ii) * per;
+      T* rp = A.rowpart + (t * R + ii) * per;
 #pragma unroll
       for (int l = 0; l < G; ++l)
         if (l < k) rp[r * k + l] = racc[l];
@@ -385,15 +433,15 @@ gauss_closure_pair_kernel(const GaussClosureArgs A) {
   }
   if (r < k) {
     for (int q = 0; q < Q; ++q) {
-      float* cp = A.colpart + (t * R + q * NP + grp) * per;
-      const float* ca = colacc + q * (G + 2) * 32 + lane;
+      T* cp = A.colpart + (t * R + q * NP + grp) * per;
+      const T* ca = colacc + q * (G + 2) * 32 + lane;
       for (int l = 0; l < k; ++l) cp[r * k + l] = ca[l * 32];
       cp[k * k + r] = ca[G * 32];
       if (r == 0) cp[k * k + k] = ca[(G + 1) * 32];
     }
   }
-  dsum = gp_warp_sum(dsum);
-  nbad = gp_warp_sum(nbad);
+  dsum = warp_sum(dsum);
+  nbad = warp_sum(nbad);
   if (lane == 0) {
     A.losspart[2 * t] = dsum;
     A.losspart[2 * t + 1] = nbad;
@@ -403,43 +451,45 @@ gauss_closure_pair_kernel(const GaussClosureArgs A) {
 // Per class c (blocks 0 .. C - 1): the slot partials of the tiles of its block row (ascending block column)
 // and block column (ascending block row) -> gPsi[c] (+ the logdet class term), gMu[c]. Block C: out =
 // {weight * sum d, #non-finite, 0} from the loss partials. Fixed order throughout.
+template <typename T>
 __global__ void __launch_bounds__(1024)
-gauss_closure_reduce_kernel(const PairTiles T, int C, int k, int dist, const float* __restrict__ rowpart,
-                            const float* __restrict__ colpart, const float* __restrict__ losspart,
-                            const float* __restrict__ Sinv, float weight, float* __restrict__ out,
-                            float* __restrict__ gPsi, float* __restrict__ gMu) {
-  extern __shared__ float sg[];  // the reduced slot of this class
+gauss_closure_reduce_kernel(const PairTiles Tl, int C, int k, int dist, const T* __restrict__ rowpart,
+                            const T* __restrict__ colpart, const T* __restrict__ losspart,
+                            const T* __restrict__ Sinv, T weight, T* __restrict__ out,
+                            T* __restrict__ gPsi, T* __restrict__ gMu) {
+  extern __shared__ __align__(16) unsigned char gc_reduce_smem[];
+  T* sg = reinterpret_cast<T*>(gc_reduce_smem);  // the reduced slot of this class
   const int c = blockIdx.x;
   if (c == C) {
-    float sum, bad;
-    reduce_loss_partials(losspart, T.ntiles, sum, bad);
+    T sum, bad;
+    reduce_loss_partials(losspart, Tl.ntiles, sum, bad);
     if (threadIdx.x == 0) {
       out[0] = weight * sum;
       out[1] = bad;
-      out[2] = 0.f;  // max |grad|, filled by closure_finish_kernel
+      out[2] = T(0);  // max |grad|, filled by closure_finish_kernel
     }
     return;
   }
-  const int per = gc_slot_floats(k), R = T.R, slot = c % R, bc = c / R;
+  const int per = gc_slot_floats(k), R = Tl.R, slot = c % R, bc = c / R;
   const int64_t pstride = (int64_t)R * per;
   for (int e = threadIdx.x; e < per; e += blockDim.x) {
-    float a = 0.f, b = 0.f;
-    if (bc >= T.bi0 && bc <= T.bi1) {  // row side: tiles (bc, 0 .. bc)
-      const float* p = rowpart + ((int64_t)bc * (bc + 1) / 2 - T.tile0) * pstride + (int64_t)slot * per + e;
+    T a = T(0), b = T(0);
+    if (bc >= Tl.bi0 && bc <= Tl.bi1) {  // row side: tiles (bc, 0 .. bc)
+      const T* p = rowpart + ((int64_t)bc * (bc + 1) / 2 - Tl.tile0) * pstride + (int64_t)slot * per + e;
 #pragma unroll 4
       for (int bj = 0; bj <= bc; ++bj) a += p[bj * pstride];
     }
-    const int i0 = max(T.bi0, bc);  // column side: tiles (i0 .. bi1, bc)
+    const int i0 = max(Tl.bi0, bc);  // column side: tiles (i0 .. bi1, bc)
 #pragma unroll 4
-    for (int bi = i0; bi <= T.bi1; ++bi)
-      b += colpart[((int64_t)bi * (bi + 1) / 2 + bc - T.tile0) * pstride + (int64_t)slot * per + e];
+    for (int bi = i0; bi <= Tl.bi1; ++bi)
+      b += colpart[((int64_t)bi * (bi + 1) / 2 + bc - Tl.tile0) * pstride + (int64_t)slot * per + e];
     sg[e] = a + b;
   }
   __syncthreads();
   const bool bhat = gauss_closure_needs_logdet(dist);
-  const float gsum = sg[k * k + k];
+  const T gsum = sg[k * k + k];
   for (int e = threadIdx.x; e < k * k + k; e += blockDim.x) {
-    if (e < k * k) gPsi[(int64_t)c * k * k + e] = bhat ? sg[e] - 0.25f * gsum * Sinv[(int64_t)c * k * k + e] : sg[e];
+    if (e < k * k) gPsi[(int64_t)c * k * k + e] = bhat ? sg[e] - T(0.25) * gsum * Sinv[(int64_t)c * k * k + e] : sg[e];
     else gMu[(int64_t)c * k + e - k * k] = sg[e];
   }
 }
@@ -518,8 +568,9 @@ cudaError_t launch_gauss_pairs(const float* muA, const float* SigA, const float*
 
 // ---- fitting closure of the mean-covariance distances ----
 // group width G and tile edge R = (32 / G) Q: Q grows with the pair count while tiles stay plentiful, up to
-// R = 16 / 8 / 4 at G <= 8 / 16 / 32, so that the partials (2 R (k^2 + k + 1) floats per tile of R^2 pairs) stay
-// below the affine-invariant closure's
+// R = 16 / 8 / 4 at G <= 8 / 16 / 32, so that the partials (2 R (k^2 + k + 1) elements per tile of R^2 pairs) stay
+// below the affine-invariant closure's. The float64 closure keeps the rule: its largest block, 4 warps at G = 32 and
+// Q = 4, takes 170 KB of shared memory (gc_pair_smem_elems).
 static int gc_group(int k) {
   int G = 2;
   while (G < k) G *= 2;
@@ -554,37 +605,52 @@ static GcWorkspace gc_workspace(int C, int k, int64_t pair_begin, int64_t pair_e
   return w;
 }
 
-size_t gauss_closure_workspace_floats(int C, int k, int64_t pair_begin, int64_t pair_end) {
+size_t gauss_closure_workspace_elems(int C, int k, int64_t pair_begin, int64_t pair_end) {
   return gc_workspace(C, k, pair_begin, pair_end).total_floats;
+}
+
+template <typename T, typename Noise>
+static cudaError_t launch_gc_class(const T* PsiPart, const T* MuPart, int nchunk, Noise noise, int C, int k, int dist,
+                                   T* Psi, T* Mu, T* logdet, T* Sinv, int32_t* flag, cudaStream_t st) {
+  cudaError_t e = cudaMemsetAsync(flag, 0, 2 * sizeof(int32_t), st);  // flag[1]: closure_finish's arrival ticket
+  if (e != cudaSuccess || C <= 0) return e;
+  const int smem = GP_WARPS * 2 * k * (k + 1) * (int)sizeof(T);
+  static int smem_set[kMaxDevices] = {0};
+  if ((e = ensure_dynamic_smem(gauss_closure_class_kernel<T, Noise>, smem, smem_set)) != cudaSuccess) return e;
+  gauss_closure_class_kernel<T, Noise><<<(C + GP_WARPS - 1) / GP_WARPS, GP_WARPS * 32, smem, st>>>(
+      PsiPart, MuPart, nchunk, noise, C, k, gauss_closure_needs_logdet(dist) ? 1 : 0, Psi, Mu, logdet, Sinv, flag);
+  return cudaGetLastError();
 }
 
 cudaError_t launch_gauss_closure_class(const float* PsiPart, const float* MuPart, int nchunk, float noise, int C, int k,
                                        int dist, float* Psi, float* Mu, float* logdet, float* Sinv, int32_t* flag,
                                        cudaStream_t st) {
-  cudaError_t e = cudaMemsetAsync(flag, 0, 2 * sizeof(int32_t), st);  // flag[1]: closure_finish's arrival ticket
-  if (e != cudaSuccess || C <= 0) return e;
-  const int smem = GP_WARPS * 2 * k * (k + 1) * (int)sizeof(float);
-  gauss_closure_class_kernel<<<(C + GP_WARPS - 1) / GP_WARPS, GP_WARPS * 32, smem, st>>>(
-      PsiPart, MuPart, nchunk, noise, C, k, gauss_closure_needs_logdet(dist) ? 1 : 0, Psi, Mu, logdet, Sinv, flag);
-  return cudaGetLastError();
+  return launch_gc_class(PsiPart, MuPart, nchunk, noise, C, k, dist, Psi, Mu, logdet, Sinv, flag, st);
 }
 
-template <int G>
-static cudaError_t launch_gc_pair(const GaussClosureArgs& A, cudaStream_t st) {
-  const int smem = GC_WARPS * A.Q * (G + 2) * 32 * (int)sizeof(float);
+cudaError_t launch_gauss_closure_class(const double* PsiPart, const double* MuPart, int nchunk, const double* noise,
+                                       int C, int k, int dist, double* Psi, double* Mu, double* logdet, double* Sinv,
+                                       int32_t* flag, cudaStream_t st) {
+  return launch_gc_class(PsiPart, MuPart, nchunk, noise, C, k, dist, Psi, Mu, logdet, Sinv, flag, st);
+}
+
+template <typename T, int G>
+static cudaError_t launch_gc_pair(const GaussClosureArgs<T>& A, cudaStream_t st) {
+  const int smem = GC_WARPS * gc_pair_smem_elems<T, G>(A.Q) * (int)sizeof(T);
   static int smem_set[kMaxDevices] = {0};
-  cudaError_t e = ensure_dynamic_smem(gauss_closure_pair_kernel<G>, smem, smem_set);
+  cudaError_t e = ensure_dynamic_smem(gauss_closure_pair_kernel<T, G>, smem, smem_set);
   if (e != cudaSuccess) return e;
   const unsigned blocks = (unsigned)((A.T.ntiles + GC_WARPS - 1) / GC_WARPS);
-  gauss_closure_pair_kernel<G><<<blocks, GC_WARPS * 32, smem, st>>>(A);
+  gauss_closure_pair_kernel<T, G><<<blocks, GC_WARPS * 32, smem, st>>>(A);
   return cudaGetLastError();
 }
 
-cudaError_t launch_gauss_closure_pairs(const float* Psi, const float* Mu, const float* logdet, const float* Sinv, int C,
-                                       int k, int dist, int64_t pair_begin, int64_t pair_end, float weight, float* out,
-                                       float* gPsi, float* gMu, float* ws, cudaStream_t st) {
+template <typename T>
+static cudaError_t launch_gc_pairs(const T* Psi, const T* Mu, const T* logdet, const T* Sinv, int C, int k, int dist,
+                                   int64_t pair_begin, int64_t pair_end, T weight, T* out, T* gPsi, T* gMu, T* ws,
+                                   cudaStream_t st) {
   const GcWorkspace W = gc_workspace(C, k, pair_begin, pair_end);
-  GaussClosureArgs A;
+  GaussClosureArgs<T> A;
   A.Psi = Psi; A.Mu = Mu; A.logdet = logdet;
   A.C = C; A.k = k; A.dist = dist; A.Q = W.Q;
   A.pair_begin = pair_begin; A.pair_end = pair_end; A.weight = weight; A.T = W.T;
@@ -592,11 +658,11 @@ cudaError_t launch_gauss_closure_pairs(const float* Psi, const float* Mu, const 
   cudaError_t e = cudaSuccess;
   if (W.T.ntiles > 0) {
     switch (gc_group(k)) {
-      case 2: e = launch_gc_pair<2>(A, st); break;
-      case 4: e = launch_gc_pair<4>(A, st); break;
-      case 8: e = launch_gc_pair<8>(A, st); break;
-      case 16: e = launch_gc_pair<16>(A, st); break;
-      case 32: e = launch_gc_pair<32>(A, st); break;
+      case 2: e = launch_gc_pair<T, 2>(A, st); break;
+      case 4: e = launch_gc_pair<T, 4>(A, st); break;
+      case 8: e = launch_gc_pair<T, 8>(A, st); break;
+      case 16: e = launch_gc_pair<T, 16>(A, st); break;
+      case 32: e = launch_gc_pair<T, 32>(A, st); break;
       default: return cudaErrorNotSupported;
     }
     if (e != cudaSuccess) return e;
@@ -604,9 +670,21 @@ cudaError_t launch_gauss_closure_pairs(const float* Psi, const float* Mu, const 
   const int per = gc_slot_floats(k), passes = (per + 1023) / 1024;
   int nt = (((per + passes - 1) / passes) + 31) & ~31;
   if (nt < 128) nt = 128;
-  gauss_closure_reduce_kernel<<<C + 1, nt, per * sizeof(float), st>>>(W.T, C, k, dist, A.rowpart, A.colpart,
-                                                                     A.losspart, Sinv, weight, out, gPsi, gMu);
+  gauss_closure_reduce_kernel<T><<<C + 1, nt, per * sizeof(T), st>>>(W.T, C, k, dist, A.rowpart, A.colpart, A.losspart,
+                                                                     Sinv, weight, out, gPsi, gMu);
   return cudaGetLastError();
+}
+
+cudaError_t launch_gauss_closure_pairs(const float* Psi, const float* Mu, const float* logdet, const float* Sinv, int C,
+                                       int k, int dist, int64_t pair_begin, int64_t pair_end, float weight, float* out,
+                                       float* gPsi, float* gMu, float* ws, cudaStream_t st) {
+  return launch_gc_pairs(Psi, Mu, logdet, Sinv, C, k, dist, pair_begin, pair_end, weight, out, gPsi, gMu, ws, st);
+}
+
+cudaError_t launch_gauss_closure_pairs(const double* Psi, const double* Mu, const double* logdet, const double* Sinv,
+                                       int C, int k, int dist, int64_t pair_begin, int64_t pair_end, double weight,
+                                       double* out, double* gPsi, double* gMu, double* ws, cudaStream_t st) {
+  return launch_gc_pairs(Psi, Mu, logdet, Sinv, C, k, dist, pair_begin, pair_end, weight, out, gPsi, gMu, ws, st);
 }
 
 }  // namespace sqfa

@@ -176,12 +176,17 @@ cudaError_t launch_fused_loss_sharded(int phase, const float* S, const float* M,
 cudaError_t launch_fused_loss(const float* S, const float* M, const float* filters, int C, int D, int k, float noise,
                               int dist, int constraint, int n_fixed, int64_t pair_begin, int64_t pair_end, float* out,
                               float* out_host, float* grad, float* ws, cudaStream_t st);
-// ---- closure64.cu (float64 closure: affine-invariant / Fisher-Rao lower bound, k <= 32) ----
+// ---- closure64.cu (float64 closures, k <= 32: affine-invariant / Fisher-Rao lower bound, and the mean-covariance
+// distances of gauss.cu; one workspace layout, sized by the distance code) ----
 size_t fused_loss_workspace_bytes_f64(int C, int D, int k, int dist, int64_t pair_begin, int64_t pair_end);
 cudaError_t launch_closure_f64(const double* S, const double* M, const double* raw_filters, int C, int D, int k,
                                const double* noise, int dist, int constraint, int n_fixed, int64_t pair_begin,
                                int64_t pair_end, double* out, double* out_host, double* grad, double* ws,
                                cudaStream_t st);
+cudaError_t launch_gauss_closure_f64(const double* S, const double* M, const double* raw_filters, int C, int D, int k,
+                                     const double* noise, int dist, int constraint, int n_fixed, int64_t pair_begin,
+                                     int64_t pair_end, double* out, double* out_host, double* grad, double* ws,
+                                     cudaStream_t st);
 }  // namespace sqfa
 
 
@@ -216,11 +221,19 @@ cudaError_t launch_gauss_pairs(const float* muA, const float* SigA, const float*
 // closure codes SQFA_DIST_MAHALANOBIS / BHATTACHARYYA / HELLINGER
 __host__ __device__ inline bool is_gauss_closure(int dist) { return (dist & 15) >= 5 && (dist & 15) <= 7; }
 __host__ __device__ inline bool gauss_closure_needs_logdet(int dist) { return (dist & 15) == 6 || (dist & 15) == 7; }
-size_t gauss_closure_workspace_floats(int C, int k, int64_t pair_begin, int64_t pair_end);
+// workspace of the pair stage in elements of the closure's scalar type (the same count in float32 and float64)
+size_t gauss_closure_workspace_elems(int C, int k, int64_t pair_begin, int64_t pair_end);
+// float32: noise by value; float64: noise from one device double
 cudaError_t launch_gauss_closure_class(const float* PsiPart, const float* MuPart, int nchunk, float noise, int C, int k,
                                        int dist, float* Psi, float* Mu, float* logdet, float* Sinv, int32_t* flag,
                                        cudaStream_t st);
+cudaError_t launch_gauss_closure_class(const double* PsiPart, const double* MuPart, int nchunk, const double* noise,
+                                       int C, int k, int dist, double* Psi, double* Mu, double* logdet, double* Sinv,
+                                       int32_t* flag, cudaStream_t st);
 cudaError_t launch_gauss_closure_pairs(const float* Psi, const float* Mu, const float* logdet, const float* Sinv, int C,
                                        int k, int dist, int64_t pair_begin, int64_t pair_end, float weight, float* out,
                                        float* gPsi, float* gMu, float* ws, cudaStream_t st);
+cudaError_t launch_gauss_closure_pairs(const double* Psi, const double* Mu, const double* logdet, const double* Sinv,
+                                       int C, int k, int dist, int64_t pair_begin, int64_t pair_end, double weight,
+                                       double* out, double* gPsi, double* gMu, double* ws, cudaStream_t st);
 }  // namespace sqfa

@@ -9,7 +9,8 @@ covariance; alternative `distance_fun` plug-ins, SURVEY.md section 8(f) row 4) r
 Cholesky kernel with an analytic backward. float64 inputs and matrices above 64 x 64 take the
 reference's own composition with device-side library calls, in the dtype of the inputs. As `distance_fun`
 of `SQFA`, `mahalanobis`, `mahalanobis_sq`, `bhattacharyya` and `hellinger` also fit through the models'
-single-call native closure (up to 32 filters); `fisher_rao_same_cov` keeps the generic path.
+single-call native closure (up to 32 filters), in float32 and, for a `.double()` model on one device, in
+float64; `fisher_rao_same_cov` keeps the generic path. The per-matrix functions stay composed in float64.
 
 Extension (not reference API): the Bures-Wasserstein distance between SPD matrices and the
 2-Wasserstein distance between Gaussians run in the same Jacobi pair kernel (up to 34 x 34) and

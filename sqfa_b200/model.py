@@ -116,8 +116,9 @@ def _check_statistics(data_statistics, needs_dict=False):
 def _statistics_to(data_statistics, dev, dtype=torch.float32):
     """The statistics on the compute device in the model's dtype (no copy if already so). float32 models
     run the native closure; a model converted with `.double()` -- the reference's remedy for NaN / inf
-    distances, _optim.py:28-30 -- keeps float64 statistics; its affine-invariant / Fisher-Rao closure is native
-    (closure64.cu), every other float64 closure uses float64 device-side library calls (SURVEY.md 8(f) row 3)."""
+    distances, _optim.py:28-30 -- keeps float64 statistics; its affine-invariant / Fisher-Rao closure and its
+    Mahalanobis / Bhattacharyya / Hellinger closure are native (closure64.cu, gauss.cu) on one device, every
+    other float64 closure uses float64 device-side library calls (SURVEY.md 8(f) row 3)."""
 
     def put(t):
         return t.detach().to(device=dev, dtype=dtype).contiguous()
@@ -310,8 +311,9 @@ class SecondMomentsSQFA(nn.Module):
         filters has a closed-form adjoint (Sphere: (I - f f^T)/|w| per row; Identity; FixedFilters:
         zero rows) -- torch's `orthogonal` keeps the autograd path. Saves the ~15 micro-kernels and
         the autograd engine round trip per evaluation that dominate small-C fits. A float64 parameter with
-        float64 statistics takes the float64 closure for the affine-invariant / Fisher-Rao distances on one
-        device, and None otherwise."""
+        float64 statistics takes a float64 closure on one device for the affine-invariant / Fisher-Rao
+        distances and for the mean-covariance distances (Mahalanobis, Bhattacharyya, Hellinger), and None
+        otherwise."""
         if not parametrize_is_parametrized(self, "filters"):
             return None
         chain = list(self.parametrizations.filters)
@@ -328,8 +330,11 @@ class SecondMomentsSQFA(nn.Module):
         if S.dtype != p.dtype or (M is not None and M.dtype != p.dtype):
             return None
         f64 = p.dtype == torch.float64
-        # float64 (a `.double()` model): the native closure covers affine-invariant / Fisher-Rao on one device
-        if f64 and ((dist & 15) not in (_ops.DIST_AI, _ops.DIST_FR) or self._process_group is not None):
+        # float64 (a `.double()` model): the native closures cover affine-invariant / Fisher-Rao and the
+        # mean-covariance distances on one device
+        gauss64 = f64 and (dist & 15) in (_ops.DIST_MAHA, _ops.DIST_BHATT, _ops.DIST_HELL)
+        if f64 and (((dist & 15) not in (_ops.DIST_AI, _ops.DIST_FR) and not gauss64)
+                    or self._process_group is not None):
             return None
         group = self._process_group
         k, D = p.shape
@@ -374,8 +379,13 @@ class SecondMomentsSQFA(nn.Module):
         # single device: ONE native call per evaluation (constraint and its adjoint included), all
         # buffers static, captured in a CUDA graph after the first evaluations
         P = C * (C - 1) // 2
-        ws_bytes = (lib.sqfa_fused_loss_workspace_bytes_f64 if f64 else lib.sqfa_fused_loss_workspace_bytes)(
-            C, D, k, dist, 0, P)
+        if gauss64:
+            ws_query, eval_f64 = lib.sqfa_gauss_closure_workspace_bytes_f64, _ops.gauss_closure_eval_f64_raw
+        elif f64:
+            ws_query, eval_f64 = lib.sqfa_fused_loss_workspace_bytes_f64, _ops.closure_eval_f64_raw
+        else:
+            ws_query = lib.sqfa_fused_loss_workspace_bytes
+        ws_bytes = ws_query(C, D, k, dist, 0, P)
         ws = torch.empty(max(int(ws_bytes), 1), dtype=torch.uint8, device=S.device)
         out = torch.zeros(_ops.N_OUT, dtype=p.dtype, device=S.device)
         out_host = torch.zeros(_ops.N_OUT, dtype=p.dtype).pin_memory()  # mirror, filled by every evaluation
@@ -385,7 +395,7 @@ class SecondMomentsSQFA(nn.Module):
             noise_dev = torch.full((1,), noise, dtype=torch.float64, device=S.device)
 
             def launch():
-                _ops.closure_eval_f64_raw(p.detach(), S, M, noise_dev, dist, sphere, n_fixed, out, grad, ws, out_host)
+                eval_f64(p.detach(), S, M, noise_dev, dist, sphere, n_fixed, out, grad, ws, out_host)
         else:
             def launch():
                 _ops.closure_eval_raw(p.detach(), S, M, noise, dist, sphere, n_fixed, out, grad, ws, out_host)
