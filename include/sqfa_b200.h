@@ -462,6 +462,18 @@ int sqfa_lbfgs_direction(const float* g, float* prev_g, float* d, float* S, floa
                          int32_t* meta, int64_t n, int32_t history, float t_prev, int first, float* param, float lr,
                          float tolerance_change, float* out_scalars, sqfa_stream_t stream);
 
+/* The same update in float64, with the same arithmetic in the same order, for a float64 parameter
+ * (every state buffer above in double; meta stays int32). The three host scalars are passed by
+ * pointer: scalars_host [3] = {t_prev, lr, tolerance_change} is PLAIN HOST memory, read during the
+ * call and not retained. out_scalars [8] has the layout above, in double, device or mapped pinned host
+ * memory. n <= sqfa_lbfgs_max_n_f64() (8 doubles per thread of the cluster), history <=
+ * sqfa_lbfgs_max_history(); otherwise SQFA_E_UNSUPPORTED. NULL pointers (param excepted), n <= 0 or
+ * history < 1: SQFA_E_INVALID. */
+int64_t sqfa_lbfgs_max_n_f64(void);
+int sqfa_lbfgs_direction_f64(const double* g, double* prev_g, double* d, double* S, double* Y, double* ro,
+                             double* hdiag, int32_t* meta, int64_t n, int32_t history, const double* scalars_host,
+                             int first, double* param, double* out_scalars, sqfa_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

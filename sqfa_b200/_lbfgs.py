@@ -1,14 +1,19 @@
 """L-BFGS with the direction update on the device (SURVEY.md section 8(f), rank 1).
 
 `LBFGS` is `torch.optim.LBFGS` -- the optimiser the reference's `fitting_loop` uses
-(reference _optim.py:78-79) -- with one change: when there is a single float32 CUDA parameter and no
-line search (the reference's configuration), the "update memory + two-loop recursion" block of
-`step` -- and the fixed step `x += t d` that follows it -- runs as ONE kernel (`sqfa_lbfgs_direction`)
-instead of 4 tiny torch kernels and 2 implicit host synchronisations per history entry; a closure that
-can be launched without a host wait is enqueued right behind it (one host wait per iteration). Same algorithm, same update rule and stopping tests, same
+(reference _optim.py:78-79) -- with one change: when there is a single float32 or float64 CUDA parameter
+and no line search (the reference's configuration), the "update memory + two-loop recursion" block of
+`step` -- and the fixed step `x += t d` that follows it -- runs as ONE kernel (`sqfa_lbfgs_direction`,
+`sqfa_lbfgs_direction_f64` for float64) instead of 4 tiny torch kernels and 2 implicit host
+synchronisations per history entry; a closure that can be launched without a host wait is enqueued right
+behind it (one host wait per iteration). Same algorithm, same update rule and stopping tests, same
 order of floating-point operations up to the summation order inside each dot product. Every other
-configuration falls through to `torch.optim.LBFGS.step` unchanged.
+configuration -- line search, several parameters, a CPU parameter, more elements than the kernel holds
+(`sqfa_lbfgs_max_n()` floats, `sqfa_lbfgs_max_n_f64()` doubles) or a longer history -- falls through to
+`torch.optim.LBFGS.step` unchanged.
 """
+
+import ctypes
 
 import torch
 
@@ -24,25 +29,26 @@ class LBFGS(torch.optim.LBFGS):
         if group["line_search_fn"] is not None or len(self._params) != 1:
             return None
         p = self._params[0]
-        if not (p.is_cuda and p.dtype == torch.float32 and p.is_contiguous()):
+        if not (p.is_cuda and p.dtype in (torch.float32, torch.float64) and p.is_contiguous()):
             return None
         lib = _lib.load()
         n, hist = p.numel(), int(group["history_size"])
-        if n > lib.sqfa_lbfgs_max_n() or hist > lib.sqfa_lbfgs_max_history() or hist < 1:
+        max_n = lib.sqfa_lbfgs_max_n() if p.dtype == torch.float32 else lib.sqfa_lbfgs_max_n_f64()
+        if n > max_n or hist > lib.sqfa_lbfgs_max_history() or hist < 1:
             return None
         state = self.state[p]
         nat = state.get("sqfa_native")
         if nat is None:
-            dev = p.device
+            dev, dt = p.device, p.dtype
             nat = {
-                "prev_g": torch.zeros(n, device=dev),
-                "d": torch.zeros(n, device=dev),
-                "S": torch.empty(hist + 1, n, device=dev),
-                "Y": torch.empty(hist + 1, n, device=dev),
-                "ro": torch.zeros(hist + 1, device=dev),
-                "hdiag": torch.ones(1, device=dev),
+                "prev_g": torch.zeros(n, dtype=dt, device=dev),
+                "d": torch.zeros(n, dtype=dt, device=dev),
+                "S": torch.empty(hist + 1, n, dtype=dt, device=dev),
+                "Y": torch.empty(hist + 1, n, dtype=dt, device=dev),
+                "ro": torch.zeros(hist + 1, dtype=dt, device=dev),
+                "hdiag": torch.ones(1, dtype=dt, device=dev),
                 "meta": torch.zeros(2, dtype=torch.int32, device=dev),
-                "out": torch.zeros(8, dtype=torch.float32).pin_memory(),  # written by the kernel (mapped)
+                "out": torch.zeros(8, dtype=dt).pin_memory(),  # written by the kernel (mapped)
                 "t": 0.0,
             }
             state["sqfa_native"] = nat
@@ -54,15 +60,18 @@ class LBFGS(torch.optim.LBFGS):
         evaluation, enqueued behind it --, and wait once. Returns (ys, g.d, max|d|, sum|g|, pairs held, t,
         step applied) as Python numbers."""
         lib, dev = _lib.load(), g.device
-        _lib.check(
-            lib.sqfa_lbfgs_direction(
-                _lib.ptr(g), _lib.ptr(nat["prev_g"]), _lib.ptr(nat["d"]), _lib.ptr(nat["S"]), _lib.ptr(nat["Y"]),
-                _lib.ptr(nat["ro"]), _lib.ptr(nat["hdiag"]), _lib.ptr(nat["meta"]), g.numel(), history,
-                float(nat["t"]), 1 if first else 0, _lib.ptr(param), float(lr), float(tolerance_change),
-                _lib.ptr(nat["out"]), _lib.stream_ptr(dev),
-            ),
-            "sqfa_lbfgs_direction",
-        )
+        bufs = (_lib.ptr(g), _lib.ptr(nat["prev_g"]), _lib.ptr(nat["d"]), _lib.ptr(nat["S"]), _lib.ptr(nat["Y"]),
+                 _lib.ptr(nat["ro"]), _lib.ptr(nat["hdiag"]), _lib.ptr(nat["meta"]), g.numel(), history)
+        if g.dtype == torch.float64:
+            # the float64 entry takes its three host scalars by pointer (the C ABI passes no double by value)
+            scalars = (ctypes.c_double * 3)(float(nat["t"]), float(lr), float(tolerance_change))
+            code = lib.sqfa_lbfgs_direction_f64(*bufs, scalars, 1 if first else 0, _lib.ptr(param),
+                                                _lib.ptr(nat["out"]), _lib.stream_ptr(dev))
+            _lib.check(code, "sqfa_lbfgs_direction_f64")
+        else:
+            code = lib.sqfa_lbfgs_direction(*bufs, float(nat["t"]), 1 if first else 0, _lib.ptr(param), float(lr),
+                                            float(tolerance_change), _lib.ptr(nat["out"]), _lib.stream_ptr(dev))
+            _lib.check(code, "sqfa_lbfgs_direction")
         if then is not None:
             then()
         ev = torch.cuda.Event()

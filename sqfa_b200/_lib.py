@@ -100,6 +100,11 @@ SIGNATURES = {
         [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_i32, c_f32, c_int, c_ptr, c_f32, c_f32, c_ptr,
          c_ptr],
     ),
+    "sqfa_lbfgs_max_n_f64": (c_i64, []),
+    "sqfa_lbfgs_direction_f64": (
+        c_int,
+        [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_i32, c_ptr, c_int, c_ptr, c_ptr, c_ptr],
+    ),
     "sqfa_project_workspace_bytes": (c_size, [c_i32, c_i32, c_i32]),
     "sqfa_project_fwd": (
         c_int,

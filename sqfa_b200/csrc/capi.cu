@@ -622,6 +622,24 @@ int sqfa_lbfgs_direction(const float* g, float* prev_g, float* d, float* S_, flo
                                                      S(stream)));
 }
 
+int64_t sqfa_lbfgs_max_n_f64(void) { return sqfa::lbfgs_max_n_f64(); }
+
+int sqfa_lbfgs_direction_f64(const double* g, double* prev_g, double* d, double* S_, double* Y, double* ro,
+                             double* hdiag, int32_t* meta, int64_t n, int32_t history, const double* scalars_host,
+                             int first, double* param, double* out_scalars, sqfa_stream_t stream) {
+  if (g == nullptr || prev_g == nullptr || d == nullptr || S_ == nullptr || Y == nullptr || ro == nullptr ||
+      hdiag == nullptr || meta == nullptr || scalars_host == nullptr || out_scalars == nullptr || n <= 0 ||
+      history < 1)
+    return fail_arg(__func__, "bad argument");
+  if (n > sqfa::lbfgs_max_n_f64() || history > sqfa::lbfgs_max_history())
+    return fail_arg(__func__, "vector or history too large for the single-cluster kernel", SQFA_E_UNSUPPORTED);
+  // {t_prev, lr, tolerance_change}: read here and passed by value, so the caller may reuse the memory at once
+  const double t_prev = scalars_host[0], lr = scalars_host[1], tolerance_change = scalars_host[2];
+  return wrap(__func__, sqfa::launch_lbfgs_direction_f64(g, prev_g, d, S_, Y, ro, hdiag, meta, n, history, t_prev,
+                                                         first ? 1 : 0, param, lr, tolerance_change, out_scalars,
+                                                         S(stream)));
+}
+
 }  // extern "C"
 
 extern "C" {

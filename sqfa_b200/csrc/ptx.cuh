@@ -317,6 +317,9 @@ __device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
 __device__ __forceinline__ void st_cluster_u32(uint32_t cluster_addr, uint32_t v) {
   asm volatile("st.shared::cluster.u32 [%0], %1;" ::"r"(cluster_addr), "r"(v) : "memory");
 }
+__device__ __forceinline__ void st_cluster_u64(uint32_t cluster_addr, uint64_t v) {
+  asm volatile("st.shared::cluster.u64 [%0], %1;" ::"r"(cluster_addr), "l"(v) : "memory");
+}
 
 // wait on a barrier that also receives arrivals from the peer CTA (cta-scope acquire: a
 // cluster-scope acquire would invalidate L1 (CCTL.IVALL) on every wake-up)

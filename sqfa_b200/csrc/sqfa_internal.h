@@ -197,6 +197,11 @@ int lbfgs_max_history();
 cudaError_t launch_lbfgs_direction(const float* g, float* prev_g, float* d, float* S, float* Y, float* ro, float* hdiag,
                                    int32_t* meta, int64_t n, int history, float t_prev, int first, float* param,
                                    float lr, float tol_change, float* out, cudaStream_t stream);
+// the same update in float64, n <= lbfgs_max_n_f64()
+int lbfgs_max_n_f64();
+cudaError_t launch_lbfgs_direction_f64(const double* g, double* prev_g, double* d, double* S, double* Y, double* ro,
+                                       double* hdiag, int32_t* meta, int64_t n, int history, double t_prev, int first,
+                                       double* param, double lr, double tol_change, double* out, cudaStream_t stream);
 }  // namespace sqfa
 
 namespace sqfa {
