@@ -417,6 +417,24 @@ int sqfa_gauss_closure_eval_f64(const double* S, const double* M, const double* 
                                 double* out, double* out_host, double* grad, void* ws, size_t ws_bytes,
                                 sqfa_stream_t stream);
 
+/* sqfa_fused_loss_sharded in float64: the classes and the pairs of a float64 closure sharded over the ranks of a
+ * multi-device caller, with the same three phases, exchange spans and contracts (S, M hold all classes on every
+ * rank, a rank reads only its own; F is the constrained filters, dF the rank's share of d loss / dF). For the codes
+ * of sqfa_closure_eval_f64 and sqfa_gauss_closure_eval_f64: SQFA_DIST_AFFINE_INVARIANT, SQFA_DIST_FISHER_RAO_LB and
+ * SQFA_DIST_MAHALANOBIS (each optionally + SQFA_DIST_SQUARED), SQFA_DIST_BHATTACHARYYA and SQFA_DIST_HELLINGER;
+ * M is required for all but the affine-invariant distance, n_filters <= 32. `noise` points to ONE double in device
+ * memory. ws: 16-byte aligned, at least the float64 workspace query of the code (sqfa_fused_loss_workspace_bytes_f64
+ * or sqfa_gauss_closure_workspace_bytes_f64) for [pair_begin, pair_end). After the second all-reduce the last 64
+ * doubles of span 1 start with {loss, #non-finite distances}. Deterministic: no floating-point atomics.
+ * Other known codes and n_filters > 32 return SQFA_E_UNSUPPORTED; every check runs before any launch. */
+int sqfa_fused_loss_exchange_span_f64(int32_t n_classes, int32_t n_dim, int32_t n_filters, int32_t dist,
+                                      int64_t pair_begin, int64_t pair_end, int32_t which, size_t* offset_bytes,
+                                      size_t* bytes);
+int sqfa_fused_loss_sharded_f64(int32_t phase, const double* S, const double* M, const double* F, int32_t n_classes,
+                                int32_t n_dim, int32_t n_filters, const double* noise, int32_t dist,
+                                int32_t class_begin, int32_t class_end, int64_t pair_begin, int64_t pair_end,
+                                double* dF, void* ws, size_t ws_bytes, sqfa_stream_t stream);
+
 /* Plug-in distances between Gaussians that use the mean covariance of the pair (distances.py:240-432),
  * one warp per pair (Cholesky of (Sigma_a + Sigma_b) / 2 in shared memory), all n_a * n_b pairs:
  *   SQFA_GAUSS_MAHALANOBIS_SQ  d^T M^-1 d                                             (:283-330)

@@ -154,6 +154,12 @@ SIGNATURES = {
         [c_ptr, c_ptr, c_ptr, c_i32, c_i32, c_i32, c_ptr, c_i32, c_i32, c_i32, c_i64, c_i64, c_ptr, c_ptr, c_ptr,
          c_ptr, c_size, c_ptr],
     ),
+    "sqfa_fused_loss_exchange_span_f64": (c_int, [c_i32, c_i32, c_i32, c_i32, c_i64, c_i64, c_i32, c_ptr, c_ptr]),
+    "sqfa_fused_loss_sharded_f64": (
+        c_int,
+        [c_i32, c_ptr, c_ptr, c_ptr, c_i32, c_i32, c_i32, c_ptr, c_i32, c_i32, c_i32, c_i64, c_i64, c_ptr, c_ptr,
+         c_size, c_ptr],
+    ),
     "sqfa_gauss_closure_workspace_bytes_f64": (c_size, [c_i32, c_i32, c_i32, c_i32, c_i64, c_i64]),
     "sqfa_gauss_closure_eval_f64": (
         c_int,

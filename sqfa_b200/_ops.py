@@ -380,6 +380,17 @@ def fused_loss_raw(F, S, M, noise, dist, group=None, ws=None):
     return packed
 
 
+def _exchange_spans(fn, C, D, k, dist, p0, p1, ws, dtype):
+    """The two exchange spans of a sharded closure's workspace, as views of `dtype`."""
+    lib = _lib.load()
+    spans = []
+    for which in (0, 1):
+        off, nbytes = ctypes.c_size_t(0), ctypes.c_size_t(0)
+        _lib.check(getattr(lib, fn)(C, D, k, dist, p0, p1, which, ctypes.byref(off), ctypes.byref(nbytes)), fn)
+        spans.append(ws[off.value : off.value + nbytes.value].view(dtype))
+    return spans
+
+
 def fused_loss_sharded_raw(F, S, M, noise, dist, group, ws=None):
     """`fused_loss_raw` with the classes AND the pairs sharded over the ranks of `group` (AI / FR): every
     rank projects only its share of the classes (the part that reads C D^2 floats) and evaluates only its
@@ -399,12 +410,7 @@ def fused_loss_sharded_raw(F, S, M, noise, dist, group, ws=None):
     p0, p1 = shard_pairs(P, C, rank, world)
     c0, c1 = class_share(C, rank, world)
     ws = _closure_workspace(lib, C, D, k, dist, p0, p1, dev, ws)
-    spans = []
-    for which in (0, 1):
-        off, nbytes = ctypes.c_size_t(0), ctypes.c_size_t(0)
-        _lib.check(lib.sqfa_fused_loss_exchange_span(C, D, k, dist, p0, p1, which, ctypes.byref(off), ctypes.byref(nbytes)),
-                   "sqfa_fused_loss_exchange_span")
-        spans.append(ws[off.value : off.value + nbytes.value].view(torch.float32))
+    spans = _exchange_spans("sqfa_fused_loss_exchange_span", C, D, k, dist, p0, p1, ws, torch.float32)
     packed = torch.empty(4 + k * D, dtype=torch.float32, device=dev)
     dF = ctypes.c_void_p(packed.data_ptr() + 16)
 
@@ -467,6 +473,83 @@ def gauss_closure_eval_f64_raw(W, S, M, noise, dist, sphere, n_fixed, out, grad,
     """`closure_eval_f64_raw` for the mean-covariance distances (Mahalanobis, Bhattacharyya, Hellinger); M, the
     class means, is required."""
     _closure_eval_f64("sqfa_gauss_closure_eval_f64", W, S, M, noise, dist, sphere, n_fixed, out, grad, ws, out_host)
+
+
+def closure_workspace_bytes_f64(C, D, k, dist, p0, p1):
+    """Workspace of the float64 closure of `dist` over pairs [p0, p1): the mean-covariance query for Mahalanobis,
+    Bhattacharyya and Hellinger, the affine-invariant / Fisher-Rao one otherwise (0 for codes neither takes)."""
+    lib = _lib.load()
+    gauss = (dist & 15) in (DIST_MAHA, DIST_BHATT, DIST_HELL)
+    query = lib.sqfa_gauss_closure_workspace_bytes_f64 if gauss else lib.sqfa_fused_loss_workspace_bytes_f64
+    return int(query(C, D, k, dist, p0, p1))
+
+
+def _group_rank(group):
+    import torch.distributed as dist_mod
+
+    return dist_mod.get_rank(group), dist_mod.get_world_size(group)
+
+
+def fused_loss_f64_raw(F, S, M, noise, dist, group, ws):
+    """`fused_loss_raw` in float64 with the pair list sharded over the ranks of `group`: every rank runs the
+    single-device float64 closure (no constraint) at the constrained filters F on its `shard_pairs` range -- the
+    losses and gradients of disjoint ranges add up -- and ONE all-reduce sums [loss, #non-finite, -, -, dF].
+    `noise` is a one-element float64 device tensor. Returns the packed float64 vector (entry 2 is meaningless)."""
+    import torch.distributed as dist_mod
+
+    lib = _lib.load()
+    C, D, _ = S.shape
+    k = F.shape[0]
+    rank, world = _group_rank(group)
+    p0, p1 = shard_pairs(C * (C - 1) // 2, C, rank, world)
+    gauss = (dist & 15) in (DIST_MAHA, DIST_BHATT, DIST_HELL)
+    fn = "sqfa_gauss_closure_eval_f64" if gauss else "sqfa_closure_eval_f64"
+    packed = torch.empty(4 + k * D, dtype=torch.float64, device=S.device)
+    _lib.check(
+        getattr(lib, fn)(
+            _lib.ptr(S), _lib.ptr(M), _lib.ptr(F), C, D, k, _lib.ptr(noise), dist, 0, 0, p0, p1, _lib.ptr(packed),
+            None, ctypes.c_void_p(packed.data_ptr() + 32), _lib.ptr(ws), ws.numel(), _lib.stream_ptr(S.device),
+        ),
+        fn,
+    )
+    dist_mod.all_reduce(packed, group=group)
+    return packed
+
+
+def fused_loss_sharded_f64_raw(F, S, M, noise, dist, group, ws):
+    """`fused_loss_sharded_raw` in float64 (affine-invariant, Fisher-Rao, Mahalanobis, Bhattacharyya, Hellinger): the
+    three phases of sqfa_fused_loss_sharded_f64 with the same three all-reduces, on float64 spans. `noise` is a
+    one-element float64 device tensor. Returns the packed float64 vector [loss, #non-finite, -, -, dF]."""
+    import torch.distributed as dist_mod
+
+    from ._stats_driver import class_share
+
+    lib = _lib.load()
+    dev = S.device
+    C, D, _ = S.shape
+    k = F.shape[0]
+    rank, world = _group_rank(group)
+    p0, p1 = shard_pairs(C * (C - 1) // 2, C, rank, world)
+    c0, c1 = class_share(C, rank, world)
+    spans = _exchange_spans("sqfa_fused_loss_exchange_span_f64", C, D, k, dist, p0, p1, ws, torch.float64)
+    packed = torch.empty(4 + k * D, dtype=torch.float64, device=dev)
+    dF = ctypes.c_void_p(packed.data_ptr() + 32)
+
+    def phase(i):
+        _lib.check(
+            lib.sqfa_fused_loss_sharded_f64(i, _lib.ptr(S), _lib.ptr(M), _lib.ptr(F), C, D, k, _lib.ptr(noise), dist,
+                                            c0, c1, p0, p1, dF, _lib.ptr(ws), ws.numel(), _lib.stream_ptr(dev)),
+            "sqfa_fused_loss_sharded_f64",
+        )
+
+    phase(0)
+    dist_mod.all_reduce(spans[0], group=group)
+    phase(1)
+    dist_mod.all_reduce(spans[1], group=group)
+    phase(2)
+    dist_mod.all_reduce(packed[4:], group=group)
+    packed[:4] = spans[1][-64:-60]  # {loss, #non-finite, -, -} summed over the ranks
+    return packed
 
 
 class FusedLoss(torch.autograd.Function):

@@ -570,6 +570,49 @@ int sqfa_gauss_closure_eval_f64(const double* S_, const double* M, const double*
                                                        static_cast<double*>(ws), S(stream)));
 }
 
+// sharded float64 closure: the codes of both float64 closures. Returns 0, or the fail_arg code for a code, n_filters
+// or pair range the layout cannot take (checked before anything else reads the layout).
+static int sharded_f64_check(const char* fn, int32_t n_classes, int32_t n_dim, int32_t n_filters, int32_t dist,
+                             int64_t pair_begin, int64_t pair_end) {
+  if (!dist_ok(dist) || n_classes <= 0 || n_dim <= 0 || n_filters <= 0) return fail_arg(fn, "bad argument");
+  if (!f64_dist_ok(dist) && !gauss_f64_dist_ok(dist))
+    return fail_arg(fn, "the sharded float64 closure supports SQFA_DIST_AFFINE_INVARIANT, SQFA_DIST_FISHER_RAO_LB and "
+                        "SQFA_DIST_MAHALANOBIS (each optionally + SQFA_DIST_SQUARED), SQFA_DIST_BHATTACHARYYA and "
+                        "SQFA_DIST_HELLINGER",
+                    SQFA_E_UNSUPPORTED);
+  if (n_filters > 32) return fail_arg(fn, "n_filters must be <= 32", SQFA_E_UNSUPPORTED);
+  const int64_t P = (int64_t)n_classes * (n_classes - 1) / 2;
+  if (pair_begin < 0 || pair_end > P || pair_begin > pair_end) return fail_arg(fn, "bad pair range");
+  return 0;
+}
+
+int sqfa_fused_loss_exchange_span_f64(int32_t n_classes, int32_t n_dim, int32_t n_filters, int32_t dist,
+                                      int64_t pair_begin, int64_t pair_end, int32_t which, size_t* offset_bytes,
+                                      size_t* bytes) {
+  if ((which != 0 && which != 1) || offset_bytes == nullptr || bytes == nullptr)
+    return fail_arg(__func__, "bad argument");
+  if (const int rc = sharded_f64_check(__func__, n_classes, n_dim, n_filters, dist, pair_begin, pair_end)) return rc;
+  sqfa::fused_loss_exchange_span_f64(n_classes, n_dim, n_filters, dist, pair_begin, pair_end, which, offset_bytes,
+                                     bytes);
+  return 0;
+}
+
+int sqfa_fused_loss_sharded_f64(int32_t phase, const double* S_, const double* M, const double* F, int32_t n_classes,
+                                int32_t n_dim, int32_t n_filters, const double* noise, int32_t dist,
+                                int32_t class_begin, int32_t class_end, int64_t pair_begin, int64_t pair_end,
+                                double* dF, void* ws, size_t ws_bytes, sqfa_stream_t stream) {
+  if (S_ == nullptr || F == nullptr || ws == nullptr || noise == nullptr || (dist_uses_means(dist) && M == nullptr) ||
+      phase < 0 || phase > 2 || (phase == 2 && dF == nullptr) || class_begin < 0 || class_end > n_classes ||
+      class_begin > class_end || (reinterpret_cast<uintptr_t>(ws) & 15) != 0)
+    return fail_arg(__func__, "bad argument");
+  if (const int rc = sharded_f64_check(__func__, n_classes, n_dim, n_filters, dist, pair_begin, pair_end)) return rc;
+  if (ws_bytes < sqfa::fused_loss_workspace_bytes_f64(n_classes, n_dim, n_filters, dist, pair_begin, pair_end))
+    return fail_arg(__func__, "workspace too small", SQFA_E_WORKSPACE);
+  return wrap(__func__, sqfa::launch_fused_loss_sharded_f64(phase, S_, M, F, n_classes, n_dim, n_filters, noise, dist,
+                                                            class_begin, class_end, pair_begin, pair_end, dF,
+                                                            static_cast<double*>(ws), S(stream)));
+}
+
 }  // extern "C"
 
 extern "C" {

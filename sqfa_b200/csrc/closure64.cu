@@ -24,6 +24,7 @@
 // Stopping rule of the Jacobi (DESIGN.md section 18): a column pair is rotated while
 // |a_p . a_q| > J64_TOL |a_p| |a_q|; a sweep whose rotations all had |a_p . a_q| <= J64_LAST |a_p| |a_q| is the
 // last one (what it leaves is of order J64_LAST^2 relative); at most J64_MAX_SWEEPS sweeps.
+#include <algorithm>
 #include <cmath>
 #include <cstdint>
 #include <cuda_runtime.h>
@@ -402,8 +403,8 @@ int p64_tile_edge(int64_t npairs) {
 }
 
 struct Closure64Layout {
-  size_t F, inv_norm, T, Mu, W, logdet, sinv, gPsi, gMu, ticket, proj, psipart, mupart, rowpart, colpart, losspart, pair,
-      total;
+  size_t F, inv_norm, T, Mu, W, logdet, sinv, gPsi, gMu, red_out, ticket, proj, psipart, mupart, rowpart, colpart,
+      losspart, pair, total;
   int rows, nsplit, nchunk, csplit;
   PairTiles tiles;
 };
@@ -436,6 +437,7 @@ Closure64Layout closure64_layout(int C, int D, int k, int dist, int64_t pair_beg
   L.sinv = o;     o += ld ? al<double>((size_t)C * k * k) : 0;
   L.gPsi = o;     o += al<double>((size_t)C * k * k);
   L.gMu = o;      o += al<double>((size_t)C * k);
+  L.red_out = o;  o += al<double>(64);  // {loss, #non-finite} of a rank's pairs: [gPsi | gMu | red_out] is one exchange span
   L.ticket = o;   o += al<double>(1);  // uint32 arrival ticket of closure_finish_kernel; int32 [2, 4): gauss class flag
   L.proj = o;     o += al<double>(fwd > bwd ? fwd : bwd);  // row-split partials of T, later the class-split partials of dF
   L.psipart = o;  o += al<double>((size_t)C * L.nchunk * k * k);
@@ -449,20 +451,34 @@ Closure64Layout closure64_layout(int C, int D, int k, int dist, int64_t pair_beg
 }
 
 template <int KT, int VEC>
-cudaError_t run_project64(const double* S, const double* F, int C, int D, int k, const Closure64Layout& L, double* part,
+cudaError_t run_project64(const double* S, const double* F, int C, int D, int k, int rows, int nsplit, double* part,
                           cudaStream_t st) {
-  const dim3 grid((D + PS64_THREADS * VEC - 1) / (PS64_THREADS * VEC), L.nsplit, C);
-  project64_stream_kernel<KT, VEC><<<grid, PS64_THREADS, 0, st>>>(S, F, C, D, k, L.rows, part);
+  const dim3 grid((D + PS64_THREADS * VEC - 1) / (PS64_THREADS * VEC), nsplit, C);
+  project64_stream_kernel<KT, VEC><<<grid, PS64_THREADS, 0, st>>>(S, F, C, D, k, rows, part);
   return cudaGetLastError();
 }
 
 template <int VEC>
-cudaError_t run_project64_k(const double* S, const double* F, int C, int D, int k, const Closure64Layout& L,
-                            double* part, cudaStream_t st) {
-  if (k <= 4) return run_project64<4, VEC>(S, F, C, D, k, L, part, st);
-  if (k <= 8) return run_project64<8, VEC>(S, F, C, D, k, L, part, st);
-  if (k <= 16) return run_project64<16, VEC>(S, F, C, D, k, L, part, st);
-  return run_project64<32, VEC>(S, F, C, D, k, L, part, st);
+cudaError_t run_project64_k(const double* S, const double* F, int C, int D, int k, int rows, int nsplit, double* part,
+                            cudaStream_t st) {
+  if (k <= 4) return run_project64<4, VEC>(S, F, C, D, k, rows, nsplit, part, st);
+  if (k <= 8) return run_project64<8, VEC>(S, F, C, D, k, rows, nsplit, part, st);
+  if (k <= 16) return run_project64<16, VEC>(S, F, C, D, k, rows, nsplit, part, st);
+  return run_project64<32, VEC>(S, F, C, D, k, rows, nsplit, part, st);
+}
+
+// The streaming pass over the n classes that S, M, T, PsiPart and MuPart start at (nsplit splits of `rows` rows,
+// partials in `part`), then T and the per-chunk partials of Psi_c and, with M, mu'_c.
+cudaError_t project64_partials(const double* S, const double* M, const double* F, int n, int D, int k, int rows,
+                               int nsplit, int nchunk, double* part, double* T, double* PsiPart, double* MuPart,
+                               cudaStream_t st) {
+  // 16-byte loads of S when every row starts 16-byte aligned
+  const bool vec2 = (D % 2 == 0) && (reinterpret_cast<uintptr_t>(S) & 15) == 0;
+  cudaError_t e = vec2 ? run_project64_k<2>(S, F, n, D, k, rows, nsplit, part, st)
+                       : run_project64_k<1>(S, F, n, D, k, rows, nsplit, part, st);
+  if (e != cudaSuccess) return e;
+  project64_finish_kernel<<<dim3(nchunk, n), PF64_COLS, 0, st>>>(part, F, M, n, D, k, nsplit, T, PsiPart, MuPart);
+  return cudaGetLastError();
 }
 
 // The front of both float64 closures: the sphere constraint (F = W / |W| into the workspace; *F_out is the
@@ -478,45 +494,27 @@ cudaError_t closure64_front(const double* S, const double* M, const double* raw_
   }
   *F_out = F;
   if ((e = cudaMemsetAsync(ws + L.ticket, 0, sizeof(unsigned int), st)) != cudaSuccess) return e;
-  // 16-byte loads of S when every row starts 16-byte aligned
-  const bool vec2 = (D % 2 == 0) && (reinterpret_cast<uintptr_t>(S) & 15) == 0;
-  e = vec2 ? run_project64_k<2>(S, F, C, D, k, L, ws + L.proj, st) : run_project64_k<1>(S, F, C, D, k, L, ws + L.proj, st);
-  if (e != cudaSuccess) return e;
-  project64_finish_kernel<<<dim3(L.nchunk, C), PF64_COLS, 0, st>>>(ws + L.proj, F, M, C, D, k, L.nsplit, ws + L.T,
-                                                                   ws + L.psipart, ws + L.mupart);
-  return cudaGetLastError();
+  return project64_partials(S, M, F, C, D, k, L.rows, L.nsplit, L.nchunk, ws + L.proj, ws + L.T, ws + L.psipart,
+                            ws + L.mupart, st);
 }
 
-// The back of both float64 closures: the projection adjoint with gMu when M is given, the constraint's adjoint,
-// the frozen rows, max |grad| and the published out.
-cudaError_t closure64_back(const double* M, int C, int D, int k, const double* F, int sphere, int n_fixed,
-                           const Closure64Layout& L, double* out, double* out_host, double* grad, double* ws,
-                           cudaStream_t st) {
-  return launch_project_bwd_constrained(ws + L.gPsi, M != nullptr ? ws + L.gMu : nullptr, ws + L.T, M, C, D, k, F,
-                                        ws + L.inv_norm, sphere, n_fixed, grad, out, out_host,
-                                        reinterpret_cast<unsigned int*>(ws + L.ticket), ws + L.proj, st);
-}
-
-}  // namespace
-
-size_t fused_loss_workspace_bytes_f64(int C, int D, int k, int dist, int64_t pair_begin, int64_t pair_end) {
-  return closure64_layout(C, D, k, dist, pair_begin, pair_end).total * sizeof(double);
-}
-
-cudaError_t launch_closure_f64(const double* S, const double* M, const double* raw_filters, int C, int D, int k,
-                               const double* noise, int dist, int constraint, int n_fixed, int64_t pair_begin,
-                               int64_t pair_end, double* out, double* out_host, double* grad, double* ws,
-                               cudaStream_t st) {
+// The middle of both float64 closures, from the per-chunk partials of all C classes: the class stage, the pair stage
+// on [pair_begin, pair_end) and the per-class reduce into (gPsi, gMu) of every class and out = {weight * sum d,
+// #non-finite, 0}. Affine-invariant / Fisher-Rao: class64, pair64, pair_reduce; the mean-covariance distances: the
+// class, pair and reduce stages of gauss.cu.
+cudaError_t closure64_middle(const double* noise, int C, int k, int dist, int64_t pair_begin, int64_t pair_end,
+                             double weight, const Closure64Layout& L, double* out, double* ws, cudaStream_t st) {
+  cudaError_t e;
+  if (is_gauss_closure(dist)) {
+    int32_t* flag = reinterpret_cast<int32_t*>(ws + L.ticket) + 2;
+    if ((e = launch_gauss_closure_class(ws + L.psipart, ws + L.mupart, L.nchunk, noise, C, k, dist, ws + L.W,
+                                        ws + L.Mu, ws + L.logdet, ws + L.sinv, flag, st)) != cudaSuccess)
+      return e;
+    return launch_gauss_closure_pairs(ws + L.W, ws + L.Mu, ws + L.logdet, ws + L.sinv, C, k, dist, pair_begin,
+                                      pair_end, weight, out, ws + L.gPsi, ws + L.gMu, ws + L.pair, st);
+  }
   const int fr = (dist & 15) == SQFA_DIST_FISHER_RAO_LB ? 1 : 0;
   const int m = fr ? k + 1 : k;
-  const Closure64Layout L = closure64_layout(C, D, k, dist, pair_begin, pair_end);
-  const int sphere = constraint == 1 ? 1 : 0;
-  const double* Mfr = fr ? M : nullptr;
-  const int64_t P = (int64_t)C * (C - 1) / 2;
-  const double weight = -1.0 / (double)(P > 0 ? P : 1);
-  const double* F;
-  cudaError_t e;
-  if ((e = closure64_front(S, Mfr, raw_filters, C, D, k, sphere, L, ws, &F, st)) != cudaSuccess) return e;
   {
     const int per_warp = class64_smem_doubles(m, k) * (int)sizeof(double);
     const int nw = warps_for(per_warp, W64);
@@ -543,10 +541,39 @@ cudaError_t launch_closure_f64(const double* S, const double* M, const double* r
     pair64_kernel<<<(unsigned)((L.tiles.ntiles + nw - 1) / nw), nw * 32, nw * per_warp, st>>>(A);
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
   }
-  double* gMu = fr ? ws + L.gMu : nullptr;
-  if ((e = launch_pair_reduce_closure(L.tiles, C, m, k, fr, ws + L.rowpart, ws + L.colpart, ws + L.losspart, weight,
-                                      ws + L.Mu, out, ws + L.gPsi, gMu, st)) != cudaSuccess)
-    return e;
+  return launch_pair_reduce_closure(L.tiles, C, m, k, fr, ws + L.rowpart, ws + L.colpart, ws + L.losspart, weight,
+                                    ws + L.Mu, out, ws + L.gPsi, fr ? ws + L.gMu : nullptr, st);
+}
+
+// The back of both float64 closures: the projection adjoint with gMu when M is given, the constraint's adjoint,
+// the frozen rows, max |grad| and the published out.
+cudaError_t closure64_back(const double* M, int C, int D, int k, const double* F, int sphere, int n_fixed,
+                           const Closure64Layout& L, double* out, double* out_host, double* grad, double* ws,
+                           cudaStream_t st) {
+  return launch_project_bwd_constrained(ws + L.gPsi, M != nullptr ? ws + L.gMu : nullptr, ws + L.T, M, C, D, k, F,
+                                        ws + L.inv_norm, sphere, n_fixed, grad, out, out_host,
+                                        reinterpret_cast<unsigned int*>(ws + L.ticket), ws + L.proj, st);
+}
+
+}  // namespace
+
+size_t fused_loss_workspace_bytes_f64(int C, int D, int k, int dist, int64_t pair_begin, int64_t pair_end) {
+  return closure64_layout(C, D, k, dist, pair_begin, pair_end).total * sizeof(double);
+}
+
+cudaError_t launch_closure_f64(const double* S, const double* M, const double* raw_filters, int C, int D, int k,
+                               const double* noise, int dist, int constraint, int n_fixed, int64_t pair_begin,
+                               int64_t pair_end, double* out, double* out_host, double* grad, double* ws,
+                               cudaStream_t st) {
+  const Closure64Layout L = closure64_layout(C, D, k, dist, pair_begin, pair_end);
+  const int sphere = constraint == 1 ? 1 : 0;
+  const double* Mfr = (dist & 15) == SQFA_DIST_FISHER_RAO_LB ? M : nullptr;
+  const int64_t P = (int64_t)C * (C - 1) / 2;
+  const double weight = -1.0 / (double)(P > 0 ? P : 1);
+  const double* F;
+  cudaError_t e;
+  if ((e = closure64_front(S, Mfr, raw_filters, C, D, k, sphere, L, ws, &F, st)) != cudaSuccess) return e;
+  if ((e = closure64_middle(noise, C, k, dist, pair_begin, pair_end, weight, L, out, ws, st)) != cudaSuccess) return e;
   return closure64_back(Mfr, C, D, k, F, sphere, n_fixed, L, out, out_host, grad, ws, st);
 }
 
@@ -563,14 +590,65 @@ cudaError_t launch_gauss_closure_f64(const double* S, const double* M, const dou
   const double* F;
   cudaError_t e;
   if ((e = closure64_front(S, M, raw_filters, C, D, k, sphere, L, ws, &F, st)) != cudaSuccess) return e;
-  int32_t* flag = reinterpret_cast<int32_t*>(ws + L.ticket) + 2;
-  if ((e = launch_gauss_closure_class(ws + L.psipart, ws + L.mupart, L.nchunk, noise, C, k, dist, ws + L.W, ws + L.Mu,
-                                      ws + L.logdet, ws + L.sinv, flag, st)) != cudaSuccess)
-    return e;
-  if ((e = launch_gauss_closure_pairs(ws + L.W, ws + L.Mu, ws + L.logdet, ws + L.sinv, C, k, dist, pair_begin,
-                                      pair_end, weight, out, ws + L.gPsi, ws + L.gMu, ws + L.pair, st)) != cudaSuccess)
-    return e;
+  if ((e = closure64_middle(noise, C, k, dist, pair_begin, pair_end, weight, L, out, ws, st)) != cudaSuccess) return e;
   return closure64_back(M, C, D, k, F, sphere, n_fixed, L, out, out_host, grad, ws, st);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// The float64 closure with the CLASSES and the PAIRS sharded over ranks: the three phases of
+// launch_fused_loss_sharded (closure.cu) on the float64 layout, for every code of the two closures above. F is the
+// constrained filters; the caller all-reduces exchange span 0 after phase 0 and span 1 after phase 1.
+//   phase 0  zero span 0 = [PsiPart | MuPart]; the streaming projection of classes [c0, c1) only, its row split
+//            chosen for c1 - c0 classes (bounded by the proj region, which the layout sizes for C classes)
+//   phase 1  class stage of all C classes from the summed partials, pair stage on [pair_begin, pair_end), reduce
+//            into span 1 = [gPsi | gMu | red_out] (every class's gPsi is written, red_out[0..1] = {weight * sum d,
+//            #non-finite}, the rest of red_out zero)
+//   phase 2  the projection adjoint over classes [c0, c1) into dF: the closure's tail with no constraint, no
+//            frozen rows and no published out
+void fused_loss_exchange_span_f64(int C, int D, int k, int dist, int64_t pair_begin, int64_t pair_end, int which,
+                                  size_t* offset_bytes, size_t* bytes) {
+  const Closure64Layout L = closure64_layout(C, D, k, dist, pair_begin, pair_end);
+  if (which == 0) {
+    *offset_bytes = L.psipart * sizeof(double);
+    *bytes = (L.rowpart - L.psipart) * sizeof(double);  // psipart and mupart are adjacent
+  } else {
+    *offset_bytes = L.gPsi * sizeof(double);
+    *bytes = (L.ticket - L.gPsi) * sizeof(double);  // gPsi | gMu | red_out
+  }
+}
+
+cudaError_t launch_fused_loss_sharded_f64(int phase, const double* S, const double* M, const double* F, int C, int D,
+                                          int k, const double* noise, int dist, int c0, int c1, int64_t pair_begin,
+                                          int64_t pair_end, double* dF, double* ws, cudaStream_t st) {
+  const Closure64Layout L = closure64_layout(C, D, k, dist, pair_begin, pair_end);
+  const bool means = (dist & 15) == SQFA_DIST_FISHER_RAO_LB || is_gauss_closure(dist);
+  const double* Mm = means ? M : nullptr;
+  const int n_own = c1 > c0 ? c1 - c0 : 0;
+  cudaError_t e;
+  if (phase == 0) {
+    if ((e = cudaMemsetAsync(ws + L.psipart, 0, (L.rowpart - L.psipart) * sizeof(double), st)) != cudaSuccess)
+      return e;
+    if (n_own == 0) return cudaSuccess;
+    const size_t per_split = (size_t)n_own * k * D;
+    const int cap = (int)std::min<size_t>((L.psipart - L.proj) / per_split, (size_t)D);
+    const int nsplit = std::max(1, std::min(p64_nsplit(n_own, D), cap));
+    const int rows = (D + nsplit - 1) / nsplit;
+    return project64_partials(S + (size_t)c0 * D * D, Mm != nullptr ? Mm + (size_t)c0 * D : nullptr, F, n_own, D, k,
+                              rows, (D + rows - 1) / rows, L.nchunk, ws + L.proj, ws + L.T + (size_t)c0 * k * D,
+                              ws + L.psipart + (size_t)c0 * L.nchunk * k * k,
+                              ws + L.mupart + (size_t)c0 * L.nchunk * k, st);
+  }
+  if (phase == 1) {
+    const int64_t P = (int64_t)C * (C - 1) / 2;
+    const double weight = -1.0 / (double)(P > 0 ? P : 1);
+    if ((e = cudaMemsetAsync(ws + L.red_out, 0, 64 * sizeof(double), st)) != cudaSuccess) return e;
+    return closure64_middle(noise, C, k, dist, pair_begin, pair_end, weight, L, ws + L.red_out, ws, st);
+  }
+  // phase 2: (gPsi, gMu) are now the sums over all pairs
+  return launch_project_bwd_constrained<double>(
+      ws + L.gPsi + (size_t)c0 * k * k, Mm != nullptr ? ws + L.gMu + (size_t)c0 * k : nullptr,
+      ws + L.T + (size_t)c0 * k * D, Mm != nullptr ? Mm + (size_t)c0 * D : nullptr, n_own, D, k, F, nullptr, 0, 0, dF,
+      nullptr, nullptr, nullptr, ws + L.proj, st);
 }
 
 }  // namespace sqfa

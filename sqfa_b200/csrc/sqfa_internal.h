@@ -187,6 +187,12 @@ cudaError_t launch_gauss_closure_f64(const double* S, const double* M, const dou
                                      const double* noise, int dist, int constraint, int n_fixed, int64_t pair_begin,
                                      int64_t pair_end, double* out, double* out_host, double* grad, double* ws,
                                      cudaStream_t st);
+// the class- and pair-sharded closure of closure.cu in float64, for every code of the two closures above
+void fused_loss_exchange_span_f64(int C, int D, int k, int dist, int64_t pair_begin, int64_t pair_end, int which,
+                                  size_t* offset_bytes, size_t* bytes);
+cudaError_t launch_fused_loss_sharded_f64(int phase, const double* S, const double* M, const double* F, int C, int D,
+                                          int k, const double* noise, int dist, int c0, int c1, int64_t pair_begin,
+                                          int64_t pair_end, double* dF, double* ws, cudaStream_t st);
 }  // namespace sqfa
 
 

@@ -311,9 +311,9 @@ class SecondMomentsSQFA(nn.Module):
         filters has a closed-form adjoint (Sphere: (I - f f^T)/|w| per row; Identity; FixedFilters:
         zero rows) -- torch's `orthogonal` keeps the autograd path. Saves the ~15 micro-kernels and
         the autograd engine round trip per evaluation that dominate small-C fits. A float64 parameter with
-        float64 statistics takes a float64 closure on one device for the affine-invariant / Fisher-Rao
-        distances and for the mean-covariance distances (Mahalanobis, Bhattacharyya, Hellinger), and None
-        otherwise."""
+        float64 statistics takes a float64 closure for the affine-invariant / Fisher-Rao distances and for the
+        mean-covariance distances (Mahalanobis, Bhattacharyya, Hellinger), on one device or sharded over a
+        process group like float32, and None otherwise."""
         if not parametrize_is_parametrized(self, "filters"):
             return None
         chain = list(self.parametrizations.filters)
@@ -331,10 +331,9 @@ class SecondMomentsSQFA(nn.Module):
             return None
         f64 = p.dtype == torch.float64
         # float64 (a `.double()` model): the native closures cover affine-invariant / Fisher-Rao and the
-        # mean-covariance distances on one device
+        # mean-covariance distances
         gauss64 = f64 and (dist & 15) in (_ops.DIST_MAHA, _ops.DIST_BHATT, _ops.DIST_HELL)
-        if f64 and (((dist & 15) not in (_ops.DIST_AI, _ops.DIST_FR) and not gauss64)
-                    or self._process_group is not None):
+        if f64 and (dist & 15) not in (_ops.DIST_AI, _ops.DIST_FR) and not gauss64:
             return None
         group = self._process_group
         k, D = p.shape
@@ -350,13 +349,20 @@ class SecondMomentsSQFA(nn.Module):
 
             rank, world = dist_mod.get_rank(group), dist_mod.get_world_size(group)
             p0, p1 = _ops.shard_pairs(C * (C - 1) // 2, C, rank, world)
-            ws = torch.empty(max(int(lib.sqfa_fused_loss_workspace_bytes(C, D, k, dist, p0, p1)), 1),
-                             dtype=torch.uint8, device=S.device)
+            nbytes = (_ops.closure_workspace_bytes_f64(C, D, k, dist, p0, p1) if f64
+                      else lib.sqfa_fused_loss_workspace_bytes(C, D, k, dist, p0, p1))
+            ws = torch.empty(max(int(nbytes), 1), dtype=torch.uint8, device=S.device)
             # AI / FR with at least one class per rank: the projection shards with the classes as well
             # (three small all-reduces per evaluation instead of one; SQFA_SHARD_CLASSES=0: pairs only)
             shard_classes = ((dist & 15) != _ops.DIST_LE and C >= world
                              and os.environ.get("SQFA_SHARD_CLASSES", "1") == "1")
-            eval_sharded = _ops.fused_loss_sharded_raw if shard_classes else _ops.fused_loss_raw
+            if f64:
+                # the float64 closures read the noise from the device
+                noise_arg = torch.full((1,), noise, dtype=torch.float64, device=S.device)
+                eval_sharded = _ops.fused_loss_sharded_f64_raw if shard_classes else _ops.fused_loss_f64_raw
+            else:
+                noise_arg = noise
+                eval_sharded = _ops.fused_loss_sharded_raw if shard_classes else _ops.fused_loss_raw
 
             @torch.no_grad()
             def run_sharded():
@@ -366,7 +372,7 @@ class SecondMomentsSQFA(nn.Module):
                     F = W / nrm
                 else:
                     F = W
-                packed = eval_sharded(F, S, M, noise, dist, group, ws)
+                packed = eval_sharded(F, S, M, noise_arg, dist, group, ws)
                 dF = packed[4:].view(k, D)
                 if n_fixed:
                     dF[:n_fixed] = 0.0  # frozen rows are detached in FixedFilters.forward
@@ -374,6 +380,7 @@ class SecondMomentsSQFA(nn.Module):
                 p.grad = dW
                 return torch.cat([packed[:2], dW.abs().max().view(1)])
 
+            run_sharded.dtype = p.dtype  # a float64 fit hands its loss to the optimiser in float64
             return run_sharded
 
         # single device: ONE native call per evaluation (constraint and its adjoint included), all
