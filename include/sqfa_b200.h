@@ -43,6 +43,8 @@ typedef void* sqfa_stream_t; /* cudaStream_t */
 #define SQFA_EST_EMPIRICAL 0
 #define SQFA_EST_OAS 1
 #define SQFA_EST_PACKED_GRAM 16 /* OR-ed in: the gram argument is the packed upper-tile list (below) */
+#define SQFA_EST_CENTRED_SUMS 32 /* OR-ed in (sqfa_stats_epilogue): the shift argument holds the class sums of
+                                    (x - s) for the s the Gram was centred on, and d = sums / n_c */
 
 /* `accumulate` argument of sqfa_class_gram: a bit set */
 #define SQFA_GRAM_ACCUMULATE 1 /* add to the existing content (streaming / chunked input) */
@@ -162,6 +164,31 @@ int64_t sqfa_class_gram_group_signals(int64_t n, int32_t n_dim, int32_t n_classe
  * collective on the counters above. No kernel is launched, no SM is occupied while waiting. */
 int sqfa_stream_wait_geq(sqfa_stream_t stream, const int32_t* flag, int32_t value);
 
+/* One-pass class means (the single-device sqfa_class_statistics runs these steps):
+ *   sqfa_class_pilot_shift      shift[c][j] = mean of the first min(n_c, 32) rows of class c in bucket order
+ *                               (0 for an empty class); rows added in a fixed order
+ *   sqfa_class_gram_sums        sqfa_class_gram (shift, accumulate 0, no completion counters) whose
+ *                               diagonal tiles also write class-sum partials of (x - shift) into
+ *                               partials[n_classes][nsplit][n_dim], nsplit = sqfa_class_gram_sum_splits(...);
+ *                               X is read once for both. The partials are zeroed by the call.
+ *                               nsplit = 0: the Gram would be split into more than 16 K parts (classes of
+ *                               ~10^5 rows); sqfa_class_gram_sums returns SQFA_E_UNSUPPORTED and
+ *                               sqfa_class_statistics takes the two passes (sums, means, Gram on the means).
+ *   sqfa_class_means_from_partials
+ *                               sums[c][j] = sum over the nsplit partials (float64, in order), then
+ *                               means[c][j] = sums[c][j] / counts[c] + shift[c][j]   (NaN when empty)
+ * followed by sqfa_stats_epilogue(shift = sums, estimator | SQFA_EST_CENTRED_SUMS). The Gram needs a shift
+ * close to the class mean, not the mean itself: the epilogue takes n d d^T (d = sums / n) off it. */
+int32_t sqfa_class_gram_sum_splits(int64_t n, int32_t n_dim, int32_t n_classes);
+int sqfa_class_pilot_shift(const float* X, int64_t ldx, const int32_t* perm, const int64_t* offsets, int32_t n_dim,
+                           int32_t n_classes, float* shift, sqfa_stream_t stream);
+int sqfa_class_gram_sums(const float* X, int64_t ldx, const int32_t* perm, const int64_t* offsets, const float* shift,
+                         int64_t n, int32_t n_dim, int32_t n_classes, float* gram, float* partials, void* ws,
+                         size_t ws_bytes, sqfa_stream_t stream);
+int sqfa_class_means_from_partials(const float* partials, int32_t nsplit, const int64_t* counts, const float* shift,
+                                   int32_t n_dim, int32_t n_classes, float* sums, float* means,
+                                   sqfa_stream_t stream);
+
 /* Class counts as two exact float32 words, out[c] = counts[c] / 2^20 and out[n_classes + c] = counts[c] mod
  * 2^20, so that a multi-device caller sums [class sums | counts] of its ranks in ONE float32 all-reduce;
  * sqfa_counts_unpack turns the summed words back into int64 (exact below 2^44 rows). */
@@ -197,12 +224,13 @@ int sqfa_stats_epilogue_reduce(const float* gram, const float* peer_slots, int64
 /* cudaMemcpyAsync(dst, src, bytes) on `stream` (copy engine; dst may be peer-mapped device memory). */
 int sqfa_peer_push(void* dst, const void* src, size_t bytes, sqfa_stream_t stream);
 
-/* class_statistics in ONE call (statistics.py:8-54) for n rows resident on one device: bucket the
- * labels, per-class sums and means, Gram of the rows centred by their class mean, epilogue. It is
- * exactly the sequence sqfa_bucket_labels -> sqfa_class_sums -> sqfa_class_means ->
- * sqfa_class_gram (shift = means) -> sqfa_stats_epilogue enqueued on `stream` from one host call
- * (no host round trips between the steps); multi-device callers use the separate entry points and
- * all-reduce the partial sums between them.
+/* class_statistics in ONE call (statistics.py:8-54) for n rows resident on one device, in one pass over X
+ * (two where sqfa_class_gram_sum_splits is 0, see above):
+ * bucket the labels, pilot shift, Gram of the rows centred by it with the class sums on the side, means,
+ * epilogue. It is exactly the sequence sqfa_bucket_labels -> sqfa_class_pilot_shift -> sqfa_class_gram_sums
+ * -> sqfa_class_means_from_partials -> sqfa_stats_epilogue (shift = the pilot shift) enqueued on `stream`
+ * from one host call (no host round trips between the steps); multi-device callers use the two-pass entry
+ * points (sqfa_class_sums, sqfa_class_gram) and all-reduce the partial sums between them.
  *   means   (n_classes, n_dim)          out
  *   cov     (n_classes, n_dim, n_dim)   out (the Gram is accumulated here, then finalised in place)
  *   sm      (n_classes, n_dim, n_dim)   out, may be NULL
@@ -241,6 +269,12 @@ int sqfa_class_gram_h(const void* X, int64_t ldx, int32_t elem, const int32_t* p
 int64_t sqfa_class_gram_group_signals_h(int64_t n, int32_t n_dim, int32_t n_classes, int32_t n_groups, int32_t group,
                                         int32_t elem);
 size_t sqfa_class_statistics_workspace_bytes_h(int64_t n, int32_t n_dim, int32_t n_classes, int32_t elem);
+int32_t sqfa_class_gram_sum_splits_h(int64_t n, int32_t n_dim, int32_t n_classes, int32_t elem);
+int sqfa_class_pilot_shift_h(const void* X, int64_t ldx, int32_t elem, const int32_t* perm, const int64_t* offsets,
+                             int32_t n_dim, int32_t n_classes, float* shift, sqfa_stream_t stream);
+int sqfa_class_gram_sums_h(const void* X, int64_t ldx, int32_t elem, const int32_t* perm, const int64_t* offsets,
+                           const float* shift, int64_t n, int32_t n_dim, int32_t n_classes, float* gram,
+                           float* partials, void* ws, size_t ws_bytes, sqfa_stream_t stream);
 int sqfa_class_statistics_h(const void* X, int64_t ldx, int32_t elem, const int64_t* labels, int64_t n, int32_t n_dim,
                             int32_t n_classes, int estimator, int ddof, float* means, float* cov, float* sm,
                             int64_t* counts, int64_t* offsets, int32_t* perm, void* ws, size_t ws_bytes,

@@ -51,6 +51,19 @@ SIGNATURES = {
     "sqfa_stream_wait_geq": (c_int, [c_ptr, c_ptr, c_i32]),
     "sqfa_gram_packed_floats": (c_size, [c_i32, c_i32]),
     "sqfa_gram_executed_tile_area": (c_i64, [c_i32]),
+    "sqfa_class_gram_sum_splits": (c_i32, [c_i64, c_i32, c_i32]),
+    "sqfa_class_pilot_shift": (c_int, [c_ptr, c_i64, c_ptr, c_ptr, c_i32, c_i32, c_ptr, c_ptr]),
+    "sqfa_class_gram_sums": (
+        c_int,
+        [c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_i64, c_i32, c_i32, c_ptr, c_ptr, c_ptr, c_size, c_ptr],
+    ),
+    "sqfa_class_means_from_partials": (c_int, [c_ptr, c_i32, c_ptr, c_ptr, c_i32, c_i32, c_ptr, c_ptr, c_ptr]),
+    "sqfa_class_gram_sum_splits_h": (c_i32, [c_i64, c_i32, c_i32, c_i32]),
+    "sqfa_class_pilot_shift_h": (c_int, [c_ptr, c_i64, c_i32, c_ptr, c_ptr, c_i32, c_i32, c_ptr, c_ptr]),
+    "sqfa_class_gram_sums_h": (
+        c_int,
+        [c_ptr, c_i64, c_i32, c_ptr, c_ptr, c_ptr, c_i64, c_i32, c_i32, c_ptr, c_ptr, c_ptr, c_size, c_ptr],
+    ),
     "sqfa_counts_pack": (c_int, [c_ptr, c_i32, c_ptr, c_ptr]),
     "sqfa_counts_unpack": (c_int, [c_ptr, c_i32, c_ptr, c_ptr]),
     "sqfa_stats_epilogue_workspace_bytes": (c_size, [c_i32]),

@@ -159,6 +159,57 @@ class CudaStatsOps:
         )
         return means
 
+    def pilot_shift(self, X, perm, offsets, C):
+        """Centring vectors of the one-pass path: the mean of the first min(n_c, 32) rows of each class."""
+        dev = X.device
+        shift = torch.empty(C, X.shape[1], dtype=torch.float32, device=dev)
+        fn, xa = self._x_fn("sqfa_class_pilot_shift")
+        _lib.check(fn(*xa(X), _lib.ptr(perm), _lib.ptr(offsets), X.shape[1], C, _lib.ptr(shift), _lib.stream_ptr(dev)),
+                   "sqfa_class_pilot_shift")
+        return shift
+
+    def one_pass_splits(self, X, C):
+        """Class-sum partials per class of `class_gram_sums` (0: this shape keeps the two passes)."""
+        return self._query("sqfa_class_gram_sum_splits", X.shape[0], X.shape[1], C)
+
+    def class_gram_sums(self, X, perm, offsets, shift, C):
+        """`class_gram` (centred on `shift`) whose diagonal tiles also write the class sums of x - shift as
+        partials [C, nsplit, D]: the one pass over X of single-device class_statistics. Returns (gram, partials)."""
+        dev = X.device
+        n, D = X.shape
+        nsplit = self._query("sqfa_class_gram_sum_splits", n, D, C)
+        gram = torch.empty(C, D, D, dtype=torch.float32, device=dev)
+        partials = torch.empty(C, nsplit, D, dtype=torch.float32, device=dev)
+        ws_bytes = self._query("sqfa_class_gram_workspace_bytes", n, D, C)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        if self.gram_events is not None:
+            ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
+            ev[0].record()
+        fn, xa = self._x_fn("sqfa_class_gram_sums")
+        _lib.check(
+            fn(*xa(X), _lib.ptr(perm), _lib.ptr(offsets), _lib.ptr(shift), n, D, C, _lib.ptr(gram), _lib.ptr(partials),
+               _lib.ptr(ws), ws_bytes, _lib.stream_ptr(dev)),
+            "sqfa_class_gram_sums",
+        )
+        if self.gram_events is not None:
+            ev[1].record()
+            self.gram_events.append(ev)
+        return gram, partials
+
+    def means_from_partials(self, partials, counts, shift):
+        """(means, sums): sums = the class sums of x - shift (sum of the partials), means = shift + sums / counts."""
+        C, nsplit, D = partials.shape
+        sums = torch.empty(C, D, dtype=torch.float32, device=partials.device)
+        means = torch.empty_like(sums)
+        _lib.check(
+            self.lib.sqfa_class_means_from_partials(
+                _lib.ptr(partials), nsplit, _lib.ptr(counts), _lib.ptr(shift), D, C, _lib.ptr(sums), _lib.ptr(means),
+                _lib.stream_ptr(partials.device),
+            ),
+            "sqfa_class_means_from_partials",
+        )
+        return means, sums
+
     supports_packed = True  # class_gram / finalize understand the packed upper-tile layout
 
     def packed_is_smaller(self, D, C):
@@ -388,9 +439,10 @@ class CudaStatsOps:
         st["free"][k] = ev
         return cov, sm
 
-    def finalize(self, gram, means, counts, estimator_id, ddof, want_sm, packed=False, class_range=None):
+    def finalize(self, gram, means, counts, estimator_id, ddof, want_sm, packed=False, class_range=None, centred_sums=None):
         """cov (in place over gram unless it is packed; mirrored), optional OAS shrinkage, second moments.
-        `class_range` (c0, c1): only those classes (a rank finalising its share of a sharded result)."""
+        `class_range` (c0, c1): only those classes (a rank finalising its share of a sharded result).
+        `centred_sums`: the class sums of (x - s) when gram was centred on vectors s other than the means."""
         lib, dev = self.lib, gram.device
         C, D = means.shape
         c0, c1 = (0, C) if class_range is None else class_range
@@ -406,12 +458,13 @@ class CudaStatsOps:
         if nc == 0:
             return cov, sm
         means_part, counts_part = means[c0:c1], counts[c0:c1]
+        sums_part = None if centred_sums is None else centred_sums[c0:c1]
         ws_bytes = lib.sqfa_stats_epilogue_workspace_bytes(nc)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         _lib.check(
             lib.sqfa_stats_epilogue(
-                _lib.ptr(gram_part), _lib.ptr(means_part), None, _lib.ptr(counts_part), D, nc,
-                estimator_id | (16 if packed else 0), ddof, _lib.ptr(cov), _lib.ptr(sm), _lib.ptr(ws), ws_bytes,
+                _lib.ptr(gram_part), _lib.ptr(means_part), _lib.ptr(sums_part), _lib.ptr(counts_part), D, nc,
+                estimator_id | (16 if packed else 0) | (32 if centred_sums is not None else 0), ddof, _lib.ptr(cov), _lib.ptr(sm), _lib.ptr(ws), ws_bytes,
                 _lib.stream_ptr(dev),
             ),
             "sqfa_stats_epilogue",
@@ -453,6 +506,7 @@ class CudaStatsOps64(CudaStatsOps):
     maximum are dtype-independent and inherited; there is no packed Gram and no one-call fused path."""
 
     supports_packed = False
+    class_gram_sums = None  # float64 keeps its two passes
     fused = None
     fused_prepare = None
     counts_pack = None
@@ -540,8 +594,13 @@ def run_class_statistics(ops, X, y, estimator_id, group=None, n_classes=None, dd
     rows held by all ranks (every rank returns the full global result, or -- `shard_output` -- the
     means of all classes and the covariances / second moments of its `class_share`).
 
-    Two passes over the local rows, like the reference (mean first, then the Gram of the centred
-    rows, statistics.py:118-120). `centre` (C, D) overrides the centring vectors.
+    On one device without `centre`, ONE pass over the rows: the Gram is centred on a pilot shift (the mean
+    of each class's first 32 rows) and writes the class sums of x - shift on the way; mean = shift + sums / n
+    and the epilogue takes n d d^T (d = mean - shift) off the Gram. That is what the single call
+    `sqfa_class_statistics` runs, step by step. Otherwise two passes over the local rows, like the
+    reference (mean first, then the Gram of the centred rows, statistics.py:118-120): a process group
+    all-reduces the sums before the Gram so that every rank centres on the same means. `centre` (C, D)
+    overrides the centring vectors.
     """
     prepared = None
     if n_classes is None:
@@ -588,6 +647,14 @@ def run_class_statistics(ops, X, y, estimator_id, group=None, n_classes=None, dd
         return ops.fused(X, y, C, estimator_id, ddof, want_sm, prepared)
     perm, offsets, counts = ops.bucket(y, C)
     D = X.shape[1]
+    if (group is None and centre is None and getattr(ops, "class_gram_sums", None) is not None
+            and ops.one_pass_splits(X, C) > 0):
+        class_counts = counts[:C].clone()
+        shift = ops.pilot_shift(X, perm, offsets, C)
+        gram, partials = ops.class_gram_sums(X, perm, offsets, shift, C)
+        means, sums = ops.means_from_partials(partials, class_counts, shift)
+        cov, sm = ops.finalize(gram, means, class_counts, estimator_id, ddof, want_sm, centred_sums=sums)
+        return means, cov, sm, (perm, offsets, counts)
     lease = None
     if (group is not None and shard_output and centre is None and getattr(ops, "peer_acquire", None) is not None
             and getattr(ops, "supports_packed", False) and ops.packed_is_smaller(D, C)

@@ -50,7 +50,11 @@ int class_sums_impl(const char* fn, const void* X, int elem, int64_t ldx, const 
 int class_gram_impl(const char* fn, const void* X, int elem, int64_t ldx, const int32_t* perm,
                     const int64_t* offsets, const float* shift, int64_t n, int32_t n_dim, int32_t n_classes,
                     float* gram, int accumulate, int chain_rows, int32_t* done, int32_t n_groups,
-                    int32_t first_class, int32_t reserve_sms, void* ws, size_t ws_bytes, sqfa_stream_t stream);
+                    int32_t first_class, int32_t reserve_sms, void* ws, size_t ws_bytes, sqfa_stream_t stream,
+                    float* sum_partials = nullptr);
+int class_pilot_shift_impl(const char* fn, const void* X, int elem, int64_t ldx, const int32_t* perm,
+                           const int64_t* offsets, int32_t n_dim, int32_t n_classes, float* shift, sqfa_stream_t stream);
+int32_t class_gram_sum_splits(int64_t n, int32_t n_dim, int32_t n_classes, int elem);
 size_t class_gram_ws(int64_t n, int32_t n_dim, int32_t n_classes, int elem);
 int64_t class_gram_signals(int64_t n, int32_t n_dim, int32_t n_classes, int32_t n_groups, int32_t group, int elem);
 size_t class_statistics_ws(int64_t n, int32_t n_dim, int32_t n_classes, int elem);
@@ -168,6 +172,60 @@ int64_t sqfa_class_gram_group_signals_h(int64_t n, int32_t n_dim, int32_t n_clas
   return e < 0 ? 0 : class_gram_signals(n, n_dim, n_classes, n_groups, group, e);
 }
 
+int32_t sqfa_class_gram_sum_splits(int64_t n, int32_t n_dim, int32_t n_classes) {
+  return class_gram_sum_splits(n, n_dim, n_classes, sqfa::ELEM_F32);
+}
+
+int32_t sqfa_class_gram_sum_splits_h(int64_t n, int32_t n_dim, int32_t n_classes, int32_t elem) {
+  const int e = half_elem(__func__, elem);
+  return e < 0 ? 0 : class_gram_sum_splits(n, n_dim, n_classes, e);
+}
+
+int sqfa_class_pilot_shift(const float* X, int64_t ldx, const int32_t* perm, const int64_t* offsets, int32_t n_dim,
+                           int32_t n_classes, float* shift, sqfa_stream_t stream) {
+  return class_pilot_shift_impl(__func__, X, sqfa::ELEM_F32, ldx, perm, offsets, n_dim, n_classes, shift, stream);
+}
+
+int sqfa_class_pilot_shift_h(const void* X, int64_t ldx, int32_t elem, const int32_t* perm, const int64_t* offsets,
+                             int32_t n_dim, int32_t n_classes, float* shift, sqfa_stream_t stream) {
+  const int e = half_elem(__func__, elem);
+  if (e < 0) return SQFA_E_INVALID;
+  return class_pilot_shift_impl(__func__, X, e, ldx, perm, offsets, n_dim, n_classes, shift, stream);
+}
+
+int sqfa_class_gram_sums(const float* X, int64_t ldx, const int32_t* perm, const int64_t* offsets, const float* shift,
+                         int64_t n, int32_t n_dim, int32_t n_classes, float* gram, float* partials, void* ws,
+                         size_t ws_bytes, sqfa_stream_t stream) {
+  if (partials == nullptr || shift == nullptr) return fail_arg(__func__, "bad argument");
+  if (class_gram_sum_splits(n, n_dim, n_classes, sqfa::ELEM_F32) == 0)
+    return fail_arg(__func__, "K split too deep for class-sum partials", SQFA_E_UNSUPPORTED);
+  return class_gram_impl(__func__, X, sqfa::ELEM_F32, ldx, perm, offsets, shift, n, n_dim, n_classes, gram, 0, 0,
+                         nullptr, 0, 0, 0, ws, ws_bytes, stream, partials);
+}
+
+int sqfa_class_gram_sums_h(const void* X, int64_t ldx, int32_t elem, const int32_t* perm, const int64_t* offsets,
+                           const float* shift, int64_t n, int32_t n_dim, int32_t n_classes, float* gram,
+                           float* partials, void* ws, size_t ws_bytes, sqfa_stream_t stream) {
+  const int e = half_elem(__func__, elem);
+  if (e < 0) return SQFA_E_INVALID;
+  if (partials == nullptr || shift == nullptr) return fail_arg(__func__, "bad argument");
+  if (class_gram_sum_splits(n, n_dim, n_classes, e) == 0)
+    return fail_arg(__func__, "K split too deep for class-sum partials", SQFA_E_UNSUPPORTED);
+  return class_gram_impl(__func__, X, e, ldx, perm, offsets, shift, n, n_dim, n_classes, gram, 0, 0, nullptr, 0, 0, 0,
+                         ws, ws_bytes, stream, partials);
+}
+
+int sqfa_class_means_from_partials(const float* partials, int32_t nsplit, const int64_t* counts, const float* shift,
+                                   int32_t n_dim, int32_t n_classes, float* sums, float* means,
+                                   sqfa_stream_t stream) {
+  if (partials == nullptr || nsplit <= 0 || counts == nullptr || shift == nullptr || sums == nullptr ||
+      means == nullptr || n_dim <= 0 || n_classes < 0)
+    return fail_arg(__func__, "bad argument");
+  const cudaError_t e = sqfa::launch_class_sums_finalize(partials, nsplit, n_dim, n_classes, sums, S(stream));
+  if (e != cudaSuccess) return wrap(__func__, e);
+  return wrap(__func__, sqfa::launch_class_means(sums, counts, shift, n_dim, n_classes, means, S(stream)));
+}
+
 // cuStreamWaitValue32 through the runtime's driver entry point lookup (no link dependency on libcuda)
 int sqfa_stream_wait_geq(sqfa_stream_t stream, const int32_t* flag, int32_t value) {
   if (flag == nullptr) return fail_arg(__func__, "bad argument");
@@ -207,15 +265,17 @@ int sqfa_stats_epilogue(const float* gram, const float* means, const float* shif
                         int32_t n_dim, int32_t n_classes, int estimator, int ddof, float* cov, float* sm, void* ws,
                         size_t ws_bytes, sqfa_stream_t stream) {
   const int packed = estimator & SQFA_EST_PACKED_GRAM;
-  estimator &= ~SQFA_EST_PACKED_GRAM;
+  const int centred_sums = estimator & SQFA_EST_CENTRED_SUMS;
+  estimator &= ~(SQFA_EST_PACKED_GRAM | SQFA_EST_CENTRED_SUMS);
   if (gram == nullptr || means == nullptr || counts == nullptr || cov == nullptr || n_dim <= 0 || n_classes < 0 ||
       (estimator != SQFA_EST_EMPIRICAL && estimator != SQFA_EST_OAS) || (ddof != 0 && ddof != 1) ||
-      (packed && cov == gram))
+      (packed && cov == gram) || (centred_sums && shift == nullptr))
     return fail_arg(__func__, "bad argument");
   if (estimator == SQFA_EST_OAS && (ws == nullptr || ws_bytes < sqfa::stats_epilogue_workspace_bytes(n_classes)))
     return fail_arg(__func__, "workspace too small", SQFA_E_WORKSPACE);
   return wrap(__func__, sqfa::launch_stats_epilogue(gram, packed, means, shift, counts, n_dim, n_classes, estimator,
-                                                    ddof, cov, sm, ws, S(stream)));
+                                                    ddof, cov, sm, ws, S(stream), sqfa::GramSources{nullptr, 0, 0, 0},
+                                                    centred_sums ? 1 : 0));
 }
 
 int sqfa_stats_epilogue_reduce(const float* gram, const float* peer_slots, int64_t slot_stride, int32_t n_sources,
@@ -784,7 +844,8 @@ size_t class_gram_ws(int64_t n, int32_t n_dim, int32_t n_classes, int elem) {
 int class_gram_impl(const char* fn, const void* X, int elem, int64_t ldx, const int32_t* perm,
                     const int64_t* offsets, const float* shift, int64_t n, int32_t n_dim, int32_t n_classes,
                     float* gram, int accumulate, int chain_rows, int32_t* done, int32_t n_groups,
-                    int32_t first_class, int32_t reserve_sms, void* ws, size_t ws_bytes, sqfa_stream_t stream) {
+                    int32_t first_class, int32_t reserve_sms, void* ws, size_t ws_bytes, sqfa_stream_t stream,
+                    float* sum_partials) {
   if (n_dim <= 0 || n_classes < 0 || offsets == nullptr || gram == nullptr || ws == nullptr || ldx < n_dim ||
       X == nullptr || perm == nullptr || (accumulate & ~(SQFA_GRAM_ACCUMULATE | SQFA_GRAM_PACKED)) ||
       (done != nullptr && (n_groups <= 0 || n_groups > 65536)) || reserve_sms < 0 || first_class < 0 ||
@@ -798,7 +859,26 @@ int class_gram_impl(const char* fn, const void* X, int elem, int64_t ldx, const 
   if (sms <= 0) return fail_arg(fn, "no CUDA device");
   return wrap(fn, sqfa::launch_class_gram(X, elem, ldx, perm, offsets, shift, n, n_dim, n_classes, gram,
                                           accumulate & SQFA_GRAM_ACCUMULATE, accumulate & SQFA_GRAM_PACKED, chain_rows,
-                                          done, n_groups, first_class, reserve_sms, ws, sms, S(stream)));
+                                          done, n_groups, first_class, reserve_sms, ws, sms, S(stream), sum_partials));
+}
+
+int class_pilot_shift_impl(const char* fn, const void* X, int elem, int64_t ldx, const int32_t* perm,
+                           const int64_t* offsets, int32_t n_dim, int32_t n_classes, float* shift, sqfa_stream_t stream) {
+  if (X == nullptr || perm == nullptr || offsets == nullptr || shift == nullptr || n_dim <= 0 || n_classes < 0 ||
+      ldx < n_dim)
+    return fail_arg(fn, "bad argument");
+  return wrap(fn, sqfa::launch_class_pilot_shift(X, elem, ldx, perm, offsets, n_dim, n_classes, shift, S(stream)));
+}
+
+// class-sum partials per class that sqfa_class_gram_sums writes: 4 sample quads x the launch's K parts; 0 when
+// the Gram is split into more than kOnePassMaxKsplit K parts (classes of ~10^5 rows, the c5 shard): the partials
+// would outgrow the workspace the two-pass sums use, and those shapes keep the two passes
+constexpr int kOnePassMaxKsplit = 16;
+int32_t class_gram_sum_splits(int64_t n, int32_t n_dim, int32_t n_classes, int elem) {
+  if (n_dim <= 0 || n_classes <= 0) return 0;
+  const int sms = sm_count_cached();
+  const int ks = sqfa::gram_ksplit_launch(n < 0 ? 0 : n, n_classes, n_dim, 0, sms > 0 ? sms : 148, sqfa::elem_bytes(elem));
+  return ks <= kOnePassMaxKsplit ? 4 * ks : 0;
 }
 
 int64_t class_gram_signals(int64_t n, int32_t n_dim, int32_t n_classes, int32_t n_groups, int32_t group, int elem) {
@@ -815,7 +895,13 @@ struct StatsWs { size_t bucket, sums_ws, sums, gram, epi, total; };
 inline StatsWs stats_ws(int64_t n, int32_t D, int32_t C, int elem) {
   StatsWs w;
   w.bucket = align256(sqfa_bucket_workspace_bytes(n, C));
-  w.sums_ws = align256(sqfa_class_sums_workspace_bytes(n, D, C));
+  // the one-pass path keeps the pilot shift and the Gram's class-sum partials where the two-pass sums kept theirs
+  const size_t splits = (size_t)class_gram_sum_splits(n, D, C, elem);
+  const size_t one_pass = splits == 0 ? 0
+                                      : align256((size_t)C * (size_t)D * sizeof(float)) +
+                                            splits * (size_t)C * (size_t)D * sizeof(float);
+  const size_t two_pass = sqfa_class_sums_workspace_bytes(n, D, C);
+  w.sums_ws = align256(one_pass > two_pass ? one_pass : two_pass);
   w.sums = align256((size_t)(C > 0 ? C : 1) * (size_t)(D > 0 ? D : 1) * sizeof(float));
   w.gram = align256(class_gram_ws(n, D, C, elem));
   w.epi = align256(sqfa_stats_epilogue_workspace_bytes(C));
@@ -838,23 +924,40 @@ int class_statistics_impl(const char* fn, const void* X, int elem, int64_t ldx, 
   if (ws_bytes < w.total) return fail_arg(fn, "workspace too small", SQFA_E_WORKSPACE);
   uint8_t* p = static_cast<uint8_t*>(ws);
   void* ws_bucket = p;
-  void* ws_sums = p + w.bucket;
+  float* shift = reinterpret_cast<float*>(p + w.bucket);
+  float* partials = reinterpret_cast<float*>(p + w.bucket + align256((size_t)n_classes * (size_t)n_dim * sizeof(float)));
   float* sums = reinterpret_cast<float*>(p + w.bucket + w.sums_ws);
   void* ws_gram = p + w.bucket + w.sums_ws + w.sums;
   void* ws_epi = p + w.bucket + w.sums_ws + w.sums + w.gram;
   int rc = sqfa_bucket_labels(labels, n, n_classes, counts, offsets, perm, ws_bucket, w.bucket, stream);
   if (rc) return rc;
-  const bool f32 = elem == sqfa::ELEM_F32;  // failures name the step, as the step's own entry point would
-  rc = class_sums_impl(f32 ? "sqfa_class_sums" : "sqfa_class_sums_h", X, elem, ldx, perm, offsets, nullptr, n, n_dim, n_classes, sums, 0, ws_sums, w.sums_ws,
-                       stream);
+  // One pass over X: the Gram centres on a pilot shift s (the first rows of each class) and its diagonal
+  // tiles write the class sums of x - s on the way; mean = s + sums / n, and the epilogue takes n d d^T,
+  // d = mean - s, off the Gram. Failures name the step, as the step's own entry point would.
+  const bool f32 = elem == sqfa::ELEM_F32;
+  const int32_t splits = class_gram_sum_splits(n, n_dim, n_classes, elem);
+  if (splits == 0) {  // deep K split: sums, means, then the Gram centred on the means
+    rc = class_sums_impl(f32 ? "sqfa_class_sums" : "sqfa_class_sums_h", X, elem, ldx, perm, offsets, nullptr, n, n_dim,
+                         n_classes, sums, 0, shift, w.sums_ws, stream);
+    if (rc) return rc;
+    rc = sqfa_class_means(sums, counts, nullptr, n_dim, n_classes, means, stream);
+    if (rc) return rc;
+    rc = class_gram_impl(f32 ? "sqfa_class_gram" : "sqfa_class_gram_h", X, elem, ldx, perm, offsets, means, n, n_dim,
+                         n_classes, cov, 0, 0, nullptr, 0, 0, 0, ws_gram, w.gram, stream);
+    if (rc) return rc;
+    return sqfa_stats_epilogue(cov, means, nullptr, counts, n_dim, n_classes, estimator, ddof, cov, sm, ws_epi, w.epi,
+                               stream);
+  }
+  rc = class_pilot_shift_impl(f32 ? "sqfa_class_pilot_shift" : "sqfa_class_pilot_shift_h", X, elem, ldx, perm,
+                              offsets, n_dim, n_classes, shift, stream);
   if (rc) return rc;
-  rc = sqfa_class_means(sums, counts, nullptr, n_dim, n_classes, means, stream);
+  rc = class_gram_impl(f32 ? "sqfa_class_gram_sums" : "sqfa_class_gram_sums_h", X, elem, ldx, perm, offsets, shift, n,
+                       n_dim, n_classes, cov, 0, 0, nullptr, 0, 0, 0, ws_gram, w.gram, stream, partials);
   if (rc) return rc;
-  rc = class_gram_impl(f32 ? "sqfa_class_gram" : "sqfa_class_gram_h", X, elem, ldx, perm, offsets, means, n, n_dim, n_classes, cov, 0, 0, nullptr, 0, 0, 0,
-                       ws_gram, w.gram, stream);
+  rc = sqfa_class_means_from_partials(partials, splits, counts, shift, n_dim, n_classes, sums, means, stream);
   if (rc) return rc;
-  return sqfa_stats_epilogue(cov, means, nullptr, counts, n_dim, n_classes, estimator, ddof, cov, sm, ws_epi, w.epi,
-                             stream);
+  return sqfa_stats_epilogue(cov, means, sums, counts, n_dim, n_classes, estimator | SQFA_EST_CENTRED_SUMS, ddof, cov,
+                             sm, ws_epi, w.epi, stream);
 }
 
 }  // namespace

@@ -82,6 +82,8 @@ struct GramParams {
   const int64_t* offsets;
   const float* shift;
   float* gram;
+  float* sums;       // optional class-sum partials [C][KS][4][D]: sum of (x - shift) over the samples of one
+                     //   K part that one sample quad of a diagonal tile saw (see produce)
   int32_t* done;     // optional completion counters: done[c G / C] += 1 per (job, CTA, epilogue warp) once the
   int n_groups;      //   job's tile is stored -- a collective on another stream can be gated on a class group
   int class_order;   // jobs in class order (so class groups finish in order) instead of largest class first
@@ -97,7 +99,7 @@ struct GramParams {
   int vecx;          // rows of X are aligned to 4 elements: LDG.128 (float32) / LDG.64 (bf16, fp16)
   int flags;         // tuning switches (env SQFA_GRAM_FLAGS): 1 = no A-as-B reuse on diagonal tiles,
                      // 2 = A / B producer warps share the A operand of diagonal tiles, 4 = scalar loads,
-                     // 8 = no early cross-term MMAs during a chain drain
+                     // 8 = no early cross-term MMAs during a chain drain (1 and 2 are off with `sums`)
 };
 
 __device__ __forceinline__ uint32_t ldg_nc_u16(const void* p) {  // zero-extended
@@ -183,7 +185,7 @@ struct JobGeom {
   int c, m0, n0, n_eff, nh;
   bool diag;  // full diagonal tile: each CTA's B half is the same data as its A operand
   int64_t row_begin, n_c;
-  int kb0, kb1;
+  int ks, kb0, kb1;
 };
 
 template <int TM, int TN>
@@ -199,6 +201,7 @@ __device__ __forceinline__ JobGeom decode_job(const GramParams& P, int j) {
   g.row_begin = P.offsets[g.c];
   g.n_c = P.offsets[g.c + 1] - g.row_begin;
   const int nkb_total = (int)((g.n_c + BK - 1) / BK);
+  g.ks = jb.w;
   g.kb0 = (int)(((int64_t)jb.w * nkb_total) / P.KS);
   g.kb1 = (int)(((int64_t)(jb.w + 1) * nkb_total) / P.KS);
   return g;
@@ -277,7 +280,13 @@ __device__ __forceinline__ void gram_body(const GramParams& P) {
       // of the job and the B warp the odd ones -- twice the global loads in flight on diagonal tiles.
       // Measured: c5 shard 77.0 -> 73.0 ms, c4 2.20 -> 2.43 ms, c2 / c3 unchanged; off by default.
       const bool share = g.diag && (P.flags & 2);
-      if (g.diag && !isA && !share) {
+      // Class sums: every column of a class lies in exactly one diagonal tile (tm == tn) per K part, where
+      // the B warps have no operand to produce. There they load the A warp's samples and columns again (L2
+      // hits) and add up x - s (fixed order) while keeping the barrier protocol going; each stores its
+      // float4 at the end of the job, one slot per (class, K part, quad, column): no atomics, and an empty
+      // K part stores zeros. The A producers and the off-diagonal jobs run exactly as without sums.
+      const bool sum_job = P.sums != nullptr && g.diag && !isA;
+      if (g.diag && !isA && !share && !sum_job) {
         for (int kb = kb0; kb < kb1; ++kb) {
           mbar_wait(&empty_bar[stage], phase ^ 1);
           __syncwarp();
@@ -286,7 +295,7 @@ __device__ __forceinline__ void gram_body(const GramParams& P) {
         }
         continue;
       }
-      const bool asA = isA || share;
+      const bool asA = isA || share || sum_job;
       const uint32_t hi_base = asA ? hi_A : hi_B;
       const uint32_t lo_base = hi_base + OP_BYTES;  // 32-bit shared addresses: no 64-bit math in the loop
       const int col = (asA ? g.m0 : g.n0) + 128 * (int)rank + 4 * lane;  // first of this thread's 4 columns
@@ -307,9 +316,11 @@ __device__ __forceinline__ void gram_body(const GramParams& P) {
       // per-load branches); scalar loads only in the last column tile of a D not divisible by 4
       const bool fastw = __all_sync(0xffffffffu, vecx && (ncol == 4 || ncol == 0));
 
-      auto produce = [&](auto fast_tag, auto share_tag) {
+      auto produce = [&](auto fast_tag, auto share_tag, auto sum_tag) {
         constexpr bool FAST = decltype(fast_tag)::value;
         constexpr bool SHARE = decltype(share_tag)::value;
+        constexpr bool SUM = decltype(sum_tag)::value;  // sums only: nothing is stored to shared memory
+        float4 psum = make_float4(0.f, 0.f, 0.f, 0.f);
         constexpr int S = SHARE ? 2 : 1;          // stride between the stages this warp produces
         const int off = (SHARE && !isA) ? 1 : 0;  // its first stage, relative to kb0
         // Register pipeline. ptxas tracks every global load of this loop on ONE scoreboard, so the
@@ -370,6 +381,11 @@ __device__ __forceinline__ void gram_body(const GramParams& P) {
             ++ring_kb;
           }
           mbar_wait(&empty_bar[stage], phase ^ 1);
+          if constexpr (SUM) {  // the stage's arrival does not wait for this warp's loads
+            __syncwarp();
+            if (lane == 0) mbar_arrive_cluster(full0 + stage * 8);
+            if (++stage == STAGES2) { stage = 0; phase ^= 1; }
+          }
           float4 b[4];
 #pragma unroll
           for (int r = 0; r < 4; ++r) b[r] = Load::widen(bq[r]);
@@ -379,6 +395,13 @@ __device__ __forceinline__ void gram_body(const GramParams& P) {
 #pragma unroll
             for (int r = 0; r < 4; ++r)
               if (r >= (int)nv) b[r] = z;
+          }
+          if constexpr (SUM) {  // padded samples are exactly zero after centring
+            psum.x += ((b[0].x - sh.x) + (b[1].x - sh.x)) + ((b[2].x - sh.x) + (b[3].x - sh.x));
+            psum.y += ((b[0].y - sh.y) + (b[1].y - sh.y)) + ((b[2].y - sh.y) + (b[3].y - sh.y));
+            psum.z += ((b[0].z - sh.z) + (b[1].z - sh.z)) + ((b[2].z - sh.z) + (b[3].z - sh.z));
+            psum.w += ((b[0].w - sh.w) + (b[1].w - sh.w)) + ((b[2].w - sh.w) + (b[3].w - sh.w));
+            return;
           }
           const uint32_t hp = hi_base + stage * STAGE2_BYTES;
           const uint32_t lp = lo_base + stage * STAGE2_BYTES;
@@ -411,11 +434,22 @@ __device__ __forceinline__ void gram_body(const GramParams& P) {
         if constexpr (SHARE) {
           while (ring_kb < kb1) skip_stage();  // trailing stages of the other warp
         }
+        if constexpr (SUM) {
+          float* const out = P.sums + (((int64_t)g.c * P.KS + g.ks) * 4 + quad) * D + col;
+          if (ncol > 0) out[0] = psum.x;
+          if (ncol > 1) out[1] = psum.y;
+          if (ncol > 2) out[2] = psum.z;
+          if (ncol > 3) out[3] = psum.w;
+        }
       };
+      using T_ = std::true_type;
+      using F_ = std::false_type;
       if (share) {
-        if (fastw) produce(std::true_type{}, std::true_type{}); else produce(std::false_type{}, std::true_type{});
+        if (fastw) produce(T_{}, T_{}, F_{}); else produce(F_{}, T_{}, F_{});
+      } else if (sum_job) {
+        if (fastw) produce(T_{}, F_{}, T_{}); else produce(F_{}, F_{}, T_{});
       } else {
-        if (fastw) produce(std::true_type{}, std::false_type{}); else produce(std::false_type{}, std::false_type{});
+        if (fastw) produce(T_{}, F_{}, F_{}); else produce(F_{}, F_{}, F_{});
       }
     }
   } else if (warp == MMA_WARP2) {
@@ -743,6 +777,11 @@ int gram_ksplit(int64_t n, int C, int D, int num_sms, int elem_size) {
   return (int)(ks < 1 ? 1 : ks);
 }
 
+// K parts per class of a launch (either variant): the class-sum partials come in 4 per K part
+int gram_ksplit_launch(int64_t n, int C, int D, int packed, int num_sms, int elem_size) {
+  return gram_use_small(D, packed) ? gram_ksplit_small(n, C, num_sms) : gram_ksplit(n, C, D, num_sms, elem_size);
+}
+
 size_t gram_workspace_bytes(int C, int D, int ksplit_max) {
   // the job plan of either variant (the single-CTA variant splits K up to 64 ways)
   const size_t pair = (size_t)C * gram_tiles_per_class(D, nullptr) * (ksplit_max > 0 ? ksplit_max : 1);
@@ -754,7 +793,7 @@ template <typename T>
 static cudaError_t launch_class_gram_t(const T* X, int64_t ldx, const int32_t* perm, const int64_t* offsets,
                                        const float* shift, int64_t n, int D, int C, float* gram, int accumulate,
                                        int packed, int chain_rows, int32_t* done, int n_groups, int first_class,
-                                       int reserve_sms, void* ws, int num_sms, cudaStream_t stream) {
+                                       int reserve_sms, void* ws, int num_sms, cudaStream_t stream, float* sums) {
   const bool small = gram_use_small(D, packed);
   static int smem_set[kMaxDevices] = {0}, smem_set1[kMaxDevices] = {0};  // per element type
   {
@@ -767,12 +806,12 @@ static cudaError_t launch_class_gram_t(const T* X, int64_t ldx, const int32_t* p
   int TT = 0;
   int T_ = gram_tiles_per_class(D, &TT);
   if (small) { TT = 1; T_ = 1; }
-  P.X = X; P.ldx = ldx; P.n = n; P.perm = perm; P.offsets = offsets; P.shift = shift; P.gram = gram;
+  P.X = X; P.ldx = ldx; P.n = n; P.perm = perm; P.offsets = offsets; P.shift = shift; P.gram = gram; P.sums = sums;
   P.done = done; P.n_groups = n_groups > 0 ? n_groups : 1; P.class_order = done != nullptr ? 1 : 0;
   P.first_class = (P.class_order && first_class > 0 && first_class < C) ? first_class : 0;
   P.jobs = reinterpret_cast<const int4*>(ws);
   P.D = D; P.C = C;
-  P.KS = small ? gram_ksplit_small(n, C, num_sms) : gram_ksplit(n, C, D, num_sms, (int)sizeof(T));
+  P.KS = gram_ksplit_launch(n, C, D, packed, num_sms, (int)sizeof(T));
   P.njobs = C * T_ * P.KS;
   const int cr = chain_rows > 0 ? chain_rows : 512;
   P.chain_kb = (cr + BK - 1) / BK;
@@ -780,7 +819,7 @@ static cudaError_t launch_class_gram_t(const T* X, int64_t ldx, const int32_t* p
   P.packed = packed ? 1 : 0; P.T = T_; P.TT = TT;
   P.vec_ok = (D % 4 == 0) && ((reinterpret_cast<uintptr_t>(gram) & 15) == 0);
   static const int env_flags = [] { const char* e = getenv("SQFA_GRAM_FLAGS"); return e ? atoi(e) : 0; }();
-  P.flags = env_flags;
+  P.flags = sums != nullptr ? env_flags & ~3 : env_flags;  // class sums need the B warps of diagonal tiles idle
   P.vecx = ((ldx % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & (4 * sizeof(T) - 1)) == 0) && !(env_flags & 4)) ? 1 : 0;
   if ((uint64_t)ldx * sizeof(T) >= (1ull << 32)) return cudaErrorInvalidValue;
   if (P.atomic_out && !accumulate) {  // K parts are summed with red.add -> start from zero
@@ -807,16 +846,16 @@ static cudaError_t launch_class_gram_t(const T* X, int64_t ldx, const int32_t* p
 cudaError_t launch_class_gram(const void* X, int elem, int64_t ldx, const int32_t* perm, const int64_t* offsets,
                               const float* shift, int64_t n, int D, int C, float* gram, int accumulate, int packed,
                               int chain_rows, int32_t* done, int n_groups, int first_class, int reserve_sms, void* ws,
-                              int num_sms, cudaStream_t stream) {
+                              int num_sms, cudaStream_t stream, float* sums) {
   if (elem == ELEM_BF16)
     return launch_class_gram_t(static_cast<const __nv_bfloat16*>(X), ldx, perm, offsets, shift, n, D, C, gram,
                                accumulate, packed, chain_rows, done, n_groups, first_class, reserve_sms, ws, num_sms,
-                               stream);
+                               stream, sums);
   if (elem == ELEM_F16)
     return launch_class_gram_t(static_cast<const __half*>(X), ldx, perm, offsets, shift, n, D, C, gram, accumulate,
-                               packed, chain_rows, done, n_groups, first_class, reserve_sms, ws, num_sms, stream);
+                               packed, chain_rows, done, n_groups, first_class, reserve_sms, ws, num_sms, stream, sums);
   return launch_class_gram_t(static_cast<const float*>(X), ldx, perm, offsets, shift, n, D, C, gram, accumulate,
-                             packed, chain_rows, done, n_groups, first_class, reserve_sms, ws, num_sms, stream);
+                             packed, chain_rows, done, n_groups, first_class, reserve_sms, ws, num_sms, stream, sums);
 }
 
 }  // namespace sqfa

@@ -52,6 +52,11 @@ cudaError_t launch_class_sums(const void* X, int elem, int64_t ldx, const int32_
                               float* partial_ws, int nsplit, cudaStream_t stream);
 cudaError_t launch_class_means(const float* sums, const int64_t* counts, const float* shift, int D, int C,
                                float* means, cudaStream_t stream);
+cudaError_t launch_class_pilot_shift(const void* X, int elem, int64_t ldx, const int32_t* perm,
+                                    const int64_t* offsets, int D, int C, float* shift, cudaStream_t stream);
+// sums[c][j] = sum over s < nsplit of partial[c][s][j], in float64, s in order
+cudaError_t launch_class_sums_finalize(const float* partial, int nsplit, int D, int C, float* sums,
+                                       cudaStream_t stream);
 cudaError_t launch_counts_pack(const int64_t* counts, int C, float* out, cudaStream_t stream);
 cudaError_t launch_counts_unpack(const float* in, int C, int64_t* counts, cudaStream_t stream);
 size_t stats_epilogue_workspace_bytes(int C);
@@ -65,17 +70,21 @@ struct GramSources {
 };
 cudaError_t launch_stats_epilogue(const float* gram, int packed, const float* means, const float* shift,
                                   const int64_t* counts, int D, int C, int estimator, int ddof, float* cov, float* sm,
-                                  void* ws, cudaStream_t stream, GramSources src = GramSources{nullptr, 0, 0, 0});
+                                  void* ws, cudaStream_t stream, GramSources src = GramSources{nullptr, 0, 0, 0},
+                                  int centred_sums = 0);
 
 // ---- gram.cu (K2: tcgen05 cta_group::2 Gram on CTA pairs) ----
 int gram_tiles_per_class(int D, int* TT_out);
 int64_t gram_executed_tile_area(int D);
 int gram_ksplit(int64_t n, int C, int D, int num_sms, int elem_size);
+int gram_ksplit_launch(int64_t n, int C, int D, int packed, int num_sms, int elem_size);
 size_t gram_workspace_bytes(int C, int D, int ksplit_max);
+// sums != nullptr: the diagonal tiles' producers also write class-sum partials sums[C][4 KS][D] of (x - shift),
+// KS = gram_ksplit_launch(...); class_sums_finalize with nsplit = 4 KS adds them up
 cudaError_t launch_class_gram(const void* X, int elem, int64_t ldx, const int32_t* perm, const int64_t* offsets,
                               const float* shift, int64_t n, int D, int C, float* gram, int accumulate, int packed,
                               int chain_rows, int32_t* done, int n_groups, int first_class, int reserve_sms, void* ws,
-                              int num_sms, cudaStream_t stream);
+                              int num_sms, cudaStream_t stream, float* sums = nullptr);
 size_t gram_packed_floats(int D, int C);  // floats of the packed upper-tile list (256 x 256 tiles)
 }  // namespace sqfa
 

@@ -1,4 +1,5 @@
-// K2a: segmented per-class column sums (-> class means), K3: statistics epilogue
+// K2a: segmented per-class column sums (-> class means) and the pilot shift of the one-pass path,
+// K3: statistics epilogue
 // (mean, unbiased covariance, covariance + mu mu^T, optional OAS shrinkage).
 //
 // Reference semantics: /root/reference/src/sqfa/statistics.py
@@ -129,6 +130,34 @@ __global__ void class_sums_finalize_kernel(const float* __restrict__ partial, in
   sums[idx] = (float)acc;
 }
 
+// Pilot shift of the one-pass class_statistics: shift[c][j] = mean of the first min(n_c, PILOT_ROWS) rows of
+// class c in bucket order (0 for an empty class). The Gram centres on it and writes sum (x - shift) on the
+// way; the epilogue corrects the Gram by n d d^T, d = mean - shift. |d| ~ sigma / sqrt(32) makes the centred
+// values (1 + 1/32) times larger in square than with the exact mean, i.e. 3 % more 3xTF32 and truncation
+// error. One thread per column, the rows added in order: a bf16 / fp16 X gives the bits of its float32 copy.
+constexpr int PILOT_ROWS = 32;
+constexpr int PILOT_THREADS = 128;
+
+template <typename T>
+__global__ void __launch_bounds__(PILOT_THREADS)
+class_pilot_shift_kernel(const T* __restrict__ X, int64_t ldx, const int32_t* __restrict__ perm,
+                         const int64_t* __restrict__ offsets, int D, float* __restrict__ shift) {
+  const int c = blockIdx.y;
+  const int col = blockIdx.x * PILOT_THREADS + threadIdx.x;
+  if (col >= D) return;
+  const int64_t begin = offsets[c];
+  const int64_t n_c = offsets[c + 1] - begin;
+  const int p = n_c < PILOT_ROWS ? (int)(n_c > 0 ? n_c : 0) : PILOT_ROWS;
+  float v[PILOT_ROWS];
+#pragma unroll
+  for (int r = 0; r < PILOT_ROWS; ++r)  // all loads in flight, then the sum
+    v[r] = r < p ? ldg_widen(X + (int64_t)__ldg(perm + begin + r) * ldx + col) : 0.f;
+  float s = 0.f;
+#pragma unroll
+  for (int r = 0; r < PILOT_ROWS; ++r) s += v[r];
+  shift[(int64_t)c * D + col] = p > 0 ? s / (float)p : 0.f;
+}
+
 // means[c][j] = sums[c][j] / n_c (+ shift[c][j]);  0/0 -> NaN for an empty class, as torch.mean does.
 __global__ void class_means_kernel(const float* __restrict__ sums, const int64_t* __restrict__ counts,
                                    const float* __restrict__ shift, int D, int C, float* __restrict__ means) {
@@ -159,10 +188,19 @@ __device__ __forceinline__ const float* gram_elem(const float* gram, int packed,
   return gram + (((int64_t)c * T + t) * 256 + (r & 255)) * 256 + (q & 255);
 }
 
+// d = mean - shift. With centred_sums, `shift` holds the class sums of (x - s) the Gram was centred for and
+// d = sums / n: exact to float32 rounding of d itself, where mean - s would lose the bits of |mean| >> |d|
+// (data far from the origin).
+__device__ __forceinline__ float centring_offset(const float* mu, const float* shift, int c, int D, int r, float n,
+                                                 int centred_sums) {
+  const float v = shift[(int64_t)c * D + r];
+  return centred_sums ? v / n : mu[r] - v;
+}
+
 __global__ void __launch_bounds__(256)
 stats_epilogue_kernel(const float* gram, int packed, const float* __restrict__ means,
                       const float* __restrict__ shift, const int64_t* __restrict__ counts, int D, int NT, int ddof,
-                      float* cov, float* sm, const GramSources src) {
+                      float* cov, float* sm, const GramSources src, int centred_sums) {
   __shared__ float s_cov[32][33];
   __shared__ float s_mu_i[32], s_mu_j[32], s_d_i[32], s_d_j[32];
   const int c = blockIdx.y;
@@ -176,15 +214,15 @@ stats_epilogue_kernel(const float* gram, int packed, const float* __restrict__ m
   const int tj = ti + t;
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;  // 32 x 8
   const float* mu = means + (int64_t)c * D;
+  const float n = (float)counts[c];
   if (threadIdx.x < 32) {
     const int r = ti * 32 + threadIdx.x, q = tj * 32 + threadIdx.x;
     s_mu_i[threadIdx.x] = r < D ? mu[r] : 0.f;
     s_mu_j[threadIdx.x] = q < D ? mu[q] : 0.f;
-    s_d_i[threadIdx.x] = (shift != nullptr && r < D) ? mu[r] - shift[(int64_t)c * D + r] : 0.f;
-    s_d_j[threadIdx.x] = (shift != nullptr && q < D) ? mu[q] - shift[(int64_t)c * D + q] : 0.f;
+    s_d_i[threadIdx.x] = (shift != nullptr && r < D) ? centring_offset(mu, shift, c, D, r, n, centred_sums) : 0.f;
+    s_d_j[threadIdx.x] = (shift != nullptr && q < D) ? centring_offset(mu, shift, c, D, q, n, centred_sums) : 0.f;
   }
   __syncthreads();
-  const float n = (float)counts[c];
   const float nm1 = n - (float)ddof;
   for (int rr = ty; rr < 32; rr += 8) {
     const int r = ti * 32 + rr, q = tj * 32 + tx;
@@ -198,7 +236,7 @@ stats_epilogue_kernel(const float* gram, int packed, const float* __restrict__ m
         for (int s = 0; s < src.n_src; ++s)
           g += *gram_elem(s == src.self ? gram : src.peers + s * src.stride, packed, c, D, r, q);
       }
-      if (shift != nullptr) g -= n * s_d_i[rr] * s_d_j[tx];
+      if (shift != nullptr && n > 0.f) g -= n * s_d_i[rr] * s_d_j[tx];  // empty class: d is NaN, n d d^T is 0
       v = g / nm1;
     }
     s_cov[rr][tx] = v;
@@ -234,7 +272,7 @@ stats_epilogue_kernel(const float* gram, int packed, const float* __restrict__ m
 __global__ void __launch_bounds__(256)
 stats_epilogue_v4_kernel(const float* gram, int packed, const float* __restrict__ means,
                          const float* __restrict__ shift, const int64_t* __restrict__ counts, int D, int NT, int ddof,
-                         float* cov, float* sm, const GramSources src) {
+                         float* cov, float* sm, const GramSources src, int centred_sums) {
   __shared__ float s_cov[64][65];
   __shared__ float s_mu_i[64], s_mu_j[64], s_d_i[64], s_d_j[64];
   const int c = blockIdx.y;
@@ -247,15 +285,15 @@ stats_epilogue_v4_kernel(const float* gram, int packed, const float* __restrict_
   const int tj = ti + t;
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;  // 16 float4 columns x 16 rows per pass
   const float* mu = means + (int64_t)c * D;
+  const float n = (float)counts[c];
   if (threadIdx.x < 64) {
     const int r = ti * 64 + threadIdx.x, q = tj * 64 + threadIdx.x;
     s_mu_i[threadIdx.x] = r < D ? mu[r] : 0.f;
     s_mu_j[threadIdx.x] = q < D ? mu[q] : 0.f;
-    s_d_i[threadIdx.x] = (shift != nullptr && r < D) ? mu[r] - shift[(int64_t)c * D + r] : 0.f;
-    s_d_j[threadIdx.x] = (shift != nullptr && q < D) ? mu[q] - shift[(int64_t)c * D + q] : 0.f;
+    s_d_i[threadIdx.x] = (shift != nullptr && r < D) ? centring_offset(mu, shift, c, D, r, n, centred_sums) : 0.f;
+    s_d_j[threadIdx.x] = (shift != nullptr && q < D) ? centring_offset(mu, shift, c, D, q, n, centred_sums) : 0.f;
   }
   __syncthreads();
-  const float n = (float)counts[c];
   const float nm1 = n - (float)ddof;
   const int q0 = tj * 64 + 4 * tx;  // D % 4 == 0: a float4 is entirely inside or outside the matrix
 #pragma unroll
@@ -272,7 +310,7 @@ stats_epilogue_v4_kernel(const float* gram, int packed, const float* __restrict_
           g.x += v.x; g.y += v.y; g.z += v.z; g.w += v.w;
         }
       }
-      if (shift != nullptr) {
+      if (shift != nullptr && n > 0.f) {  // empty class: d is NaN, n d d^T is 0
         const float a = n * s_d_i[rr];
         g.x -= a * s_d_j[4 * tx]; g.y -= a * s_d_j[4 * tx + 1];
         g.z -= a * s_d_j[4 * tx + 2]; g.w -= a * s_d_j[4 * tx + 3];
@@ -460,6 +498,30 @@ cudaError_t launch_class_sums(const void* X, int elem, int64_t ldx, const int32_
   return cudaGetLastError();
 }
 
+cudaError_t launch_class_pilot_shift(const void* X, int elem, int64_t ldx, const int32_t* perm,
+                                    const int64_t* offsets, int D, int C, float* shift, cudaStream_t stream) {
+  if (C <= 0 || D <= 0) return cudaSuccess;
+  const dim3 grid((D + PILOT_THREADS - 1) / PILOT_THREADS, C);
+  if (elem == ELEM_BF16)
+    class_pilot_shift_kernel<<<grid, PILOT_THREADS, 0, stream>>>(static_cast<const __nv_bfloat16*>(X), ldx, perm,
+                                                                 offsets, D, shift);
+  else if (elem == ELEM_F16)
+    class_pilot_shift_kernel<<<grid, PILOT_THREADS, 0, stream>>>(static_cast<const __half*>(X), ldx, perm, offsets, D,
+                                                                 shift);
+  else
+    class_pilot_shift_kernel<<<grid, PILOT_THREADS, 0, stream>>>(static_cast<const float*>(X), ldx, perm, offsets, D,
+                                                                 shift);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_class_sums_finalize(const float* partial, int nsplit, int D, int C, float* sums,
+                                       cudaStream_t stream) {
+  const int64_t total = (int64_t)C * D;
+  if (total <= 0) return cudaSuccess;
+  class_sums_finalize_kernel<<<(int)((total + 255) / 256), 256, 0, stream>>>(partial, nsplit, D, C, sums, 0);
+  return cudaGetLastError();
+}
+
 cudaError_t launch_class_means(const float* sums, const int64_t* counts, const float* shift, int D, int C,
                                float* means, cudaStream_t stream) {
   const int64_t total = (int64_t)C * D;
@@ -472,7 +534,7 @@ size_t stats_epilogue_workspace_bytes(int C) { return (size_t)(C > 0 ? C : 1) * 
 
 cudaError_t launch_stats_epilogue(const float* gram, int packed, const float* means, const float* shift,
                                   const int64_t* counts, int D, int C, int estimator, int ddof, float* cov, float* sm,
-                                  void* ws, cudaStream_t stream, GramSources src) {
+                                  void* ws, cudaStream_t stream, GramSources src, int centred_sums) {
   if (C <= 0 || D <= 0) return cudaSuccess;
   const bool al16 = ((reinterpret_cast<uintptr_t>(gram) | reinterpret_cast<uintptr_t>(cov) |
                       reinterpret_cast<uintptr_t>(sm) | reinterpret_cast<uintptr_t>(src.peers) |
@@ -480,11 +542,11 @@ cudaError_t launch_stats_epilogue(const float* gram, int packed, const float* me
   if (D % 4 == 0 && al16) {
     const int NT = (D + 63) / 64;
     stats_epilogue_v4_kernel<<<dim3(NT * (NT + 1) / 2, C), 256, 0, stream>>>(gram, packed, means, shift, counts, D, NT,
-                                                                             ddof, cov, sm, src);
+                                                                             ddof, cov, sm, src, centred_sums);
   } else {
     const int NT = (D + 31) / 32;
     stats_epilogue_kernel<<<dim3(NT * (NT + 1) / 2, C), 256, 0, stream>>>(gram, packed, means, shift, counts, D, NT, ddof,
-                                                                          cov, sm, src);
+                                                                          cov, sm, src, centred_sums);
   }
   if (estimator == 1) {
     double* partial = static_cast<double*>(ws);
